@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the FFT cross-correlation hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): xcorr pairs/sec at L = 1,440,000 (N = 2,880,000), batched.
 A step is one pass of the whole path (forward FFTs, conj-multiply, inverse FFT,
@@ -109,7 +109,9 @@ def emit(line):
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps (repetitions) of every throughput leg; the latency legs time a fixed "
+                         "number of calls and the CPU baseline about 12 s")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--pairs", type=int, default=PAIRS_PER_GPU, help="pairs per GPU per step")
@@ -121,7 +123,28 @@ def parse():
     ap.add_argument("--no-latency", action="store_true")
     ap.add_argument("--no-inlib", action="store_true", help="skip the in-library multi-GPU leg (N > 1)")
     ap.add_argument("--inlib-pairs", type=int, default=1024, help="device-resident pairs per GPU in the in-library leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path returned in its last step as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, arrays):
+    """Writes equal-length 1-D arrays as `path`/<name>.npy in float64 (every field of a result
+    record, integers included, is exact in float64).  Above DUMP_BYTES in all, a fixed seeded
+    sample of the rows is written; `pair_id` says which pairs the rows belong to."""
+    import numpy as np
+    n = len(arrays["pair_id"])
+    keep = (DUMP_BYTES - 1024 * len(arrays)) // (8 * len(arrays))     # 1 KiB per .npy header: headroom
+    rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False)) if n > keep else slice(None)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64)[rows])
 
 
 def measured_peaks():
@@ -252,10 +275,12 @@ def run_reference_arm(args):
     for _ in range(args.warmup):
         cpu_reference_run(L, callers, callers, SEED)
     times = []
-    kind = backend = None
+    kind = backend = lags = None
     for _ in range(args.steps):
-        dt, kind, backend, _ = cpu_reference_run(L, per_step, callers, SEED)
+        dt, kind, backend, lags = cpu_reference_run(L, per_step, callers, SEED)
         times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pair_id": range(per_step), "lag": lags})
     total = sum(times)
     value = per_step * args.steps / total
     line = {
@@ -265,7 +290,7 @@ def run_reference_arm(args):
         "data": "synthetic (seeded integer generator, SURVEY 8d)",
         "config": {"workload": "reference CPU path (src/cross_correlation.c) on %d-pair samples of "
                                "config[3]: L=%d, N=%d" % (per_step, L, 2 * L),
-                   "sample_len": L, "pairs_per_step": per_step},
+                   "sample_len": L, "pairs_per_step": per_step, "seed": SEED},
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": kind,
                          "sample": "%d pairs/step x %d steps, %d concurrent callers x 2 FFT threads, "
                                    "FFT backend %s (in place of FFTW3, which is not installed)"
@@ -412,7 +437,7 @@ def measure_in_library(ac, torch, n_dev, L, args, per_gpu_process_value):
 
         from concurrent.futures import ThreadPoolExecutor
         gate = threading.Barrier(n_dev)
-        steps = max(args.steps, 8)
+        steps = args.steps
         with ThreadPoolExecutor(n_dev) as pool:
             list(pool.map(lambda g: drive(g, max(2, args.warmup), False), range(n_dev)))
             t0 = time.perf_counter()
@@ -540,6 +565,12 @@ def main():
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
     launches = ctx.launch_count() - launches0
+    res = d_res.cpu().numpy().view(ac.RESULT_DTYPE)      # what the last timed step returned
+    if args.dump_outputs:
+        everyone = ac.gather_results(res, world * n, dst=0)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"pair_id": range(world * n),
+                                             **{f: everyone[f] for f in ac.RESULT_DTYPE.names}})
     # per-kernel durations: the same K steps again, every launch bracketed by CUDA events on its
     # own stream (kept out of the timed region above: the event records sit between the
     # PDL-chained stage launches)
@@ -556,7 +587,6 @@ def main():
     ctx.profile_enable(False)
 
     # correctness of what was timed: every pair recovers its injected lag
-    res = d_res.cpu().numpy().view(ac.RESULT_DTYPE)
     from oracle import capi   # checker only (synth_true_lag), never the thing measured
     bad = sum(1 for i in range(0, n, max(1, n // 256))
               if int(res["lag"][i]) != capi.synth_true_lag(SEED, first_pair + i, L))
@@ -617,15 +647,15 @@ def main():
                     "bound": "pcie + host copy threads (%.2f MB of host input per pair)" % (3 * L * esz / 1e6),
                     "api": "audiosync_cuda_xcorr_batch(memspace=HOST)"}
         ne = min(args.e2e_pairs, n)
-        reps = max(2, args.steps)
+        reps = args.steps
         e2e = e2e_leg(torch.float64, ac.F64, True, max(1, ne // 2), reps)
         if os.environ.get("E2E_ONLY_HEADLINE") == "1":            # tools/e2e_feed.sh: feed-policy sweeps
             emit({"e2e": e2e, "e2e_variants": {}})
             return
         e2e_variants["f64_pinned_narrowing_off"] = e2e_leg(torch.float64, ac.F64, True, max(1, ne // 2), reps, narrow=ac.NARROW_OFF)
         e2e_variants["f32_pinned"] = e2e_leg(torch.float32, ac.F32, True, ne, reps)
-        e2e_variants["f64_pageable"] = e2e_leg(torch.float64, ac.F64, False, max(1, ne // 4), 2)
-        e2e_variants["f64_pageable_narrowing_off"] = e2e_leg(torch.float64, ac.F64, False, max(1, ne // 4), 2, narrow=ac.NARROW_OFF)
+        e2e_variants["f64_pageable"] = e2e_leg(torch.float64, ac.F64, False, max(1, ne // 4), reps)
+        e2e_variants["f64_pageable_narrowing_off"] = e2e_leg(torch.float64, ac.F64, False, max(1, ne // 4), reps, narrow=ac.NARROW_OFF)
 
     # ---- config 3: single-pair latency at this length (rank 0 only) --------------------------
     latency = None
@@ -695,7 +725,7 @@ def main():
             "generator, SURVEY 8d; generated on device)",
             "config": {"workload": "config[3]: %d pairs/GPU of L=%d frames (N=%d real points), "
                                    "device-resident fp32, whole path incl. argmax + Pearson" % (n, L, 2 * L),
-                       "sample_len": L, "pairs_per_gpu": n, "total_pairs": world * n, "plan": plan,
+                       "sample_len": L, "pairs_per_gpu": n, "total_pairs": world * n, "plan": plan, "seed": SEED,
                        "inputs_larger_than_l2": bool(n * 3 * L * 4 > 126e6),
                        "input_bytes_per_gpu": n * 3 * L * 4, "sharding": "contiguous pair blocks, no collective"},
             "roofline": {"bound": "hbm", "kernel": dom, "achieved": achieved, "peak": peak, "unit": "GB/s",
