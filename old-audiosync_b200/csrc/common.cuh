@@ -62,6 +62,11 @@ __host__ __device__ __forceinline__ uint32_t argmax_key_index(uint64_t key) {
     return ~((lo >> 1) | 0x80000000u);
 }
 
+// the seed's key (index 0): abs keys carry an index >= 1 < 2^31, so their low word differs
+__host__ __device__ __forceinline__ bool argmax_key_is_seed(uint64_t key) {
+    return ((uint32_t)(key & 0xffffffffu) >> 1) == 0x7fffffffu;
+}
+
 // signed value of the winning entry
 __host__ __device__ __forceinline__ float argmax_key_value(uint64_t key) {
     float m = float_from_order_bits((uint32_t)(key >> 32));
@@ -76,18 +81,29 @@ struct PairPeak {
     double peak;              // r[raw_index]
     double second;            // resolved second peak (direct path)
     int resolved;             // 1 if raw_index/peak/second are already final
-    unsigned int second_bits; // fp32 path: order bits of the largest |r[i]|, i != argmax (0: none yet)
+    unsigned int second_bits; // fp32 path: order bits of the largest |r[i]|, i >= 1, i != argmax (0: none yet)
+    unsigned int seed_bits;   // fp32 path: order bits of |r[0]| (0: not written yet)
 };
 
 __host__ __device__ __forceinline__ PairPeak cleared_peak() {
     PairPeak z;
-    z.key = 0ull; z.raw_index = 0; z.peak = 0.0; z.second = 0.0; z.resolved = 0; z.second_bits = 0u;
+    z.key = 0ull; z.raw_index = 0; z.peak = 0.0; z.second = 0.0; z.resolved = 0; z.second_bits = 0u; z.seed_bits = 0u;
     return z;
 }
 
 // |value| carried by a packed key (abs keys hold |v|, the seed key holds the signed r[0]).
 __host__ __device__ __forceinline__ float argmax_key_mag(uint64_t key) {
     return fabsf(float_from_order_bits((uint32_t)(key >> 32)));
+}
+
+// Second peak of the fp32 transform path: the largest |r[i]| over i >= 1 other than the peak
+// (second_bits), joined by |r[0]| unless r[0] is the peak.  r[0] is kept out of second_bits
+// because second_bits is also the threshold below which the kernels skip candidates, and a
+// negative r[0] may lose while being the largest magnitude (see ArgmaxAcc).
+__host__ __device__ __forceinline__ float pair_second(const PairPeak& p) {
+    float s = p.second_bits != 0u ? float_from_order_bits(p.second_bits) : 0.0f;
+    if (p.seed_bits != 0u && argmax_key_index(p.key) != 0u) s = fmaxf(s, float_from_order_bits(p.seed_bits));
+    return s;
 }
 
 // Fold of src/cross_correlation.c:256-271.  Window = x[xoff .. xoff+n) of the

@@ -690,7 +690,7 @@ struct GenColInvKernel {
                                 constexpr int k = decltype(K)::value;
                                 const unsigned i_re = i_first + 2u * (unsigned)k * Wt * (unsigned)M2;
                                 if (i_re < limit) {
-                                    if (i_re == 0u) acc.consider_seed(v[k].x);
+                                    if (i_re == 0u) acc.consider_seed(v[k].x, &p.peaks[pair]);
                                     else acc.consider(v[k].x, i_re);
                                 }
                                 if (i_re + 1u < limit) acc.consider(v[k].y, i_re + 1u);

@@ -93,9 +93,17 @@ ASC_HD cplx load_packed<double>(const double* __restrict__ x, long long n) {
 
 // Running |r| argmax of one thread (reference src/cross_correlation.c:52-67 as
 // a max over packed keys, see common.cuh) plus the SECOND peak: the largest
-// |r[i]| over every entry other than the winner (SURVEY 8f rank 4; the oracle's
-// `second`, which makes "the peak is unique" observable).  The packed key is only
-// built for candidates that can still change either; a NaN never passes `a >= thr`.
+// |r[i]| over every entry i >= 1 other than the winner (SURVEY 8f rank 4; the
+// oracle's `second`, which makes "the peak is unique" observable).  The packed key
+// is only built for candidates that can still change either; a NaN never passes
+// `a >= thr`.
+//
+// The threshold argument -- a value below the running second peak can be neither the
+// peak nor the second -- holds for every entry i >= 1 but not for the signed seed
+// r[0]: a negative r[0] loses to any |r[i]| while possibly being the largest magnitude,
+// so its |r[0]| must not raise `thr`, the warp's bound or the pair's published
+// second_bits.  It never enters `second`; the seed's thread stores it in
+// PairPeak::seed_bits, and pair_second() joins it to the second peak at the end.
 struct ArgmaxPair {
     unsigned long long best;
     float second;
@@ -107,7 +115,7 @@ struct ArgmaxAcc {
     float thr = 0.0f;                // lower bound of the pair's final second peak: smaller magnitudes are skipped
     ASC_HD void update(unsigned long long key, float a) {
         if (key > best) {
-            if (best != 0ull) second = fmaxf(second, argmax_key_mag(best));   // NaN seed: fmaxf drops it
+            if (best != 0ull && !argmax_key_is_seed(best)) second = fmaxf(second, argmax_key_mag(best));
             best = key;
         } else {
             second = fmaxf(second, a);
@@ -118,8 +126,12 @@ struct ArgmaxAcc {
         const float a = fabsf(v);
         if (a >= thr) update(argmax_key_abs(v, index), a);
     }
-    ASC_HD void consider_seed(float v) { update(argmax_key_seed(v), fabsf(v)); }   // index 0, signed
-    ASC_HD float best_mag() const { return best != 0ull ? argmax_key_mag(best) : 0.0f; }
+    ASC_HD void consider_seed(float v, PairPeak* pk) {   // index 0, signed
+        update(argmax_key_seed(v), 0.0f);
+        pk->seed_bits = float_order_bits(fabsf(v));
+    }
+    // bound for the warp's threshold: the seed's magnitude is none (see above)
+    ASC_HD float best_mag() const { return best != 0ull && !argmax_key_is_seed(best) ? argmax_key_mag(best) : 0.0f; }
     ASC_HD ArgmaxPair result() const { ArgmaxPair r; r.best = best; r.second = second; return r; }
 };
 
@@ -553,7 +565,7 @@ struct ColInvKernel {
                                     constexpr int k = decltype(K)::value;
                                     const int n1 = f0 + k * Wt;
                                     const uint32_t i_re = 2u * ((uint32_t)n1 * (uint32_t)M2 + (uint32_t)(c0 + c));
-                                    if (has_seed && n1 == 0) acc.consider_seed(v[k].x);
+                                    if (has_seed && n1 == 0) acc.consider_seed(v[k].x, &p.peaks[pair]);
                                     else acc.consider(v[k].x, i_re);
                                     acc.consider(v[k].y, i_re + 1u);
                                 });
@@ -1016,7 +1028,7 @@ struct DeviceExec {
     }
     // CTA-wide (peak key, second peak) of the per-thread pairs, then one atomicMax on *dst
     // and one on *dst_second.  Pairs merge associatively: the larger key leads, the smaller
-    // key's magnitude joins the two seconds.  At grid level the key the atomicMax displaces
+    // key's magnitude joins the two seconds (unless it is the seed's, see ArgmaxAcc).  At grid level the key the atomicMax displaces
     // (or fails to displace) is a second-peak candidate too: over all CTAs max(min(old, mine))
     // is exactly the second largest CTA peak.  `scratch`: at least 32 * 12 bytes of the CTA's
     // dynamic shared memory; it may alias data f() reads (a barrier separates the two uses).
@@ -1027,7 +1039,7 @@ struct DeviceExec {
         const unsigned long long lose = ob > best ? best : ob;
         best = ob > best ? ob : best;
         second = fmaxf(second, os);
-        if (lose != 0ull) second = fmaxf(second, argmax_key_mag(lose));
+        if (lose != 0ull && !argmax_key_is_seed(lose)) second = fmaxf(second, argmax_key_mag(lose));
     }
 #endif
     template <class F>

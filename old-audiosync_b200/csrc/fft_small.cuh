@@ -138,7 +138,7 @@ struct SmallXcorrKernel {
                 for (int n = tid; n < M; n += THREADS) {
                     const cplx v = buf[n];
                     const uint32_t i_re = (uint32_t)(2 * n);
-                    if (n == 0) acc.consider_seed(v.x);
+                    if (n == 0) acc.consider_seed(v.x, &p.peaks[pair]);
                     else acc.consider(v.x, i_re);
                     acc.consider(v.y, i_re + 1u);
                 }

@@ -236,8 +236,7 @@ __device__ __forceinline__ void pearson_block(
         const PairPeak p = peaks[pair];
         raw = p.resolved ? p.raw_index : (long long)argmax_key_index(p.key);
         peak = p.resolved ? p.peak : (double)argmax_key_value(p.key);
-        second = p.resolved ? p.second
-                            : (p.second_bits != 0u ? (double)float_from_order_bits(p.second_bits) : 0.0);
+        second = p.resolved ? p.second : (double)pair_second(p);
         // the transform's own scale -> the reference's (FFTW c2r: x N); powers of two for the static plans
         peak *= peak_scale;
         second *= peak_scale;

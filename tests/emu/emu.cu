@@ -40,13 +40,13 @@ struct HostExec {
             const ArgmaxPair k = f(t);
             const unsigned long long lose = k.best > best ? best : k.best;
             if (k.best > best) best = k.best;
-            if (lose != 0) second = fmaxf(second, argmax_key_mag(lose));
+            if (lose != 0 && !argmax_key_is_seed(lose)) second = fmaxf(second, argmax_key_mag(lose));
             second = fmaxf(second, k.second);
         }
         const unsigned long long old = *dst;
         const unsigned long long loser = old < best ? old : best;
         if (best > old) *dst = best;
-        if (loser != 0 && old != best) second = fmaxf(second, argmax_key_mag(loser));
+        if (loser != 0 && old != best && !argmax_key_is_seed(loser)) second = fmaxf(second, argmax_key_mag(loser));
         const unsigned int sb = float_order_bits(second);
         if (sb > *dst_second) *dst_second = sb;
     }
@@ -66,7 +66,7 @@ static int run_static(const InT* source, const InT* sample, PairPeak* peak, cplx
     std::vector<cplx> row_tab = build_row_tab<Row>(M, M1);
     std::vector<cplx> m_lo, m_hi;
     build_two_level(M, M - 1, m_lo, m_hi);
-    peak->key = 12345ull; peak->second_bits = 777u;   // garbage: K_A must clear both
+    peak->key = 12345ull; peak->second_bits = 777u; peak->seed_bits = 777u;   // garbage: K_A must clear them
 
     {
         // fp32: the TMA-staged variant (the product's default; host emulation copies the same boxes
@@ -110,7 +110,7 @@ static int run_small(const InT* source, const InT* sample, long long L, PairPeak
     using K = SmallXcorrKernel<InT>;
     typename K::Params p{source, sample, peak, wm.data(), wn.data(), pl};
     std::vector<cplx> smem(K::smem_bytes((int)L) / sizeof(cplx));
-    peak->key = 12345ull; peak->second_bits = 777u;   // garbage: the kernel must clear both
+    peak->key = 12345ull; peak->second_bits = 777u; peak->seed_bits = 777u;   // garbage: the kernel must clear them
     HostExec ex{0, 0, 0, K::THREADS};
     K::run(ex, p, smem.data());
     return 0;
@@ -128,7 +128,7 @@ static int run_generic(const InT* source, const InT* sample, long long L, long l
     std::vector<C> planes(2 * sh.M);
     PairPeak pk;
     memset(&pk, 0, sizeof(pk));
-    pk.key = 12345ull; pk.second_bits = 777u;   // garbage: G_A must clear both
+    pk.key = 12345ull; pk.second_bits = 777u; pk.seed_bits = 777u;   // garbage: G_A must clear them
     auto col_fwd = [&](auto KK) {
         using K = decltype(KK);
         typename K::Params p{source, sample, planes.data(), &pk, tb.wcol.data(), tb.m_lo.data(), tb.m_hi.data(),
@@ -168,7 +168,7 @@ static int run_generic(const InT* source, const InT* sample, long long L, long l
     if (sizeof(T) == 4) {
         *raw_index = (long long)argmax_key_index(pk.key);
         *peak_value = (double)argmax_key_value(pk.key) * scale;
-        *second_value = (pk.second_bits ? (double)float_from_order_bits(pk.second_bits) : 0.0) * scale;
+        *second_value = (double)pair_second(pk) * scale;
     } else {
         // fp64: r[0 .. 2L) sits in plane 1; resolve like argmax_f64_kernel (reference :52-67)
         const T* r = reinterpret_cast<const T*>(planes.data()) + 2 * sh.M;
@@ -214,7 +214,7 @@ static int emu_any(const InT* source, const InT* sample, long long L, int forced
     if (rc != 0) return rc;
     *raw_index = (long long)argmax_key_index(pk.key);
     *peak_value = (double)argmax_key_value(pk.key);
-    g_last_second = pk.second_bits ? (double)float_from_order_bits(pk.second_bits) : 0.0;
+    g_last_second = (double)pair_second(pk);
     return 0;
 }
 
