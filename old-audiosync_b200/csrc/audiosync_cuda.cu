@@ -1131,7 +1131,7 @@ struct audiosync_cuda_pool {
     audiosync_cuda_ctx* ctx = nullptr;
     asc::DeviceState* dev = nullptr;
     size_t n_slots = 0, max_len = 0;
-    long long src_pitch = 0, smp_pitch = 0;      // elements; multiples of 4 (16-byte rows for cp.async)
+    long long src_pitch = 0, smp_pitch = 0;      // elements; multiples of 4 (16-byte rows for TMA-staged tiles)
     int dtype = AUDIOSYNC_CUDA_F64;
     asc::DevBuf src, smp;
     // fp32 slots: arriving doubles land in one of two staging buffers (copy stream) and are

@@ -122,7 +122,39 @@ ASC_HD cplx cmul_const(cplx v, float wr, float wi) {
     return cmake(fmaf(-v.y, wi, v.x * wr), fmaf(v.x, wi, v.y * wr));
 #endif
 }
-ASC_HD cplx cconj(cplx a) { return cmake(a.x, -a.y); }
+// a + conj(b), a - conj(b)
+ASC_HD cplx cconj_add(cplx a, cplx b) {
+#if ASC_PACKED
+    return __fadd2_rn(a, cmake(b.x, -b.y));
+#else
+    return cmake(a.x + b.x, a.y - b.y);
+#endif
+}
+ASC_HD cplx cconj_sub(cplx a, cplx b) {
+#if ASC_PACKED
+    return __fadd2_rn(a, cmake(-b.x, b.y));
+#else
+    return cmake(a.x - b.x, a.y + b.y);
+#endif
+}
+// acc + a * conj(b)
+ASC_HD cplx cmulc_acc(cplx a, cplx b, cplx acc) {
+#if ASC_PACKED
+    const cplx t = __ffma2_rn(cmake(a.y, -a.x), cmake(b.y, b.y), acc);
+    return __ffma2_rn(a, cmake(b.x, b.x), t);
+#else
+    return cmake(fmaf(a.x, b.x, fmaf(a.y, b.y, acc.x)), fmaf(a.y, b.x, fmaf(-a.x, b.y, acc.y)));
+#endif
+}
+// acc - a * conj(b)
+ASC_HD cplx cmulc_nacc(cplx a, cplx b, cplx acc) {
+#if ASC_PACKED
+    const cplx t = __ffma2_rn(cmake(-a.y, a.x), cmake(b.y, b.y), acc);
+    return __ffma2_rn(a, cmake(-b.x, -b.x), t);
+#else
+    return cmake(fmaf(-a.x, b.x, fmaf(-a.y, b.y, acc.x)), fmaf(-a.y, b.x, fmaf(a.x, b.y, acc.y)));
+#endif
+}
 // multiply by +i / -i
 ASC_HD cplx cmul_pi(cplx a) { return cmake(-a.y, a.x); }
 ASC_HD cplx cmul_ni(cplx a) { return cmake(a.y, -a.x); }
@@ -142,7 +174,14 @@ ASC_HD cplxd csub_i(cplxd a, cplxd b) { return cmake(a.x + b.y, a.y - b.x); }
 ASC_HD cplxd caxpy_i(double s, cplxd b, cplxd a) { return cmake(fma(-b.y, s, a.x), fma(b.x, s, a.y)); }
 ASC_HD cplxd caxmy_i(double s, cplxd b, cplxd a) { return cmake(fma(b.y, s, a.x), fma(-b.x, s, a.y)); }
 ASC_HD cplxd cmul_const(cplxd v, double wr, double wi) { return cmake(fma(-v.y, wi, v.x * wr), fma(v.x, wi, v.y * wr)); }
-ASC_HD cplxd cconj(cplxd a) { return cmake(a.x, -a.y); }
+ASC_HD cplxd cconj_add(cplxd a, cplxd b) { return cmake(a.x + b.x, a.y - b.y); }
+ASC_HD cplxd cconj_sub(cplxd a, cplxd b) { return cmake(a.x - b.x, a.y + b.y); }
+ASC_HD cplxd cmulc_acc(cplxd a, cplxd b, cplxd acc) {
+    return cmake(fma(a.x, b.x, fma(a.y, b.y, acc.x)), fma(a.y, b.x, fma(-a.x, b.y, acc.y)));
+}
+ASC_HD cplxd cmulc_nacc(cplxd a, cplxd b, cplxd acc) {
+    return cmake(fma(-a.x, b.x, fma(-a.y, b.y, acc.x)), fma(-a.y, b.x, fma(a.x, b.y, acc.y)));
+}
 ASC_HD cplxd cmul_pi(cplxd a) { return cmake(-a.y, a.x); }
 ASC_HD cplxd cmul_ni(cplxd a) { return cmake(a.y, -a.x); }
 
@@ -185,9 +224,6 @@ ASC_HD void cp_async_wait_all() {
 #if defined(__CUDA_ARCH__)
     asm volatile("cp.async.wait_all;" ::: "memory");
 #endif
-}
-ASC_HD void smem_zero16(void* smem_dst) {
-    *reinterpret_cast<float4*>(smem_dst) = make_float4(0.f, 0.f, 0.f, 0.f);
 }
 // Makes this thread's earlier shared-memory writes visible to the async proxy
 // (required between st.shared and a bulk store that reads the same bytes).

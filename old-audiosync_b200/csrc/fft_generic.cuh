@@ -28,14 +28,13 @@
 
 namespace asc {
 
-#ifndef ASC_GEN_MIN_CTAS
-#define ASC_GEN_MIN_CTAS 3       // resident CTAs per SM the fp32 runtime-radix kernels are compiled for (85 registers)
-#endif
 constexpr int GEN_MAX_PASSES = 8;
 constexpr int GEN_THREADS = 256;       // CTA size of the large shapes
 constexpr int GEN_THREADS_SMALL = 64;  // ... and of shapes whose passes have fewer than ~128 butterflies per CTA
-// resident CTAs per SM a runtime-radix kernel is compiled for: 85 registers per thread (fp32)
-constexpr int gen_min_ctas(int nt, bool is_double) { return is_double ? (nt >= 256 ? 1 : 4) : (ASC_GEN_MIN_CTAS * 256) / nt; }
+// Resident CTAs per SM a runtime-radix kernel is compiled for.  fp32: GEN_MIN_CTAS CTAs of 256
+// threads (85 registers per thread), the occupancy the planner sizes tiles and rows for; fp64: 256 threads.
+constexpr int GEN_MIN_CTAS = 3;
+constexpr int gen_min_ctas(int nt, bool is_double) { return is_double ? (nt >= 256 ? 1 : 4) : (GEN_MIN_CTAS * 256) / nt; }
 
 // Division of a small unsigned number by a runtime constant without a divide: q = n / d for
 // n < 2^31 (Granlund-Montgomery: m = ceil(2^(31 + ceil(log2 d)) / d)); powers of two shift.
@@ -102,33 +101,6 @@ template <> struct GenTraits<double> {
     static constexpr int CT = 8;
     static constexpr int PADSH = 3;
 };
-
-// a + conj(b), a - conj(b), acc +- a conj(b) for the fp64 type (fp32: fft_kernels.cuh)
-ASC_HD cplxd cconj_add(cplxd a, cplxd b) { return cmake(a.x + b.x, a.y - b.y); }
-ASC_HD cplxd cconj_sub(cplxd a, cplxd b) { return cmake(a.x - b.x, a.y + b.y); }
-ASC_HD cplxd cmulc_acc(cplxd a, cplxd b, cplxd acc) {
-    return cmake(fma(a.x, b.x, fma(a.y, b.y, acc.x)), fma(a.y, b.x, fma(-a.x, b.y, acc.y)));
-}
-ASC_HD cplxd cmulc_nacc(cplxd a, cplxd b, cplxd acc) {
-    return cmake(fma(-a.x, b.x, fma(-a.y, b.y, acc.x)), fma(-a.y, b.x, fma(a.x, b.y, acc.y)));
-}
-// split / conj-multiply / merge with the twiddle folded (see split_mul_merge_w2): 2 Q[k], 2 Q[M-k]
-template <class C>
-ASC_HD void gen_split_mul_merge(C a, C b, C c, C d, C w2, C& qk2, C& qmk2) {
-    const C s = cconj_add(a, b), t = cconj_sub(a, b);
-    const C s2 = cconj_add(c, d), t2 = cconj_sub(c, d);
-    const C g = cmulc_acc(t, t2, cmulc(s, s2));
-    const C x = cmulc(s, t2);
-    const C h = cmulc_nacc(x, w2, cmulc(t, s2));
-    qk2 = cadd(g, h);
-    const C e = csub(g, h);
-    qmk2 = cmake(e.x, -e.y);
-}
-
-template <class C>
-ASC_HD C gen_tw2(const C* __restrict__ lo, const C* __restrict__ hi, unsigned a) {
-    return cmul(ldg(lo + (a & TW2_MASK)), ldg(hi + (a >> TW2_BITS)));
-}
 
 // Packed point n = (real 2n, real 2n + 1) of a signal.  Source: x[i mod 2L] for i < src_ext, zero
 // beyond; sample: y[i] for i < L, zero beyond (the zero pad of reference :159-166).  Points below
@@ -301,7 +273,7 @@ struct GenColFwdKernel {
                         C g[9];
                         static_for<0, 4>([&](auto I) {
                             constexpr int k = 1 << decltype(I)::value;
-                            if constexpr (k < R) g[k] = gen_tw2<C>(p.m_lo, p.m_hi, n2 * Wt * (unsigned)k);
+                            if constexpr (k < R) g[k] = tw2<C>(p.m_lo, p.m_hi, n2 * Wt * (unsigned)k);
                         });
                         for (int bf = tid / CT; bf < nbf; bf += TR) {
                             const int i0 = bf * R;
@@ -309,7 +281,7 @@ struct GenColFwdKernel {
                             load(i0, v);
                             dft_reg<R, -1, C>(v);
                             const unsigned f0 = (unsigned)ldg(p.p2f_col + i0);
-                            const C t0 = gen_tw2<C>(p.m_lo, p.m_hi, n2 * f0);
+                            const C t0 = tw2<C>(p.m_lo, p.m_hi, n2 * f0);
                             C* __restrict__ o = out + (f0 * (unsigned)M2 + n2);
                             o[0] = cmul(v[0], t0);
                             static_for<1, R>([&](auto K) {
@@ -448,7 +420,7 @@ struct GenRowFusedKernel {
         }
         // split + conj-multiply (reference :232-233) + merge, into the source rows
         ex.phase([&](int tid) {
-            const C wk1 = gen_tw2<C>(p.m_lo, p.m_hi, (unsigned)k1a);
+            const C wk1 = tw2<C>(p.m_lo, p.m_hi, (unsigned)k1a);
             if (two) {
                 C* __restrict__ zs_a = buf;
                 C* __restrict__ zs_b = buf + RP;
@@ -458,7 +430,7 @@ struct GenRowFusedKernel {
                     const int pa = phys(e), pb = phys(M2 - 1 - e);
                     const C w2 = cmul(ldg(p.wpos + e), wk1);
                     C qk, qmk;
-                    gen_split_mul_merge<C>(zs_a[pa], zs_b[pb], zp_a[pa], zp_b[pb], w2, qk, qmk);
+                    split_mul_merge_w2<C>(zs_a[pa], zs_b[pb], zp_a[pa], zp_b[pb], w2, qk, qmk);
                     zs_a[pa] = qk;
                     zs_b[pb] = qmk;
                 }
@@ -478,7 +450,7 @@ struct GenRowFusedKernel {
                     const C w2 = cmul(ldg(p.wpos + ea), wk1);
                     const int pa = phys(ea), pb = phys(eb);
                     C qk, qmk;
-                    gen_split_mul_merge<C>(zs[pa], zs[pb], zp[pa], zp[pb], w2, qk, qmk);
+                    split_mul_merge_w2<C>(zs[pa], zs[pb], zp[pa], zp[pb], w2, qk, qmk);
                     zs[pa] = qk;
                     if (pa != pb) zs[pb] = qmk;
                 }
@@ -567,9 +539,9 @@ struct GenRowFusedKernel {
                             C g[9];
                             static_for<0, 4>([&](auto I) {
                                 constexpr int k = 1 << decltype(I)::value;
-                                if constexpr (k < R) g[k] = gen_tw2<C>(p.m_lo, p.m_hi, (unsigned)(S * k) * k1);
+                                if constexpr (k < R) g[k] = tw2<C>(p.m_lo, p.m_hi, (unsigned)(S * k) * k1);
                             });
-                            const C t0 = gen_tw2<C>(p.m_lo, p.m_hi, (unsigned)j * k1);
+                            const C t0 = tw2<C>(p.m_lo, p.m_hi, (unsigned)j * k1);
                             o[j] = cmulc(v[0], t0);
                             static_for<1, R>([&](auto K) {
                                 constexpr int k = decltype(K)::value;

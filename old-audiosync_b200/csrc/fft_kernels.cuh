@@ -22,9 +22,10 @@
 // column tiles (cp.async.bulk.tensor), plain bulk copies for the contiguous rows,
 // completion on an mbarrier -- so that no thread spends instructions on the load
 // and the load of one CTA overlaps the butterflies of the other CTAs on the SM;
-// K_B's product rows leave the same way (cp.async.bulk shared -> global).  A
-// cp.async (LDGSTS) variant of each staging step remains selectable at compile
-// time.  The last pass is fused with the global store / epilogue.
+// K_B's product rows leave the same way (cp.async.bulk shared -> global).  Only
+// K_A has a second path: its first pass loads through registers where the input
+// cannot be staged (fp64, or fp32 not 16-byte aligned).  The last pass is fused
+// with the global store / epilogue.
 //
 // Kernel bodies are written against an executor (DeviceExec on the GPU,
 // tests/emu's HostExec on the CPU) that runs one "phase" for every thread and
@@ -35,19 +36,6 @@
 #include "fft_device.cuh"
 
 namespace asc {
-
-#ifndef ASC_ROW_TMA
-#define ASC_ROW_TMA 1        // K_B stages its rows with TMA bulk copies (0: cp.async / LDGSTS)
-#endif
-#ifndef ASC_COLFWD_GPOW
-#define ASC_COLFWD_GPOW 1    // K_A last pass: per-thread constants W_M^(n2*Wt*k) as powers of the k = 1 value
-#endif
-#ifndef ASC_COLFWD_STEP
-#define ASC_COLFWD_STEP 1    // K_A last pass: W_M^(n2*f0) stepped from item to item (see ColFwdKernel)
-#endif
-#ifndef ASC_SPLIT_FENCE_EVERY
-#define ASC_SPLIT_FENCE_EVERY 2   // split phase: compiler fence after every n-th e1 step (0: none): four items in flight (none: +0.14, 1: +0.1 us/pair)
-#endif
 
 constexpr int COL_T = 16;          // columns per tile: 16 * 8 B = one 128-byte line
 
@@ -64,8 +52,9 @@ constexpr unsigned TW2_BITS = 10;  // two-level twiddle tables: a = hi * 1024 + 
 constexpr unsigned TW2_MASK = (1u << TW2_BITS) - 1u;
 
 // exp(-2*pi*i*a/base) from the two-level tables (both halves correctly rounded
-// from fp64 on the host; one fp32 complex product here).
-ASC_HD cplx tw2(const cplx* __restrict__ lo, const cplx* __restrict__ hi, unsigned a) {
+// from fp64 on the host; one complex product here).
+template <class C>
+ASC_HD C tw2(const C* __restrict__ lo, const C* __restrict__ hi, unsigned a) {
     return cmul(ldg(lo + (a & TW2_MASK)), ldg(hi + (a >> TW2_BITS)));
 }
 
@@ -135,20 +124,30 @@ struct ArgmaxAcc {
     ASC_HD ArgmaxPair result() const { ArgmaxPair r; r.best = best; r.second = second; return r; }
 };
 
+// Merges the (peak key, second peak) pair (ob, os) into (best, second).  Pairs merge
+// associatively: the larger key leads, the smaller key's magnitude joins the two seconds
+// (unless it is the seed's, see ArgmaxAcc).  At grid level the key an atomicMax displaces (or
+// fails to displace) is merged with os = 0: over all CTAs max(min(old, mine)) is exactly the
+// second largest CTA peak.
+ASC_HD void argmax_merge(unsigned long long& best, float& second, unsigned long long ob, float os) {
+    const unsigned long long lose = ob > best ? best : ob;
+    best = ob > best ? ob : best;
+    second = fmaxf(second, os);
+    if (lose != 0ull && !argmax_key_is_seed(lose)) second = fmaxf(second, argmax_key_mag(lose));
+}
+
 // --------------------------------------------------------------------- K_A
-// STAGE 1 / 2 (fp32 input, 16-byte aligned): the tile is staged in shared memory before pass 0
-// -- 1: cp.async (LDGSTS), 2: boxes of a tensor map through the TMA unit, completion on an
-// mbarrier -- and the zero half of the padded sample is never touched; STAGE 0 (fp64 input or
-// unaligned pointers): the first pass loads, converts and packs through registers.
+// TMA (fp32 input, 16-byte aligned): the tile is staged in shared memory before pass 0 as boxes
+// of a tensor map through the TMA unit, completion on an mbarrier, and the zero half of the
+// padded sample is never touched; otherwise (fp64 input or unaligned pointers) the first pass
+// loads, converts and packs through registers.
 //
 // TMA staging of the SOURCE tile: the CTA's shared memory is exactly the tile, so the 8-byte
 // mbarrier sits at its very end and the last tile row (128 bytes) is not staged; pass 0 reads
 // that row from global memory, and the thread whose butterfly writes the barrier's bytes
 // invalidates it first.  (The sample tile has its unstaged upper half to spare.)
-template <class RL, int M2_, int NT, typename InT, int STAGE>
+template <class RL, int M2_, int NT, typename InT, bool TMA>
 struct ColFwdKernel {
-    static constexpr bool ASYNC = STAGE != 0;
-    static constexpr bool TMA = STAGE == 2;
     static constexpr int M1 = RL::n;
     static constexpr int M2 = M2_;                  // row length (compile time: index products fold)
     static constexpr int P = RL::count;
@@ -157,7 +156,8 @@ struct ColFwdKernel {
     static constexpr int MIN_CTAS = ctas_per_sm(SMEM, NT);
     static_assert(NT % COL_T == 0, "a thread must keep its column across items");
     static_assert(P >= 2, "column plans need at least two passes");
-    static_assert(!ASYNC || sizeof(InT) == 4, "async staging copies packed fp32 pairs verbatim");
+    static_assert(!TMA || sizeof(InT) == 4, "TMA staging copies packed fp32 pairs verbatim");
+    static_assert(!TMA || M1 >= 4, "tile too small for a box");
     static_assert(M1 % 2 == 0, "the zero half of the sample must be whole tile rows");
 
     struct Params {
@@ -172,7 +172,7 @@ struct ColFwdKernel {
         long long L;             // sample_len == M = M1 * M2
         long long src_pitch;     // elements between consecutive pairs' sources / samples;
         long long smp_pitch;     // 0 = packed ([pair][2L] and [pair][L])
-        // STAGE 2: [pair][M1 or M1/2 rows][2*M2 floats] views of sources / samples, boxes of
+        // TMA: [pair][M1 or M1/2 rows][2*M2 floats] views of sources / samples, boxes of
         // 32 floats x tile_box_rows(M1 - 1) resp. tile_box_rows(M1 / 2) rows
         CUtensorMap tm_src, tm_smp;
     };
@@ -194,7 +194,6 @@ struct ColFwdKernel {
 
         [[maybe_unused]] void* mbar = reinterpret_cast<char*>(buf) + SMEM - 8;
         if constexpr (TMA) {
-            static_assert(!TMA || M1 >= 4, "tile too small for a box");
             ex.phase([&](int tid) {
                 if (tid == 0) {
                     if (clears_peak) p.peaks[pair] = cleared_peak();
@@ -223,28 +222,6 @@ struct ColFwdKernel {
                 }
                 mbar_wait(mbar, 0);
             });
-        } else if constexpr (ASYNC) {
-            // tile row n1 = 16 packed points = 128 bytes = 8 chunks; shared tile has the same pitch
-            ex.phase([&](int tid) {
-                if (clears_peak && tid == 0) p.peaks[pair] = cleared_peak();
-                // thread -> (row tid/8 + i*NT/8, 16-byte part tid%8): both pointers advance by
-                // compile-time constants, so the unrolled loop is one LDGSTS per chunk
-                static_assert(NT % 8 == 0, "a thread keeps its 16-byte part across rows");
-                constexpr int RSTEP = NT / 8;
-                const int rows_valid = sig == 0 ? M1 : M1 / 2;
-                const int row0 = tid >> 3;
-                const char* __restrict__ g = reinterpret_cast<const char*>(x) + (size_t)c0 * sizeof(cplx) +
-                                             (size_t)row0 * (M2 * sizeof(cplx)) + (tid & 7) * 16;
-                char* __restrict__ sm = reinterpret_cast<char*>(buf) + tid * 16;
-#pragma unroll
-                for (int i = 0; i < (M1 + RSTEP - 1) / RSTEP; i++) {
-                    const int row = row0 + i * RSTEP;
-                    // rows of the zero pad are neither staged nor cleared: pass 0 below treats
-                    // them as zeros in registers and overwrites every position of the tile
-                    if (row < rows_valid) cp_async16(sm + i * (NT * 16), g + (size_t)i * (RSTEP * M2 * sizeof(cplx)));
-                }
-                cp_async_wait_all();
-            });
         }
 
         static_for<0, P>([&](auto PP) {
@@ -252,7 +229,7 @@ struct ColFwdKernel {
             constexpr int R = RL::r(ps);
             constexpr int S = RL::stride(ps);
             constexpr bool first = ps == 0, last = ps == P - 1;
-            constexpr bool from_global = first && !ASYNC;
+            constexpr bool from_global = first && !TMA;
             constexpr int items = (M1 / R) * COL_T;
             ex.phase([&](int tid) {
                 if (from_global && clears_peak && tid == 0) p.peaks[pair] = cleared_peak();
@@ -301,7 +278,7 @@ struct ColFwdKernel {
                             });
                         }
                     };
-                    if constexpr (first && ASYNC) {
+                    if constexpr (first && TMA) {
                         static_assert(R % 2 == 0 && S * R == M1, "zero-pad rows must be the inputs q >= R/2 of pass 0");
                         if (sig == 1) items_loop(std::true_type{});
                         else items_loop(std::false_type{});
@@ -319,9 +296,10 @@ struct ColFwdKernel {
                     // so the per-thread constants do not crowd out the butterfly's registers.
                     constexpr bool lean_g = R > 8;
                     cplx g[R];
-                    if constexpr (!lean_g && ASC_COLFWD_GPOW != 0) {
+                    if constexpr (!lean_g) {
                         // g[k] = g[1]^k by products (k = 2: g1*g1, 3: g2*g1, 4: g2*g2, 5: g4*g1, ...:
-                        // at most three roundings) instead of two scattered table reads per k
+                        // at most three roundings) instead of two scattered table reads per k, which
+                        // miss the small L1 left beside the tiles (K_A 7.32 -> 6.81 us/pair)
                         static_assert(R <= 8, "power chain written for k < 8");
                         g[1] = tw2(p.m_lo, p.m_hi, n2 * (unsigned)Wt);
                         static_for<2, R>([&](auto K) {
@@ -344,9 +322,9 @@ struct ColFwdKernel {
                     // whole number MSTEP of units of the leading digit (M1/r0 positions), the bin
                     // f0 advances by MSTEP per item and W_M^(n2*f0) by the per-thread constant
                     // W_M^(n2*MSTEP): one product per item instead of the digit reversal, three
-                    // table reads (L2 latency) and two products.
+                    // table reads (L2 latency) and two products (K_A 7.87 -> 7.31 us/pair).
                     constexpr int DB = NT / COL_T, UNIT = RL::stride(0) / R;
-                    constexpr bool STEP = ASC_COLFWD_STEP != 0 && ITER > 1 && DB % UNIT == 0;
+                    constexpr bool STEP = ITER > 1 && DB % UNIT == 0;
                     constexpr int MSTEP = STEP ? DB / UNIT : 0;
                     [[maybe_unused]] int f0_run = 0;
                     [[maybe_unused]] cplx t0_run = cmake(1.f, 0.f), gstep = cmake(1.f, 0.f);
@@ -416,10 +394,12 @@ struct ColFwdKernel {
 };
 
 // --------------------------------------------------------------------- K_C
-// TMA: the tile is staged with boxes of a tensor map over plane 0 (rows 0 .. M1-2; the last row
-// and the mbarrier as in ColFwdKernel); otherwise with cp.async.
-template <class RL, int M2_, int NT, bool TMA = false>
+// The tile is staged with boxes of a tensor map over plane 0 (rows 0 .. M1-2; the last row and
+// the mbarrier as in ColFwdKernel).  TMA staging is the only path; the TMA parameter is kept,
+// fixed to true, so that callers which name ColInvKernel<..., true> (tests/emu) keep building.
+template <class RL, int M2_, int NT, bool TMA = true>
 struct ColInvKernel {
+    static_assert(TMA, "K_C's tiles are always staged by the TMA unit");
     static constexpr int M1 = RL::n;
     static constexpr int M2 = M2_;
     static constexpr int P = RL::count;
@@ -435,7 +415,7 @@ struct ColInvKernel {
         PairPeak* peaks;         // [pair]
         const cplx* tw;          // RL pass tables (forward sign; conjugated here)
         long long L;
-        CUtensorMap tm;          // TMA: [2 * pair][M1 rows][2*M2 floats] view of the planes
+        CUtensorMap tm;          // [2 * pair][M1 rows][2*M2 floats] view of the planes
     };
     static constexpr int TMA_ROWS = M1 - 1;
 
@@ -448,37 +428,23 @@ struct ColInvKernel {
         const long long M = p.L;
         const cplx* __restrict__ in = p.planes + pair * 2 * M;
 
-        // stage the tile: row n1 = 128 bytes = 8 chunks of 16 bytes
-        [[maybe_unused]] void* mbar = reinterpret_cast<char*>(buf) + SMEM - 8;
-        if constexpr (TMA) {
-            ex.phase([&](int tid) {
-                if (tid == 0) mbar_init(mbar, 1);
-            });
-            ex.phase([&](int tid) {
-                if (tid == 0) {
-                    constexpr int NB = tile_boxes(TMA_ROWS), BR = tile_box_rows(TMA_ROWS);
-                    constexpr size_t pitch = (size_t)M2 * sizeof(cplx);
-                    const char* __restrict__ raw = reinterpret_cast<const char*>(in + c0);
-                    mbar_expect_tx(mbar, (unsigned)(NB * BR * 128));
-                    static_for<0, NB>([&](auto I) {
-                        constexpr int r0 = tile_box_start(TMA_ROWS, decltype(I)::value);
-                        tma_load_rows(buf + r0 * COL_T, &p.tm, 2 * c0, r0, (int)(2 * pair), mbar, raw + r0 * pitch, pitch, BR);
-                    });
-                }
-                mbar_wait(mbar, 0);
-            });
-        } else
+        // stage the tile
+        void* mbar = reinterpret_cast<char*>(buf) + SMEM - 8;
         ex.phase([&](int tid) {
-            static_assert(NT % 8 == 0, "a thread keeps its 16-byte part across rows");
-            constexpr int RSTEP = NT / 8;
-            const int row0 = tid >> 3;
-            const char* __restrict__ g = reinterpret_cast<const char*>(in + c0) +
-                                         (size_t)row0 * (M2 * sizeof(cplx)) + (tid & 7) * 16;
-            char* __restrict__ sm = reinterpret_cast<char*>(buf) + tid * 16;
-#pragma unroll
-            for (int i = 0; i < (M1 + RSTEP - 1) / RSTEP; i++)
-                if (row0 + i * RSTEP < M1) cp_async16(sm + i * (NT * 16), g + (size_t)i * (RSTEP * M2 * sizeof(cplx)));
-            cp_async_wait_all();
+            if (tid == 0) mbar_init(mbar, 1);
+        });
+        ex.phase([&](int tid) {
+            if (tid == 0) {
+                constexpr int NB = tile_boxes(TMA_ROWS), BR = tile_box_rows(TMA_ROWS);
+                constexpr size_t pitch = (size_t)M2 * sizeof(cplx);
+                const char* __restrict__ raw = reinterpret_cast<const char*>(in + c0);
+                mbar_expect_tx(mbar, (unsigned)(NB * BR * 128));
+                static_for<0, NB>([&](auto I) {
+                    constexpr int r0 = tile_box_start(TMA_ROWS, decltype(I)::value);
+                    tma_load_rows(buf + r0 * COL_T, &p.tm, 2 * c0, r0, (int)(2 * pair), mbar, raw + r0 * pitch, pitch, BR);
+                });
+            }
+            mbar_wait(mbar, 0);
         });
 
         static_for<0, P - 1>([&](auto PP) {
@@ -497,7 +463,7 @@ struct ColInvKernel {
                     cplx v[R];
                     static_for<0, R>([&](auto Q) {
                         constexpr int q = decltype(Q)::value;
-                        if constexpr (TMA && ps == 0 && q == R - 1) {
+                        if constexpr (ps == 0 && q == R - 1) {
                             // tile row M1 - 1 is not staged (the mbarrier sits there)
                             if (i0 == S - 1) v[q] = ldg(in + ((long long)(M1 - 1) * M2 + c0 + c));
                             else v[q] = buf[(i0 + q * S) * COL_T + c];
@@ -505,7 +471,7 @@ struct ColInvKernel {
                             v[q] = buf[(i0 + q * S) * COL_T + c];
                         }
                     });
-                    if constexpr (TMA && ps == 0) {
+                    if constexpr (ps == 0) {
                         if (i0 == S - 1 && c == COL_T - 1) mbar_inval(mbar);   // overwritten below
                     }
                     dft_reg<R, +1>(v);
@@ -611,46 +577,16 @@ ASC_HD void split_mul_merge(cplx a, cplx b, cplx c, cplx d, cplx w, cplx& qk, cp
 //   i conj(w) (p1 - p2) / 2 = H = t conj(s') - conj(w^2) s conj(t')
 // so only w^2 = exp(-2*pi*i*k/M) is needed.  Returns 2 Q[k] = G + H and 2 Q[M-k] = conj(G - H):
 // the caller folds the factor 1/2 into a later twiddle.  18 packed instructions instead of 34.
-ASC_HD cplx cconj_add(cplx a, cplx b) {   // a + conj(b)
-#if ASC_PACKED
-    return __fadd2_rn(a, cmake(b.x, -b.y));
-#else
-    return cmake(a.x + b.x, a.y - b.y);
-#endif
-}
-ASC_HD cplx cconj_sub(cplx a, cplx b) {   // a - conj(b)
-#if ASC_PACKED
-    return __fadd2_rn(a, cmake(-b.x, b.y));
-#else
-    return cmake(a.x - b.x, a.y + b.y);
-#endif
-}
-// acc + a * conj(b)
-ASC_HD cplx cmulc_acc(cplx a, cplx b, cplx acc) {
-#if ASC_PACKED
-    const cplx t = __ffma2_rn(cmake(a.y, -a.x), cmake(b.y, b.y), acc);
-    return __ffma2_rn(a, cmake(b.x, b.x), t);
-#else
-    return cmake(fmaf(a.x, b.x, fmaf(a.y, b.y, acc.x)), fmaf(a.y, b.x, fmaf(-a.x, b.y, acc.y)));
-#endif
-}
-// acc - a * conj(b)
-ASC_HD cplx cmulc_nacc(cplx a, cplx b, cplx acc) {
-#if ASC_PACKED
-    const cplx t = __ffma2_rn(cmake(-a.y, a.x), cmake(b.y, b.y), acc);
-    return __ffma2_rn(a, cmake(-b.x, -b.x), t);
-#else
-    return cmake(fmaf(-a.x, b.x, fmaf(-a.y, b.y, acc.x)), fmaf(-a.y, b.x, fmaf(a.x, b.y, acc.y)));
-#endif
-}
-ASC_HD void split_mul_merge_w2(cplx a, cplx b, cplx c, cplx d, cplx w2, cplx& qk2, cplx& qmk2) {
-    const cplx s = cconj_add(a, b), t = cconj_sub(a, b);
-    const cplx s2 = cconj_add(c, d), t2 = cconj_sub(c, d);
-    const cplx g = cmulc_acc(t, t2, cmulc(s, s2));
-    const cplx x = cmulc(s, t2);
-    const cplx h = cmulc_nacc(x, w2, cmulc(t, s2));
+// C: cplx (the product) or cplxd (the runtime-radix kernels' fp64 mode).
+template <class C>
+ASC_HD void split_mul_merge_w2(C a, C b, C c, C d, C w2, C& qk2, C& qmk2) {
+    const C s = cconj_add(a, b), t = cconj_sub(a, b);
+    const C s2 = cconj_add(c, d), t2 = cconj_sub(c, d);
+    const C g = cmulc_acc(t, t2, cmulc(s, s2));
+    const C x = cmulc(s, t2);
+    const C h = cmulc_nacc(x, w2, cmulc(t, s2));
     qk2 = cadd(g, h);
-    const cplx e = csub(g, h);
+    const C e = csub(g, h);
     qmk2 = cmake(e.x, -e.y);
 }
 
@@ -668,8 +604,7 @@ struct RowFusedKernel {
     static constexpr int S0 = RL::stride(0);
     static_assert(M2 % 2 == 0, "row length must be even (16-byte chunks, bulk store size)");
     static_assert(P >= 2, "row plans need at least two passes");
-    static constexpr bool ROW_TMA = ASC_ROW_TMA != 0;
-    static_assert(!ROW_TMA || (S0 * R0 == M2 && S0 >= 16), "pass 0 must own the last two points of a row as its last two items");
+    static_assert(S0 * R0 == M2 && S0 >= 16, "pass 0 must own the last two points of a row as its last two items");
 
     // A pass whose sub-stride S is below 16 (but not 1) would have half-warps
     // straddle blocks and collide in the banks; give each block 16 thread slots
@@ -714,12 +649,12 @@ struct RowFusedKernel {
         void* tabbar = buf + 2 * RP + 2 * TABP;               // mbarrier of that copy
 
         // ---- stage the 2*nrows rows.  smem slots: 0,1 source rows; 2,3 sample rows.
-        // ROW_TMA: four bulk copies of the TMA unit, issued by one thread, awaited by all.
+        // Four bulk copies of the TMA unit, issued by one thread, awaited by all.
         // The CTA's shared memory is exactly the four rows, so the 8-byte mbarrier sits on the
         // last point of slot 3; the last two points of that row are not staged -- forward pass 0
         // reads them from global memory instead -- and the thread whose butterfly writes them
         // first invalidates the barrier.
-        if constexpr (ROW_TMA) {
+        {
             void* mbar = buf + 4 * RP - 1;
             ex.phase([&](int tid) {
                 if (tid == 0) mbar_init(mbar, 1);
@@ -737,23 +672,7 @@ struct RowFusedKernel {
                 }
                 mbar_wait(mbar, 0);
             });
-        } else
-        ex.phase([&](int tid) {
-            constexpr int cpr = M2 / 2;                       // 16-byte chunks per row
-            static_for<0, 4>([&](auto B) {
-                constexpr int slot = decltype(B)::value;      // 0,1 source rows; 2,3 sample rows
-                constexpr int rr = slot & 1;
-                if (rr == 0 || two) {
-                    const cplx* __restrict__ g = (slot >= 2 ? plane_p : plane_s) + (long long)(rr ? k1b : k1a) * M2;
-                    const char* __restrict__ gs = reinterpret_cast<const char*>(g) + tid * 16;
-                    char* __restrict__ sm = reinterpret_cast<char*>(buf + slot * RP) + tid * 16;
-#pragma unroll
-                    for (int i = 0; i < (cpr + NT - 1) / NT; i++)
-                        if (tid + i * NT < cpr) cp_async16(sm + i * (NT * 16), gs + i * (NT * 16));
-                }
-            });
-            cp_async_wait_all();
-        });
+        }
 
         // ---- forward DIF on 2*nrows rows.  One pass over the nb rows in shared-memory slots
         // slot0, slot0 + sstep, ... by threads t = 0 .. nt-1.
@@ -764,8 +683,8 @@ struct RowFusedKernel {
             constexpr int SL = slots(S);
             constexpr int per_row = (M2 / (S * R)) * SL;
             const int items = per_row * nb;
-            // ROW_TMA, pass 0: items (slot 3, i0 = S-2) and (slot 3, i0 = S-1) are the last two of
-            // a call whose last row is slot 3
+            // pass 0: items (slot 3, i0 = S-2) and (slot 3, i0 = S-1) are the last two of a call
+            // whose last row is slot 3
             [[maybe_unused]] const int tail_w = (slot0 + (nb - 1) * sstep == 3) ? items - 2 : 0x7fffffff;
             {
                 for (int w = t; w < items; w += nt) {
@@ -781,7 +700,7 @@ struct RowFusedKernel {
                         constexpr int q = decltype(Q)::value;
                         v[q] = row[i0 + q * S];
                     });
-                    if constexpr (ROW_TMA && ps == 0) {
+                    if constexpr (ps == 0) {
                         // the two points of slot 3 the staging left out (see above): the last two
                         // items of the pass; what the shared-memory read returned for them was the
                         // barrier's bytes
@@ -843,8 +762,9 @@ struct RowFusedKernel {
                     });
                     static_for<0, SPLIT_MN>([&](auto Mm) {
 #if defined(__CUDA_ARCH__)
-                        if constexpr (ASC_SPLIT_FENCE_EVERY > 0 && decltype(Mm)::value > 0 &&
-                                      decltype(Mm)::value % (ASC_SPLIT_FENCE_EVERY > 0 ? ASC_SPLIT_FENCE_EVERY : 1) == 0)
+                        // compiler fence after every second e1 step: four items in flight per
+                        // thread (no fence: +0.14 us/pair, a fence after every step: +0.1)
+                        if constexpr (decltype(Mm)::value > 0 && decltype(Mm)::value % 2 == 0)
                             asm volatile("" ::: "memory");
 #endif
                         static_for<0, SPLIT_XN>([&](auto X) {
@@ -1026,22 +946,10 @@ struct DeviceExec {
         return *k;
 #endif
     }
-    // CTA-wide (peak key, second peak) of the per-thread pairs, then one atomicMax on *dst
-    // and one on *dst_second.  Pairs merge associatively: the larger key leads, the smaller
-    // key's magnitude joins the two seconds (unless it is the seed's, see ArgmaxAcc).  At grid level the key the atomicMax displaces
-    // (or fails to displace) is a second-peak candidate too: over all CTAs max(min(old, mine))
-    // is exactly the second largest CTA peak.  `scratch`: at least 32 * 12 bytes of the CTA's
+    // CTA-wide (peak key, second peak) of the per-thread pairs (argmax_merge), then one
+    // atomicMax on *dst and one on *dst_second.  `scratch`: at least 32 * 12 bytes of the CTA's
     // dynamic shared memory; it may alias data f() reads (a barrier separates the two uses).
     // No static shared memory, so the column kernels keep 3 CTAs per SM.
-#if defined(__CUDA_ARCH__)
-    static __device__ __forceinline__ void merge_pairs(unsigned long long& best, float& second,
-                                                       unsigned long long ob, float os) {
-        const unsigned long long lose = ob > best ? best : ob;
-        best = ob > best ? ob : best;
-        second = fmaxf(second, os);
-        if (lose != 0ull && !argmax_key_is_seed(lose)) second = fmaxf(second, argmax_key_mag(lose));
-    }
-#endif
     template <class F>
     ASC_HD void phase_argmax(F&& f, unsigned long long* dst, unsigned int* dst_second, void* scratch) {
 #if defined(__CUDA_ARCH__)
@@ -1051,7 +959,7 @@ struct DeviceExec {
         unsigned long long best = mine.best;
         float second = mine.second;
         for (int o = 16; o > 0; o >>= 1)
-            merge_pairs(best, second, __shfl_xor_sync(0xffffffffu, best, o), __shfl_xor_sync(0xffffffffu, second, o));
+            argmax_merge(best, second, __shfl_xor_sync(0xffffffffu, best, o), __shfl_xor_sync(0xffffffffu, second, o));
         const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
         const int nw = (blockDim.x + 31) >> 5;
         __syncthreads();                      // every warp is done reading what `scratch` aliases
@@ -1061,10 +969,10 @@ struct DeviceExec {
             best = lane < nw ? s_best[lane] : 0ull;
             second = lane < nw ? s_sec[lane] : 0.0f;
             for (int o = 16; o > 0; o >>= 1)
-                merge_pairs(best, second, __shfl_xor_sync(0xffffffffu, best, o), __shfl_xor_sync(0xffffffffu, second, o));
+                argmax_merge(best, second, __shfl_xor_sync(0xffffffffu, best, o), __shfl_xor_sync(0xffffffffu, second, o));
             if (lane == 0) {
                 const unsigned long long old = atomicMax(dst, best);
-                if (old != best) merge_pairs(best, second, old, 0.0f);
+                if (old != best) argmax_merge(best, second, old, 0.0f);
                 atomicMax(dst_second, float_order_bits(second));
             }
         }

@@ -88,7 +88,6 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 static EncodeTiledFn tensor_map_encoder() {
     static const EncodeTiledFn fn = [] {
-        if (getenv("AUDIOSYNC_CUDA_NO_TMA_TILES")) return (EncodeTiledFn) nullptr;   // diagnostic knob: cp.async staging of the column tiles
         void* f = nullptr;
         cudaDriverEntryPointQueryResult q;
         if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess ||
@@ -113,7 +112,7 @@ static int make_tile_map(CUtensorMap* tm, const void* base, int M2, int rows, si
     const CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(base), gdim, gstride, box, estride,
                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    return r == CUDA_SUCCESS ? 0 : -1;   // the caller falls back to cp.async staging
+    return r == CUDA_SUCCESS ? 0 : -1;
 }
 
 // Stage launches of the static path: programmatic dependent launch (see pdl_prologue).

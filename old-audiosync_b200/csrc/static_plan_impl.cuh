@@ -21,41 +21,45 @@ static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& 
     const cplx* row_tab = static_cast<const cplx*>(plan->row_tab.p);
     const cplx* m_lo = static_cast<const cplx*>(plan->m_lo.p);
     const cplx* m_hi = static_cast<const cplx*>(plan->m_hi.p);
+    // K_C always stages its tiles through the TMA unit: its map is encoded before anything is
+    // enqueued, so that a failure leaves no partial wave behind
+    using KC = ColInvKernel<Col, Row::n, P::NT_COL>;
+    typename KC::Params pc{planes, peaks, col_tw, P::L};
+    if (make_tile_map(&pc.tm, planes, M2, M1, (size_t)P::L * sizeof(cplx), (size_t)2 * pairs,
+                      tile_box_rows(KC::TMA_ROWS)) != 0) {
+        set_last_error("L = %lld: cuTensorMapEncodeTiled %s for the workspace planes", P::L,
+                       tensor_map_encoder() ? "failed" : "is not exported by the driver");
+        return -1;
+    }
     const dim3 grid_a(M2 / COL_T, 2, pairs);
-    auto col_fwd = [&](auto KK, const auto* s_in, const auto* m_in) -> int {
+    auto col_fwd = [&](auto KK, const typename decltype(KK)::Params& p) -> int {
         using K = decltype(KK);
-        typename K::Params p{s_in, m_in, planes, peaks, col_tw, col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch};
         return launch(ctx, d, KC_COL_FWD, st, [&] {
             launch_stage(fft_kernel_entry<K>, grid_a, dim3(K::THREADS), K::SMEM, st, p);
         });
     };
     if (dtype == AUDIOSYNC_CUDA_F32) {
-        // cp.async staging needs 16-byte aligned rows: every pair / row offset is a multiple
-        // of 16 bytes, so only the base pointers decide.
-        static const bool no_async = getenv("AUDIOSYNC_CUDA_NOASYNC") != nullptr;   // experiment knob
-        const bool aligned = !no_async && ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(smp)) & 15u) == 0 &&
+        // TMA boxes need 16-byte aligned rows: every pair / row offset is a multiple of 16 bytes,
+        // so only the base pointers decide.  Other fp32 inputs load through registers.
+        const bool aligned = ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(smp)) & 15u) == 0 &&
                              src_pitch % 4 == 0 && smp_pitch % 4 == 0;
         const float* s_in = static_cast<const float*>(src);
         const float* m_in = static_cast<const float*>(smp);
-        int rc;
-        using KT = ColFwdKernel<Col, Row::n, P::NT_COL, float, 2>;
+        using KT = ColFwdKernel<Col, Row::n, P::NT_COL, float, true>;
+        using KR = ColFwdKernel<Col, Row::n, P::NT_COL, float, false>;
         typename KT::Params pt{s_in, m_in, planes, peaks, col_tw, col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch};
-        if (aligned && tensor_map_encoder() &&
-            make_tile_map(&pt.tm_src, s_in, M2, M1, (size_t)src_pitch * sizeof(float), (size_t)pairs,
-                          tile_box_rows(KT::SRC_ROWS)) == 0 &&
-            make_tile_map(&pt.tm_smp, m_in, M2, M1 / 2, (size_t)smp_pitch * sizeof(float), (size_t)pairs,
-                          tile_box_rows(KT::SMP_ROWS)) == 0) {
-            rc = launch(ctx, d, KC_COL_FWD, st, [&] {
-                launch_stage(fft_kernel_entry<KT>, grid_a, dim3(KT::THREADS), KT::SMEM, st, pt);
-            });
-        } else {
-            rc = aligned ? col_fwd(ColFwdKernel<Col, Row::n, P::NT_COL, float, 1>{}, s_in, m_in)
-                         : col_fwd(ColFwdKernel<Col, Row::n, P::NT_COL, float, 0>{}, s_in, m_in);
-        }
-        if (rc != 0) return -1;
+        const bool tma = aligned &&
+                         make_tile_map(&pt.tm_src, s_in, M2, M1, (size_t)src_pitch * sizeof(float), (size_t)pairs,
+                                       tile_box_rows(KT::SRC_ROWS)) == 0 &&
+                         make_tile_map(&pt.tm_smp, m_in, M2, M1 / 2, (size_t)smp_pitch * sizeof(float), (size_t)pairs,
+                                       tile_box_rows(KT::SMP_ROWS)) == 0;
+        if ((tma ? col_fwd(KT{}, pt)
+                 : col_fwd(KR{}, {s_in, m_in, planes, peaks, col_tw, col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch})) != 0)
+            return -1;
     } else {
-        if (col_fwd(ColFwdKernel<Col, Row::n, P::NT_COL, double, 0>{}, static_cast<const double*>(src),
-                    static_cast<const double*>(smp)) != 0) return -1;
+        using K = ColFwdKernel<Col, Row::n, P::NT_COL, double, false>;
+        if (col_fwd(K{}, {static_cast<const double*>(src), static_cast<const double*>(smp), planes, peaks, col_tw,
+                          col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch}) != 0) return -1;
     }
     {
         using K = RowFusedKernel<Row, Col::n, P::NT_ROW>;
@@ -65,21 +69,10 @@ static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& 
                 launch_stage(fft_kernel_entry<K>, grid, dim3(K::THREADS), K::SMEM, st, p);
             }) != 0) return -1;
     }
-    using KCT = ColInvKernel<Col, Row::n, P::NT_COL, true>;
-    typename KCT::Params pct{planes, peaks, col_tw, P::L};
-    if (tensor_map_encoder() &&
-        make_tile_map(&pct.tm, planes, M2, M1, (size_t)P::L * sizeof(cplx), (size_t)2 * pairs,
-                      tile_box_rows(KCT::TMA_ROWS)) == 0) {
+    {
         const dim3 grid(pairs, M2 / COL_T, 1);
         if (launch(ctx, d, KC_COL_INV, st, [&] {
-                launch_stage(fft_kernel_entry<KCT>, grid, dim3(KCT::THREADS), KCT::SMEM, st, pct);
-            }) != 0) return -1;
-    } else {
-        using K = ColInvKernel<Col, Row::n, P::NT_COL>;
-        typename K::Params p{planes, peaks, col_tw, P::L};
-        const dim3 grid(pairs, M2 / COL_T, 1);
-        if (launch(ctx, d, KC_COL_INV, st, [&] {
-                launch_stage(fft_kernel_entry<K>, grid, dim3(K::THREADS), K::SMEM, st, p);
+                launch_stage(fft_kernel_entry<KC>, grid, dim3(KC::THREADS), KC::SMEM, st, pc);
             }) != 0) return -1;
     }
     return 0;
@@ -111,13 +104,13 @@ int build_static_plan(FftPlan* plan) {
         upload(plan->row_tab, build_row_tab<Row>(P::L, Col::n)) != 0 ||
         upload(plan->m_lo, m_lo) != 0 || upload(plan->m_hi, m_hi) != 0)
         return -1;
-    if (prepare_kernel<ColFwdKernel<Col, Row::n, P::NT_COL, float, 2>>(ColFwdKernel<Col, Row::n, P::NT_COL, float, 2>::SMEM) != 0 ||
-        prepare_kernel<ColFwdKernel<Col, Row::n, P::NT_COL, float, 1>>(ColFwdKernel<Col, Row::n, P::NT_COL, float, 1>::SMEM) != 0 ||
-        prepare_kernel<ColFwdKernel<Col, Row::n, P::NT_COL, float, 0>>(ColFwdKernel<Col, Row::n, P::NT_COL, float, 0>::SMEM) != 0 ||
-        prepare_kernel<ColFwdKernel<Col, Row::n, P::NT_COL, double, 0>>(ColFwdKernel<Col, Row::n, P::NT_COL, double, 0>::SMEM) != 0 ||
-        prepare_kernel<RowFusedKernel<Row, Col::n, P::NT_ROW>>(RowFusedKernel<Row, Col::n, P::NT_ROW>::SMEM) != 0 ||
-        prepare_kernel<ColInvKernel<Col, Row::n, P::NT_COL, true>>(ColInvKernel<Col, Row::n, P::NT_COL, true>::SMEM) != 0 ||
-        prepare_kernel<ColInvKernel<Col, Row::n, P::NT_COL>>(ColInvKernel<Col, Row::n, P::NT_COL>::SMEM) != 0)
+    using KT = ColFwdKernel<Col, Row::n, P::NT_COL, float, true>;
+    using KR = ColFwdKernel<Col, Row::n, P::NT_COL, float, false>;
+    using KD = ColFwdKernel<Col, Row::n, P::NT_COL, double, false>;
+    using KB = RowFusedKernel<Row, Col::n, P::NT_ROW>;
+    using KC = ColInvKernel<Col, Row::n, P::NT_COL>;
+    if (prepare_kernel<KT>(KT::SMEM) != 0 || prepare_kernel<KR>(KR::SMEM) != 0 || prepare_kernel<KD>(KD::SMEM) != 0 ||
+        prepare_kernel<KB>(KB::SMEM) != 0 || prepare_kernel<KC>(KC::SMEM) != 0)
         return -1;
     plan->run_wave = [plan](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
                             int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,

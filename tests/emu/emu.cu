@@ -38,21 +38,18 @@ struct HostExec {
         float second = 0.0f;
         for (int t = 0; t < nt; t++) {
             const ArgmaxPair k = f(t);
-            const unsigned long long lose = k.best > best ? best : k.best;
-            if (k.best > best) best = k.best;
-            if (lose != 0 && !argmax_key_is_seed(lose)) second = fmaxf(second, argmax_key_mag(lose));
-            second = fmaxf(second, k.second);
+            argmax_merge(best, second, k.best, k.second);
         }
         const unsigned long long old = *dst;
-        const unsigned long long loser = old < best ? old : best;
         if (best > old) *dst = best;
-        if (loser != 0 && old != best && !argmax_key_is_seed(loser)) second = fmaxf(second, argmax_key_mag(loser));
+        if (old != best) argmax_merge(best, second, old, 0.0f);
         const unsigned int sb = float_order_bits(second);
         if (sb > *dst_second) *dst_second = sb;
     }
 };
 
-template <class P, typename InT>
+// TMA: K_A stages its tiles (fp32 only), otherwise its first pass loads through registers
+template <class P, typename InT, bool TMA>
 static int run_static(const InT* source, const InT* sample, PairPeak* peak, cplx* planes_out) {
     using Col = typename P::Col;
     using Row = typename P::Row;
@@ -69,9 +66,8 @@ static int run_static(const InT* source, const InT* sample, PairPeak* peak, cplx
     peak->key = 12345ull; peak->second_bits = 777u; peak->seed_bits = 777u;   // garbage: K_A must clear them
 
     {
-        // fp32: the TMA-staged variant (the product's default; host emulation copies the same boxes
-        // and leaves the last tile row unstaged), fp64: through registers
-        using K = ColFwdKernel<Col, Row::n, P::NT_COL, InT, sizeof(InT) == 4 ? 2 : 0>;
+        // TMA: host emulation copies the same boxes and leaves the last tile row unstaged
+        using K = ColFwdKernel<Col, Row::n, P::NT_COL, InT, TMA>;
         typename K::Params p{source, sample, planes.data(), peak, col_tw.data(), col_tc.data(), m_lo.data(), m_hi.data(), M};
         std::vector<cplx> smem(K::SMEM / sizeof(cplx));
         for (int sig = 0; sig < 2; sig++)
@@ -91,7 +87,7 @@ static int run_static(const InT* source, const InT* sample, PairPeak* peak, cplx
     }
     if (planes_out) memcpy(planes_out, planes.data(), sizeof(cplx) * M);
     {
-        using K = ColInvKernel<Col, Row::n, P::NT_COL, true>;
+        using K = ColInvKernel<Col, Row::n, P::NT_COL>;
         typename K::Params p{planes.data(), peak, col_tw.data(), M};
         std::vector<cplx> smem(K::SMEM / sizeof(cplx));
         for (int tile = 0; tile < M2 / COL_T; tile++) {
@@ -188,9 +184,10 @@ static int run_generic(const InT* source, const InT* sample, long long L, long l
 
 static double g_last_second = 0.0;   // second peak of the last emu_any call
 
+// ka_registers: static plans run K_A's register load even where the product stages fp32 tiles
 template <typename InT>
 static int emu_any(const InT* source, const InT* sample, long long L, int forced,
-                   long long* raw_index, double* peak_value, int* path) {
+                   long long* raw_index, double* peak_value, int* path, bool ka_registers = false) {
     PairPeak pk;
     memset(&pk, 0, sizeof(pk));
     PathKind kind = choose_path(L, forced);
@@ -199,7 +196,12 @@ static int emu_any(const InT* source, const InT* sample, long long L, int forced
     if (kind == PATH_STATIC_FFT) {
         for_each_static_plan([&](auto P) {
             using PT = decltype(P);
-            if (PT::L == L) rc = run_static<PT, InT>(source, sample, &pk, nullptr);
+            if (PT::L != L) return;
+            if constexpr (sizeof(InT) == 4)
+                rc = ka_registers ? run_static<PT, InT, false>(source, sample, &pk, nullptr)
+                                  : run_static<PT, InT, true>(source, sample, &pk, nullptr);
+            else
+                rc = run_static<PT, InT, false>(source, sample, &pk, nullptr);
         });
     } else if (kind == PATH_SMALL_FFT) {
         rc = run_small<InT>(source, sample, L, &pk);
@@ -254,6 +256,13 @@ int emu_generic_describe(long long L, int precise, char* desc, size_t desc_len) 
 int emu_xcorr_f32(const float* source, const float* sample, long long L, int forced,
                   long long* raw_index, double* peak_value, int* path) {
     return emu_any<float>(source, sample, L, forced, raw_index, peak_value, path);
+}
+
+// the same with K_A's fp32 first pass through registers (the product's path for fp32 inputs
+// that are not 16-byte aligned)
+int emu_xcorr_f32_ka_registers(const float* source, const float* sample, long long L, int forced,
+                               long long* raw_index, double* peak_value, int* path) {
+    return emu_any<float>(source, sample, L, forced, raw_index, peak_value, path, true);
 }
 
 int emu_xcorr_f64(const double* source, const double* sample, long long L, int forced,

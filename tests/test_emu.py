@@ -28,6 +28,7 @@ def emu():
     sig = [C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.POINTER(C.c_longlong),
            C.POINTER(C.c_double), C.POINTER(C.c_int)]
     E.emu_xcorr_f32.argtypes = sig
+    E.emu_xcorr_f32_ka_registers.argtypes = sig
     E.emu_xcorr_f64.argtypes = sig
     E.emu_fold.argtypes = [C.c_longlong, C.c_longlong] + [C.POINTER(C.c_longlong)] * 4
     E.emu_key_abs.restype = C.c_ulonglong
@@ -52,33 +53,40 @@ def emu():
 PATH_AUTO, PATH_FFT = 0, 1
 
 
-def run_emu(E, src, smp, f64=False, forced=PATH_FFT):
+def run_emu(E, src, smp, f64=False, forced=PATH_FFT, ka_registers=False):
+    """ka_registers: the static plans' K_A takes fp32 through its register load instead of TMA staging."""
     L = len(smp)
     idx, pk, path = C.c_longlong(), C.c_double(), C.c_int()
     dt = np.float64 if f64 else np.float32
     s = np.ascontiguousarray(src, dt); p = np.ascontiguousarray(smp, dt)
-    fn = E.emu_xcorr_f64 if f64 else E.emu_xcorr_f32
+    fn = E.emu_xcorr_f64 if f64 else (E.emu_xcorr_f32_ka_registers if ka_registers else E.emu_xcorr_f32)
     rc = fn(s.ctypes.data, p.ctypes.data, L, forced, C.byref(idx), C.byref(pk), C.byref(path))
     assert rc == 0
     return idx.value, pk.value, path.value
+
+
+STATIC_LENGTHS = (144000, 288000, 480000, 720000, 960000, 1440000)
 
 
 def _fft_cases():
     out = []
     for c in SYNTH["cases"]:
         if c["L"] % 2 == 0 and c["tag"] == "pair" and c["pair_id"] in (0, 3):
-            out.append(c)
+            out.append(pytest.param(c, False, id="L%d-p%d" % (c["L"], c["pair_id"])))
+            # fp32 at a static length: also through K_A's register load (unaligned inputs)
+            if c["pair_id"] == 0 and c["L"] in STATIC_LENGTHS:
+                out.append(pytest.param(c, True, id="L%d-p%d-ka_registers" % (c["L"], c["pair_id"])))
     return out
 
 
-@pytest.mark.parametrize("case", _fft_cases(), ids=lambda c: "L%d-p%d" % (c["L"], c["pair_id"]))
-def test_emulated_kernels_match_golden(emu, case):
+@pytest.mark.parametrize("case,ka_registers", _fft_cases())
+def test_emulated_kernels_match_golden(emu, case, ka_registers):
     L = case["L"]
     path = emu.emu_path_for(L, PATH_FFT)
     if path == 2:
         pytest.skip("length has no FFT plan (direct path: nothing to emulate)")
     src, smp = capi.synth_pair(case["seed"], case["pair_id"], L)
-    idx, peak, used = run_emu(emu, src, smp, f64=(case["pair_id"] == 3))
+    idx, peak, used = run_emu(emu, src, smp, f64=(case["pair_id"] == 3), ka_registers=ka_registers)
     assert used == path
     assert case["margin"] > 1e-4                     # unique peak => index must be exact
     assert idx == case["raw_index"]
@@ -93,7 +101,7 @@ def test_emulated_kernels_match_golden(emu, case):
 
 
 def test_static_plans_cover_interval_schedule(emu):
-    for L in (144000, 288000, 480000, 720000, 960000, 1440000):
+    for L in STATIC_LENGTHS:
         assert emu.emu_path_for(L, PATH_AUTO) == 0          # PATH_STATIC_FFT
     for L in (4096, 4320, 5000, 6250, 8192):
         assert emu.emu_path_for(L, PATH_AUTO) == 1          # PATH_SMALL_FFT

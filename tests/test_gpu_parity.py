@@ -1023,13 +1023,14 @@ import sys, json
 sys.path.insert(0, {root!r}); sys.path.insert(0, {pkg!r})
 import numpy as np, torch
 import audiosync_cuda as ac
-L, n = {L}, 5
+L, n, off = {L}, 5, {off}
 with ac.Context([0]) as c:
-    d_src = torch.empty(n * 2 * L, dtype=torch.float32, device="cuda:0")
+    d_src = torch.empty(n * 2 * L + off, dtype=torch.float32, device="cuda:0")
     d_smp = torch.empty(n * L, dtype=torch.float32, device="cuda:0")
     d_res = torch.zeros(n * ac.RESULT_DTYPE.itemsize, dtype=torch.uint8, device="cuda:0")
-    c.synth_pairs(0, {seed}, 0, n, L, ac.F32, d_src.data_ptr(), d_smp.data_ptr())
-    c.xcorr_batch_device(0, d_src.data_ptr(), d_smp.data_ptr(), n, L, ac.F32, d_res.data_ptr())
+    src = d_src.data_ptr() + 4 * off
+    c.synth_pairs(0, {seed}, 0, n, L, ac.F32, src, d_smp.data_ptr())
+    c.xcorr_batch_device(0, src, d_smp.data_ptr(), n, L, ac.F32, d_res.data_ptr())
     c.synchronize(0)
     r = d_res.cpu().numpy().view(ac.RESULT_DTYPE)
 print(json.dumps({{k: [float(x).hex() for x in r[k]] for k in ("raw_index", "lag", "peak", "coef", "second", "ret")}}))
@@ -1038,15 +1039,16 @@ print(json.dumps({{k: [float(x).hex() for x in r[k]] for k in ("raw_index", "lag
 
 @pytest.mark.parametrize("L", [144000, 1440000])
 def test_staging_and_launch_variants_are_bit_identical(L):
-    """The TMA-staged tiles / programmatic dependent launch (default) and the diagnostic
-    fallbacks (cp.async staging of the column tiles, plain stream-ordered launches) run the
-    same arithmetic: every field of the result records must agree bit for bit."""
+    """The TMA-staged column tiles with programmatic dependent launch (default), the first column
+    pass loading through registers (source base 8 bytes off a 16-byte boundary) and plain
+    stream-ordered launches run the same arithmetic: every field of the result records must agree
+    bit for bit.  The offset is two floats, not one: the register path loads float2."""
     import subprocess
     import sys
     root = os.path.dirname(HERE)
-    code = _VARIANT_SNIPPET.format(root=root, pkg=os.path.join(root, "old-audiosync_b200"), L=L, seed=SEED)
     outs = []
-    for extra in ({}, {"AUDIOSYNC_CUDA_NO_TMA_TILES": "1"}, {"AUDIOSYNC_CUDA_NO_PDL": "1"}):
+    for extra, off in (({}, 0), ({}, 2), ({"AUDIOSYNC_CUDA_NO_PDL": "1"}, 0)):
+        code = _VARIANT_SNIPPET.format(root=root, pkg=os.path.join(root, "old-audiosync_b200"), L=L, seed=SEED, off=off)
         env = dict(os.environ, **extra)
         p = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
         assert p.returncode == 0, p.stderr[-2000:]
