@@ -107,7 +107,20 @@ int audiosync_cuda_dropin_max_inflight(int reset);
 
 typedef struct audiosync_cuda_ctx audiosync_cuda_ctx;
 
-enum { AUDIOSYNC_CUDA_F32 = 0, AUDIOSYNC_CUDA_F64 = 1 };
+/* Element type of the batch calls' sources / samples.
+ *   F32, F64: float / double samples.
+ *   S16: 16-bit signed PCM, little-endian (ffmpeg's s16le), the value of a sample s being
+ *        s * 2^-15 = s / 32768.0 -- the scaling ffmpeg/libswresample and libsndfile apply when they
+ *        decode s16 to float or double.  Every int16 maps exactly into fp32 and fp64 under it, and
+ *        the library widens on the device, in the first transform pass and in the Pearson step: an
+ *        S16 call returns, bit for bit in every field of each record, what the same call returns
+ *        with dtype F64 on the doubles s / 32768.0 (every path, precise mode included).  A quarter
+ *        of the F64 bytes cross the link (8.64 MB per pair at sample_len 1,440,000, against 17.28
+ *        MB in F32 and 34.56 MB in F64).  Shapes, layouts and memspaces are those of F32 / F64; any
+ *        2-byte-aligned base is accepted.  Accepted by audiosync_cuda_xcorr_batch,
+ *        audiosync_cuda_xcorr_batch_results and audiosync_cuda_xcorr_batch_device only: the session
+ *        pool and audiosync_cuda_synth_pairs refuse it, and host narrowing does not apply to it. */
+enum { AUDIOSYNC_CUDA_F32 = 0, AUDIOSYNC_CUDA_F64 = 1, AUDIOSYNC_CUDA_S16 = 2 };
 enum { AUDIOSYNC_CUDA_HOST = 0, AUDIOSYNC_CUDA_DEVICE = 1 };
 
 /* Which transform path a given sample_len takes.  AUTO: the static four-step kernels for the

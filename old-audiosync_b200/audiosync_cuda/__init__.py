@@ -22,15 +22,17 @@ import numpy as np
 __all__ = [
     "AudiosyncCudaError", "lib", "lib_path", "cross_correlation", "pearson_coefficient",
     "interval_loop", "Context", "RESULT_DTYPE", "MIN_CONFIDENCE", "SAMPLE_RATE",
-    "INTERV_SAMPLE", "frames_to_ms", "F32", "F64", "HOST", "DEVICE",
+    "INTERV_SAMPLE", "frames_to_ms", "F32", "F64", "S16", "HOST", "DEVICE",
     "PATH_AUTO", "PATH_FFT", "PATH_DIRECT", "NARROW_OFF", "NARROW_LOSSLESS", "NARROW_ALWAYS", "EXPORTED_SYMBOLS", "shard_pairs", "gather_results", "host_narrow", "copy_threads",
     "cross_correlation_ptr", "RealBuffer", "set_residency", "dropin_stats", "dropin_max_inflight", "SessionPool",
 ]
 
-F32, F64 = 0, 1
+F32, F64, S16 = 0, 1, 2          # S16: int16 PCM, value s / 32768 (records == F64 on those doubles, bit for bit)
 HOST, DEVICE = 0, 1
 PATH_AUTO, PATH_FFT, PATH_DIRECT = 0, 1, 2
 NARROW_OFF, NARROW_LOSSLESS, NARROW_ALWAYS = 0, 1, 2
+
+_NP_DTYPES = {np.dtype(np.float32): F32, np.dtype(np.float64): F64, np.dtype(np.int16): S16}
 
 MIN_CONFIDENCE = 0.95                                             # audiosync.h:24
 SAMPLE_RATE = 48000                                               # audiosync.h:14
@@ -451,12 +453,12 @@ class Context:
 
     # -- host-facing batch call ------------------------------------------------
     def xcorr_batch(self, sources: np.ndarray, samples: np.ndarray):
-        """sources [n][2L], samples [n][L], float32 or float64 host arrays.
+        """sources [n][2L], samples [n][L], float32, float64 or int16 (16-bit PCM, S16) host arrays.
 
         Returns a dict of numpy arrays: lags (int64), coefs, rets (int32), peaks.
         """
-        if sources.dtype != samples.dtype or sources.dtype not in (np.float32, np.float64):
-            raise TypeError("sources/samples must both be float32 or float64")
+        if sources.dtype != samples.dtype or sources.dtype not in _NP_DTYPES:
+            raise TypeError("sources/samples must both be float32, float64 or int16")
         sources = np.ascontiguousarray(sources)
         samples = np.ascontiguousarray(samples)
         if sources.ndim != 2 or samples.ndim != 2 or sources.shape[0] != samples.shape[0] \
@@ -465,7 +467,7 @@ class Context:
         n, L = samples.shape
         lags = np.zeros(n, np.int64); coefs = np.zeros(n, np.float64)
         rets = np.zeros(n, np.int32); peaks = np.zeros(n, np.float64)
-        dt = F32 if sources.dtype == np.float32 else F64
+        dt = _NP_DTYPES[sources.dtype]
         rc = lib().audiosync_cuda_xcorr_batch(self._h, sources.ctypes.data, samples.ctypes.data, n, L,
                                               dt, HOST, lags.ctypes.data, coefs.ctypes.data,
                                               rets.ctypes.data, peaks.ctypes.data)
@@ -474,7 +476,7 @@ class Context:
 
     def xcorr_batch_ptr(self, sources_ptr: int, samples_ptr: int, n_pairs: int, sample_len: int,
                         dtype: int, memspace: int):
-        """Same call on raw pointers (pinned host buffers or device memory)."""
+        """Same call on raw pointers (pinned host buffers or device memory); dtype F32, F64 or S16."""
         lags = np.zeros(n_pairs, np.int64); coefs = np.zeros(n_pairs, np.float64)
         rets = np.zeros(n_pairs, np.int32); peaks = np.zeros(n_pairs, np.float64)
         rc = lib().audiosync_cuda_xcorr_batch(self._h, sources_ptr, samples_ptr, n_pairs, sample_len,
@@ -485,7 +487,8 @@ class Context:
 
     def xcorr_batch_records(self, sources_ptr: int, samples_ptr: int, n_pairs: int, sample_len: int,
                             dtype: int, memspace: int) -> np.ndarray:
-        """Whole result records (``RESULT_DTYPE``: lag, coef, peak, ret, success, raw_index, second, margin, ncc)."""
+        """Whole result records (``RESULT_DTYPE``: lag, coef, peak, ret, success, raw_index, second, margin, ncc);
+        dtype F32, F64 or S16."""
         res = np.zeros(n_pairs, RESULT_DTYPE)
         rc = lib().audiosync_cuda_xcorr_batch_results(self._h, sources_ptr, samples_ptr, n_pairs, sample_len,
                                                       dtype, memspace, res.ctypes.data)
@@ -495,7 +498,7 @@ class Context:
     def xcorr_batch_torch(self, sources, samples, out=None, sync: bool = True):
         """Zero-copy batch call on torch CUDA tensors (SURVEY 8f rank 3).
 
-        ``sources`` [n, 2L] and ``samples`` [n, L]: contiguous float32 or float64 tensors on one
+        ``sources`` [n, 2L] and ``samples`` [n, L]: contiguous float32, float64 or int16 (S16) tensors on one
         device of this context.  The kernels are enqueued on torch's CURRENT stream of that
         device, reading the tensors in place; the 48-byte records land in ``out`` (a uint8
         CUDA tensor of n * 64 bytes, allocated when omitted).  With ``sync`` the records come
@@ -505,8 +508,9 @@ class Context:
         import torch
         if not (sources.is_cuda and samples.is_cuda) or sources.device != samples.device:
             raise ValueError("sources and samples must be CUDA tensors on the same device")
-        if sources.dtype != samples.dtype or sources.dtype not in (torch.float32, torch.float64):
-            raise TypeError("sources/samples must both be float32 or float64")
+        dts = {torch.float32: F32, torch.float64: F64, torch.int16: S16}
+        if sources.dtype != samples.dtype or sources.dtype not in dts:
+            raise TypeError("sources/samples must both be float32, float64 or int16")
         if sources.dim() != 2 or samples.dim() != 2 or sources.shape[0] != samples.shape[0] \
                 or sources.shape[1] != 2 * samples.shape[1]:
             raise ValueError("expected sources [n, 2L] and samples [n, L]")
@@ -523,7 +527,7 @@ class Context:
             # a NULL handle would select the library's own stream: order it after torch's default
             # stream by draining that one first, and synchronise the device afterwards
             torch.cuda.current_stream(dev).synchronize()
-        dt = F32 if sources.dtype == torch.float32 else F64
+        dt = dts[sources.dtype]
         if n:
             self.xcorr_batch_device(dev.index, sources.data_ptr(), samples.data_ptr(), n, L, dt,
                                     out.data_ptr(), stream)
@@ -536,12 +540,14 @@ class Context:
     # -- stream-ordered device calls --------------------------------------------
     def xcorr_batch_device(self, device: int, d_sources: int, d_samples: int, n_pairs: int,
                            sample_len: int, dtype: int, d_results: int, stream: int = 0):
+        """Stream-ordered call on device pointers; dtype F32, F64 or S16."""
         rc = lib().audiosync_cuda_xcorr_batch_device(self._h, device, d_sources, d_samples, n_pairs,
                                                      sample_len, dtype, d_results, stream or None)
         self._check(rc, "xcorr_batch_device")
 
     def synth_pairs(self, device: int, seed: int, first_pair: int, n_pairs: int, sample_len: int,
                     dtype: int, d_sources: int, d_samples: int, stream: int = 0):
+        """Seeded synthetic pairs in device memory; dtype F32 or F64 (S16 is refused)."""
         rc = lib().audiosync_cuda_synth_pairs(self._h, device, seed, first_pair, n_pairs, sample_len,
                                               dtype, d_sources, d_samples, stream or None)
         self._check(rc, "synth_pairs")

@@ -88,9 +88,12 @@ static int run_small_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d
                           const void* smp, long long sp, long long mp, PairPeak* peaks, int pairs,
                           cudaStream_t st) {
     using K = SmallXcorrKernel<InT>;
+    // int16: one 4-byte load per packed point where every pair's base is 4-byte aligned
+    const int vec_src = reinterpret_cast<uintptr_t>(src) % 4 == 0 && sp % 2 == 0;
+    const int vec_smp = reinterpret_cast<uintptr_t>(smp) % 4 == 0 && mp % 2 == 0;
     typename K::Params p{static_cast<const InT*>(src), static_cast<const InT*>(smp), peaks,
                          static_cast<const cplx*>(plan->wm.p), static_cast<const cplx*>(plan->wn.p),
-                         plan->small, sp, mp};
+                         plan->small, sp, mp, vec_src, vec_smp};
     const size_t smem = K::smem_bytes(plan->small.M);
     const dim3 grid(1, 1, pairs);
     return launch(ctx, d, KC_SMALL_FFT, st, [&] {
@@ -116,12 +119,19 @@ static int build_small_plan(FftPlan* plan, long long L) {
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
         ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<SmallXcorrKernel<double>>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
+        ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<SmallXcorrKernel<int16_t>>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
     }
     plan->run_wave = [plan](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
                             int dtype, long long sp, long long mp, void*, PairPeak* peaks, int pairs,
                             cudaStream_t st) {
-        return dtype == AUDIOSYNC_CUDA_F32 ? run_small_wave<float>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st)
-                                           : run_small_wave<double>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
+        switch (dtype) {
+            case AUDIOSYNC_CUDA_F32: return run_small_wave<float>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
+            case AUDIOSYNC_CUDA_F64: return run_small_wave<double>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
+            case AUDIOSYNC_CUDA_S16: return run_small_wave<int16_t>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
+        }
+        set_last_error("bad dtype %d", dtype);
+        return -1;
     };
     return 0;
 }
@@ -194,8 +204,13 @@ static int build_direct_plan(FftPlan* plan, long long L) {
     plan->run_wave = [L](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
                          int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,
                          cudaStream_t st) {
-        return dtype == AUDIOSYNC_CUDA_F32 ? run_direct_wave<float>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st)
-                                           : run_direct_wave<double>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st);
+        switch (dtype) {
+            case AUDIOSYNC_CUDA_F32: return run_direct_wave<float>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st);
+            case AUDIOSYNC_CUDA_F64: return run_direct_wave<double>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st);
+            case AUDIOSYNC_CUDA_S16: return run_direct_wave<int16_t>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st);
+        }
+        set_last_error("bad dtype %d", dtype);
+        return -1;
     };
     return 0;
 }
@@ -279,8 +294,9 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
     ASC_CUDA_OK(cudaSetDevice(d.device));
     FftPlan* plan = get_plan(ctx, d, L);
     if (!plan) return -1;
-    const size_t esz = dtype == AUDIOSYNC_CUDA_F64 ? 8 : 4;
-    const int in_dtype = dtype == AUDIOSYNC_CUDA_F64 ? AUDIOSYNC_CUDA_F64 : AUDIOSYNC_CUDA_F32;   // what the transform loads
+    const size_t esz = dtype_bytes(dtype);
+    if (esz == 0) { set_last_error("bad dtype %d", dtype); return -1; }
+    const int in_dtype = dtype == ASC_DTYPE_F32_EXACT ? AUDIOSYNC_CUDA_F32 : dtype;   // what the transform loads
     int wave = ctx->wave_pairs > 0 ? ctx->wave_pairs : default_wave_pairs(plan, n_pairs);
     wave = (int)std::min<size_t>((size_t)wave, n_pairs);
     wave = std::min(wave, 65535);
@@ -315,10 +331,16 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
                     reinterpret_cast<const float*>(s), reinterpret_cast<const float*>(m), src_pitch, smp_pitch, L,
                     (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
             });
-        } else {
+        } else if (dtype == AUDIOSYNC_CUDA_F64) {
             rc = launch(ctx, d, KC_PEARSON, st, [&] {
                 launch_stage(pearson_kernel<double, true>, grid, dim3(PEARSON_THREADS), 0, st,
                     reinterpret_cast<const double*>(s), reinterpret_cast<const double*>(m), src_pitch, smp_pitch, L,
+                    (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
+            });
+        } else {   // S16 (esz above admits nothing else): the f64 path's arithmetic on s * 2^-15
+            rc = launch(ctx, d, KC_PEARSON, st, [&] {
+                launch_stage(pearson_kernel<int16_t, true>, grid, dim3(PEARSON_THREADS), 0, st,
+                    reinterpret_cast<const int16_t*>(s), reinterpret_cast<const int16_t*>(m), src_pitch, smp_pitch, L,
                     (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
             });
         }
@@ -612,7 +634,7 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
     if (p1 <= p0) return 0;
     std::lock_guard<std::mutex> dlk(d.mu);
     ASC_CUDA_OK(cudaSetDevice(d.device));
-    const size_t esz = dtype == AUDIOSYNC_CUDA_F32 ? 4 : 8;
+    const size_t esz = dtype_bytes(dtype);
     const size_t src_n = (size_t)(2 * L), smp_n = (size_t)L;
     const size_t src_bytes = src_n * esz, smp_bytes = smp_n * esz;
     const bool pageable = host_pointer_is_pageable(sources) || host_pointer_is_pageable(samples);
@@ -1006,6 +1028,7 @@ int audiosync_cuda_synth_pairs(audiosync_cuda_ctx* ctx, int device, uint64_t see
                                size_t n_pairs, size_t sample_len, int dtype, void* d_sources,
                                void* d_samples, void* stream) {
     if (!ctx || !d_sources || !d_samples) return -1;
+    if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64) { set_last_error("bad dtype"); return -1; }   // F32 / F64 only
     DeviceState* d = ctx->find(device);
     if (!d) { set_last_error("device %d is not part of this context", device); return -1; }
     if (n_pairs == 0) return 0;
@@ -1013,20 +1036,20 @@ int audiosync_cuda_synth_pairs(audiosync_cuda_ctx* ctx, int device, uint64_t see
     ASC_CUDA_OK(cudaSetDevice(d->device));
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
     const long long L = (long long)sample_len;
-    const size_t esz = dtype == AUDIOSYNC_CUDA_F32 ? 4 : 8;
+    const size_t esz = dtype_bytes(dtype);
     const unsigned bx = (unsigned)std::min<long long>((3 * L + 255) / 256, 4096);
     for (size_t p0 = 0; p0 < n_pairs; p0 += 32768) {
         const unsigned np = (unsigned)std::min<size_t>(32768, n_pairs - p0);
         const dim3 grid(bx, np);
         char* s = static_cast<char*>(d_sources) + p0 * (size_t)(2 * L) * esz;
         char* m = static_cast<char*>(d_samples) + p0 * (size_t)L * esz;
-        int rc;
+        int rc = -1;
         if (dtype == AUDIOSYNC_CUDA_F32)
             rc = launch(ctx, *d, KC_SYNTH, st, [&] {
                 synth_kernel<float><<<grid, 256, 0, st>>>(reinterpret_cast<float*>(s),
                                                           reinterpret_cast<float*>(m), seed, first_pair + p0, L);
             });
-        else
+        else if (dtype == AUDIOSYNC_CUDA_F64)
             rc = launch(ctx, *d, KC_SYNTH, st, [&] {
                 synth_kernel<double><<<grid, 256, 0, st>>>(reinterpret_cast<double*>(s),
                                                            reinterpret_cast<double*>(m), seed, first_pair + p0, L);
@@ -1040,7 +1063,7 @@ int audiosync_cuda_xcorr_batch_device(audiosync_cuda_ctx* ctx, int device, const
                                       const void* d_samples, size_t n_pairs, size_t sample_len,
                                       int dtype, audiosync_cuda_result* d_results, void* stream) {
     if (!ctx || !d_sources || !d_samples || !d_results) { set_last_error("null argument"); return -1; }
-    if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64) { set_last_error("bad dtype"); return -1; }
+    if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64 && dtype != AUDIOSYNC_CUDA_S16) { set_last_error("bad dtype"); return -1; }
     DeviceState* d = ctx->find(device);
     if (!d) { set_last_error("device %d is not part of this context", device); return -1; }
     std::lock_guard<std::mutex> lk(d->mu);      // per device: threads driving different devices do not serialise
@@ -1052,7 +1075,7 @@ int audiosync_cuda_xcorr_batch_results(audiosync_cuda_ctx* ctx, const void* sour
                                        size_t n_pairs, size_t sample_len, int dtype, int memspace,
                                        audiosync_cuda_result* results) {
     if (!ctx || !sources || !samples || (!results && n_pairs)) { set_last_error("null argument"); return -1; }
-    if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64) { set_last_error("bad dtype"); return -1; }
+    if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64 && dtype != AUDIOSYNC_CUDA_S16) { set_last_error("bad dtype"); return -1; }
     if (n_pairs == 0) return 0;
     if (sample_len == 0) { set_last_error("sample_len must be > 0"); return -1; }
     std::lock_guard<std::mutex> lk(ctx->mu);
@@ -1204,7 +1227,7 @@ int audiosync_cuda_pool_create(audiosync_cuda_ctx* ctx, int device, size_t n_slo
     pool->ctx = ctx; pool->dev = d; pool->n_slots = n_slots; pool->max_len = max_sample_len; pool->dtype = dtype;
     pool->smp_pitch = (long long)((max_sample_len + 3) / 4 * 4);
     pool->src_pitch = 2 * pool->smp_pitch;
-    const size_t esz = dtype == AUDIOSYNC_CUDA_F32 ? 4 : 8;
+    const size_t esz = dtype_bytes(dtype);
     if (pool->src.ensure(esz * (size_t)pool->src_pitch * n_slots) != 0 ||
         pool->smp.ensure(esz * (size_t)pool->smp_pitch * n_slots) != 0) {
         audiosync_cuda_pool_destroy(pool);
@@ -1316,7 +1339,7 @@ int audiosync_cuda_pool_run(audiosync_cuda_pool* pool, size_t first_slot, size_t
     if (d.results.ensure(sizeof(audiosync_cuda_result) * n_slots) != 0 ||
         d.h_results.ensure(sizeof(audiosync_cuda_result) * n_slots) != 0)
         return -1;
-    const size_t esz = pool->dtype == AUDIOSYNC_CUDA_F32 ? 4 : 8;
+    const size_t esz = dtype_bytes(pool->dtype);
     const char* s0 = static_cast<const char*>(pool->src.p) + first_slot * (size_t)pool->src_pitch * esz;
     const char* m0 = static_cast<const char*>(pool->smp.p) + first_slot * (size_t)pool->smp_pitch * esz;
     auto* d_res = static_cast<audiosync_cuda_result*>(d.results.p);

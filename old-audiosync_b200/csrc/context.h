@@ -60,15 +60,25 @@ struct PinnedBuf {
     void release();
 };
 
+// Internal input type of enqueue_batch beside the public F32 / F64 / S16: fp32 values that are the
+// EXACT images of the caller's doubles (lossless host narrowing).  The transform reads them as any
+// fp32 batch; the Pearson step widens them and runs the f64 path's arithmetic, so the result record
+// is the f64 call's bit for bit.
+constexpr int ASC_DTYPE_F32_EXACT = 100;
+
+// Bytes of one input element of `dtype`; 0 for a value that is not an input type.
+inline size_t dtype_bytes(int dtype) {
+    switch (dtype) {
+        case AUDIOSYNC_CUDA_F32: case ASC_DTYPE_F32_EXACT: return 4;
+        case AUDIOSYNC_CUDA_F64: return 8;
+        case AUDIOSYNC_CUDA_S16: return 2;
+    }
+    return 0;
+}
+
 // Pinned bounce buffers for PAGEABLE host inputs: the host memcpy of piece k + 1 overlaps the
 // DMA of piece k and the stream stays asynchronous (a cudaMemcpyAsync straight from pageable
 // memory is staged by the driver and blocks the calling thread for the whole transfer).
-// Internal input type of enqueue_batch beside the public F32 / F64: fp32 values that are the EXACT
-// images of the caller's doubles (lossless host narrowing).  The transform reads them as any fp32
-// batch; the Pearson step widens them and runs the f64 path's arithmetic, so the result record is
-// the f64 call's bit for bit.
-constexpr int ASC_DTYPE_F32_EXACT = 100;
-
 struct StageRing {
     static constexpr int N = 6;
     static constexpr size_t PIECE = (size_t)8 << 20;

@@ -198,6 +198,20 @@ ASC_HD T ldg(const T* p) {
 #endif
 }
 
+// One input element as a real of the arithmetic type R: fp32 / fp64 inputs as they are (rounded to
+// R), 16-bit PCM as s * 2^-15 -- the scaling decoders apply (ffmpeg, libsndfile), exact in fp32 and
+// fp64, so an int16 input computes what the f64 call on the doubles s / 32768 computes.
+template <typename R, typename InT>
+ASC_HD R in_real(InT v) {
+    if constexpr (std::is_same<InT, int16_t>::value) return (R)v * (R)0x1p-15;
+    else return (R)v;
+}
+// Two consecutive input elements as one vector load (the address is aligned to two elements).
+template <typename InT> struct in_pair;
+template <> struct in_pair<float> { typedef float2 type; };
+template <> struct in_pair<double> { typedef double2 type; };
+template <> struct in_pair<int16_t> { typedef short2 type; };
+
 // ------------------------------------------------------- asynchronous staging
 // Global -> shared copies that bypass the register file (LDGSTS / cp.async,
 // 16 bytes per thread, L1 bypass) and the shared -> global bulk store of the

@@ -112,24 +112,19 @@ ASC_HD C gen_load_point(const InT* __restrict__ x, unsigned n, int sig, long lon
     typedef typename scalar_of<C>::type real;
     if (n < fast_pts) {
         if (vec) {
-            if constexpr (sizeof(InT) == 4) {
-                const float2 d = ldg(reinterpret_cast<const float2*>(x) + n);
-                return cmake((real)d.x, (real)d.y);
-            } else {
-                const double2 d = ldg(reinterpret_cast<const double2*>(x) + n);
-                return cmake((real)d.x, (real)d.y);
-            }
+            const typename in_pair<InT>::type d = ldg(reinterpret_cast<const typename in_pair<InT>::type*>(x) + n);
+            return cmake(in_real<real>(d.x), in_real<real>(d.y));
         }
-        return cmake((real)ldg(x + 2 * (size_t)n), (real)ldg(x + 2 * (size_t)n + 1));
+        return cmake(in_real<real>(ldg(x + 2 * (size_t)n)), in_real<real>(ldg(x + 2 * (size_t)n + 1)));
     }
     const long long i0 = 2 * (long long)n, i1 = i0 + 1;
     real a = (real)0, b = (real)0;
     if (sig == 0) {
-        if (i0 < src_ext) a = (real)ldg(x + (i0 < 2 * L ? i0 : i0 - 2 * L));
-        if (i1 < src_ext) b = (real)ldg(x + (i1 < 2 * L ? i1 : i1 - 2 * L));
+        if (i0 < src_ext) a = in_real<real>(ldg(x + (i0 < 2 * L ? i0 : i0 - 2 * L)));
+        if (i1 < src_ext) b = in_real<real>(ldg(x + (i1 < 2 * L ? i1 : i1 - 2 * L)));
     } else {
-        if (i0 < L) a = (real)ldg(x + i0);
-        if (i1 < L) b = (real)ldg(x + i1);
+        if (i0 < L) a = in_real<real>(ldg(x + i0));
+        if (i1 < L) b = in_real<real>(ldg(x + i1));
     }
     return cmake(a, b);
 }
@@ -227,19 +222,12 @@ struct GenColFwdKernel {
                             typedef typename scalar_of<C>::type real;
                             const unsigned nfirst = (unsigned)i0 * (unsigned)M2 + n2, dn = (unsigned)S * (unsigned)M2;
                             if (vec && nfirst + (unsigned)(R - 1) * dn < fast_pts) {
-                                if constexpr (sizeof(InT) == 4) {
-                                    const float2* __restrict__ px = reinterpret_cast<const float2*>(x) + nfirst;
-                                    static_for<0, R>([&](auto Q) {
-                                        const float2 d2 = ldg(px + (size_t)decltype(Q)::value * dn);
-                                        v[decltype(Q)::value] = cmake((real)d2.x, (real)d2.y);
-                                    });
-                                } else {
-                                    const double2* __restrict__ px = reinterpret_cast<const double2*>(x) + nfirst;
-                                    static_for<0, R>([&](auto Q) {
-                                        const double2 d2 = ldg(px + (size_t)decltype(Q)::value * dn);
-                                        v[decltype(Q)::value] = cmake((real)d2.x, (real)d2.y);
-                                    });
-                                }
+                                typedef typename in_pair<InT>::type V;
+                                const V* __restrict__ px = reinterpret_cast<const V*>(x) + nfirst;
+                                static_for<0, R>([&](auto Q) {
+                                    const V d2 = ldg(px + (size_t)decltype(Q)::value * dn);
+                                    v[decltype(Q)::value] = cmake(in_real<real>(d2.x), in_real<real>(d2.y));
+                                });
                             } else {
                                 static_for<0, R>([&](auto Q) {
                                     constexpr int q = decltype(Q)::value;

@@ -24,7 +24,7 @@
 // and the load of one CTA overlaps the butterflies of the other CTAs on the SM;
 // K_B's product rows leave the same way (cp.async.bulk shared -> global).  Only
 // K_A has a second path: its first pass loads through registers where the input
-// cannot be staged (fp64, or fp32 not 16-byte aligned).  The last pass is fused
+// cannot be staged (fp64, int16, or fp32 not 16-byte aligned).  The last pass is fused
 // with the global store / epilogue.
 //
 // Kernel bodies are written against an executor (DeviceExec on the GPU,
@@ -67,17 +67,28 @@ constexpr int tile_box_start(int rows, int i) {
     return i * tile_box_rows(rows) + tile_box_rows(rows) <= rows ? i * tile_box_rows(rows) : rows - tile_box_rows(rows);
 }
 
+// Packed point n = (x[2n], x[2n + 1]).  vec: one 4-byte load per int16 point (the base is 4-byte
+// aligned); otherwise two 2-byte loads.  The fp32 / fp64 loads need their natural pair alignment,
+// which every caller's base has, and ignore it.
 template <typename InT>
-ASC_HD cplx load_packed(const InT* __restrict__ x, long long n);
+ASC_HD cplx load_packed(const InT* __restrict__ x, long long n, bool vec = true);
 
 template <>
-ASC_HD cplx load_packed<float>(const float* __restrict__ x, long long n) {
+ASC_HD cplx load_packed<float>(const float* __restrict__ x, long long n, bool) {
     return ldg(reinterpret_cast<const float2*>(x) + n);
 }
 template <>
-ASC_HD cplx load_packed<double>(const double* __restrict__ x, long long n) {
+ASC_HD cplx load_packed<double>(const double* __restrict__ x, long long n, bool) {
     double2 d = ldg(reinterpret_cast<const double2*>(x) + n);
-    return cmake((float)d.x, (float)d.y);
+    return cmake(in_real<float>(d.x), in_real<float>(d.y));
+}
+template <>
+ASC_HD cplx load_packed<int16_t>(const int16_t* __restrict__ x, long long n, bool vec) {
+    if (vec) {
+        const short2 s = ldg(reinterpret_cast<const short2*>(x) + n);
+        return cmake(in_real<float>(s.x), in_real<float>(s.y));
+    }
+    return cmake(in_real<float>(ldg(x + 2 * n)), in_real<float>(ldg(x + 2 * n + 1)));
 }
 
 // Running |r| argmax of one thread (reference src/cross_correlation.c:52-67 as
@@ -139,8 +150,8 @@ ASC_HD void argmax_merge(unsigned long long& best, float& second, unsigned long 
 // --------------------------------------------------------------------- K_A
 // TMA (fp32 input, 16-byte aligned): the tile is staged in shared memory before pass 0 as boxes
 // of a tensor map through the TMA unit, completion on an mbarrier, and the zero half of the
-// padded sample is never touched; otherwise (fp64 input or unaligned pointers) the first pass
-// loads, converts and packs through registers.
+// padded sample is never touched; otherwise (fp64 or int16 input, or unaligned fp32 pointers) the
+// first pass loads, converts and packs through registers.
 //
 // TMA staging of the SOURCE tile: the CTA's shared memory is exactly the tile, so the 8-byte
 // mbarrier sits at its very end and the last tile row (128 bytes) is not staged; pass 0 reads
@@ -156,7 +167,7 @@ struct ColFwdKernel {
     static constexpr int MIN_CTAS = ctas_per_sm(SMEM, NT);
     static_assert(NT % COL_T == 0, "a thread must keep its column across items");
     static_assert(P >= 2, "column plans need at least two passes");
-    static_assert(!TMA || sizeof(InT) == 4, "TMA staging copies packed fp32 pairs verbatim");
+    static_assert(!TMA || std::is_same<InT, float>::value, "TMA staging copies packed fp32 pairs verbatim");
     static_assert(!TMA || M1 >= 4, "tile too small for a box");
     static_assert(M1 % 2 == 0, "the zero half of the sample must be whole tile rows");
 
@@ -172,6 +183,9 @@ struct ColFwdKernel {
         long long L;             // sample_len == M = M1 * M2
         long long src_pitch;     // elements between consecutive pairs' sources / samples;
         long long smp_pitch;     // 0 = packed ([pair][2L] and [pair][L])
+        // int16 input: every pair's sources / samples start 4-byte aligned (one load per packed
+        // point); CTA-uniform.  These sit in the padding before the tensor maps.
+        int vec_src, vec_smp;
         // TMA: [pair][M1 or M1/2 rows][2*M2 floats] views of sources / samples, boxes of
         // 32 floats x tile_box_rows(M1 - 1) resp. tile_box_rows(M1 / 2) rows
         CUtensorMap tm_src, tm_smp;
@@ -189,6 +203,7 @@ struct ColFwdKernel {
                                              : p.samples + pair * (p.smp_pitch ? p.smp_pitch : M);
         // number of valid packed points: source M, sample M/2 (upper half is the zero pad)
         const long long nvalid = sig == 0 ? M : M / 2;
+        [[maybe_unused]] const bool vec = sig == 0 ? p.vec_src != 0 : p.vec_smp != 0;
         cplx* __restrict__ out = p.planes + (pair * 2 + sig) * M;
         const bool clears_peak = ex.bx() == 0 && sig == 0;
 
@@ -250,7 +265,7 @@ struct ColFwdKernel {
                                 static_for<0, R>([&](auto Q) {
                                     constexpr int q = decltype(Q)::value;
                                     const long long n = (long long)(i0 + q * S) * M2 + c0 + c;
-                                    v[q] = n < nvalid ? load_packed<InT>(x, n) : cmake(0.f, 0.f);
+                                    v[q] = n < nvalid ? load_packed<InT>(x, n, vec) : cmake(0.f, 0.f);
                                 });
                             } else {
                                 static_for<0, R>([&](auto Q) {

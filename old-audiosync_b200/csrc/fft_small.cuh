@@ -48,6 +48,7 @@ struct SmallXcorrKernel {
         SmallPlan plan;
         long long src_pitch;  // elements between consecutive pairs; 0 = packed (2M / M)
         long long smp_pitch;
+        int vec_src, vec_smp; // int16 input: one 4-byte load per packed point (every pair's base is 4-byte aligned)
     };
     // two rows of M points + 512 bytes of reduction scratch (phase_argmax needs 392)
     static size_t smem_bytes(int M) { return (size_t)2 * M * sizeof(cplx) + 512; }
@@ -76,8 +77,8 @@ struct SmallXcorrKernel {
                     static_for<0, R>([&](auto Q) {
                         constexpr int q = decltype(Q)::value;
                         const long long n = i0 + q * S;
-                        if (rr == 0) v[q] = load_packed<InT>(p.sources + pair * (p.src_pitch ? p.src_pitch : 2 * M), n);
-                        else v[q] = n < M / 2 ? load_packed<InT>(p.samples + pair * (p.smp_pitch ? p.smp_pitch : M), n)
+                        if (rr == 0) v[q] = load_packed<InT>(p.sources + pair * (p.src_pitch ? p.src_pitch : 2 * M), n, p.vec_src != 0);
+                        else v[q] = n < M / 2 ? load_packed<InT>(p.samples + pair * (p.smp_pitch ? p.smp_pitch : M), n, p.vec_smp != 0)
                                               : cmake(0.f, 0.f);
                     });
                 } else {

@@ -37,6 +37,7 @@ int GenStage<T, NT>::prepare_cols(const GenShape& sh) {
         constexpr int CT = decltype(CTC)::value;
         return prepare_gen_kernel<GenColFwdKernel<T, float, CT, NT>>(GenColFwdKernel<T, float, CT, NT>::smem_bytes(sh)) != 0 ||
                prepare_gen_kernel<GenColFwdKernel<T, double, CT, NT>>(GenColFwdKernel<T, double, CT, NT>::smem_bytes(sh)) != 0 ||
+               prepare_gen_kernel<GenColFwdKernel<T, int16_t, CT, NT>>(GenColFwdKernel<T, int16_t, CT, NT>::smem_bytes(sh)) != 0 ||
                prepare_gen_kernel<GenColInvKernel<T, CT, NT>>(GenColInvKernel<T, CT, NT>::smem_bytes(sh)) != 0 ? -1 : 0;
     });
 }
@@ -69,7 +70,13 @@ int GenStage<T, NT>::col_fwd(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState
             });
         });
     };
-    return dtype == AUDIOSYNC_CUDA_F32 ? go(float{}) : go(double{});
+    switch (dtype) {
+        case AUDIOSYNC_CUDA_F32: return go(float{});
+        case AUDIOSYNC_CUDA_F64: return go(double{});
+        case AUDIOSYNC_CUDA_S16: return go(int16_t{});
+    }
+    set_last_error("bad dtype %d", dtype);
+    return -1;
 }
 
 template <typename T, int NT>

@@ -3,6 +3,7 @@
 #pragma once
 
 #include "common.cuh"
+#include "fft_device.cuh"   // in_real: the input element as a real
 
 namespace asc {
 
@@ -71,9 +72,9 @@ direct_corr_kernel(const T* __restrict__ sources, const T* __restrict__ samples,
     const int t = threadIdx.x;
     double acc = 0.0;
     for (long long n0 = 0; n0 < L; n0 += DIRECT_TILE) {
-        s_smp[t] = (n0 + t < L) ? (double)smp[n0 + t] : 0.0;
-        s_src[t] = (double)src[(j0 + n0 + t) % N];
-        s_src[t + DIRECT_TILE] = (double)src[(j0 + n0 + t + DIRECT_TILE) % N];
+        s_smp[t] = (n0 + t < L) ? in_real<double>(smp[n0 + t]) : 0.0;
+        s_src[t] = in_real<double>(src[(j0 + n0 + t) % N]);
+        s_src[t + DIRECT_TILE] = in_real<double>(src[(j0 + n0 + t + DIRECT_TILE) % N]);
         __syncthreads();
 #pragma unroll 8
         for (int i = 0; i < DIRECT_TILE; i++) acc = fma(s_smp[i], s_src[t + i], acc);
@@ -215,10 +216,12 @@ __device__ __forceinline__ void pearson_finish(const PearsonPartial& s, const Wi
 // CTA of a pair to finish (ticket counter, self-resetting) sums the chunk partials in a fixed
 // order and writes the result record, so the whole Pearson step needs no second launch.
 // Every thread of the CTA must call it (barriers inside).
-// WIDE: fp64 arithmetic on the widened inputs whatever T is.  T = float with WIDE is the path of
-// host-narrowed batches whose floats are the exact images of the caller's doubles: element for
-// element the same operations as T = double, so the record is the f64 call's bit for bit.
-template <typename T, int NTP, bool WIDE = (sizeof(T) == 8)>
+// WIDE: fp64 arithmetic on the widened inputs (in_real) whatever T is.  T = float with WIDE is the
+// path of host-narrowed batches whose floats are the exact images of the caller's doubles, T =
+// int16_t that of 16-bit PCM (s * 2^-15, exact): element for element the same operations as
+// T = double, so the record is the f64 call's on those doubles bit for bit.  Only fp32 inputs have
+// the fp32 path.
+template <typename T, int NTP, bool WIDE = !std::is_same<T, float>::value>
 __device__ __forceinline__ void pearson_block(
     const T* __restrict__ sources, const T* __restrict__ samples,
     long long src_pitch, long long smp_pitch, long long L,
@@ -250,7 +253,7 @@ __device__ __forceinline__ void pearson_block(
     if (lo < w.n) {
         if (t < 32) {
             long long k = ((long long)t * w.n) >> 5;
-            double px = (double)x[k], py = (double)y[k];
+            double px = in_real<double>(x[k]), py = in_real<double>(y[k]);
             for (int o = 16; o > 0; o >>= 1) {
                 px += __shfl_xor_sync(0xffffffffu, px, o);
                 py += __shfl_xor_sync(0xffffffffu, py, o);
@@ -312,13 +315,13 @@ __device__ __forceinline__ void pearson_block(
                 for (int u = 0; u < UN; u++) { xv[u] = x[i + u * NTP]; yv[u] = y[i + u * NTP]; }
 #pragma unroll
                 for (int u = 0; u < UN; u++) {
-                    const double dx = (double)xv[u] - px, dy = (double)yv[u] - py;
+                    const double dx = in_real<double>(xv[u]) - px, dy = in_real<double>(yv[u]) - py;
                     acc.sx += dx; acc.sy += dy;
                     acc.sxx = fma(dx, dx, acc.sxx); acc.syy = fma(dy, dy, acc.syy); acc.sxy = fma(dx, dy, acc.sxy);
                 }
             }
             for (; i < hi; i += NTP) {
-                const double dx = (double)x[i] - px, dy = (double)y[i] - py;
+                const double dx = in_real<double>(x[i]) - px, dy = in_real<double>(y[i]) - py;
                 acc.sx += dx; acc.sy += dy;
                 acc.sxx = fma(dx, dx, acc.sxx); acc.syy = fma(dy, dy, acc.syy); acc.sxy = fma(dx, dy, acc.sxy);
             }
@@ -371,7 +374,7 @@ __device__ __forceinline__ void pearson_block(
         double px = 0.0, py = 0.0;
         if (w.n > 0) {
             const long long k = ((long long)t * w.n) >> 5;
-            px = (double)x[k]; py = (double)y[k];
+            px = in_real<double>(x[k]); py = in_real<double>(y[k]);
             for (int o = 16; o > 0; o >>= 1) {
                 px += __shfl_xor_sync(0xffffffffu, px, o);
                 py += __shfl_xor_sync(0xffffffffu, py, o);
@@ -387,7 +390,7 @@ __device__ __forceinline__ void pearson_block(
 }
 
 // grid = (n_chunks, n_pairs), block = 256.
-template <typename T, bool WIDE = (sizeof(T) == 8)>
+template <typename T, bool WIDE = !std::is_same<T, float>::value>
 __global__ void __launch_bounds__(PEARSON_THREADS)
 pearson_kernel(const T* __restrict__ sources, const T* __restrict__ samples,
                long long src_pitch, long long smp_pitch, long long L,

@@ -56,10 +56,21 @@ static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& 
         if ((tma ? col_fwd(KT{}, pt)
                  : col_fwd(KR{}, {s_in, m_in, planes, peaks, col_tw, col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch})) != 0)
             return -1;
-    } else {
+    } else if (dtype == AUDIOSYNC_CUDA_F64) {
         using K = ColFwdKernel<Col, Row::n, P::NT_COL, double, false>;
         if (col_fwd(K{}, {static_cast<const double*>(src), static_cast<const double*>(smp), planes, peaks, col_tw,
                           col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch}) != 0) return -1;
+    } else if (dtype == AUDIOSYNC_CUDA_S16) {
+        // one 4-byte load per packed point where every pair's base is 4-byte aligned (a view at an
+        // odd element offset, e.g. x[1:], is not: two 2-byte loads then)
+        const int vec_src = reinterpret_cast<uintptr_t>(src) % 4 == 0 && src_pitch % 2 == 0;
+        const int vec_smp = reinterpret_cast<uintptr_t>(smp) % 4 == 0 && smp_pitch % 2 == 0;
+        using K = ColFwdKernel<Col, Row::n, P::NT_COL, int16_t, false>;
+        if (col_fwd(K{}, {static_cast<const int16_t*>(src), static_cast<const int16_t*>(smp), planes, peaks, col_tw,
+                          col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch, vec_src, vec_smp}) != 0) return -1;
+    } else {
+        set_last_error("bad dtype %d", dtype);
+        return -1;
     }
     {
         using K = RowFusedKernel<Row, Col::n, P::NT_ROW>;
@@ -107,9 +118,11 @@ int build_static_plan(FftPlan* plan) {
     using KT = ColFwdKernel<Col, Row::n, P::NT_COL, float, true>;
     using KR = ColFwdKernel<Col, Row::n, P::NT_COL, float, false>;
     using KD = ColFwdKernel<Col, Row::n, P::NT_COL, double, false>;
+    using KS = ColFwdKernel<Col, Row::n, P::NT_COL, int16_t, false>;
     using KB = RowFusedKernel<Row, Col::n, P::NT_ROW>;
     using KC = ColInvKernel<Col, Row::n, P::NT_COL>;
     if (prepare_kernel<KT>(KT::SMEM) != 0 || prepare_kernel<KR>(KR::SMEM) != 0 || prepare_kernel<KD>(KD::SMEM) != 0 ||
+        prepare_kernel<KS>(KS::SMEM) != 0 ||
         prepare_kernel<KB>(KB::SMEM) != 0 || prepare_kernel<KC>(KC::SMEM) != 0)
         return -1;
     plan->run_wave = [plan](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
