@@ -151,6 +151,7 @@ typedef struct audiosync_cuda_result {
     double  margin;     /* (|peak| - second) / |peak| (0 when peak == 0): the peak is      */
                         /* unique when this is well above the arithmetic's 1e-6            */
     double  ncc;        /* normalised correlation at the peak: peak / (N * sqrt(Sx2*Sy2)), */
+                        /* (PHAT weighting: peak / N, see audiosync_cuda_set_weighting)     */
                         /* N = 2*sample_len, Sx2 / Sy2 = sum of squares of the two aligned */
                         /* windows the coefficient is taken over (cross_correlation.c      */
                         /* :256-271); for lag >= 0 the cosine similarity of the windows.   */
@@ -283,9 +284,33 @@ int  audiosync_cuda_copy_threads(void);
  * than the fp32 product path, peak values within 1e-12 of an fp64 FFT.  A second oracle for the
  * fp32 kernels; env AUDIOSYNC_CUDA_PRECISE=1 selects it for the drop-in cross_correlation(). */
 int  audiosync_cuda_set_precise(audiosync_cuda_ctx *ctx, int on);
+/* Cross-spectrum weighting of the batch calls, per context (default NONE: the reference's plain
+ * correlation).  PHAT is the generalised cross-correlation with phase transform (GCC-PHAT), the
+ * standard delay estimator for reverberant or spectrally coloured recordings: with N = 2L,
+ * X = DFT_N(source[0, 2L)) and Y = DFT_N(zero-padded sample),
+ *     W[k]   = X[k] conj(Y[k]) / (|X[k]| |Y[k]|)    (0 where |X[k]|^2 or |Y[k]|^2 is 0 in the arithmetic type)
+ *     r_w[j] = sum_k W[k] e^(2 pi i j k / N)        (unnormalised like FFTW's c2r, so |r_w| <= N)
+ * and the record is derived from r_w: raw_index by the reference's argmax rule (signed r_w[0] seed,
+ * strict >, first index wins), lag by the same fold, peak / second / margin over r_w, and coef, ret,
+ * success the Pearson coefficient of the aligned windows of the original inputs at that lag.  ncc
+ * becomes peak / N, the phase coherence at the peak: in [-1, 1], 1 for a pure circular shift, 0
+ * when the peak is 0.  The peak is a near-delta whatever the spectral colour or level of either
+ * signal; scaling an input by a power of two leaves every record field unchanged.
+ * PHAT is defined on the N = 2L spectrum and is served wherever the plan transforms at N = 2L: the
+ * six static lengths, the single-CTA kernel (short even 2/3/5-smooth lengths; under AUTO also
+ * below 4,096 frames, PHAT never takes the time-domain kernel) and the runtime-radix kernels for
+ * 2/3/5-smooth lengths of at least 256 frames, in fp32 and in precise mode.  With PHAT on, a call
+ * returns -1 with a message (audiosync_cuda_last_error) and writes no output for PATH_DIRECT, for
+ * lengths that would be embedded (not 2/3/5-smooth: a weighted N'-point spectrum is a different
+ * function) and for lengths without such a plan.  It applies to xcorr_batch, xcorr_batch_results,
+ * xcorr_batch_device and pool_run, every dtype, memspace and host-narrowing mode; the drop-in
+ * cross_correlation() never weights.  Returns -1 for an unknown value. */
+enum { AUDIOSYNC_CUDA_WEIGHT_NONE = 0, AUDIOSYNC_CUDA_WEIGHT_PHAT = 1 };
+int  audiosync_cuda_set_weighting(audiosync_cuda_ctx *ctx, int weighting);
 void audiosync_cuda_set_debug(int on);                                    /* same effect as global_debug */
 /* Describes the plan for a length, e.g.
- * "fft L=1440000 M1=600 M2=2400 col=6x10x10 row=8x10x30 static". Returns the
+ * "fft L=1440000 M1=600 M2=2400 col=6x10x10 row=8x10x30 static", followed by " phat" under
+ * PHAT weighting. Returns the
  * number of characters written (excluding the NUL), -1 if buf is too small. */
 int audiosync_cuda_describe_plan(audiosync_cuda_ctx *ctx, size_t sample_len,
                                  char *buf, size_t buf_len);

@@ -23,13 +23,14 @@ __all__ = [
     "AudiosyncCudaError", "lib", "lib_path", "cross_correlation", "pearson_coefficient",
     "interval_loop", "Context", "RESULT_DTYPE", "MIN_CONFIDENCE", "SAMPLE_RATE",
     "INTERV_SAMPLE", "frames_to_ms", "F32", "F64", "S16", "HOST", "DEVICE",
-    "PATH_AUTO", "PATH_FFT", "PATH_DIRECT", "NARROW_OFF", "NARROW_LOSSLESS", "NARROW_ALWAYS", "EXPORTED_SYMBOLS", "shard_pairs", "gather_results", "host_narrow", "copy_threads",
+    "PATH_AUTO", "PATH_FFT", "PATH_DIRECT", "WEIGHT_NONE", "WEIGHT_PHAT", "NARROW_OFF", "NARROW_LOSSLESS", "NARROW_ALWAYS", "EXPORTED_SYMBOLS", "shard_pairs", "gather_results", "host_narrow", "copy_threads",
     "cross_correlation_ptr", "RealBuffer", "set_residency", "dropin_stats", "dropin_max_inflight", "SessionPool",
 ]
 
 F32, F64, S16 = 0, 1, 2          # S16: int16 PCM, value s / 32768 (records == F64 on those doubles, bit for bit)
 HOST, DEVICE = 0, 1
 PATH_AUTO, PATH_FFT, PATH_DIRECT = 0, 1, 2
+WEIGHT_NONE, WEIGHT_PHAT = 0, 1  # cross-spectrum weighting of the batch calls (GCC-PHAT: ncc = peak / N)
 NARROW_OFF, NARROW_LOSSLESS, NARROW_ALWAYS = 0, 1, 2
 
 _NP_DTYPES = {np.dtype(np.float32): F32, np.dtype(np.float64): F64, np.dtype(np.int16): S16}
@@ -51,7 +52,7 @@ EXPORTED_SYMBOLS = [
     "audiosync_cuda_create", "audiosync_cuda_destroy", "audiosync_cuda_device_count",
     "audiosync_cuda_xcorr_batch", "audiosync_cuda_xcorr_batch_results", "audiosync_cuda_xcorr_batch_device",
     "audiosync_cuda_synth_pairs", "audiosync_cuda_synchronize",
-    "audiosync_cuda_set_path", "audiosync_cuda_set_wave_pairs", "audiosync_cuda_set_debug", "audiosync_cuda_set_precise",
+    "audiosync_cuda_set_path", "audiosync_cuda_set_wave_pairs", "audiosync_cuda_set_debug", "audiosync_cuda_set_precise", "audiosync_cuda_set_weighting",
     "audiosync_cuda_set_host_narrowing", "audiosync_cuda_host_narrow", "audiosync_cuda_copy_threads",
     "audiosync_cuda_set_residency", "audiosync_cuda_dropin_stats", "audiosync_cuda_dropin_max_inflight",
     "audiosync_cuda_pool_create", "audiosync_cuda_pool_destroy", "audiosync_cuda_pool_reset",
@@ -125,6 +126,8 @@ def lib() -> C.CDLL:
     L.audiosync_cuda_host_narrow.argtypes = [vp, vp, C.c_size_t]
     L.audiosync_cuda_set_precise.restype = i32
     L.audiosync_cuda_set_precise.argtypes = [vp, i32]
+    L.audiosync_cuda_set_weighting.restype = i32
+    L.audiosync_cuda_set_weighting.argtypes = [vp, i32]
     L.audiosync_cuda_set_wave_pairs.restype = i32
     L.audiosync_cuda_set_wave_pairs.argtypes = [vp, i32]
     L.audiosync_cuda_set_residency.restype = None
@@ -423,6 +426,11 @@ class Context:
     def set_precise(self, on: bool):
         """fp64 arithmetic in the transforms (validation mode; see include/audiosync_cuda.h)."""
         self._check(lib().audiosync_cuda_set_precise(self._h, 1 if on else 0), "set_precise")
+
+    def set_weighting(self, mode: int):
+        """Cross-spectrum weighting of this context's batch calls: WEIGHT_NONE (the plain correlation)
+        or WEIGHT_PHAT (GCC-PHAT, the whitened cross-spectrum; see include/audiosync_cuda.h)."""
+        self._check(lib().audiosync_cuda_set_weighting(self._h, int(mode)), "set_weighting")
 
     def set_host_narrowing(self, mode: int):
         """f64 HOST batches converted to fp32 on the host while staged (half the PCIe bytes):

@@ -83,11 +83,11 @@ int PinnedBuf::ensure(size_t need) {
 }
 void PinnedBuf::release() { if (p) cudaFreeHost(p); p = nullptr; bytes = 0; }
 
-template <typename InT>
+template <typename InT, bool PHAT>
 static int run_small_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src,
                           const void* smp, long long sp, long long mp, PairPeak* peaks, int pairs,
                           cudaStream_t st) {
-    using K = SmallXcorrKernel<InT>;
+    using K = SmallXcorrKernel<InT, PHAT>;
     // int16: one 4-byte load per packed point where every pair's base is 4-byte aligned
     const int vec_src = reinterpret_cast<uintptr_t>(src) % 4 == 0 && sp % 2 == 0;
     const int vec_smp = reinterpret_cast<uintptr_t>(smp) % 4 == 0 && mp % 2 == 0;
@@ -115,23 +115,32 @@ static int build_small_plan(FftPlan* plan, long long L) {
     const size_t smem = SmallXcorrKernel<float>::smem_bytes((int)L);
     if (smem > 48 * 1024) {
         const int cap = (int)SmallXcorrKernel<float>::smem_bytes(SMALL_MAX_M);
-        ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<SmallXcorrKernel<float>>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
-        ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<SmallXcorrKernel<double>>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
-        ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<SmallXcorrKernel<int16_t>>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
+        auto allow = [&](auto KK) -> int {
+            ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<decltype(KK)>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
+            return 0;
+        };
+        if ((plan->phat ? allow(SmallXcorrKernel<float, true>{}) | allow(SmallXcorrKernel<double, true>{}) |
+                              allow(SmallXcorrKernel<int16_t, true>{})
+                        : allow(SmallXcorrKernel<float>{}) | allow(SmallXcorrKernel<double>{}) |
+                              allow(SmallXcorrKernel<int16_t>{})) != 0)
+            return -1;
     }
-    plan->run_wave = [plan](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
-                            int dtype, long long sp, long long mp, void*, PairPeak* peaks, int pairs,
-                            cudaStream_t st) {
+    auto run = [plan](auto PH, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp, int dtype,
+                      long long sp, long long mp, PairPeak* peaks, int pairs, cudaStream_t st) -> int {
+        constexpr bool PHAT = decltype(PH)::value;
         switch (dtype) {
-            case AUDIOSYNC_CUDA_F32: return run_small_wave<float>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
-            case AUDIOSYNC_CUDA_F64: return run_small_wave<double>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
-            case AUDIOSYNC_CUDA_S16: return run_small_wave<int16_t>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
+            case AUDIOSYNC_CUDA_F32: return run_small_wave<float, PHAT>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
+            case AUDIOSYNC_CUDA_F64: return run_small_wave<double, PHAT>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
+            case AUDIOSYNC_CUDA_S16: return run_small_wave<int16_t, PHAT>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
         }
         set_last_error("bad dtype %d", dtype);
         return -1;
+    };
+    plan->run_wave = [plan, run](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
+                                 int dtype, long long sp, long long mp, void*, PairPeak* peaks, int pairs,
+                                 cudaStream_t st) {
+        return plan->phat ? run(std::true_type{}, ctx, d, src, smp, dtype, sp, mp, peaks, pairs, st)
+                          : run(std::false_type{}, ctx, d, src, smp, dtype, sp, mp, peaks, pairs, st);
     };
     return 0;
 }
@@ -151,9 +160,15 @@ static int build_generic_plan_t(FftPlan* plan) {
     static const bool no_static_rows = getenv("AUDIOSYNC_CUDA_NO_STATIC_ROWS") != nullptr;      // diagnostics / A-B runs
     const bool static_rows = sizeof(T) == 4 && sh.static_rows != 0 && !no_static_rows;
     if (static_rows) plan->peak_scale *= 2.0;
+    // PHAT: the split's half-angle tables in the runtime-radix row kernel's position order (a static
+    // row kernel uploads its own)
+    if (plan->phat && !static_rows &&
+        (upload(plan->phat_rev, tb.phat_pos) != 0 || upload(plan->phat_lo, tb.phat_lo) != 0 || upload(plan->phat_hi, tb.phat_hi) != 0))
+        return -1;
     if ((small_col ? GenStage<T, GEN_THREADS_SMALL>::prepare_cols(sh) : GenStage<T, GEN_THREADS>::prepare_cols(sh)) != 0 ||
         (static_rows ? static_rows_prepare(plan)
-                     : small_row ? GenStage<T, GEN_THREADS_SMALL>::prepare_rows(sh) : GenStage<T, GEN_THREADS>::prepare_rows(sh)) != 0)
+                     : small_row ? GenStage<T, GEN_THREADS_SMALL>::prepare_rows(sh, plan->phat)
+                                 : GenStage<T, GEN_THREADS>::prepare_rows(sh, plan->phat)) != 0)
         return -1;
     plan->run_wave = [plan, small_col, small_row, static_rows](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
                                                   int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,
@@ -215,18 +230,22 @@ static int build_direct_plan(FftPlan* plan, long long L) {
     return 0;
 }
 
-// plans are cached per device and per (L, forced path)
+// plans are cached per device and per (L, forced path, precise, weighting)
 static FftPlan* get_plan(audiosync_cuda_ctx* ctx, DeviceState& d, long long L) {
     std::lock_guard<std::mutex> plk(d.plan_mu);
-    const size_t key = (size_t)L * 8 + (size_t)ctx->path * 2 + (ctx->precise ? 1 : 0);
+    const bool phat = ctx->weighting == AUDIOSYNC_CUDA_WEIGHT_PHAT;
+    const size_t key = ((size_t)L * 8 + (size_t)ctx->path * 2 + (ctx->precise ? 1 : 0)) * 2 + (phat ? 1 : 0);
     auto it = d.plans.find(key);
     if (it != d.plans.end()) return it->second.get();
     auto plan = std::make_shared<FftPlan>();
-    const PathKind kind = choose_path(L, ctx->path, ctx->precise);
+    plan->phat = phat;
+    const char* why = nullptr;
+    const PathKind kind = phat ? choose_path_phat(L, ctx->path, ctx->precise, &why) : choose_path(L, ctx->path, ctx->precise);
     int rc = -1;
     if (kind == PATH_NONE) {
-        set_last_error("sample_len %lld: no transform plan fits the device and the O(L^2) kernel is not used above %lld frames",
-                       L, DIRECT_MAX_L);
+        if (why) set_last_error("sample_len %lld: %s", L, why);
+        else set_last_error("sample_len %lld: no transform plan fits the device and the O(L^2) kernel is not used above %lld frames",
+                            L, DIRECT_MAX_L);
         return nullptr;
     }
     if (kind == PATH_STATIC_FFT) {
@@ -245,6 +264,7 @@ static FftPlan* get_plan(audiosync_cuda_ctx* ctx, DeviceState& d, long long L) {
         if (g_last_error[0] == 0) set_last_error("could not build a plan for sample_len %lld", L);
         return nullptr;
     }
+    if (phat) plan->desc += " phat";
     d.plans[key] = plan;
     return plan.get();
 }
@@ -321,25 +341,25 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
         int rc;
         if (dtype == AUDIOSYNC_CUDA_F32) {
             rc = launch(ctx, d, KC_PEARSON, st, [&] {
-                launch_stage(pearson_kernel<float, false>, grid, dim3(PEARSON_THREADS), 0, st,
+                launch_stage(plan->phat ? pearson_kernel<float, false, true> : pearson_kernel<float, false>, grid, dim3(PEARSON_THREADS), 0, st,
                     reinterpret_cast<const float*>(s), reinterpret_cast<const float*>(m), src_pitch, smp_pitch, L,
                     (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
             });
         } else if (dtype == ASC_DTYPE_F32_EXACT) {
             rc = launch(ctx, d, KC_PEARSON, st, [&] {
-                launch_stage(pearson_kernel<float, true>, grid, dim3(PEARSON_THREADS), 0, st,
+                launch_stage(plan->phat ? pearson_kernel<float, true, true> : pearson_kernel<float, true>, grid, dim3(PEARSON_THREADS), 0, st,
                     reinterpret_cast<const float*>(s), reinterpret_cast<const float*>(m), src_pitch, smp_pitch, L,
                     (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
             });
         } else if (dtype == AUDIOSYNC_CUDA_F64) {
             rc = launch(ctx, d, KC_PEARSON, st, [&] {
-                launch_stage(pearson_kernel<double, true>, grid, dim3(PEARSON_THREADS), 0, st,
+                launch_stage(plan->phat ? pearson_kernel<double, true, true> : pearson_kernel<double, true>, grid, dim3(PEARSON_THREADS), 0, st,
                     reinterpret_cast<const double*>(s), reinterpret_cast<const double*>(m), src_pitch, smp_pitch, L,
                     (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
             });
         } else {   // S16 (esz above admits nothing else): the f64 path's arithmetic on s * 2^-15
             rc = launch(ctx, d, KC_PEARSON, st, [&] {
-                launch_stage(pearson_kernel<int16_t, true>, grid, dim3(PEARSON_THREADS), 0, st,
+                launch_stage(plan->phat ? pearson_kernel<int16_t, true, true> : pearson_kernel<int16_t, true>, grid, dim3(PEARSON_THREADS), 0, st,
                     reinterpret_cast<const int16_t*>(s), reinterpret_cast<const int16_t*>(m), src_pitch, smp_pitch, L,
                     (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
             });
@@ -938,6 +958,15 @@ int audiosync_cuda_set_path(audiosync_cuda_ctx* ctx, int path) {
 int audiosync_cuda_set_precise(audiosync_cuda_ctx* ctx, int on) {
     if (!ctx) return -1;
     ctx->precise = on != 0;
+    return 0;
+}
+
+int audiosync_cuda_set_weighting(audiosync_cuda_ctx* ctx, int mode) {
+    if (!ctx || (mode != AUDIOSYNC_CUDA_WEIGHT_NONE && mode != AUDIOSYNC_CUDA_WEIGHT_PHAT)) {
+        set_last_error("unknown weighting %d", mode);
+        return -1;
+    }
+    ctx->weighting = mode;
     return 0;
 }
 

@@ -288,7 +288,8 @@ struct GenColFwdKernel {
 // Forward rows of both planes, split / conj-multiply / merge, inverse rows: grid = (M1/2 + 1, 1, pairs).
 // Rows are padded by one point per 128 bytes (phys), which keeps every pass -- also the stride-1
 // pass of an even radix, e.g. power-of-two lengths -- free of bank conflicts.
-template <typename T, int NT_ = GEN_THREADS>
+// PHAT: the split step whitens the spectra (split_phat_merge) with w = W_N^k1 * phat_pos[e].
+template <typename T, int NT_ = GEN_THREADS, bool PHAT = false>
 struct GenRowFusedKernel {
     typedef typename GenTraits<T>::C C;
     static constexpr int PADSH = GenTraits<T>::PADSH;
@@ -303,6 +304,11 @@ struct GenRowFusedKernel {
         const C* m_hi;
         const int* f2p_row;      // position of frequency
         GenShape sh;
+        // PHAT only: the split's w = exp(-2*pi*i*k/N), N = 2M, as exp(-2*pi*i*freq_of_pos(e)/(2*M2))
+        // in position order times W_N^k1 from two-level tables
+        const C* phat_pos;
+        const C* phat_lo;
+        const C* phat_hi;
     };
     static ASC_HD int row_pitch(int M2) { return (M2 + (M2 >> PADSH) + 2) & ~1; }     // even: 16-byte rows for bulk copies
     static size_t smem_bytes(const GenShape& sh) { return (size_t)4 * row_pitch(sh.M2) * sizeof(C) + 16; }
@@ -408,7 +414,7 @@ struct GenRowFusedKernel {
         }
         // split + conj-multiply (reference :232-233) + merge, into the source rows
         ex.phase([&](int tid) {
-            const C wk1 = tw2<C>(p.m_lo, p.m_hi, (unsigned)k1a);
+            const C wk1 = PHAT ? tw2<C>(p.phat_lo, p.phat_hi, (unsigned)k1a) : tw2<C>(p.m_lo, p.m_hi, (unsigned)k1a);
             if (two) {
                 C* __restrict__ zs_a = buf;
                 C* __restrict__ zs_b = buf + RP;
@@ -416,9 +422,10 @@ struct GenRowFusedKernel {
                 C* __restrict__ zp_b = buf + 3 * RP;
                 for (int e = tid; e < M2; e += THREADS) {
                     const int pa = phys(e), pb = phys(M2 - 1 - e);
-                    const C w2 = cmul(ldg(p.wpos + e), wk1);
+                    const C w2 = cmul(ldg((PHAT ? p.phat_pos : p.wpos) + e), wk1);      // PHAT: w
                     C qk, qmk;
-                    split_mul_merge_w2<C>(zs_a[pa], zs_b[pb], zp_a[pa], zp_b[pb], w2, qk, qmk);
+                    if constexpr (PHAT) split_phat_merge<2, C>(zs_a[pa], zs_b[pb], zp_a[pa], zp_b[pb], w2, qk, qmk);
+                    else split_mul_merge_w2<C>(zs_a[pa], zs_b[pb], zp_a[pa], zp_b[pb], w2, qk, qmk);
                     zs_a[pa] = qk;
                     zs_b[pb] = qmk;
                 }
@@ -435,10 +442,11 @@ struct GenRowFusedKernel {
                         ea = e;
                         eb = M2 - 1 - e;
                     }
-                    const C w2 = cmul(ldg(p.wpos + ea), wk1);
+                    const C w2 = cmul(ldg((PHAT ? p.phat_pos : p.wpos) + ea), wk1);     // PHAT: w
                     const int pa = phys(ea), pb = phys(eb);
                     C qk, qmk;
-                    split_mul_merge_w2<C>(zs[pa], zs[pb], zp[pa], zp[pb], w2, qk, qmk);
+                    if constexpr (PHAT) split_phat_merge<2, C>(zs[pa], zs[pb], zp[pa], zp[pb], w2, qk, qmk);
+                    else split_mul_merge_w2<C>(zs[pa], zs[pb], zp[pa], zp[pb], w2, qk, qmk);
                     zs[pa] = qk;
                     if (pa != pb) zs[pb] = qmk;
                 }

@@ -605,7 +605,84 @@ ASC_HD void split_mul_merge_w2(C a, C b, C c, C d, C w2, C& qk2, C& qmk2) {
     qmk2 = cmake(e.x, -e.y);
 }
 
-template <class RL, int M1_, int NT>
+// GCC-PHAT weighting: one spectrum value as a unit phasor, 0 where its squared magnitude is 0.
+// The value is first scaled by the power of two that brings its larger component into [1, 2):
+// exact, it keeps the squares in range at any input level, and it makes the phasor a function of
+// the value's direction alone, so that scaling either input by a power of two leaves the weighted
+// correlation unchanged bit for bit.
+ASC_HD float phat_rsqrt(float q) {
+#if defined(__CUDA_ARCH__)
+    return rsqrtf(q);
+#else
+    return 1.0f / sqrtf(q);
+#endif
+}
+ASC_HD double phat_rsqrt(double q) {
+#if defined(__CUDA_ARCH__)
+    return rsqrt(q);
+#else
+    return 1.0 / sqrt(q);
+#endif
+}
+ASC_HD cplx unit_phasor(cplx z) {
+    const float m = fmaxf(fabsf(z.x), fabsf(z.y));
+    uint32_t b;
+    memcpy(&b, &m, 4);
+    int e = (int)(b >> 23);                                   // m in [2^(e-127), 2^(e-126))
+    e = e < 1 ? 1 : (e > 253 ? 253 : e);
+    const uint32_t sb = (uint32_t)(254 - e) << 23;            // 2^(127 - e)
+    float s;
+    memcpy(&s, &sb, 4);
+    const float x = z.x * s, y = z.y * s;
+    const float q = fmaf(x, x, y * y);
+    const float r = q > 0.0f ? phat_rsqrt(q) : 0.0f;
+    return cmake(x * r, y * r);
+}
+ASC_HD cplxd unit_phasor(cplxd z) {
+    const double m = fmax(fabs(z.x), fabs(z.y));
+    uint64_t b;
+    memcpy(&b, &m, 8);
+    int e = (int)(b >> 52);                                   // m in [2^(e-1023), 2^(e-1022))
+    e = e < 1 ? 1 : (e > 2045 ? 2045 : e);
+    const uint64_t sb = (uint64_t)(2046 - e) << 52;           // 2^(1023 - e)
+    double s;
+    memcpy(&s, &sb, 8);
+    const double x = z.x * s, y = z.y * s;
+    const double q = fma(x, x, y * y);
+    const double r = q > 0.0 ? phat_rsqrt(q) : 0.0;
+    return cmake(x * r, y * r);
+}
+
+// The PHAT form of the split / multiply / merge step: W[k] = X[k] conj(Y[k]) / (|X[k]| |Y[k]|) takes
+// the place of the product.  Whitening needs X and Y themselves, hence w = exp(-2*pi*i*k/N) rather
+// than w^2: 2X[k] = s + u and conj(2X[M-k]) = s - u with u = -i w t (s, t from a, b as in
+// split_mul_merge_w2; Y from c, d alike).  X and Y are normalised separately (unit_phasor), then
+// p1 = W[k], p2 = conj(W[M-k]) are merged as in split_mul_merge.  SCALE is the output convention of
+// the step this replaces: 1 gives Q[k] (split_mul_merge), 2 gives 2 Q[k] (split_mul_merge_w2), so
+// that the inverse passes, the argmax and peak_scale are those of the unweighted path.
+template <int SCALE, class C>
+ASC_HD void split_phat_merge(C a, C b, C c, C d, C w, C& qk, C& qmk) {
+    static_assert(SCALE == 1 || SCALE == 2, "output convention of split_mul_merge or split_mul_merge_w2");
+    const C s = cconj_add(a, b), t = cconj_sub(a, b);
+    const C s2 = cconj_add(c, d), t2 = cconj_sub(c, d);
+    const C u = cmul_ni(cmul(w, t)), u2 = cmul_ni(cmul(w, t2));
+    const C p1 = cmulc(unit_phasor(cadd(s, u)), unit_phasor(cadd(s2, u2)));
+    const C p2 = cmulc(unit_phasor(csub(s, u)), unit_phasor(csub(s2, u2)));
+    C g = cadd(p1, p2);
+    C h = cmul_pi(cmulc(csub(p1, p2), w));                    // i conj(w) (p1 - p2)
+    if constexpr (SCALE == 2) {
+        g = cadd(g, g);
+        h = cadd(h, h);
+    }
+    qk = cadd(g, h);
+    const C e = csub(g, h);
+    qmk = cmake(e.x, -e.y);
+}
+
+// PHAT: the forward spectra are whitened in the split step (split_phat_merge) and the rest of the
+// kernel is unchanged.  Params::rev, m_lo and m_hi then hold the split's half-angle tables,
+// exp(-2*pi*i*freq_of_pos(e)/(2*M2)) and W_N (N = 2M), so that w = W_N^k1 * rev[e] factors like w^2.
+template <class RL, int M1_, int NT, bool PHAT = false>
 struct RowFusedKernel {
     static constexpr int M2 = RL::n;
     static constexpr int M1 = M1_;  // 0: the number of rows is a launch parameter (Params::m1) -- the rows of a
@@ -790,7 +867,8 @@ struct RowFusedKernel {
                                 const int pb = M2 - 1 - e;
                                 const cplx w2 = cmul(ax[decltype(X)::value], cm[decltype(Mm)::value]);
                                 cplx qk, qmk;
-                                split_mul_merge_w2(zs_a[e], zs_b[pb], zp_a[e], zp_b[pb], w2, qk, qmk);
+                                if constexpr (PHAT) split_phat_merge<2>(zs_a[e], zs_b[pb], zp_a[e], zp_b[pb], w2, qk, qmk);
+                                else split_mul_merge_w2(zs_a[e], zs_b[pb], zp_a[e], zp_b[pb], w2, qk, qmk);
                                 zs_a[e] = qk;
                                 zs_b[pb] = qmk;
                             }
@@ -811,7 +889,8 @@ struct RowFusedKernel {
                         }
                         const cplx w2 = cmul(ldg(p.rev + pa), wk1);
                         cplx qk, qmk;
-                        split_mul_merge_w2(zs[pa], zs[pb], zp[pa], zp[pb], w2, qk, qmk);
+                        if constexpr (PHAT) split_phat_merge<2>(zs[pa], zs[pb], zp[pa], zp[pb], w2, qk, qmk);
+                        else split_mul_merge_w2(zs[pa], zs[pb], zp[pa], zp[pb], w2, qk, qmk);
                         zs[pa] = qk;
                         if (pa != pb) zs[pb] = qmk;
                     }

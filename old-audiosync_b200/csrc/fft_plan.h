@@ -162,6 +162,16 @@ inline std::vector<cplx> build_row_rev() {
     return t;
 }
 
+// PHAT split tables (split_phat_merge needs w = exp(-2*pi*i*k/N), N = 2M, where the product needs
+// w^2): in POSITION order exp(-2*pi*i*freq_of_pos(e)/(2*M2)), the half angles of build_row_rev; the
+// W_N^k1 part comes from build_two_level(2M, M1 / 2).
+template <class RL>
+inline std::vector<cplx> build_row_rev_half() {
+    std::vector<cplx> t(RL::n);
+    for (int e = 0; e < RL::n; e++) t[e] = unit_root(RL::freq_of_pos(e), 2 * (long long)RL::n);
+    return t;
+}
+
 // K_B final-pass tables, one row per k1 (layout: RowFusedKernel::TABP): S0 entries
 // 0.5 * exp(-2*pi*i*j*k1/M), then R0 entries exp(-2*pi*i*k*S0*k1/M), zero padded to an even count.
 template <class RL>

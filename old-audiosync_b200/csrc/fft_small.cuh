@@ -35,7 +35,8 @@ ASC_HD int small_pos_of_freq(const SmallPlan& pl, int k) {
     return pos;
 }
 
-template <typename InT>
+// PHAT: the split step whitens the spectra (split_phat_merge); w is wn[k] as for the product.
+template <typename InT, bool PHAT = false>
 struct SmallXcorrKernel {
     static constexpr int THREADS = SMALL_THREADS;
 
@@ -126,7 +127,8 @@ struct SmallXcorrKernel {
                 const int pa = small_pos_of_freq(p.plan, e);
                 const int pb = small_pos_of_freq(p.plan, e == 0 ? 0 : M - e);
                 cplx qk, qmk;
-                split_mul_merge(buf[pa], buf[pb], buf[M + pa], buf[M + pb], ldg(p.wn + e), qk, qmk);
+                if constexpr (PHAT) split_phat_merge<1>(buf[pa], buf[pb], buf[M + pa], buf[M + pb], ldg(p.wn + e), qk, qmk);
+                else split_mul_merge(buf[pa], buf[pb], buf[M + pa], buf[M + pb], ldg(p.wn + e), qk, qmk);
                 buf[pa] = qk;
                 if (pa != pb) buf[pb] = qmk;
             }

@@ -43,8 +43,9 @@ int GenStage<T, NT>::prepare_cols(const GenShape& sh) {
 }
 
 template <typename T, int NT>
-int GenStage<T, NT>::prepare_rows(const GenShape& sh) {
-    return prepare_gen_kernel<GenRowFusedKernel<T, NT>>(GenRowFusedKernel<T, NT>::smem_bytes(sh));
+int GenStage<T, NT>::prepare_rows(const GenShape& sh, bool phat) {
+    return phat ? prepare_gen_kernel<GenRowFusedKernel<T, NT, true>>(GenRowFusedKernel<T, NT, true>::smem_bytes(sh))
+                : prepare_gen_kernel<GenRowFusedKernel<T, NT>>(GenRowFusedKernel<T, NT>::smem_bytes(sh));
 }
 
 template <typename T, int NT>
@@ -83,14 +84,18 @@ template <typename T, int NT>
 int GenStage<T, NT>::rows(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st) {
     typedef typename GenTraits<T>::C C;
     const GenShape& sh = plan->gen;
-    using K = GenRowFusedKernel<T, NT>;
-    typename K::Params p{static_cast<C*>(ws), static_cast<const C*>(plan->g_wrow.p), static_cast<const C*>(plan->g_wpos.p),
-                         static_cast<const C*>(plan->g_lo.p), static_cast<const C*>(plan->g_hi.p),
-                         static_cast<const int*>(plan->g_f2p_row.p), sh};
-    const dim3 grid(sh.M1 / 2 + 1, 1, pairs);
-    return launch(ctx, d, KC_ROW_FUSED, st, [&] {
-        launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), st, p);
-    });
+    auto go = [&](auto KK) -> int {
+        using K = decltype(KK);
+        typename K::Params p{static_cast<C*>(ws), static_cast<const C*>(plan->g_wrow.p), static_cast<const C*>(plan->g_wpos.p),
+                             static_cast<const C*>(plan->g_lo.p), static_cast<const C*>(plan->g_hi.p),
+                             static_cast<const int*>(plan->g_f2p_row.p), sh, static_cast<const C*>(plan->phat_rev.p),
+                             static_cast<const C*>(plan->phat_lo.p), static_cast<const C*>(plan->phat_hi.p)};
+        const dim3 grid(sh.M1 / 2 + 1, 1, pairs);
+        return launch(ctx, d, KC_ROW_FUSED, st, [&] {
+            launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), st, p);
+        });
+    };
+    return plan->phat ? go(GenRowFusedKernel<T, NT, true>{}) : go(GenRowFusedKernel<T, NT>{});
 }
 
 template <typename T, int NT>

@@ -232,6 +232,7 @@ inline double gen_peak_scale(const GenShape& sh) { return 0.5 * (double)sh.L / (
 template <class C>
 struct GenTables {
     std::vector<C> wcol, wrow, wpos, m_lo, m_hi;
+    std::vector<C> phat_pos, phat_lo, phat_hi;    // PHAT split: w = W_N^k1 * phat_pos[e], N = 2M
     std::vector<int> p2f_col, p2f_row, f2p_row;
 };
 
@@ -252,6 +253,12 @@ inline GenTables<C> gen_build_tables(const GenShape& sh) {
     t.f2p_row = gen_freq2pos(sh.row);
     t.wpos.resize(sh.M2);
     for (int e = 0; e < sh.M2; e++) t.wpos[e] = t.wrow[t.p2f_row[e]];
+    t.phat_pos.resize(sh.M2);
+    for (int e = 0; e < sh.M2; e++) t.phat_pos[e] = unit_root_as<C>(t.p2f_row[e], 2LL * sh.M2);
+    t.phat_lo.resize(1u << TW2_BITS);
+    for (long long a = 0; a < (long long)t.phat_lo.size(); a++) t.phat_lo[a] = unit_root_as<C>(a, 2 * sh.M);
+    t.phat_hi.resize(((sh.M1 / 2) >> TW2_BITS) + 1);      // k1 <= M1 / 2
+    for (long long b = 0; b < (long long)t.phat_hi.size(); b++) t.phat_hi[b] = unit_root_as<C>(b << TW2_BITS, 2 * sh.M);
     return t;
 }
 
@@ -298,6 +305,31 @@ inline PathKind choose_path(long long L, int forced, bool precise = false) {
     if (make_small_plan(L, &sp)) return PATH_SMALL_FFT;
     if (L >= GEN_MIN_L && gen_make_shape(L, false, &gs)) return PATH_GENERIC_FFT;
     return L <= DIRECT_MAX_L ? PATH_DIRECT : PATH_NONE;   // short lengths without a plan (FFT forced on a tiny odd L)
+}
+
+// The path of a PHAT-weighted context.  PHAT is defined on the N = 2L spectrum, so only plans that
+// transform at N = 2L serve it: the static plans, the single-CTA kernel (also below 4,096 frames)
+// and the runtime-radix plans at the length's own size (precise: fp64 arithmetic).  Never the
+// time-domain kernel, which has no spectrum, nor an embedded plan, whose weighted N'-point spectrum
+// is a different function and would depend on the planner's choice of M.  PATH_NONE comes with the
+// reason in *why.
+inline PathKind choose_path_phat(long long L, int forced, bool precise, const char** why) {
+    *why = nullptr;
+    if (forced == AUDIOSYNC_CUDA_PATH_DIRECT) {
+        *why = "PHAT weighting needs a transform; PATH_DIRECT has none";
+        return PATH_NONE;
+    }
+    SmallPlan sp;
+    if (!precise && has_static_plan(L)) return PATH_STATIC_FFT;
+    if (!precise && make_small_plan(L, &sp)) return PATH_SMALL_FFT;
+    GenShape gs;
+    if (L >= GEN_MIN_L && gen_make_shape(L, precise, &gs)) {
+        if (gs.M == L) return PATH_GENERIC_FFT;
+        *why = "PHAT weighting is defined on the N = 2L spectrum; this length is not 2/3/5-smooth and would be embedded in N' = 2M >= 3L";
+        return PATH_NONE;
+    }
+    *why = "no transform plan at N = 2L for PHAT weighting";
+    return PATH_NONE;
 }
 
 }  // namespace asc

@@ -34,6 +34,8 @@ struct FftPlan {
     SmallPlan small;
     GenShape gen{};                                  // runtime-radix four-step kernels
     DevBuf g_wcol, g_wrow, g_wpos, g_lo, g_hi, g_p2f_col, g_f2p_row;
+    bool phat = false;                               // PHAT weighting in the split step (AUDIOSYNC_CUDA_WEIGHT_PHAT)
+    DevBuf phat_rev, phat_lo, phat_hi;               // its twiddle w = W_N^k1 * phat_rev[e] (row kernel's position order)
     double peak_scale = 1.0;                         // r_reference = r_kernel * peak_scale
     // enqueues the transform kernels for `pairs` pairs (planes/r in ws)
     // (src, smp, dtype, src_pitch, smp_pitch [elements between pairs], workspace, peaks, pairs, stream)
@@ -44,6 +46,7 @@ struct FftPlan {
         wm.release(); wn.release();
         g_wcol.release(); g_wrow.release(); g_lo.release(); g_hi.release();
         g_wpos.release(); g_p2f_col.release(); g_f2p_row.release();
+        phat_rev.release(); phat_lo.release(); phat_hi.release();
     }
 };
 
@@ -146,7 +149,7 @@ template <class P> int build_static_plan(FftPlan* plan);     // static_plan_impl
 template <typename T, int NT>
 struct GenStage {
     static int prepare_cols(const GenShape& sh);
-    static int prepare_rows(const GenShape& sh);
+    static int prepare_rows(const GenShape& sh, bool phat);
     static int col_fwd(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp, int dtype,
                        long long sp, long long mp, void* ws, PairPeak* peaks, int pairs, cudaStream_t st);
     static int rows(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st);

@@ -184,6 +184,9 @@ struct PearsonShared {
 
 // Finishes one pair from the summed statistics (thread 0 of the finishing CTA).
 // px, py: the pivots the sums were shifted by (sum x^2 = sxx + 2 px sx + n px^2).
+// PHAT: the peak is that of the whitened correlation, and ncc = peak / N is its phase coherence
+// (the window energies have no meaning under whitening).
+template <bool PHAT>
 __device__ __forceinline__ void pearson_finish(const PearsonPartial& s, const Window& w, long long raw,
                                                double peak, double second, double px, double py, long long L,
                                                audiosync_cuda_result* __restrict__ out)
@@ -206,9 +209,13 @@ __device__ __forceinline__ void pearson_finish(const PearsonPartial& s, const Wi
     // normalised by the energies of the two windows (unshifted sums of squares)
     const double ap = fabs(peak);
     r.margin = ap > 0.0 ? (ap - second) / ap : (ap == 0.0 ? 0.0 : peak);   // NaN peak -> NaN
-    const double ex = s.sxx + 2.0 * px * s.sx + n * px * px;
-    const double ey = s.syy + 2.0 * py * s.sy + n * py * py;
-    r.ncc = peak / (2.0 * (double)L * sqrt(ex * ey));
+    if constexpr (PHAT) {
+        r.ncc = peak / (2.0 * (double)L);
+    } else {
+        const double ex = s.sxx + 2.0 * px * s.sx + n * px * px;
+        const double ey = s.syy + 2.0 * py * s.sy + n * py * py;
+        r.ncc = peak / (2.0 * (double)L * sqrt(ex * ey));
+    }
     *out = r;
 }
 
@@ -221,7 +228,7 @@ __device__ __forceinline__ void pearson_finish(const PearsonPartial& s, const Wi
 // int16_t that of 16-bit PCM (s * 2^-15, exact): element for element the same operations as
 // T = double, so the record is the f64 call's on those doubles bit for bit.  Only fp32 inputs have
 // the fp32 path.
-template <typename T, int NTP, bool WIDE = !std::is_same<T, float>::value>
+template <typename T, int NTP, bool WIDE = !std::is_same<T, float>::value, bool PHAT = false>
 __device__ __forceinline__ void pearson_block(
     const T* __restrict__ sources, const T* __restrict__ samples,
     long long src_pitch, long long smp_pitch, long long L,
@@ -383,14 +390,14 @@ __device__ __forceinline__ void pearson_block(
             if constexpr (!WIDE) { px = (double)(float)px; py = (double)(float)py; }
         }
         if (t == 0) {
-            pearson_finish(s, w, raw, peak, second, px, py, L, results + pair);
+            pearson_finish<PHAT>(s, w, raw, peak, second, px, py, L, results + pair);
             tickets[pair] = 0u;       // ready for the next wave
         }
     }
 }
 
-// grid = (n_chunks, n_pairs), block = 256.
-template <typename T, bool WIDE = !std::is_same<T, float>::value>
+// grid = (n_chunks, n_pairs), block = 256.  PHAT: records of a PHAT-weighted correlation (ncc rule).
+template <typename T, bool WIDE = !std::is_same<T, float>::value, bool PHAT = false>
 __global__ void __launch_bounds__(PEARSON_THREADS)
 pearson_kernel(const T* __restrict__ sources, const T* __restrict__ samples,
                long long src_pitch, long long smp_pitch, long long L,
@@ -400,7 +407,7 @@ pearson_kernel(const T* __restrict__ sources, const T* __restrict__ samples,
 {
     __shared__ PearsonShared<PEARSON_THREADS> sh;
     pdl_prologue();
-    pearson_block<T, PEARSON_THREADS, WIDE>(sources, samples, src_pitch, smp_pitch, L, peaks, explicit_n, peak_scale, partials,
+    pearson_block<T, PEARSON_THREADS, WIDE, PHAT>(sources, samples, src_pitch, smp_pitch, L, peaks, explicit_n, peak_scale, partials,
                                       tickets, n_chunks, results, (int)blockIdx.y, (int)blockIdx.x,
                                       (int)threadIdx.x, sh);
 }

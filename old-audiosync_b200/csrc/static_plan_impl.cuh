@@ -73,12 +73,18 @@ static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& 
         return -1;
     }
     {
-        using K = RowFusedKernel<Row, Col::n, P::NT_ROW>;
-        typename K::Params p{planes, row_tw, row_rev, m_lo, m_hi, P::L, row_tab};
-        const dim3 grid(M1 / 2 + 1, 1, pairs);
-        if (launch(ctx, d, KC_ROW_FUSED, st, [&] {
+        auto rows = [&](auto KK, const cplx* rev, const cplx* lo, const cplx* hi) -> int {
+            using K = decltype(KK);
+            typename K::Params p{planes, row_tw, rev, lo, hi, P::L, row_tab};
+            const dim3 grid(M1 / 2 + 1, 1, pairs);
+            return launch(ctx, d, KC_ROW_FUSED, st, [&] {
                 launch_stage(fft_kernel_entry<K>, grid, dim3(K::THREADS), K::SMEM, st, p);
-            }) != 0) return -1;
+            });
+        };
+        if ((plan->phat ? rows(RowFusedKernel<Row, Col::n, P::NT_ROW, true>{}, static_cast<const cplx*>(plan->phat_rev.p),
+                               static_cast<const cplx*>(plan->phat_lo.p), static_cast<const cplx*>(plan->phat_hi.p))
+                        : rows(RowFusedKernel<Row, Col::n, P::NT_ROW>{}, row_rev, m_lo, m_hi)) != 0)
+            return -1;
     }
     {
         const dim3 grid(pairs, M2 / COL_T, 1);
@@ -115,15 +121,23 @@ int build_static_plan(FftPlan* plan) {
         upload(plan->row_tab, build_row_tab<Row>(P::L, Col::n)) != 0 ||
         upload(plan->m_lo, m_lo) != 0 || upload(plan->m_hi, m_hi) != 0)
         return -1;
+    if (plan->phat) {
+        std::vector<cplx> n_lo, n_hi;
+        build_two_level(2 * P::L, Col::n / 2, n_lo, n_hi);
+        if (upload(plan->phat_rev, build_row_rev_half<Row>()) != 0 || upload(plan->phat_lo, n_lo) != 0 ||
+            upload(plan->phat_hi, n_hi) != 0)
+            return -1;
+    }
     using KT = ColFwdKernel<Col, Row::n, P::NT_COL, float, true>;
     using KR = ColFwdKernel<Col, Row::n, P::NT_COL, float, false>;
     using KD = ColFwdKernel<Col, Row::n, P::NT_COL, double, false>;
     using KS = ColFwdKernel<Col, Row::n, P::NT_COL, int16_t, false>;
     using KB = RowFusedKernel<Row, Col::n, P::NT_ROW>;
+    using KBP = RowFusedKernel<Row, Col::n, P::NT_ROW, true>;
     using KC = ColInvKernel<Col, Row::n, P::NT_COL>;
     if (prepare_kernel<KT>(KT::SMEM) != 0 || prepare_kernel<KR>(KR::SMEM) != 0 || prepare_kernel<KD>(KD::SMEM) != 0 ||
         prepare_kernel<KS>(KS::SMEM) != 0 ||
-        prepare_kernel<KB>(KB::SMEM) != 0 || prepare_kernel<KC>(KC::SMEM) != 0)
+        (plan->phat ? prepare_kernel<KBP>(KBP::SMEM) : prepare_kernel<KB>(KB::SMEM)) != 0 || prepare_kernel<KC>(KC::SMEM) != 0)
         return -1;
     plan->run_wave = [plan](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
                             int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,

@@ -6,9 +6,11 @@
 
 namespace asc {
 
+// PHAT plans run the PHAT twin of the row kernel, its split twiddle from the half-angle tables.
 template <class RL, int NT>
 struct StaticRows {
     using K = RowFusedKernel<RL, 0, NT>;
+    using KP = RowFusedKernel<RL, 0, NT, true>;
     static int prepare(FftPlan* plan) {
         const GenShape& sh = plan->gen;
         std::vector<cplx> m_lo, m_hi;
@@ -18,17 +20,29 @@ struct StaticRows {
             upload(plan->row_tab, build_row_tab<RL>(sh.M, sh.M1)) != 0 ||
             upload(plan->m_lo, m_lo) != 0 || upload(plan->m_hi, m_hi) != 0)
             return -1;
-        return prepare_kernel<K>(K::SMEM);
+        if (!plan->phat) return prepare_kernel<K>(K::SMEM);
+        std::vector<cplx> n_lo, n_hi;
+        build_two_level(2 * sh.M, sh.M1 / 2, n_lo, n_hi);
+        if (upload(plan->phat_rev, build_row_rev_half<RL>()) != 0 || upload(plan->phat_lo, n_lo) != 0 ||
+            upload(plan->phat_hi, n_hi) != 0)
+            return -1;
+        return prepare_kernel<KP>(KP::SMEM);
     }
-    static int launch_rows(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st) {
+    template <class KK>
+    static int launch_k(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st,
+                        const DevBuf& rev, const DevBuf& lo, const DevBuf& hi) {
         const GenShape& sh = plan->gen;
-        typename K::Params p{static_cast<cplx*>(ws), static_cast<const cplx*>(plan->row_tw.p),
-                             static_cast<const cplx*>(plan->row_rev.p), static_cast<const cplx*>(plan->m_lo.p),
-                             static_cast<const cplx*>(plan->m_hi.p), sh.M, static_cast<const cplx*>(plan->row_tab.p), sh.M1};
+        typename KK::Params p{static_cast<cplx*>(ws), static_cast<const cplx*>(plan->row_tw.p),
+                              static_cast<const cplx*>(rev.p), static_cast<const cplx*>(lo.p),
+                              static_cast<const cplx*>(hi.p), sh.M, static_cast<const cplx*>(plan->row_tab.p), sh.M1};
         const dim3 grid(sh.M1 / 2 + 1, 1, pairs);
         return launch(ctx, d, KC_ROW_FUSED, st, [&] {
-            launch_stage(fft_kernel_entry<K>, grid, dim3(K::THREADS), K::SMEM, st, p);
+            launch_stage(fft_kernel_entry<KK>, grid, dim3(KK::THREADS), KK::SMEM, st, p);
         });
+    }
+    static int launch_rows(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st) {
+        return plan->phat ? launch_k<KP>(plan, ctx, d, ws, pairs, st, plan->phat_rev, plan->phat_lo, plan->phat_hi)
+                          : launch_k<K>(plan, ctx, d, ws, pairs, st, plan->row_rev, plan->m_lo, plan->m_hi);
     }
 };
 
