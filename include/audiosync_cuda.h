@@ -116,10 +116,14 @@ typedef struct audiosync_cuda_ctx audiosync_cuda_ctx;
  *        S16 call returns, bit for bit in every field of each record, what the same call returns
  *        with dtype F64 on the doubles s / 32768.0 (every path, precise mode included).  A quarter
  *        of the F64 bytes cross the link (8.64 MB per pair at sample_len 1,440,000, against 17.28
- *        MB in F32 and 34.56 MB in F64).  Shapes, layouts and memspaces are those of F32 / F64; any
- *        2-byte-aligned base is accepted.  Accepted by audiosync_cuda_xcorr_batch,
- *        audiosync_cuda_xcorr_batch_results and audiosync_cuda_xcorr_batch_device only: the session
- *        pool and audiosync_cuda_synth_pairs refuse it, and host narrowing does not apply to it. */
+ *        MB in F32 and 34.56 MB in F64).  Shapes, layouts and memspaces are those of F32 / F64.
+ *        Accepted by audiosync_cuda_xcorr_batch, audiosync_cuda_xcorr_batch_results and
+ *        audiosync_cuda_xcorr_batch_device only: the session pool and audiosync_cuda_synth_pairs
+ *        refuse it, and host narrowing does not apply to it.
+ * In every dtype any base aligned to its element (4, 8 or 2 bytes) is accepted, such as a view at
+ * an odd element offset, x[1:]; the kernels then read it one element at a time where they would
+ * read two.  A device base that is not aligned to its element is refused with -1 and nothing is
+ * launched (host bases are copied into the library's own device buffers first). */
 enum { AUDIOSYNC_CUDA_F32 = 0, AUDIOSYNC_CUDA_F64 = 1, AUDIOSYNC_CUDA_S16 = 2 };
 enum { AUDIOSYNC_CUDA_HOST = 0, AUDIOSYNC_CUDA_DEVICE = 1 };
 

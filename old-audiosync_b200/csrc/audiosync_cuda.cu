@@ -88,9 +88,10 @@ static int run_small_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d
                           const void* smp, long long sp, long long mp, PairPeak* peaks, int pairs,
                           cudaStream_t st) {
     using K = SmallXcorrKernel<InT, PHAT>;
-    // int16: one 4-byte load per packed point where every pair's base is 4-byte aligned
-    const int vec_src = reinterpret_cast<uintptr_t>(src) % 4 == 0 && sp % 2 == 0;
-    const int vec_smp = reinterpret_cast<uintptr_t>(smp) % 4 == 0 && mp % 2 == 0;
+    // one load per packed point where every pair's base is aligned to two elements
+    const size_t al = 2 * sizeof(InT);
+    const int vec_src = reinterpret_cast<uintptr_t>(src) % al == 0 && sp % 2 == 0;
+    const int vec_smp = reinterpret_cast<uintptr_t>(smp) % al == 0 && mp % 2 == 0;
     typename K::Params p{static_cast<const InT*>(src), static_cast<const InT*>(smp), peaks,
                          static_cast<const cplx*>(plan->wm.p), static_cast<const cplx*>(plan->wn.p),
                          plan->small, sp, mp, vec_src, vec_smp};
@@ -311,11 +312,16 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
     if (smp_pitch == 0) smp_pitch = L;
     const bool packed = src_pitch == 2 * L && smp_pitch == L;
     if (L <= 0 || L > (1LL << 30)) { set_last_error("unsupported sample_len %lld", L); return -1; }
+    const size_t esz = dtype_bytes(dtype);
+    if (esz == 0) { set_last_error("bad dtype %d", dtype); return -1; }
+    // every kernel reads whole elements: a base between two elements is no array of this dtype
+    if (reinterpret_cast<uintptr_t>(src) % esz != 0 || reinterpret_cast<uintptr_t>(smp) % esz != 0) {
+        set_last_error("sources / samples base is not aligned to its %zu-byte element", esz);
+        return -1;
+    }
     ASC_CUDA_OK(cudaSetDevice(d.device));
     FftPlan* plan = get_plan(ctx, d, L);
     if (!plan) return -1;
-    const size_t esz = dtype_bytes(dtype);
-    if (esz == 0) { set_last_error("bad dtype %d", dtype); return -1; }
     const int in_dtype = dtype == ASC_DTYPE_F32_EXACT ? AUDIOSYNC_CUDA_F32 : dtype;   // what the transform loads
     int wave = ctx->wave_pairs > 0 ? ctx->wave_pairs : default_wave_pairs(plan, n_pairs);
     wave = (int)std::min<size_t>((size_t)wave, n_pairs);

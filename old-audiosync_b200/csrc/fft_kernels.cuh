@@ -67,20 +67,24 @@ constexpr int tile_box_start(int rows, int i) {
     return i * tile_box_rows(rows) + tile_box_rows(rows) <= rows ? i * tile_box_rows(rows) : rows - tile_box_rows(rows);
 }
 
-// Packed point n = (x[2n], x[2n + 1]).  vec: one 4-byte load per int16 point (the base is 4-byte
-// aligned); otherwise two 2-byte loads.  The fp32 / fp64 loads need their natural pair alignment,
-// which every caller's base has, and ignore it.
+// Packed point n = (x[2n], x[2n + 1]).  vec: one load of both elements (float2, double2, short2;
+// the base is aligned to two elements); otherwise two element loads.  A base is only guaranteed
+// element alignment: a view at an odd element offset, such as x[1:], has no more.
 template <typename InT>
 ASC_HD cplx load_packed(const InT* __restrict__ x, long long n, bool vec = true);
 
 template <>
-ASC_HD cplx load_packed<float>(const float* __restrict__ x, long long n, bool) {
-    return ldg(reinterpret_cast<const float2*>(x) + n);
+ASC_HD cplx load_packed<float>(const float* __restrict__ x, long long n, bool vec) {
+    if (vec) return ldg(reinterpret_cast<const float2*>(x) + n);
+    return cmake(ldg(x + 2 * n), ldg(x + 2 * n + 1));
 }
 template <>
-ASC_HD cplx load_packed<double>(const double* __restrict__ x, long long n, bool) {
-    double2 d = ldg(reinterpret_cast<const double2*>(x) + n);
-    return cmake(in_real<float>(d.x), in_real<float>(d.y));
+ASC_HD cplx load_packed<double>(const double* __restrict__ x, long long n, bool vec) {
+    if (vec) {
+        const double2 d = ldg(reinterpret_cast<const double2*>(x) + n);
+        return cmake(in_real<float>(d.x), in_real<float>(d.y));
+    }
+    return cmake(in_real<float>(ldg(x + 2 * n)), in_real<float>(ldg(x + 2 * n + 1)));
 }
 template <>
 ASC_HD cplx load_packed<int16_t>(const int16_t* __restrict__ x, long long n, bool vec) {
@@ -183,8 +187,8 @@ struct ColFwdKernel {
         long long L;             // sample_len == M = M1 * M2
         long long src_pitch;     // elements between consecutive pairs' sources / samples;
         long long smp_pitch;     // 0 = packed ([pair][2L] and [pair][L])
-        // int16 input: every pair's sources / samples start 4-byte aligned (one load per packed
-        // point); CTA-uniform.  These sit in the padding before the tensor maps.
+        // register path: every pair's sources / samples start aligned to two elements (one load
+        // per packed point); CTA-uniform.  These sit in the padding before the tensor maps.
         int vec_src, vec_smp;
         // TMA: [pair][M1 or M1/2 rows][2*M2 floats] views of sources / samples, boxes of
         // 32 floats x tile_box_rows(M1 - 1) resp. tile_box_rows(M1 / 2) rows

@@ -49,7 +49,7 @@ struct SmallXcorrKernel {
         SmallPlan plan;
         long long src_pitch;  // elements between consecutive pairs; 0 = packed (2M / M)
         long long smp_pitch;
-        int vec_src, vec_smp; // int16 input: one 4-byte load per packed point (every pair's base is 4-byte aligned)
+        int vec_src, vec_smp; // one load per packed point (every pair's base is aligned to two elements)
     };
     // two rows of M points + 512 bytes of reduction scratch (phase_argmax needs 392)
     static size_t smem_bytes(int M) { return (size_t)2 * M * sizeof(cplx) + 512; }

@@ -38,6 +38,11 @@ static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& 
             launch_stage(fft_kernel_entry<K>, grid_a, dim3(K::THREADS), K::SMEM, st, p);
         });
     };
+    // register path: one load per packed point where every pair's base is aligned to two elements
+    // (a view at an odd element offset, e.g. x[1:], is not: two element loads then)
+    auto vec_ok = [](const void* p, long long pitch, size_t esz) -> int {
+        return reinterpret_cast<uintptr_t>(p) % (2 * esz) == 0 && pitch % 2 == 0;
+    };
     if (dtype == AUDIOSYNC_CUDA_F32) {
         // TMA boxes need 16-byte aligned rows: every pair / row offset is a multiple of 16 bytes,
         // so only the base pointers decide.  Other fp32 inputs load through registers.
@@ -54,17 +59,17 @@ static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& 
                          make_tile_map(&pt.tm_smp, m_in, M2, M1 / 2, (size_t)smp_pitch * sizeof(float), (size_t)pairs,
                                        tile_box_rows(KT::SMP_ROWS)) == 0;
         if ((tma ? col_fwd(KT{}, pt)
-                 : col_fwd(KR{}, {s_in, m_in, planes, peaks, col_tw, col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch})) != 0)
+                 : col_fwd(KR{}, {s_in, m_in, planes, peaks, col_tw, col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch,
+                                  vec_ok(src, src_pitch, sizeof(float)), vec_ok(smp, smp_pitch, sizeof(float))})) != 0)
             return -1;
     } else if (dtype == AUDIOSYNC_CUDA_F64) {
         using K = ColFwdKernel<Col, Row::n, P::NT_COL, double, false>;
         if (col_fwd(K{}, {static_cast<const double*>(src), static_cast<const double*>(smp), planes, peaks, col_tw,
-                          col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch}) != 0) return -1;
+                          col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch, vec_ok(src, src_pitch, sizeof(double)),
+                          vec_ok(smp, smp_pitch, sizeof(double))}) != 0) return -1;
     } else if (dtype == AUDIOSYNC_CUDA_S16) {
-        // one 4-byte load per packed point where every pair's base is 4-byte aligned (a view at an
-        // odd element offset, e.g. x[1:], is not: two 2-byte loads then)
-        const int vec_src = reinterpret_cast<uintptr_t>(src) % 4 == 0 && src_pitch % 2 == 0;
-        const int vec_smp = reinterpret_cast<uintptr_t>(smp) % 4 == 0 && smp_pitch % 2 == 0;
+        const int vec_src = vec_ok(src, src_pitch, sizeof(int16_t));
+        const int vec_smp = vec_ok(smp, smp_pitch, sizeof(int16_t));
         using K = ColFwdKernel<Col, Row::n, P::NT_COL, int16_t, false>;
         if (col_fwd(K{}, {static_cast<const int16_t*>(src), static_cast<const int16_t*>(smp), planes, peaks, col_tw,
                           col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch, vec_src, vec_smp}) != 0) return -1;

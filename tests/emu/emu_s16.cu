@@ -1,9 +1,10 @@
 // tests/emu/emu_s16.cu -- CPU emulation of the kernel bodies for 16-bit PCM inputs (TEST ONLY).
 //
-// Runs the kernel bodies like emu.cu, with runners that set the kernels' int16 load flags the way the
-// product does: one 4-byte load per packed point where the base is 4-byte aligned, two 2-byte loads
-// otherwise.  Every runner is a template on the input type, so the int16_t instantiation and the
-// double instantiation it is compared with run the same host code, and every runner returns the whole
+// Runs the kernel bodies like emu.cu, with runners that set the kernels' load flags the way the
+// product does: one load of both elements of a packed point where the base is aligned to two elements
+// (4 bytes for int16), two element loads otherwise; the fp32 / fp64 runners can force either.  Every
+// runner is a template on the input type, so the int16_t instantiation and the double instantiation
+// it is compared with run the same host code, and every runner returns the whole
 // peak record (packed key, second-peak and seed order bits) next to the resolved index / peak /
 // second peak.  Compiled by tests/test_pcm_s16_emu.py; never linked into the product.  It does not
 // include emu.cu, whose other instantiations would double the compile time.
@@ -59,8 +60,14 @@ struct Rec {
 
 namespace {
 
-// the product's rule (static_plan_impl.cuh, run_small_wave, GenStage::col_fwd) for one packed pair
-int vec_ok(const void* p, long long pitch) { return reinterpret_cast<uintptr_t>(p) % 4 == 0 && pitch % 2 == 0; }
+// the product's rule (static_plan_impl.cuh, run_small_wave, GenStage::col_fwd) for one packed pair:
+// one load of two elements where the base is aligned to two elements and the pitch is even.  vec >= 0
+// overrides it (the emulator reads any address, so both branches can run on the same arrays).
+template <typename InT>
+int vec_ok(const InT* p, long long pitch, int vec = -1) {
+    if (vec >= 0) return vec;
+    return reinterpret_cast<uintptr_t>(p) % (2 * sizeof(InT)) == 0 && pitch % 2 == 0;
+}
 
 void from_peak(const PairPeak& pk, double scale, Rec* r) {
     r->raw_index = (long long)argmax_key_index(pk.key);
@@ -71,7 +78,7 @@ void from_peak(const PairPeak& pk, double scale, Rec* r) {
 
 // static four-step plan: K_A through its register path, K_B, K_C
 template <class P, typename InT>
-void static_plan(const InT* source, const InT* sample, PairPeak* peak) {
+void static_plan(const InT* source, const InT* sample, PairPeak* peak, int vec = -1) {
     using Col = typename P::Col;
     using Row = typename P::Row;
     constexpr int M1 = Col::n, M2 = Row::n;
@@ -88,7 +95,7 @@ void static_plan(const InT* source, const InT* sample, PairPeak* peak) {
     {
         using K = ColFwdKernel<Col, Row::n, P::NT_COL, InT, false>;
         typename K::Params p{source, sample, planes.data(), peak, col_tw.data(), col_tc.data(), m_lo.data(), m_hi.data(), M,
-                             2 * M, M, vec_ok(source, 2 * M), vec_ok(sample, M)};
+                             2 * M, M, vec_ok(source, 2 * M, vec), vec_ok(sample, M, vec)};
         std::vector<cplx> smem(K::SMEM / sizeof(cplx));
         for (int sig = 0; sig < 2; sig++)
             for (int tile = 0; tile < M2 / COL_T; tile++) {
@@ -116,13 +123,14 @@ void static_plan(const InT* source, const InT* sample, PairPeak* peak) {
     }
 }
 
-template <typename InT>
-int small_plan(const InT* source, const InT* sample, long long L, PairPeak* peak) {
+template <typename InT, bool PHAT = false>
+int small_plan(const InT* source, const InT* sample, long long L, PairPeak* peak, int vec = -1) {
     SmallPlan pl;
     if (!make_small_plan(L, &pl)) return -1;
     std::vector<cplx> wm = build_full_table(L, L), wn = build_full_table(2 * L, L);
-    using K = SmallXcorrKernel<InT>;
-    typename K::Params p{source, sample, peak, wm.data(), wn.data(), pl, 2 * L, L, vec_ok(source, 2 * L), vec_ok(sample, L)};
+    using K = SmallXcorrKernel<InT, PHAT>;
+    typename K::Params p{source, sample, peak, wm.data(), wn.data(), pl, 2 * L, L, vec_ok(source, 2 * L, vec),
+                         vec_ok(sample, L, vec)};
     std::vector<cplx> smem(K::smem_bytes((int)L) / sizeof(cplx));
     peak->key = 12345ull; peak->second_bits = 777u; peak->seed_bits = 777u;   // garbage: the kernel must clear them
     HostExec ex{0, 0, 0, K::THREADS};
@@ -194,9 +202,10 @@ int generic_plan(const InT* source, const InT* sample, long long L, Rec* out) {
     return 0;
 }
 
-// the product's AUTO / FFT choice of plan; the direct path has no transform to emulate (-2)
-template <typename InT>
-int xcorr(const InT* source, const InT* sample, long long L, int forced, Rec* out, int* path) {
+// the product's AUTO / FFT choice of plan; the direct path has no transform to emulate (-2).  PHAT:
+// the single-CTA kernel's PHAT twin (-3 for the four-step plans, whose PHAT rows are not emulated here)
+template <typename InT, bool PHAT = false>
+int xcorr(const InT* source, const InT* sample, long long L, int forced, Rec* out, int* path, int vec = -1) {
     const PathKind kind = choose_path(L, forced);
     *path = (int)kind;
     PairPeak pk;
@@ -206,13 +215,15 @@ int xcorr(const InT* source, const InT* sample, long long L, int forced, Rec* ou
         for_each_static_plan([&](auto P) {
             using PT = decltype(P);
             if (PT::L != L) return;
-            static_plan<PT, InT>(source, sample, &pk);
+            if (PHAT) { rc = -3; return; }
+            static_plan<PT, InT>(source, sample, &pk, vec);
             rc = 0;
         });
         if (rc != 0) return rc;
     } else if (kind == PATH_SMALL_FFT) {
-        if (small_plan<InT>(source, sample, L, &pk) != 0) return -1;
+        if (small_plan<InT, PHAT>(source, sample, L, &pk, vec) != 0) return -1;
     } else if (kind == PATH_GENERIC_FFT) {
+        if (PHAT) return -3;
         return generic_plan<float, InT>(source, sample, L, out);
     } else {
         return -2;
@@ -238,6 +249,14 @@ int emu16_generic_s16(const int16_t* source, const int16_t* sample, long long L,
 }
 int emu16_generic_f64(const double* source, const double* sample, long long L, int precise, Rec* out) {
     return precise ? generic_plan<double, double>(source, sample, L, out) : generic_plan<float, double>(source, sample, L, out);
+}
+// fp32 / fp64 inputs through K_A's register path (static lengths) or the single-CTA kernel (phat != 0:
+// its PHAT twin) with both load flags forced to `vec`: one load of two elements, or two element loads
+int emu16_xcorr_vec_f32(const float* source, const float* sample, long long L, int phat, int vec, Rec* out, int* path) {
+    return phat ? xcorr<float, true>(source, sample, L, 0, out, path, vec) : xcorr<float>(source, sample, L, 0, out, path, vec);
+}
+int emu16_xcorr_vec_f64(const double* source, const double* sample, long long L, int phat, int vec, Rec* out, int* path) {
+    return phat ? xcorr<double, true>(source, sample, L, 0, out, path, vec) : xcorr<double>(source, sample, L, 0, out, path, vec);
 }
 
 }

@@ -3,8 +3,9 @@
 An S16 sample s stands for the value s / 32768 (= s * 2^-15, exact in fp32 and fp64).  The kernels
 instantiated for int16_t must therefore produce exactly what their f64-input instantiation produces
 on the doubles s / 32768: the same packed peak key, second-peak bits and seed bits on the fp32-argmax
-paths, the same resolved index / peak / second peak in fp64 arithmetic.  tests/emu/emu_s16.cu holds
-the runners; this module compiles it (g++, no GPU) into a temporary directory.
+paths, the same resolved index / peak / second peak in fp64 arithmetic.  The same runners also check
+the element-load branch that fp32 / fp64 bases at an odd element offset take.  tests/emu/emu_s16.cu
+holds the runners; this module compiles it (g++, no GPU) into a temporary directory.
 """
 import ctypes as C
 import os
@@ -47,6 +48,9 @@ def emu16(tmp_path_factory):
     gsig = [C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.POINTER(Rec)]
     E.emu16_generic_s16.argtypes = gsig
     E.emu16_generic_f64.argtypes = gsig
+    vsig = [C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.POINTER(Rec), C.POINTER(C.c_int)]
+    E.emu16_xcorr_vec_f32.argtypes = vsig
+    E.emu16_xcorr_vec_f64.argtypes = vsig
     return E
 
 
@@ -144,3 +148,24 @@ def test_full_scale_inputs(emu16, L):
     src = np.where(rng.random(2 * L) < 0.5, -32768, 32767).astype(np.int16)
     _check_xcorr(emu16, src, src[17:17 + L].copy(), path)
     _check_xcorr(emu16, np.full(2 * L, -32768, np.int16), np.full(L, 32767, np.int16), path)
+
+
+@pytest.mark.parametrize("L,phat", [(144000, False), (960000, False), (4096, False), (4096, True),
+                                    (6000, False), (6000, True)])
+def test_fp_element_loads_equal_pair_loads(emu16, L, phat):
+    """fp32 / fp64 inputs at an odd element offset are read one element at a time (vec = 0) by K_A's
+    register path and the single-CTA kernel (both weightings): the same peak key, second-peak and seed
+    bits as one float2 / double2 load per packed point (vec = 1).  On the host no load can be
+    misaligned, so this checks the arithmetic of the element-load branch, not the alignment."""
+    path = PATH_STATIC if L >= 144000 else PATH_SMALL         # K_A is the same kernel under PHAT
+    src, smp = pcm_pair(L, seed=L + 5)
+    for dt, fn in ((np.float32, emu16.emu16_xcorr_vec_f32), (np.float64, emu16.emu16_xcorr_vec_f64)):
+        s, m = widen(src).astype(dt), widen(smp).astype(dt)
+        got = []
+        for vec in (0, 1):
+            r, p = Rec(), C.c_int()
+            assert fn(s.ctypes.data, m.ctypes.data, L, int(phat), vec, C.byref(r), C.byref(p)) == 0
+            assert p.value == path
+            got.append(r.tuple())
+        assert got[0] == got[1], (dt, got)
+        assert got[0][3] != 12345                   # the kernels cleared the planted peak key
