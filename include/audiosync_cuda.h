@@ -311,10 +311,33 @@ int  audiosync_cuda_set_precise(audiosync_cuda_ctx *ctx, int on);
  * cross_correlation() never weights.  Returns -1 for an unknown value. */
 enum { AUDIOSYNC_CUDA_WEIGHT_NONE = 0, AUDIOSYNC_CUDA_WEIGHT_PHAT = 1 };
 int  audiosync_cuda_set_weighting(audiosync_cuda_ctx *ctx, int weighting);
+/* Lag window of the batch calls, per context: the search for the peak is restricted to the folded
+ * lags (the record's `lag` convention) of [lag_lo, lag_hi], inclusive.  The default,
+ * [INT64_MIN, INT64_MAX], is no restriction; passing those values restores it.  lag_lo > lag_hi
+ * returns -1 with a message and leaves the setting unchanged.
+ * Per call the effective window is [max(lag_lo, -L), min(lag_hi, L - 1)]: a call whose effective
+ * window is empty returns -1 with a message and writes no output; one that covers all of [-L, L-1]
+ * is the unwindowed call, bit for bit.  The allowed raw indices are raw = lag for lag >= 0 and
+ * raw = lag + 2L below, and over them, in ascending raw order:
+ *   raw_index  the reference's argmax rule restricted to them: r[0] is the signed seed only when
+ *              the window holds lag 0, otherwise every allowed index competes by |r|; strict >, the
+ *              first index wins ties (at equal |r| a positive lag beats a negative one).  A NaN never
+ *              wins; when no allowed value is a number, raw_index is the lowest allowed index and
+ *              peak its (NaN) value, as with a NaN r[0] seed.
+ *   second     the largest |r| over the allowed indices other than raw_index (|r[0]| only when the
+ *              window holds lag 0); margin follows from it as before.
+ *   lag, coef, ret, success, ncc  the same functions of raw_index as without a window.
+ * Use it when bounds on the answer are known (the recording started after the track, the offset is
+ * within a few seconds) or to keep out lags whose aligned windows overlap by only a few frames.  It
+ * applies to xcorr_batch, xcorr_batch_results, xcorr_batch_device and pool_run, in every dtype,
+ * memspace, host-narrowing mode, path, precise mode and weighting; the drop-in cross_correlation()
+ * never uses it. */
+int  audiosync_cuda_set_lag_window(audiosync_cuda_ctx *ctx, int64_t lag_lo, int64_t lag_hi);
 void audiosync_cuda_set_debug(int on);                                    /* same effect as global_debug */
 /* Describes the plan for a length, e.g.
  * "fft L=1440000 M1=600 M2=2400 col=6x10x10 row=8x10x30 static", followed by " phat" under
- * PHAT weighting. Returns the
+ * PHAT weighting and " lags=[lo,hi]" (the effective window) when the lag window restricts the
+ * search at this length. Returns the
  * number of characters written (excluding the NUL), -1 if buf is too small. */
 int audiosync_cuda_describe_plan(audiosync_cuda_ctx *ctx, size_t sample_len,
                                  char *buf, size_t buf_len);

@@ -53,6 +53,7 @@ EXPORTED_SYMBOLS = [
     "audiosync_cuda_xcorr_batch", "audiosync_cuda_xcorr_batch_results", "audiosync_cuda_xcorr_batch_device",
     "audiosync_cuda_synth_pairs", "audiosync_cuda_synchronize",
     "audiosync_cuda_set_path", "audiosync_cuda_set_wave_pairs", "audiosync_cuda_set_debug", "audiosync_cuda_set_precise", "audiosync_cuda_set_weighting",
+    "audiosync_cuda_set_lag_window",
     "audiosync_cuda_set_host_narrowing", "audiosync_cuda_host_narrow", "audiosync_cuda_copy_threads",
     "audiosync_cuda_set_residency", "audiosync_cuda_dropin_stats", "audiosync_cuda_dropin_max_inflight",
     "audiosync_cuda_pool_create", "audiosync_cuda_pool_destroy", "audiosync_cuda_pool_reset",
@@ -128,6 +129,8 @@ def lib() -> C.CDLL:
     L.audiosync_cuda_set_precise.argtypes = [vp, i32]
     L.audiosync_cuda_set_weighting.restype = i32
     L.audiosync_cuda_set_weighting.argtypes = [vp, i32]
+    L.audiosync_cuda_set_lag_window.restype = i32
+    L.audiosync_cuda_set_lag_window.argtypes = [vp, C.c_int64, C.c_int64]
     L.audiosync_cuda_set_wave_pairs.restype = i32
     L.audiosync_cuda_set_wave_pairs.argtypes = [vp, i32]
     L.audiosync_cuda_set_residency.restype = None
@@ -431,6 +434,13 @@ class Context:
         """Cross-spectrum weighting of this context's batch calls: WEIGHT_NONE (the plain correlation)
         or WEIGHT_PHAT (GCC-PHAT, the whitened cross-spectrum; see include/audiosync_cuda.h)."""
         self._check(lib().audiosync_cuda_set_weighting(self._h, int(mode)), "set_weighting")
+
+    def set_lag_window(self, lo: int | None = None, hi: int | None = None):
+        """Restrict this context's batch calls to the folded lags [lo, hi] (inclusive); None leaves
+        that side unbounded, and set_lag_window() restores the full search (see include/audiosync_cuda.h)."""
+        lo = -(1 << 63) if lo is None else int(lo)
+        hi = (1 << 63) - 1 if hi is None else int(hi)
+        self._check(lib().audiosync_cuda_set_lag_window(self._h, lo, hi), "set_lag_window")
 
     def set_host_narrowing(self, mode: int):
         """f64 HOST batches converted to fp32 on the host while staged (half the PCIe bytes):

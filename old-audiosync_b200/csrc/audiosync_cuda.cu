@@ -83,11 +83,11 @@ int PinnedBuf::ensure(size_t need) {
 }
 void PinnedBuf::release() { if (p) cudaFreeHost(p); p = nullptr; bytes = 0; }
 
-template <typename InT, bool PHAT>
+template <typename InT, bool PHAT, bool WIN>
 static int run_small_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src,
                           const void* smp, long long sp, long long mp, PairPeak* peaks, int pairs,
-                          cudaStream_t st) {
-    using K = SmallXcorrKernel<InT, PHAT>;
+                          cudaStream_t st, const RawWindow* win) {
+    using K = SmallXcorrKernel<InT, PHAT, WIN>;
     // one load per packed point where every pair's base is aligned to two elements
     const size_t al = 2 * sizeof(InT);
     const int vec_src = reinterpret_cast<uintptr_t>(src) % al == 0 && sp % 2 == 0;
@@ -95,6 +95,7 @@ static int run_small_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d
     typename K::Params p{static_cast<const InT*>(src), static_cast<const InT*>(smp), peaks,
                          static_cast<const cplx*>(plan->wm.p), static_cast<const cplx*>(plan->wn.p),
                          plan->small, sp, mp, vec_src, vec_smp};
+    if constexpr (WIN) p.win = *win;
     const size_t smem = K::smem_bytes(plan->small.M);
     const dim3 grid(1, 1, pairs);
     return launch(ctx, d, KC_SMALL_FFT, st, [&] {
@@ -120,28 +121,34 @@ static int build_small_plan(FftPlan* plan, long long L) {
             ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<decltype(KK)>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
             return 0;
         };
-        if ((plan->phat ? allow(SmallXcorrKernel<float, true>{}) | allow(SmallXcorrKernel<double, true>{}) |
-                              allow(SmallXcorrKernel<int16_t, true>{})
-                        : allow(SmallXcorrKernel<float>{}) | allow(SmallXcorrKernel<double>{}) |
-                              allow(SmallXcorrKernel<int16_t>{})) != 0)
+        auto allow_all = [&](auto PH, auto W) -> int {
+            constexpr bool PHAT = decltype(PH)::value, WIN = decltype(W)::value;
+            return allow(SmallXcorrKernel<float, PHAT, WIN>{}) | allow(SmallXcorrKernel<double, PHAT, WIN>{}) |
+                   allow(SmallXcorrKernel<int16_t, PHAT, WIN>{});
+        };
+        if ((plan->phat ? allow_all(std::true_type{}, std::false_type{}) | allow_all(std::true_type{}, std::true_type{})
+                        : allow_all(std::false_type{}, std::false_type{}) | allow_all(std::false_type{}, std::true_type{})) != 0)
             return -1;
     }
-    auto run = [plan](auto PH, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp, int dtype,
-                      long long sp, long long mp, PairPeak* peaks, int pairs, cudaStream_t st) -> int {
-        constexpr bool PHAT = decltype(PH)::value;
+    auto run = [plan](auto PH, auto W, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp, int dtype,
+                      long long sp, long long mp, PairPeak* peaks, int pairs, cudaStream_t st, const RawWindow* win) -> int {
+        constexpr bool PHAT = decltype(PH)::value, WIN = decltype(W)::value;
         switch (dtype) {
-            case AUDIOSYNC_CUDA_F32: return run_small_wave<float, PHAT>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
-            case AUDIOSYNC_CUDA_F64: return run_small_wave<double, PHAT>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
-            case AUDIOSYNC_CUDA_S16: return run_small_wave<int16_t, PHAT>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st);
+            case AUDIOSYNC_CUDA_F32: return run_small_wave<float, PHAT, WIN>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st, win);
+            case AUDIOSYNC_CUDA_F64: return run_small_wave<double, PHAT, WIN>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st, win);
+            case AUDIOSYNC_CUDA_S16: return run_small_wave<int16_t, PHAT, WIN>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st, win);
         }
         set_last_error("bad dtype %d", dtype);
         return -1;
     };
     plan->run_wave = [plan, run](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
                                  int dtype, long long sp, long long mp, void*, PairPeak* peaks, int pairs,
-                                 cudaStream_t st) {
-        return plan->phat ? run(std::true_type{}, ctx, d, src, smp, dtype, sp, mp, peaks, pairs, st)
-                          : run(std::false_type{}, ctx, d, src, smp, dtype, sp, mp, peaks, pairs, st);
+                                 cudaStream_t st, const RawWindow* win) {
+        auto with_phat = [&](auto PH) {
+            return win ? run(PH, std::true_type{}, ctx, d, src, smp, dtype, sp, mp, peaks, pairs, st, win)
+                       : run(PH, std::false_type{}, ctx, d, src, smp, dtype, sp, mp, peaks, pairs, st, win);
+        };
+        return plan->phat ? with_phat(std::true_type{}) : with_phat(std::false_type{});
     };
     return 0;
 }
@@ -173,14 +180,14 @@ static int build_generic_plan_t(FftPlan* plan) {
         return -1;
     plan->run_wave = [plan, small_col, small_row, static_rows](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
                                                   int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,
-                                                  cudaStream_t st) {
+                                                  cudaStream_t st, const RawWindow* win) {
         using Big = GenStage<T, GEN_THREADS>;
         using Small = GenStage<T, GEN_THREADS_SMALL>;
         if ((small_col ? Small::col_fwd(plan, ctx, d, src, smp, dtype, sp, mp, ws, peaks, pairs, st)
                        : Big::col_fwd(plan, ctx, d, src, smp, dtype, sp, mp, ws, peaks, pairs, st)) != 0) return -1;
         if ((static_rows ? static_rows_launch(plan, ctx, d, ws, pairs, st)
                          : small_row ? Small::rows(plan, ctx, d, ws, pairs, st) : Big::rows(plan, ctx, d, ws, pairs, st)) != 0) return -1;
-        return small_col ? Small::col_inv(plan, ctx, d, ws, peaks, pairs, st) : Big::col_inv(plan, ctx, d, ws, peaks, pairs, st);
+        return small_col ? Small::col_inv(plan, ctx, d, ws, peaks, pairs, st, win) : Big::col_inv(plan, ctx, d, ws, peaks, pairs, st, win);
     };
     return 0;
 }
@@ -199,7 +206,7 @@ static int build_generic_plan(FftPlan* plan, long long L, bool precise) {
 template <typename InT>
 static int run_direct_wave(long long L, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src,
                            const void* smp, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,
-                           cudaStream_t st) {
+                           cudaStream_t st, const RawWindow* win) {
     const long long N = 2 * L;
     double* r = static_cast<double*>(ws);
     const dim3 grid((unsigned)((N + DIRECT_TILE - 1) / DIRECT_TILE), pairs);
@@ -208,7 +215,8 @@ static int run_direct_wave(long long L, audiosync_cuda_ctx* ctx, DeviceState& d,
                                                                   static_cast<const InT*>(smp), r, L, sp, mp);
         }) != 0) return -1;
     return launch(ctx, d, KC_ARGMAX_F64, st, [&] {
-        argmax_f64_kernel<<<pairs, 1024, 0, st>>>(r, N, N, peaks);
+        if (win) argmax_f64_window_kernel<<<pairs, 1024, 0, st>>>(r, N, N, peaks, *win);
+        else argmax_f64_kernel<<<pairs, 1024, 0, st>>>(r, N, N, peaks);
     });
 }
 
@@ -219,11 +227,11 @@ static int build_direct_plan(FftPlan* plan, long long L) {
     plan->desc = "direct L=" + std::to_string(L) + " time-domain O(L^2) fp64";
     plan->run_wave = [L](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
                          int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,
-                         cudaStream_t st) {
+                         cudaStream_t st, const RawWindow* win) {
         switch (dtype) {
-            case AUDIOSYNC_CUDA_F32: return run_direct_wave<float>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st);
-            case AUDIOSYNC_CUDA_F64: return run_direct_wave<double>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st);
-            case AUDIOSYNC_CUDA_S16: return run_direct_wave<int16_t>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st);
+            case AUDIOSYNC_CUDA_F32: return run_direct_wave<float>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st, win);
+            case AUDIOSYNC_CUDA_F64: return run_direct_wave<double>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st, win);
+            case AUDIOSYNC_CUDA_S16: return run_direct_wave<int16_t>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st, win);
         }
         set_last_error("bad dtype %d", dtype);
         return -1;
@@ -292,6 +300,16 @@ static int default_wave_pairs(const FftPlan* plan, size_t n_pairs) {
     return (int)std::min<long long>(w, (long long)std::max<size_t>(n_pairs, 1));
 }
 
+// The context's lag window at sample_len L: -1 (message set) when no lag of [-L, L - 1] is in it,
+// 0 when it holds them all (the unwindowed kernels), 1 with *w set otherwise.
+static int lag_window(const audiosync_cuda_ctx* ctx, long long L, RawWindow* w) {
+    const int rc = raw_window_of(ctx->lag_lo, ctx->lag_hi, L, w);
+    if (rc < 0)
+        set_last_error("lag window [%lld, %lld] holds no lag of [%lld, %lld] at sample_len %lld",
+                       ctx->lag_lo, ctx->lag_hi, -L, L - 1, L);
+    return rc;
+}
+
 // Ticket counters of the Pearson kernel: zeroed once, self-resetting afterwards.
 static int ensure_tickets(WorkSet& w, size_t n) {
     const size_t need = sizeof(unsigned int) * n;
@@ -319,6 +337,10 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
         set_last_error("sources / samples base is not aligned to its %zu-byte element", esz);
         return -1;
     }
+    RawWindow raw_win;
+    const int windowed = lag_window(ctx, L, &raw_win);
+    if (windowed < 0) return -1;
+    const RawWindow* win = windowed ? &raw_win : nullptr;
     ASC_CUDA_OK(cudaSetDevice(d.device));
     FftPlan* plan = get_plan(ctx, d, L);
     if (!plan) return -1;
@@ -342,7 +364,7 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
         const int pairs = (int)std::min<size_t>((size_t)wave, n_pairs - p0);
         const char* s = static_cast<const char*>(src) + p0 * (size_t)src_pitch * esz;
         const char* m = static_cast<const char*>(smp) + p0 * (size_t)smp_pitch * esz;
-        if (plan->run_wave(ctx, d, s, m, in_dtype, src_pitch, smp_pitch, work.ws.p, peaks, pairs, st) != 0) return -1;
+        if (plan->run_wave(ctx, d, s, m, in_dtype, src_pitch, smp_pitch, work.ws.p, peaks, pairs, st, win) != 0) return -1;
         const dim3 grid(n_chunks, pairs);
         int rc;
         if (dtype == AUDIOSYNC_CUDA_F32) {
@@ -976,6 +998,17 @@ int audiosync_cuda_set_weighting(audiosync_cuda_ctx* ctx, int mode) {
     return 0;
 }
 
+int audiosync_cuda_set_lag_window(audiosync_cuda_ctx* ctx, int64_t lag_lo, int64_t lag_hi) {
+    if (!ctx) { set_last_error("null argument"); return -1; }
+    if (lag_lo > lag_hi) {
+        set_last_error("lag window [%lld, %lld]: lag_lo > lag_hi", (long long)lag_lo, (long long)lag_hi);
+        return -1;
+    }
+    ctx->lag_lo = lag_lo;
+    ctx->lag_hi = lag_hi;
+    return 0;
+}
+
 int audiosync_cuda_set_host_narrowing(audiosync_cuda_ctx* ctx, int mode) {
     if (!ctx || mode < AUDIOSYNC_CUDA_NARROW_OFF || mode > AUDIOSYNC_CUDA_NARROW_ALWAYS) return -1;
     ctx->narrow_host = mode;
@@ -1013,9 +1046,15 @@ int audiosync_cuda_describe_plan(audiosync_cuda_ctx* ctx, size_t sample_len, cha
     DeviceState& d = ctx->devs[0];
     if (cudaSetDevice(d.device) != cudaSuccess) return -1;
     FftPlan* plan = get_plan(ctx, d, (long long)sample_len);
-    if (!plan || plan->desc.size() + 1 > buf_len) return -1;
-    memcpy(buf, plan->desc.c_str(), plan->desc.size() + 1);
-    return (int)plan->desc.size();
+    if (!plan) return -1;
+    std::string desc = plan->desc;
+    RawWindow w;
+    long long lo = 0, hi = 0;
+    if (raw_window_of(ctx->lag_lo, ctx->lag_hi, (long long)sample_len, &w, &lo, &hi) > 0)
+        desc += " lags=[" + std::to_string(lo) + "," + std::to_string(hi) + "]";
+    if (desc.size() + 1 > buf_len) return -1;
+    memcpy(buf, desc.c_str(), desc.size() + 1);
+    return (int)desc.size();
 }
 
 int audiosync_cuda_profile_enable(audiosync_cuda_ctx* ctx, int on) {
@@ -1115,6 +1154,8 @@ int audiosync_cuda_xcorr_batch_results(audiosync_cuda_ctx* ctx, const void* sour
     if (sample_len == 0) { set_last_error("sample_len must be > 0"); return -1; }
     std::lock_guard<std::mutex> lk(ctx->mu);
     const long long L = (long long)sample_len;
+    RawWindow win;
+    if (lag_window(ctx, L, &win) < 0) return -1;     // before any copy: nothing is written
     int rc = 0;
     if (memspace == AUDIOSYNC_CUDA_DEVICE) {
         cudaPointerAttributes at;

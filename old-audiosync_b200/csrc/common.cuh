@@ -5,6 +5,7 @@
 #include <stdint.h>
 #include <stddef.h>
 #include <math.h>
+#include <type_traits>
 
 #include "../../include/audiosync_cuda.h"
 
@@ -104,6 +105,32 @@ __host__ __device__ __forceinline__ float pair_second(const PairPeak& p) {
     float s = p.second_bits != 0u ? float_from_order_bits(p.second_bits) : 0.0f;
     if (p.seed_bits != 0u && argmax_key_index(p.key) != 0u) s = fmaxf(s, float_from_order_bits(p.seed_bits));
     return s;
+}
+
+// Lag window of the batch calls (audiosync_cuda_set_lag_window) as the raw indices it allows:
+// [lo0, lo0 + n0) and [lo1, lo1 + n1) of [0, 2L), lo0 the lowest allowed index (n1 = 0: one range).
+struct RawWindow {
+    uint32_t lo0, n0, lo1, n1;
+    __host__ __device__ __forceinline__ bool allows(uint32_t i) const { return i - lo0 < n0 || i - lo1 < n1; }
+};
+// the unwindowed kernels' (empty) window parameter
+struct NoWindow {};
+
+// Effective window [max(lo, -L), min(hi, L - 1)] of folded lags as raw ranges: raw = lag for lag >= 0,
+// lag + 2L below.  Returns -1 when it is empty, 0 when it is all of [-L, L - 1] (the unwindowed call),
+// 1 otherwise (*w filled, *elo / *ehi the effective lags).
+__host__ __device__ __forceinline__ int raw_window_of(long long lo, long long hi, long long L, RawWindow* w,
+                                                      long long* elo = nullptr, long long* ehi = nullptr) {
+    if (lo < -L) lo = -L;
+    if (hi > L - 1) hi = L - 1;
+    if (lo > hi) return -1;
+    if (elo) *elo = lo;
+    if (ehi) *ehi = hi;
+    if (lo == -L && hi == L - 1) return 0;
+    if (lo >= 0) *w = RawWindow{(uint32_t)lo, (uint32_t)(hi - lo + 1), 0u, 0u};
+    else if (hi < 0) *w = RawWindow{(uint32_t)(lo + 2 * L), (uint32_t)(hi - lo + 1), 0u, 0u};
+    else *w = RawWindow{0u, (uint32_t)(hi + 1), (uint32_t)(lo + 2 * L), (uint32_t)(-lo)};
+    return 1;
 }
 
 // Fold of src/cross_correlation.c:256-271.  Window = x[xoff .. xoff+n) of the

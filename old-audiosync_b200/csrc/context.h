@@ -195,6 +195,7 @@ struct audiosync_cuda_ctx {
     int wave_pairs = 0;
     bool precise = false;     // fp64 ARITHMETIC in the transforms (validation mode)
     int weighting = AUDIOSYNC_CUDA_WEIGHT_NONE;   // AUDIOSYNC_CUDA_WEIGHT_*: cross-spectrum weighting of the batch calls
+    long long lag_lo = INT64_MIN, lag_hi = INT64_MAX;   // lag window of the batch calls (folded lags, inclusive)
     int narrow_host = 1;      // AUDIOSYNC_CUDA_NARROW_*: f64 HOST batches converted to fp32 on the host while staged
     bool profile = false;
     std::atomic<uint64_t> launches{0};

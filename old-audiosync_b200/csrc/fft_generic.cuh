@@ -555,7 +555,9 @@ struct GenRowFusedKernel {
 // Inverse column pass.  fp32: |r| argmax epilogue over the indices < limit (= 2L), the correlation
 // is never written.  fp64: r[0 .. limit) is written to `r_out` (the dead sample plane) and resolved
 // by argmax_f64_kernel, which keeps full double keys.  grid = (pairs, ceil(M2 / CT)).
-template <typename T, int CT_ = GenTraits<T>::CT, int NT_ = GEN_THREADS>
+// WIN (fp32 only): the windowed twin -- the raw indices Params::win allows take the place of
+// [0, limit); fp64 plans apply the window in argmax_f64_window_kernel instead.
+template <typename T, int CT_ = GenTraits<T>::CT, int NT_ = GEN_THREADS, bool WIN = false>
 struct GenColInvKernel {
     typedef typename GenTraits<T>::C C;
     static constexpr int CT = CT_;
@@ -570,7 +572,9 @@ struct GenColInvKernel {
         const int* p2f_col;
         GenShape sh;
         T* r_out;                // fp64 only: [pair][2M] reals (aliases plane 1 of the pair)
+        [[no_unique_address]] std::conditional_t<WIN, RawWindow, NoWindow> win;   // WIN only
     };
+    static_assert(!WIN || sizeof(T) == 4, "fp64 plans window in argmax_f64_window_kernel");
     static size_t smem_bytes(const GenShape& sh) {
         const size_t tile = (size_t)sh.M1 * CT * sizeof(C);
         return (tile > 512 ? tile : 512) + 16;
@@ -650,6 +654,35 @@ struct GenColInvKernel {
                         for (int bf = tid / CT; bf < nbf; bf += TR) {
                             C v[R];
                             const unsigned i_first = butterfly(bf, c, n2, v);
+                            if constexpr (WIN) {
+                                // the threshold test sees allowed outputs only (see ColInvKernel): the
+                                // unmasked bound rejects first (it is the cheap test), then the allowed
+                                // outputs are tested; the butterfly of the lowest allowed index always
+                                // takes the exact path
+                                const unsigned step = 2u * Wt * (unsigned)M2;
+                                const bool has_floor = p.win.lo0 - i_first < (unsigned)R * step &&
+                                                       (p.win.lo0 - i_first) % step < 2u;
+                                if (!has_floor) {
+                                    float gm = fmaxf(fabsf(v[0].x), fabsf(v[0].y));
+                                    static_for<1, R>([&](auto K) { gm = fmaxf(gm, fmaxf(fabsf(v[decltype(K)::value].x), fabsf(v[decltype(K)::value].y))); });
+                                    if (!(gm >= acc.thr)) continue;
+                                    gm = -1.0f;
+                                    static_for<0, R>([&](auto K) {
+                                        constexpr int k = decltype(K)::value;
+                                        const unsigned i_re = i_first + (unsigned)k * step;
+                                        if (p.win.allows(i_re)) gm = fmaxf(gm, fabsf(v[k].x));
+                                        if (p.win.allows(i_re + 1u)) gm = fmaxf(gm, fabsf(v[k].y));
+                                    });
+                                    if (!(gm >= acc.thr)) continue;
+                                }
+                                static_for<0, R>([&](auto K) {
+                                    constexpr int k = decltype(K)::value;
+                                    const unsigned i_re = i_first + 2u * (unsigned)k * Wt * (unsigned)M2;
+                                    acc.consider_win(v[k].x, i_re, p.win, &p.peaks[pair]);
+                                    acc.consider_win(v[k].y, i_re + 1u, p.win, &p.peaks[pair]);
+                                });
+                                continue;
+                            }
                             // only values that reach the running second peak can matter
                             float gm = fmaxf(fabsf(v[0].x), fabsf(v[0].y));
                             static_for<1, R>([&](auto K) { gm = fmaxf(gm, fmaxf(fabsf(v[decltype(K)::value].x), fabsf(v[decltype(K)::value].y))); });

@@ -134,6 +134,19 @@ struct ArgmaxAcc {
         update(argmax_key_seed(v), 0.0f);
         pk->seed_bits = float_order_bits(fabsf(v));
     }
+    // Windowed twins: only allowed indices compete.  Raw 0 is the seed when the window allows it;
+    // otherwise the lowest allowed index always enters, past the threshold: a NaN there gets the
+    // lowest real key (argmax_key_abs maps it to 0 high bits), below every number, so when no
+    // allowed value is a number the pair resolves to that index with a NaN peak, as a NaN seed does.
+    // A NaN's magnitude never joins `second` (fmaxf drops it).
+    ASC_HD void consider_win(float v, uint32_t index, const RawWindow& w, PairPeak* pk) {
+        if (index == w.lo0) {
+            if (index == 0u) consider_seed(v, pk);
+            else update(argmax_key_abs(v, index), fabsf(v));
+        } else if (w.allows(index)) {
+            consider(v, index);
+        }
+    }
     // bound for the warp's threshold: the seed's magnitude is none (see above)
     ASC_HD float best_mag() const { return best != 0ull && !argmax_key_is_seed(best) ? argmax_key_mag(best) : 0.0f; }
     ASC_HD ArgmaxPair result() const { ArgmaxPair r; r.best = best; r.second = second; return r; }
@@ -416,7 +429,9 @@ struct ColFwdKernel {
 // The tile is staged with boxes of a tensor map over plane 0 (rows 0 .. M1-2; the last row and
 // the mbarrier as in ColFwdKernel).  TMA staging is the only path; the TMA parameter is kept,
 // fixed to true, so that callers which name ColInvKernel<..., true> (tests/emu) keep building.
-template <class RL, int M2_, int NT, bool TMA = true>
+// WIN: the windowed twin (audiosync_cuda_set_lag_window): only the raw indices Params::win allows
+// compete, and only they raise the threshold (see the epilogue).
+template <class RL, int M2_, int NT, bool TMA = true, bool WIN = false>
 struct ColInvKernel {
     static_assert(TMA, "K_C's tiles are always staged by the TMA unit");
     static constexpr int M1 = RL::n;
@@ -434,6 +449,8 @@ struct ColInvKernel {
         PairPeak* peaks;         // [pair]
         const cplx* tw;          // RL pass tables (forward sign; conjugated here)
         long long L;
+        // WIN only; it sits in the padding before the 64-byte aligned map, so the size is the same
+        [[no_unique_address]] std::conditional_t<WIN, RawWindow, NoWindow> win;
         CUtensorMap tm;          // [2 * pair][M1 rows][2*M2 floats] view of the planes
     };
     static constexpr int TMA_ROWS = M1 - 1;
@@ -525,6 +542,13 @@ struct ColInvKernel {
                     if (seen != 0u) acc.thr = float_from_order_bits(seen);
                     const int c = tid & (COL_T - 1);
                     const bool col0 = (c0 + c) == 0;
+                    // WIN: the column and row n1 of the packed point of the lowest allowed index
+                    [[maybe_unused]] bool floor_col = false;
+                    [[maybe_unused]] int floor_n1 = 0;
+                    if constexpr (WIN) {
+                        floor_col = (p.win.lo0 >> 1) % (uint32_t)M2 == (uint32_t)(c0 + c);
+                        floor_n1 = (int)((p.win.lo0 >> 1) / (uint32_t)M2);
+                    }
                     for (int w0 = 0; w0 < items; w0 += NT) {      // warp-uniform trip count
                         const int w = w0 + tid;
                         const bool act = w < items;
@@ -536,13 +560,46 @@ struct ColInvKernel {
                             v[q] = buf[(i0 + q) * COL_T + c];
                         });
                         dft_reg<R, +1>(v);
-                        float gm = fmaxf(fabsf(v[0].x), fabsf(v[0].y));
-                        static_for<1, R>([&](auto K) {
-                            constexpr int k = decltype(K)::value;
-                            gm = fmaxf(gm, fmaxf(fabsf(v[k].x), fabsf(v[k].y)));
-                        });
-                        const bool has_seed = col0 && i0 == 0;      // r[0]: signed seed, exact path always
-                        const bool need = act && (gm >= acc.thr || has_seed);
+                        const bool has_seed = col0 && i0 == 0;          // r[0]: signed seed, exact path always
+                        bool need;
+                        if constexpr (WIN) {
+                            // the threshold test sees allowed outputs only: an excluded value that
+                            // passed it could never raise the threshold, and a window without the
+                            // global peak would send the warp down the exact path again and again.
+                            // The unmasked bound rejects first (the sibling's cheap test); survivors
+                            // are tested on their allowed outputs.  The butterfly of the lowest
+                            // allowed index always takes the exact path.
+                            float gm = fmaxf(fabsf(v[0].x), fabsf(v[0].y));
+                            static_for<1, R>([&](auto K) {
+                                constexpr int k = decltype(K)::value;
+                                gm = fmaxf(gm, fmaxf(fabsf(v[k].x), fabsf(v[k].y)));
+                            });
+                            bool has_floor = false;
+                            if (floor_col) {
+                                const int f0 = RL::freq_of_pos(i0);
+                                static_for<0, R>([&](auto K) { has_floor |= f0 + decltype(K)::value * Wt == floor_n1; });
+                            }
+                            bool pass = gm >= acc.thr;
+                            if (pass && !has_floor) {
+                                const int f0 = RL::freq_of_pos(i0);
+                                gm = -1.0f;
+                                static_for<0, R>([&](auto K) {
+                                    constexpr int k = decltype(K)::value;
+                                    const uint32_t i_re = 2u * ((uint32_t)(f0 + k * Wt) * (uint32_t)M2 + (uint32_t)(c0 + c));
+                                    if (p.win.allows(i_re)) gm = fmaxf(gm, fabsf(v[k].x));
+                                    if (p.win.allows(i_re + 1u)) gm = fmaxf(gm, fabsf(v[k].y));
+                                });
+                                pass = gm >= acc.thr;
+                            }
+                            need = act && (pass || has_floor);
+                        } else {
+                            float gm = fmaxf(fabsf(v[0].x), fabsf(v[0].y));
+                            static_for<1, R>([&](auto K) {
+                                constexpr int k = decltype(K)::value;
+                                gm = fmaxf(gm, fmaxf(fabsf(v[k].x), fabsf(v[k].y)));
+                            });
+                            need = act && (gm >= acc.thr || has_seed);
+                        }
                         if (ex.any(need)) {
                             if (need) {
                                 const int f0 = RL::freq_of_pos(i0);
@@ -550,9 +607,14 @@ struct ColInvKernel {
                                     constexpr int k = decltype(K)::value;
                                     const int n1 = f0 + k * Wt;
                                     const uint32_t i_re = 2u * ((uint32_t)n1 * (uint32_t)M2 + (uint32_t)(c0 + c));
-                                    if (has_seed && n1 == 0) acc.consider_seed(v[k].x, &p.peaks[pair]);
-                                    else acc.consider(v[k].x, i_re);
-                                    acc.consider(v[k].y, i_re + 1u);
+                                    if constexpr (WIN) {
+                                        acc.consider_win(v[k].x, i_re, p.win, &p.peaks[pair]);
+                                        acc.consider_win(v[k].y, i_re + 1u, p.win, &p.peaks[pair]);
+                                    } else {
+                                        if (has_seed && n1 == 0) acc.consider_seed(v[k].x, &p.peaks[pair]);
+                                        else acc.consider(v[k].x, i_re);
+                                        acc.consider(v[k].y, i_re + 1u);
+                                    }
                                 });
                             }
                             acc.thr = fmaxf(acc.thr, ex.warp_second(acc.best_mag(), acc.second));

@@ -36,7 +36,8 @@ ASC_HD int small_pos_of_freq(const SmallPlan& pl, int k) {
 }
 
 // PHAT: the split step whitens the spectra (split_phat_merge); w is wn[k] as for the product.
-template <typename InT, bool PHAT = false>
+// WIN: the windowed twin -- only the raw indices Params::win allows compete (ArgmaxAcc::consider_win).
+template <typename InT, bool PHAT = false, bool WIN = false>
 struct SmallXcorrKernel {
     static constexpr int THREADS = SMALL_THREADS;
 
@@ -50,6 +51,7 @@ struct SmallXcorrKernel {
         long long src_pitch;  // elements between consecutive pairs; 0 = packed (2M / M)
         long long smp_pitch;
         int vec_src, vec_smp; // one load per packed point (every pair's base is aligned to two elements)
+        [[no_unique_address]] std::conditional_t<WIN, RawWindow, NoWindow> win;   // WIN only
     };
     // two rows of M points + 512 bytes of reduction scratch (phase_argmax needs 392)
     static size_t smem_bytes(int M) { return (size_t)2 * M * sizeof(cplx) + 512; }
@@ -141,9 +143,14 @@ struct SmallXcorrKernel {
                 for (int n = tid; n < M; n += THREADS) {
                     const cplx v = buf[n];
                     const uint32_t i_re = (uint32_t)(2 * n);
-                    if (n == 0) acc.consider_seed(v.x, &p.peaks[pair]);
-                    else acc.consider(v.x, i_re);
-                    acc.consider(v.y, i_re + 1u);
+                    if constexpr (WIN) {
+                        acc.consider_win(v.x, i_re, p.win, &p.peaks[pair]);
+                        acc.consider_win(v.y, i_re + 1u, p.win, &p.peaks[pair]);
+                    } else {
+                        if (n == 0) acc.consider_seed(v.x, &p.peaks[pair]);
+                        else acc.consider(v.x, i_re);
+                        acc.consider(v.y, i_re + 1u);
+                    }
                 }
                 return acc.result();
             },

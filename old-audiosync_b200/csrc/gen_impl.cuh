@@ -22,6 +22,13 @@ static int prepare_gen_kernel(size_t smem) {
     return 0;
 }
 
+// the windowed twin of the fp32 inverse column kernel (fp64 plans window in argmax_f64_window_kernel)
+template <typename T, int CT, int NT>
+static int prepare_col_inv_window(const GenShape& sh) {
+    if constexpr (sizeof(T) == 4) return prepare_gen_kernel<GenColInvKernel<T, CT, NT, true>>(GenColInvKernel<T, CT, NT, true>::smem_bytes(sh));
+    return 0;
+}
+
 // fp32 arithmetic has 16- and 8-column tiles, fp64 only 8
 template <typename T, class F>
 static int gen_for_tile_width(int ct, F&& f) {
@@ -38,7 +45,8 @@ int GenStage<T, NT>::prepare_cols(const GenShape& sh) {
         return prepare_gen_kernel<GenColFwdKernel<T, float, CT, NT>>(GenColFwdKernel<T, float, CT, NT>::smem_bytes(sh)) != 0 ||
                prepare_gen_kernel<GenColFwdKernel<T, double, CT, NT>>(GenColFwdKernel<T, double, CT, NT>::smem_bytes(sh)) != 0 ||
                prepare_gen_kernel<GenColFwdKernel<T, int16_t, CT, NT>>(GenColFwdKernel<T, int16_t, CT, NT>::smem_bytes(sh)) != 0 ||
-               prepare_gen_kernel<GenColInvKernel<T, CT, NT>>(GenColInvKernel<T, CT, NT>::smem_bytes(sh)) != 0 ? -1 : 0;
+               prepare_gen_kernel<GenColInvKernel<T, CT, NT>>(GenColInvKernel<T, CT, NT>::smem_bytes(sh)) != 0 ||
+               prepare_col_inv_window<T, CT, NT>(sh) != 0 ? -1 : 0;
     });
 }
 
@@ -100,25 +108,34 @@ int GenStage<T, NT>::rows(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d
 
 template <typename T, int NT>
 int GenStage<T, NT>::col_inv(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, PairPeak* peaks, int pairs,
-                             cudaStream_t st) {
+                             cudaStream_t st, const RawWindow* win) {
     typedef typename GenTraits<T>::C C;
     const GenShape& sh = plan->gen;
     C* planes = static_cast<C*>(ws);
     const int rc = gen_for_tile_width<T>(sh.ct, [&](auto CTC) -> int {
-        using K = GenColInvKernel<T, decltype(CTC)::value, NT>;
-        typename K::Params p{planes, peaks, static_cast<const C*>(plan->g_wcol.p), static_cast<const int*>(plan->g_p2f_col.p),
-                             sh, reinterpret_cast<T*>(planes)};
-        const dim3 grid(pairs, (sh.M2 + K::CT - 1) / K::CT, 1);
-        return launch(ctx, d, KC_COL_INV, st, [&] {
-            launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), st, p);
-        });
+        auto go = [&](auto KK, auto fill) -> int {
+            using K = decltype(KK);
+            typename K::Params p{planes, peaks, static_cast<const C*>(plan->g_wcol.p), static_cast<const int*>(plan->g_p2f_col.p),
+                                 sh, reinterpret_cast<T*>(planes)};
+            fill(p);
+            const dim3 grid(pairs, (sh.M2 + K::CT - 1) / K::CT, 1);
+            return launch(ctx, d, KC_COL_INV, st, [&] {
+                launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), st, p);
+            });
+        };
+        constexpr int CT = decltype(CTC)::value;
+        if constexpr (sizeof(T) == 4) {
+            if (win) return go(GenColInvKernel<T, CT, NT, true>{}, [&](auto& p) { p.win = *win; });
+        }
+        return go(GenColInvKernel<T, CT, NT>{}, [](auto&) {});
     });
     if (rc != 0) return -1;
     if constexpr (sizeof(T) == 8) {
         // fp64: r[0 .. 2L) of pair i sits in its (dead) sample plane; full double keys
         const double* r = reinterpret_cast<const double*>(planes) + 2 * sh.M;
         return launch(ctx, d, KC_ARGMAX_F64, st, [&] {
-            argmax_f64_kernel<<<pairs, 1024, 0, st>>>(r, 2 * sh.L, 4 * sh.M, peaks);
+            if (win) argmax_f64_window_kernel<<<pairs, 1024, 0, st>>>(r, 2 * sh.L, 4 * sh.M, peaks, *win);
+            else argmax_f64_kernel<<<pairs, 1024, 0, st>>>(r, 2 * sh.L, 4 * sh.M, peaks);
         });
     }
     return 0;

@@ -38,9 +38,10 @@ struct FftPlan {
     DevBuf phat_rev, phat_lo, phat_hi;               // its twiddle w = W_N^k1 * phat_rev[e] (row kernel's position order)
     double peak_scale = 1.0;                         // r_reference = r_kernel * peak_scale
     // enqueues the transform kernels for `pairs` pairs (planes/r in ws)
-    // (src, smp, dtype, src_pitch, smp_pitch [elements between pairs], workspace, peaks, pairs, stream)
+    // (src, smp, dtype, src_pitch, smp_pitch [elements between pairs], workspace, peaks, pairs, stream,
+    //  lag window: nullptr for the unwindowed kernels, else the windowed twins of the argmax step)
     std::function<int(audiosync_cuda_ctx*, DeviceState&, const void*, const void*, int, long long, long long,
-                      void*, PairPeak*, int, cudaStream_t)> run_wave;
+                      void*, PairPeak*, int, cudaStream_t, const RawWindow*)> run_wave;
     ~FftPlan() {
         col_tw.release(); col_tc.release(); row_tw.release(); row_rev.release(); row_tab.release(); m_lo.release(); m_hi.release();
         wm.release(); wn.release();
@@ -154,7 +155,7 @@ struct GenStage {
                        long long sp, long long mp, void* ws, PairPeak* peaks, int pairs, cudaStream_t st);
     static int rows(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st);
     static int col_inv(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, PairPeak* peaks, int pairs,
-                       cudaStream_t st);
+                       cudaStream_t st, const RawWindow* win);
 };
 
 // static_rows.cu: the rows of a runtime-radix fp32 plan on a static row kernel (RowFusedKernel<RL, 0, NT>)

@@ -153,6 +153,55 @@ argmax_f64_kernel(const double* __restrict__ r, long long N, long long pitch, Pa
     }
 }
 
+// The windowed twin (audiosync_cuda_set_lag_window): only the indices `win` allows are read, and
+// i == 0 is the seed only when it is one of them.  A NaN candidate (ninf) still beats the sentinel
+// on index order, so when no allowed value is a number the lowest allowed index is the answer with
+// its NaN value, as a NaN seed is.  The rest is argmax_f64_kernel's (kept apart so that its code is
+// unchanged).
+static __global__ void __launch_bounds__(1024)
+argmax_f64_window_kernel(const double* __restrict__ r, long long N, long long pitch, PairPeak* __restrict__ peaks,
+                         RawWindow win)
+{
+    (void)N;
+    __shared__ KeyF64 s_k[32];
+    const double* rp = r + (size_t)blockIdx.x * (size_t)pitch;
+    const double ninf = -INFINITY, pinf = INFINITY;
+    KeyF64 best; best.v = ninf; best.i = 0x7fffffffffffffffLL; best.a = 0.0; best.s = 0.0;
+    for (int g = 0; g < 2; g++) {
+        const long long beg = g ? win.lo1 : win.lo0;
+        const long long end = beg + (g ? win.n1 : win.n0);
+        for (long long i = beg + threadIdx.x; i < end; i += blockDim.x) {
+            const double x = rp[i];
+            KeyF64 c;
+            c.i = i;
+            const double a = fabs(x);
+            c.a = (a != a) ? 0.0 : a;
+            c.s = 0.0;
+            if (i == 0) c.v = (x != x) ? pinf : x;
+            else c.v = (a != a) ? ninf : a;
+            best = key_better(best, c);
+        }
+    }
+    for (int o = 16; o > 0; o >>= 1) best = key_better(best, key_shfl_xor(best, o));
+    const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+    if (l == 0) s_k[w] = best;
+    __syncthreads();
+    if (w == 0) {
+        const int nw = (blockDim.x + 31) >> 5;
+        if (l < nw) best = s_k[l];
+        else { best.v = ninf; best.i = 0x7fffffffffffffffLL; best.a = 0.0; best.s = 0.0; }
+        for (int o = 16; o > 0; o >>= 1) best = key_better(best, key_shfl_xor(best, o));
+        if (l == 0) {
+            PairPeak p = cleared_peak();
+            p.raw_index = best.i;
+            p.peak = rp[best.i];
+            p.second = best.s;
+            p.resolved = 1;
+            peaks[blockIdx.x] = p;
+        }
+    }
+}
+
 // ---------------------------------------------------------------------------
 // Pearson coefficient of the aligned windows (reference
 // src/cross_correlation.c:74-116 on the windows of :256-271).

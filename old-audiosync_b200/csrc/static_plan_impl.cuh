@@ -9,7 +9,8 @@ namespace asc {
 template <class P>
 static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d,
                            const void* src, const void* smp, int dtype, long long src_pitch,
-                           long long smp_pitch, void* ws, PairPeak* peaks, int pairs, cudaStream_t st) {
+                           long long smp_pitch, void* ws, PairPeak* peaks, int pairs, cudaStream_t st,
+                           const RawWindow* win) {
     using Col = typename P::Col;
     using Row = typename P::Row;
     constexpr int M1 = Col::n, M2 = Row::n;
@@ -93,9 +94,15 @@ static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& 
     }
     {
         const dim3 grid(pairs, M2 / COL_T, 1);
-        if (launch(ctx, d, KC_COL_INV, st, [&] {
-                launch_stage(fft_kernel_entry<KC>, grid, dim3(KC::THREADS), KC::SMEM, st, pc);
-            }) != 0) return -1;
+        if (win) {
+            using KCW = ColInvKernel<Col, Row::n, P::NT_COL, true, true>;
+            typename KCW::Params pw{planes, peaks, col_tw, P::L, *win, pc.tm};
+            if (launch(ctx, d, KC_COL_INV, st, [&] {
+                    launch_stage(fft_kernel_entry<KCW>, grid, dim3(KCW::THREADS), KCW::SMEM, st, pw);
+                }) != 0) return -1;
+        } else if (launch(ctx, d, KC_COL_INV, st, [&] {
+                       launch_stage(fft_kernel_entry<KC>, grid, dim3(KC::THREADS), KC::SMEM, st, pc);
+                   }) != 0) return -1;
     }
     return 0;
 }
@@ -140,14 +147,16 @@ int build_static_plan(FftPlan* plan) {
     using KB = RowFusedKernel<Row, Col::n, P::NT_ROW>;
     using KBP = RowFusedKernel<Row, Col::n, P::NT_ROW, true>;
     using KC = ColInvKernel<Col, Row::n, P::NT_COL>;
+    using KCW = ColInvKernel<Col, Row::n, P::NT_COL, true, true>;
     if (prepare_kernel<KT>(KT::SMEM) != 0 || prepare_kernel<KR>(KR::SMEM) != 0 || prepare_kernel<KD>(KD::SMEM) != 0 ||
         prepare_kernel<KS>(KS::SMEM) != 0 ||
-        (plan->phat ? prepare_kernel<KBP>(KBP::SMEM) : prepare_kernel<KB>(KB::SMEM)) != 0 || prepare_kernel<KC>(KC::SMEM) != 0)
+        (plan->phat ? prepare_kernel<KBP>(KBP::SMEM) : prepare_kernel<KB>(KB::SMEM)) != 0 || prepare_kernel<KC>(KC::SMEM) != 0 ||
+        prepare_kernel<KCW>(KCW::SMEM) != 0)
         return -1;
     plan->run_wave = [plan](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
                             int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,
-                            cudaStream_t st) {
-        return run_static_wave<P>(plan, ctx, d, src, smp, dtype, sp, mp, ws, peaks, pairs, st);
+                            cudaStream_t st, const RawWindow* win) {
+        return run_static_wave<P>(plan, ctx, d, src, smp, dtype, sp, mp, ws, peaks, pairs, st, win);
     };
     return 0;
 }
