@@ -203,6 +203,32 @@ int audiosync_cuda_xcorr_batch_device(audiosync_cuda_ctx *ctx, int device,
                                       size_t n_pairs, size_t sample_len, int dtype,
                                       audiosync_cuda_result *d_results, void *stream);
 
+/* One source against n_pairs samples: record i is, bit for bit in every field, what
+ * audiosync_cuda_xcorr_batch_results returns for the pair (source, samples[i]) with the source
+ * replicated n_pairs times.  source: 2*sample_len elements; samples: [n_pairs][sample_len].
+ * For many recordings synced to one master track, or one track against every interval of a long
+ * recording: the source is passed, uploaded and (on the six static lengths) transformed once per
+ * call and device instead of once per pair.
+ *   Every dtype (F32, F64, S16), with the batch calls' alignment rule: any base aligned to its
+ *   element; an unaligned device base returns -1 before anything is launched.
+ *   Every context setting applies: path, precise mode, weighting (PHAT, with the same refusals), lag
+ *   window and wave size.
+ *   HOST: pairs are split over the context's devices as in xcorr_batch; the source is uploaded once
+ *   per device and only the samples are chunked.  Host narrowing does not apply: an F64 HOST call
+ *   equals the replicated call with NARROW_OFF (under the default LOSSLESS mode, the same records).
+ *   DEVICE: both pointers live on one device of the context; no copies.
+ *   n_pairs == 0 returns 0 and launches nothing.  results: host array of n_pairs records.
+ * The static plans compute the source's forward transform once per call and device (kernel class
+ * "src_spectrum" of the profile API) and feed it to every pair's split step; every other plan reads
+ * the one source in every pair's transform. */
+int audiosync_cuda_xcorr_shared_source(audiosync_cuda_ctx *ctx, const void *source, const void *samples,
+                                       size_t n_pairs, size_t sample_len, int dtype, int memspace,
+                                       audiosync_cuda_result *results);
+/* Stream-ordered form on device pointers of one device of the context (as xcorr_batch_device). */
+int audiosync_cuda_xcorr_shared_source_device(audiosync_cuda_ctx *ctx, int device, const void *d_source,
+                                              const void *d_samples, size_t n_pairs, size_t sample_len,
+                                              int dtype, audiosync_cuda_result *d_results, void *stream);
+
 /* ------------------------------------------------------------------------
  * Session pool (SURVEY 8f rank 1): many concurrent audiosync sessions on one device.
  * Each slot owns device-resident source / sample buffers that grow as audio arrives

@@ -51,6 +51,7 @@ EXPORTED_SYMBOLS = [
     "fftw_malloc", "fftw_alloc_real", "fftw_alloc_complex", "fftw_free",
     "audiosync_cuda_create", "audiosync_cuda_destroy", "audiosync_cuda_device_count",
     "audiosync_cuda_xcorr_batch", "audiosync_cuda_xcorr_batch_results", "audiosync_cuda_xcorr_batch_device",
+    "audiosync_cuda_xcorr_shared_source", "audiosync_cuda_xcorr_shared_source_device",
     "audiosync_cuda_synth_pairs", "audiosync_cuda_synchronize",
     "audiosync_cuda_set_path", "audiosync_cuda_set_wave_pairs", "audiosync_cuda_set_debug", "audiosync_cuda_set_precise", "audiosync_cuda_set_weighting",
     "audiosync_cuda_set_lag_window",
@@ -113,6 +114,10 @@ def lib() -> C.CDLL:
     L.audiosync_cuda_xcorr_batch_results.argtypes = [vp, vp, vp, sz, sz, i32, i32, vp]
     L.audiosync_cuda_xcorr_batch_device.restype = i32
     L.audiosync_cuda_xcorr_batch_device.argtypes = [vp, i32, vp, vp, sz, sz, i32, vp, vp]
+    L.audiosync_cuda_xcorr_shared_source.restype = i32
+    L.audiosync_cuda_xcorr_shared_source.argtypes = [vp, vp, vp, sz, sz, i32, i32, vp]
+    L.audiosync_cuda_xcorr_shared_source_device.restype = i32
+    L.audiosync_cuda_xcorr_shared_source_device.argtypes = [vp, i32, vp, vp, sz, sz, i32, vp, vp]
     L.audiosync_cuda_synth_pairs.restype = i32
     L.audiosync_cuda_synth_pairs.argtypes = [vp, i32, u64, u64, sz, sz, i32, vp, vp, vp]
     L.audiosync_cuda_synchronize.restype = i32
@@ -513,6 +518,57 @@ class Context:
         self._check(rc, "xcorr_batch_results")
         return res
 
+    def xcorr_shared_source(self, source: np.ndarray, samples: np.ndarray) -> np.ndarray:
+        """One source against many samples: ``source`` 1-D with at least 2L elements (only [0, 2L) is
+        read), ``samples`` [n][L], both float32, float64 or int16 (S16) host arrays.  Record i is, bit
+        for bit, the ``xcorr_batch_records`` record of (source, samples[i]) with the source replicated
+        (see include/audiosync_cuda.h); the source is uploaded and transformed once per device."""
+        if source.dtype != samples.dtype or source.dtype not in _NP_DTYPES:
+            raise TypeError("source/samples must both be float32, float64 or int16")
+        if source.ndim != 1 or samples.ndim != 2 or source.shape[0] < 2 * samples.shape[1]:
+            raise ValueError("expected source [>= 2L] and samples [n][L]")
+        n, L = samples.shape
+        source = np.ascontiguousarray(source[: 2 * L])
+        samples = np.ascontiguousarray(samples)
+        res = np.zeros(n, RESULT_DTYPE)
+        rc = lib().audiosync_cuda_xcorr_shared_source(self._h, source.ctypes.data, samples.ctypes.data, n, L,
+                                                      _NP_DTYPES[source.dtype], HOST, res.ctypes.data)
+        self._check(rc, "xcorr_shared_source")
+        return res
+
+    def xcorr_shared_source_torch(self, source, samples, out=None, sync: bool = True):
+        """``xcorr_shared_source`` on torch CUDA tensors, zero copy: ``source`` 1-D (at least 2L
+        elements, [0, 2L) is read) and ``samples`` [n, L] of one dtype on one device of this context,
+        enqueued on torch's current stream; ``out`` and ``sync`` as in ``xcorr_batch_torch``."""
+        import torch
+        if not (source.is_cuda and samples.is_cuda) or source.device != samples.device:
+            raise ValueError("source and samples must be CUDA tensors on the same device")
+        dts = {torch.float32: F32, torch.float64: F64, torch.int16: S16}
+        if source.dtype != samples.dtype or source.dtype not in dts:
+            raise TypeError("source/samples must both be float32, float64 or int16")
+        if source.dim() != 1 or samples.dim() != 2 or source.shape[0] < 2 * samples.shape[1]:
+            raise ValueError("expected source [>= 2L] and samples [n, L]")
+        if not (source.is_contiguous() and samples.is_contiguous()):
+            raise ValueError("tensors must be contiguous (no hidden copies on this path)")
+        n, L = samples.shape
+        dev = source.device
+        if out is None:
+            out = torch.empty(n * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev)
+        elif out.device != dev or out.dtype != torch.uint8 or out.numel() < n * RESULT_DTYPE.itemsize:
+            raise ValueError("out must be a uint8 tensor of n * 64 bytes on the same device")
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        if stream == 0:
+            # as in xcorr_batch_torch: a NULL handle selects the library's own stream
+            torch.cuda.current_stream(dev).synchronize()
+        if n:
+            self.xcorr_shared_source_device(dev.index, source.data_ptr(), samples.data_ptr(), n, L, dts[source.dtype],
+                                            out.data_ptr(), stream)
+        if stream == 0:
+            self.synchronize(dev.index)
+        if not sync:
+            return out
+        return out[: n * RESULT_DTYPE.itemsize].cpu().numpy().view(RESULT_DTYPE)
+
     def xcorr_batch_torch(self, sources, samples, out=None, sync: bool = True):
         """Zero-copy batch call on torch CUDA tensors (SURVEY 8f rank 3).
 
@@ -562,6 +618,13 @@ class Context:
         rc = lib().audiosync_cuda_xcorr_batch_device(self._h, device, d_sources, d_samples, n_pairs,
                                                      sample_len, dtype, d_results, stream or None)
         self._check(rc, "xcorr_batch_device")
+
+    def xcorr_shared_source_device(self, device: int, d_source: int, d_samples: int, n_pairs: int,
+                                   sample_len: int, dtype: int, d_results: int, stream: int = 0):
+        """Stream-ordered shared-source call on device pointers; dtype F32, F64 or S16."""
+        rc = lib().audiosync_cuda_xcorr_shared_source_device(self._h, device, d_source, d_samples, n_pairs,
+                                                             sample_len, dtype, d_results, stream or None)
+        self._check(rc, "xcorr_shared_source_device")
 
     def synth_pairs(self, device: int, seed: int, first_pair: int, n_pairs: int, sample_len: int,
                     dtype: int, d_sources: int, d_samples: int, stream: int = 0):

@@ -55,7 +55,7 @@ static bool debug_on() { return g_debug_flag || (&global_debug != nullptr && glo
 const char* kernel_class_name(int k) {
     static const char* names[KC_COUNT] = {
         "synth", "direct_corr", "argmax_f64", "col_fwd", "row_fused",
-        "col_inv_argmax", "small_fft", "pearson"};
+        "col_inv_argmax", "small_fft", "pearson", "src_spectrum"};
     return (k >= 0 && k < KC_COUNT) ? names[k] : "?";
 }
 
@@ -87,20 +87,24 @@ template <typename InT, bool PHAT, bool WIN>
 static int run_small_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src,
                           const void* smp, long long sp, long long mp, PairPeak* peaks, int pairs,
                           cudaStream_t st, const RawWindow* win) {
-    using K = SmallXcorrKernel<InT, PHAT, WIN>;
-    // one load per packed point where every pair's base is aligned to two elements
-    const size_t al = 2 * sizeof(InT);
-    const int vec_src = reinterpret_cast<uintptr_t>(src) % al == 0 && sp % 2 == 0;
-    const int vec_smp = reinterpret_cast<uintptr_t>(smp) % al == 0 && mp % 2 == 0;
-    typename K::Params p{static_cast<const InT*>(src), static_cast<const InT*>(smp), peaks,
-                         static_cast<const cplx*>(plan->wm.p), static_cast<const cplx*>(plan->wn.p),
-                         plan->small, sp, mp, vec_src, vec_smp};
-    if constexpr (WIN) p.win = *win;
-    const size_t smem = K::smem_bytes(plan->small.M);
-    const dim3 grid(1, 1, pairs);
-    return launch(ctx, d, KC_SMALL_FFT, st, [&] {
-        fft_kernel_entry<K><<<grid, K::THREADS, smem, st>>>(p);
-    });
+    auto go = [&](auto KK) -> int {
+        using K = decltype(KK);
+        // one load per packed point where every pair's base is aligned to two elements
+        const size_t al = 2 * sizeof(InT);
+        const int vec_src = reinterpret_cast<uintptr_t>(src) % al == 0 && sp % 2 == 0;
+        const int vec_smp = reinterpret_cast<uintptr_t>(smp) % al == 0 && mp % 2 == 0;
+        typename K::Params p{static_cast<const InT*>(src), static_cast<const InT*>(smp), peaks,
+                             static_cast<const cplx*>(plan->wm.p), static_cast<const cplx*>(plan->wn.p),
+                             plan->small, sp, mp, vec_src, vec_smp};
+        if constexpr (WIN) p.win = *win;
+        const size_t smem = K::smem_bytes(plan->small.M);
+        const dim3 grid(1, 1, pairs);
+        return launch(ctx, d, KC_SMALL_FFT, st, [&] {
+            fft_kernel_entry<K><<<grid, K::THREADS, smem, st>>>(p);
+        });
+    };
+    // sp == 0: every pair reads the one source (the shared-source call; the kernel's 0 means packed)
+    return sp == 0 ? go(SmallXcorrKernel<InT, PHAT, WIN, true>{}) : go(SmallXcorrKernel<InT, PHAT, WIN>{});
 }
 
 static int build_small_plan(FftPlan* plan, long long L) {
@@ -124,7 +128,8 @@ static int build_small_plan(FftPlan* plan, long long L) {
         auto allow_all = [&](auto PH, auto W) -> int {
             constexpr bool PHAT = decltype(PH)::value, WIN = decltype(W)::value;
             return allow(SmallXcorrKernel<float, PHAT, WIN>{}) | allow(SmallXcorrKernel<double, PHAT, WIN>{}) |
-                   allow(SmallXcorrKernel<int16_t, PHAT, WIN>{});
+                   allow(SmallXcorrKernel<int16_t, PHAT, WIN>{}) | allow(SmallXcorrKernel<float, PHAT, WIN, true>{}) |
+                   allow(SmallXcorrKernel<double, PHAT, WIN, true>{}) | allow(SmallXcorrKernel<int16_t, PHAT, WIN, true>{});
         };
         if ((plan->phat ? allow_all(std::true_type{}, std::false_type{}) | allow_all(std::true_type{}, std::true_type{})
                         : allow_all(std::false_type{}, std::false_type{}) | allow_all(std::false_type{}, std::true_type{})) != 0)
@@ -322,11 +327,17 @@ static int ensure_tickets(WorkSet& w, size_t n) {
 
 // Enqueue the whole path for device-resident pairs on `st` (no sync).
 // src_pitch / smp_pitch: elements between consecutive pairs (0 = packed [pair][2L] / [pair][L]).
+// shared_src: every pair reads the one source at `src` (audiosync_cuda_xcorr_shared_source); the
+// kernels then get a source pitch of 0, and a static plan transforms the source into work.spec.
+// spectrum_ready: an earlier enqueue of the same call, on this work set and stream, already left that
+// source's spectrum in work.spec (the chunks of a host-fed call), so it is not computed again.
 static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work, const void* src, const void* smp,
                          size_t n_pairs, long long L, int dtype, audiosync_cuda_result* d_results,
-                         cudaStream_t st, long long src_pitch = 0, long long smp_pitch = 0) {
+                         cudaStream_t st, long long src_pitch = 0, long long smp_pitch = 0, bool shared_src = false,
+                         bool spectrum_ready = false) {
     if (n_pairs == 0) return 0;
-    if (src_pitch == 0) src_pitch = 2 * L;
+    if (shared_src) src_pitch = 0;
+    else if (src_pitch == 0) src_pitch = 2 * L;
     if (smp_pitch == 0) smp_pitch = L;
     const bool packed = src_pitch == 2 * L && smp_pitch == L;
     if (L <= 0 || L > (1LL << 30)) { set_last_error("unsupported sample_len %lld", L); return -1; }
@@ -360,11 +371,19 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
     PearsonPartial* partials = static_cast<PearsonPartial*>(work.partials.p);
     if (ensure_tickets(work, (size_t)wave) != 0) return -1;
     unsigned int* tickets = static_cast<unsigned int*>(work.tickets.p);
+    // the source's forward rows, once per call, where the plan can reuse them (the static plans);
+    // every other plan reads the one source in every pair's transform
+    const bool reuse = shared_src && plan->run_shared_wave;
+    if (reuse && !spectrum_ready &&
+        (work.spec.ensure(sizeof(cplx) * (size_t)L) != 0 || plan->source_spectrum(ctx, d, src, in_dtype, work.spec.p, peaks, st) != 0))
+        return -1;
     for (size_t p0 = 0; p0 < n_pairs; p0 += (size_t)wave) {
         const int pairs = (int)std::min<size_t>((size_t)wave, n_pairs - p0);
         const char* s = static_cast<const char*>(src) + p0 * (size_t)src_pitch * esz;
         const char* m = static_cast<const char*>(smp) + p0 * (size_t)smp_pitch * esz;
-        if (plan->run_wave(ctx, d, s, m, in_dtype, src_pitch, smp_pitch, work.ws.p, peaks, pairs, st, win) != 0) return -1;
+        if ((reuse ? plan->run_shared_wave(ctx, d, work.spec.p, m, in_dtype, smp_pitch, work.ws.p, peaks, pairs, st, win)
+                   : plan->run_wave(ctx, d, s, m, in_dtype, src_pitch, smp_pitch, work.ws.p, peaks, pairs, st, win)) != 0)
+            return -1;
         const dim3 grid(n_chunks, pairs);
         int rc;
         if (dtype == AUDIOSYNC_CUDA_F32) {
@@ -676,9 +695,11 @@ static int direct_in_flight(DeviceState& d) {
 // is used and neither side waits for the other.  The two sub-batches [0, k) (doubles) and [k, n) (exact fp32 images) are
 // enqueued separately.  solo: this call drives a single device (several devices of one context
 // share the copy threads; each then feeds its device with direct uploads only).
+// shared_src: `sources` is one source for every pair; it is uploaded once (into in_src[0]) and only
+// the samples are chunked, as they are (host narrowing does not apply).
 static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* sources,
                           const char* samples, size_t p0, size_t p1, long long L, int dtype,
-                          audiosync_cuda_result* out, bool solo) {
+                          audiosync_cuda_result* out, bool solo, bool shared_src = false) {
     if (p1 <= p0) return 0;
     std::lock_guard<std::mutex> dlk(d.mu);
     ASC_CUDA_OK(cudaSetDevice(d.device));
@@ -686,7 +707,7 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
     const size_t src_n = (size_t)(2 * L), smp_n = (size_t)L;
     const size_t src_bytes = src_n * esz, smp_bytes = smp_n * esz;
     const bool pageable = host_pointer_is_pageable(sources) || host_pointer_is_pageable(samples);
-    int mode = (dtype == AUDIOSYNC_CUDA_F64 && !ctx->precise) ? ctx->narrow_host : AUDIOSYNC_CUDA_NARROW_OFF;
+    int mode = (dtype == AUDIOSYNC_CUDA_F64 && !ctx->precise && !shared_src) ? ctx->narrow_host : AUDIOSYNC_CUDA_NARROW_OFF;
     if (mode == AUDIOSYNC_CUDA_NARROW_LOSSLESS && !pageable && (!solo || copy_pool().threads() < narrow_min_threads()))
         mode = AUDIOSYNC_CUDA_NARROW_OFF;
     static const int feed_depth = [] { const char* e = getenv("AUDIOSYNC_CUDA_FEED_DEPTH");
@@ -697,10 +718,12 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
     // what narrowed pairs are enqueued as: exact images keep the f64 call's arithmetic, ALWAYS answers as an fp32 batch
     const int narrowed_dtype = mode == AUDIOSYNC_CUDA_NARROW_ALWAYS ? AUDIOSYNC_CUDA_F32 : ASC_DTYPE_F32_EXACT;
     // chunk: about 192 MB of input per buffer (twice that when pairs are fed both ways), at least one pair
-    size_t chunk = std::max<size_t>(1, ((size_t)(hybrid ? 384u : 192u) << 20) / (src_bytes + smp_bytes));
+    const size_t src_chunk_bytes = shared_src ? 0 : src_bytes;      // source bytes per chunked pair
+    size_t chunk = std::max<size_t>(1, ((size_t)(hybrid ? 384u : 192u) << 20) / (src_chunk_bytes + smp_bytes));
     chunk = std::min(chunk, p1 - p0);
     for (int b = 0; b < 2; b++) {
-        if (d.in_src[b].ensure(src_bytes * chunk) != 0 || d.in_smp[b].ensure(smp_bytes * chunk) != 0) return -1;
+        if (d.in_src[b].ensure(shared_src ? src_bytes : src_bytes * chunk) != 0 || d.in_smp[b].ensure(smp_bytes * chunk) != 0)
+            return -1;
         if (mode != AUDIOSYNC_CUDA_NARROW_OFF &&
             (d.in_src32[b].ensure(sizeof(float) * src_n * chunk) != 0 || d.in_smp32[b].ensure(sizeof(float) * smp_n * chunk) != 0))
             return -1;
@@ -716,11 +739,12 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
     if (d.results.ensure(sizeof(audiosync_cuda_result) * total) != 0) return -1;
     if (d.h_results.ensure(sizeof(audiosync_cuda_result) * total) != 0) return -1;
     audiosync_cuda_result* d_res = static_cast<audiosync_cuda_result*>(d.results.p);
+    if (shared_src && upload_from_host(d.in_src[0].p, sources, src_bytes, d.copy_stream, d.stage, pageable) != 0) return -1;
     int it = 0;
     for (size_t c0 = 0; c0 < total; c0 += chunk, it++) {
         const size_t n = std::min(chunk, total - c0);
         const int b = it & 1;
-        const char* hs = sources + (p0 + c0) * src_bytes;
+        const char* hs = sources + (shared_src ? 0 : (p0 + c0) * src_bytes);
         const char* hm = samples + (p0 + c0) * smp_bytes;
         if (it >= 2) {
             ASC_CUDA_OK(cudaStreamWaitEvent(d.copy_stream, d.ev_done[b], 0));
@@ -735,7 +759,7 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
         auto unit_pairs = [&](size_t u) { return std::min(g, n - u * g); };
         size_t lo = 0, hi = nu, dir_off = 0;
         if (mode == AUDIOSYNC_CUDA_NARROW_OFF) {
-            if (upload_from_host(d.in_src[b].p, hs, src_bytes * n, d.copy_stream, d.stage, pageable) != 0 ||
+            if ((!shared_src && upload_from_host(d.in_src[b].p, hs, src_bytes * n, d.copy_stream, d.stage, pageable) != 0) ||
                 upload_from_host(d.in_smp[b].p, hm, smp_bytes * n, d.copy_stream, d.stage, pageable) != 0)
                 return -1;
             lo = nu;
@@ -814,7 +838,10 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
         if (n_dbl > 0) {
             ASC_CUDA_OK(cudaEventRecord(d.ev_up[b], d.copy_stream));
             ASC_CUDA_OK(cudaStreamWaitEvent(d.stream, d.ev_up[b], 0));
-            if (enqueue_batch(ctx, d, d.work, d.in_src[b].p, d.in_smp[b].p, n_dbl, L, dtype, d_res + c0, d.stream) != 0) return -1;
+            // shared_src: the first chunk transforms the source, the later ones reuse its spectrum
+            if (enqueue_batch(ctx, d, d.work, d.in_src[shared_src ? 0 : b].p, d.in_smp[b].p, n_dbl, L, dtype, d_res + c0, d.stream,
+                              0, 0, shared_src, shared_src && c0 > 0) != 0)
+                return -1;
         }
         if (p_nar < n) {
             ASC_CUDA_OK(cudaEventRecord(d.ev_up32[b], d.narrow_stream));
@@ -1133,21 +1160,34 @@ int audiosync_cuda_synth_pairs(audiosync_cuda_ctx* ctx, int device, uint64_t see
     return 0;
 }
 
-int audiosync_cuda_xcorr_batch_device(audiosync_cuda_ctx* ctx, int device, const void* d_sources,
-                                      const void* d_samples, size_t n_pairs, size_t sample_len,
-                                      int dtype, audiosync_cuda_result* d_results, void* stream) {
+// xcorr_batch_device and xcorr_shared_source_device
+static int batch_device(audiosync_cuda_ctx* ctx, int device, const void* d_sources, const void* d_samples, size_t n_pairs,
+                        size_t sample_len, int dtype, audiosync_cuda_result* d_results, void* stream, bool shared_src) {
     if (!ctx || !d_sources || !d_samples || !d_results) { set_last_error("null argument"); return -1; }
     if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64 && dtype != AUDIOSYNC_CUDA_S16) { set_last_error("bad dtype"); return -1; }
     DeviceState* d = ctx->find(device);
     if (!d) { set_last_error("device %d is not part of this context", device); return -1; }
     std::lock_guard<std::mutex> lk(d->mu);      // per device: threads driving different devices do not serialise
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
-    return enqueue_batch(ctx, *d, d->work, d_sources, d_samples, n_pairs, (long long)sample_len, dtype, d_results, st);
+    return enqueue_batch(ctx, *d, d->work, d_sources, d_samples, n_pairs, (long long)sample_len, dtype, d_results, st,
+                         0, 0, shared_src);
 }
 
-int audiosync_cuda_xcorr_batch_results(audiosync_cuda_ctx* ctx, const void* sources, const void* samples,
-                                       size_t n_pairs, size_t sample_len, int dtype, int memspace,
-                                       audiosync_cuda_result* results) {
+int audiosync_cuda_xcorr_batch_device(audiosync_cuda_ctx* ctx, int device, const void* d_sources,
+                                      const void* d_samples, size_t n_pairs, size_t sample_len,
+                                      int dtype, audiosync_cuda_result* d_results, void* stream) {
+    return batch_device(ctx, device, d_sources, d_samples, n_pairs, sample_len, dtype, d_results, stream, false);
+}
+
+int audiosync_cuda_xcorr_shared_source_device(audiosync_cuda_ctx* ctx, int device, const void* d_source,
+                                              const void* d_samples, size_t n_pairs, size_t sample_len,
+                                              int dtype, audiosync_cuda_result* d_results, void* stream) {
+    return batch_device(ctx, device, d_source, d_samples, n_pairs, sample_len, dtype, d_results, stream, true);
+}
+
+// xcorr_batch_results and xcorr_shared_source
+static int batch_results(audiosync_cuda_ctx* ctx, const void* sources, const void* samples, size_t n_pairs,
+                         size_t sample_len, int dtype, int memspace, audiosync_cuda_result* results, bool shared_src) {
     if (!ctx || !sources || !samples || (!results && n_pairs)) { set_last_error("null argument"); return -1; }
     if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64 && dtype != AUDIOSYNC_CUDA_S16) { set_last_error("bad dtype"); return -1; }
     if (n_pairs == 0) return 0;
@@ -1169,7 +1209,7 @@ int audiosync_cuda_xcorr_batch_results(audiosync_cuda_ctx* ctx, const void* sour
         ASC_CUDA_OK(cudaSetDevice(d->device));
         if (d->results.ensure(sizeof(audiosync_cuda_result) * n_pairs) != 0) return -1;
         auto* d_res = static_cast<audiosync_cuda_result*>(d->results.p);
-        if (enqueue_batch(ctx, *d, d->work, sources, samples, n_pairs, L, dtype, d_res, d->stream) != 0) return -1;
+        if (enqueue_batch(ctx, *d, d->work, sources, samples, n_pairs, L, dtype, d_res, d->stream, 0, 0, shared_src) != 0) return -1;
         ASC_CUDA_OK(cudaMemcpyAsync(results, d_res, sizeof(audiosync_cuda_result) * n_pairs,
                                     cudaMemcpyDeviceToHost, d->stream));
         ASC_CUDA_OK(cudaStreamSynchronize(d->stream));
@@ -1189,7 +1229,7 @@ int audiosync_cuda_xcorr_batch_results(audiosync_cuda_ctx* ctx, const void* sour
             if (cnt == 0) continue;
             auto work = [&, g, a, b] {
                 rcs[g] = run_host_range(ctx, ctx->devs[g], static_cast<const char*>(sources),
-                                        static_cast<const char*>(samples), a, b, L, dtype, results, solo);
+                                        static_cast<const char*>(samples), a, b, L, dtype, results, solo, shared_src);
                 if (rcs[g] != 0) errs[g] = take_last_error();   // the worker's thread-local message
             };
             if (G == 1) work(); else th.emplace_back(work);
@@ -1203,6 +1243,18 @@ int audiosync_cuda_xcorr_batch_results(audiosync_cuda_ctx* ctx, const void* sour
         if (rc != 0) return -1;
     }
     return 0;
+}
+
+int audiosync_cuda_xcorr_batch_results(audiosync_cuda_ctx* ctx, const void* sources, const void* samples,
+                                       size_t n_pairs, size_t sample_len, int dtype, int memspace,
+                                       audiosync_cuda_result* results) {
+    return batch_results(ctx, sources, samples, n_pairs, sample_len, dtype, memspace, results, false);
+}
+
+int audiosync_cuda_xcorr_shared_source(audiosync_cuda_ctx* ctx, const void* source, const void* samples,
+                                       size_t n_pairs, size_t sample_len, int dtype, int memspace,
+                                       audiosync_cuda_result* results) {
+    return batch_results(ctx, source, samples, n_pairs, sample_len, dtype, memspace, results, true);
 }
 
 int audiosync_cuda_xcorr_batch(audiosync_cuda_ctx* ctx, const void* sources, const void* samples,

@@ -41,6 +41,7 @@ enum KernelClass {
     KC_COL_INV,      // K_C  inverse column pass + |r| argmax epilogue
     KC_SMALL_FFT,    // single-CTA transform for short lengths
     KC_PEARSON,      // window statistics + coefficient + result record
+    KC_SRC_SPECTRUM, // forward rows of a shared source, once per call (RowFusedKernel ROWS_SRC_SPECTRUM)
     KC_COUNT
 };
 
@@ -108,11 +109,12 @@ struct WorkSet {
     DevBuf peaks;         // PairPeak per in-flight pair
     DevBuf partials;      // PearsonPartial
     DevBuf tickets;       // per-pair completion counters of the Pearson kernel
+    DevBuf spec;          // shared-source calls on a static plan: the source's forward rows (M complex)
     cudaEvent_t done = nullptr;
     cudaStream_t last_stream = nullptr;
     bool used = false;
     void release() {
-        ws.release(); peaks.release(); partials.release(); tickets.release();
+        ws.release(); peaks.release(); partials.release(); tickets.release(); spec.release();
         if (done) cudaEventDestroy(done);
         done = nullptr; used = false;
     }

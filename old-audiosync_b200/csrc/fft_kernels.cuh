@@ -174,7 +174,11 @@ ASC_HD void argmax_merge(unsigned long long& best, float& second, unsigned long 
 // mbarrier sits at its very end and the last tile row (128 bytes) is not staged; pass 0 reads
 // that row from global memory, and the thread whose butterfly writes the barrier's bytes
 // invalidates it first.  (The sample tile has its unstaged upper half to spare.)
-template <class RL, int M2_, int NT, typename InT, bool TMA>
+//
+// SMP_ONLY: the sample plane alone (grid y = 1), for a call whose pairs share one source whose
+// spectrum is computed once (RowFusedKernel's ROWS_SRC_SPECTRUM); Params::sources is not read and the
+// pair's peak record is cleared by a sample CTA.
+template <class RL, int M2_, int NT, typename InT, bool TMA, bool SMP_ONLY = false>
 struct ColFwdKernel {
     static constexpr int M1 = RL::n;
     static constexpr int M2 = M2_;                  // row length (compile time: index products fold)
@@ -209,11 +213,11 @@ struct ColFwdKernel {
     };
     static constexpr int SRC_ROWS = M1 - 1, SMP_ROWS = M1 / 2;   // rows the TMA unit stages
 
-    // grid = (M2 / 16, 2, pairs)
+    // grid = (M2 / 16, 2, pairs); SMP_ONLY: (M2 / 16, 1, pairs)
     template <class Ex>
     static ASC_HD void run(Ex& ex, const Params& p, cplx* __restrict__ buf) {
         const int c0 = ex.bx() * COL_T;
-        const int sig = ex.by();
+        const int sig = ex.by() + (SMP_ONLY ? 1 : 0);   // SMP_ONLY: a run-time 1 keeps the sibling's register budget
         const long long pair = ex.bz();
         const long long M = p.L;
         const InT* __restrict__ x = sig == 0 ? p.sources + pair * (p.src_pitch ? p.src_pitch : 2 * M)
@@ -222,7 +226,7 @@ struct ColFwdKernel {
         const long long nvalid = sig == 0 ? M : M / 2;
         [[maybe_unused]] const bool vec = sig == 0 ? p.vec_src != 0 : p.vec_smp != 0;
         cplx* __restrict__ out = p.planes + (pair * 2 + sig) * M;
-        const bool clears_peak = ex.bx() == 0 && sig == 0;
+        const bool clears_peak = ex.bx() == 0 && sig == (SMP_ONLY ? 1 : 0);
 
         [[maybe_unused]] void* mbar = reinterpret_cast<char*>(buf) + SMEM - 8;
         if constexpr (TMA) {
@@ -748,7 +752,19 @@ ASC_HD void split_phat_merge(C a, C b, C c, C d, C w, C& qk, C& qmk) {
 // PHAT: the forward spectra are whitened in the split step (split_phat_merge) and the rest of the
 // kernel is unchanged.  Params::rev, m_lo and m_hi then hold the split's half-angle tables,
 // exp(-2*pi*i*freq_of_pos(e)/(2*M2)) and W_N (N = 2M), so that w = W_N^k1 * rev[e] factors like w^2.
-template <class RL, int M1_, int NT, bool PHAT = false>
+//
+// MODE: what a CTA does with its rows.  A batch whose pairs share one source computes that source's
+// forward rows once and feeds them, unchanged, into every pair's split step, so that each pair's
+// product is bit for bit the one of ROWS_PAIR on the replicated source:
+//   ROWS_PAIR          the pair's source and sample rows (plane 0 and 1), as above.
+//   ROWS_SRC_SPECTRUM  the forward passes of the source rows of plane 0 only, stored back in place
+//                      in their shared-memory position order (a CTA owns rows k1 and M1 - k1).
+//   ROWS_SHARED_SRC    slots 0/1 staged from Params::spec (the rows ROWS_SRC_SPECTRUM left), the
+//                      forward passes on the sample rows only, then the split and inverse as above;
+//                      plane 0 is not read, it only receives the product.
+enum RowMode { ROWS_PAIR = 0, ROWS_SRC_SPECTRUM = 1, ROWS_SHARED_SRC = 2 };
+
+template <class RL, int M1_, int NT, bool PHAT = false, int MODE = ROWS_PAIR>
 struct RowFusedKernel {
     static constexpr int M2 = RL::n;
     static constexpr int M1 = M1_;  // 0: the number of rows is a launch parameter (Params::m1) -- the rows of a
@@ -769,7 +785,7 @@ struct RowFusedKernel {
     // (S active) instead.  S == 1 passes must use an odd radix (conflict-free).
     static constexpr int slots(int S) { return (S > 1 && S < 16) ? 16 : S; }
 
-    struct Params {
+    struct PairParams {
         cplx* planes;            // [pair][2][M1*M2]
         const cplx* tw;          // RL pass tables (forward sign, power-of-two multiples)
         const cplx* rev;         // [M2]: exp(-2*pi*i*freq_of_pos(e)/M2), position order
@@ -779,6 +795,12 @@ struct RowFusedKernel {
         const cplx* rtab;        // [M1][TABP]: per row k1 the final-pass tables (fft_plan.h: build_row_tab)
         int m1 = 0;              // rows per plane when M1_ == 0
     };
+    // ROWS_SHARED_SRC appends the spectrum pointer; the other modes keep PairParams, so that their
+    // parameter block is the same on the host and the device and the same as before the modes existed
+    struct SharedParams : PairParams {
+        const cplx* spec;        // [M1][M2] the source's forward rows, position order
+    };
+    using Params = std::conditional_t<MODE == ROWS_SHARED_SRC, SharedParams, PairParams>;
     // Final-pass twiddle tables of one row k1: S0 entries 0.5 * W_M^(j*k1) (the factor 1/2 of the
     // merge step rides here, exactly), then R0 entries W_M^(k*S0*k1); padded to an even count so
     // that a row is a whole number of 16-byte units for the bulk copy.
@@ -802,6 +824,9 @@ struct RowFusedKernel {
         const int k1a = r, k1b = m1 - r;   // k1b unused when !two
         cplx* __restrict__ plane_s = p.planes + pair * 2 * M;
         cplx* __restrict__ plane_p = plane_s + M;
+        // where slots 0/1 are staged from
+        const cplx* __restrict__ src_rows = plane_s;
+        if constexpr (MODE == ROWS_SHARED_SRC) src_rows = p.spec;
         // final-pass twiddle tables of the two rows, copied into the (then dead) sample rows
         cplx* __restrict__ tab = buf + 2 * RP;                // [2][TABP]
         void* tabbar = buf + 2 * RP + 2 * TABP;               // mbarrier of that copy
@@ -811,7 +836,7 @@ struct RowFusedKernel {
         // The CTA's shared memory is exactly the four rows, so the 8-byte mbarrier sits on the
         // last point of slot 3; the last two points of that row are not staged -- forward pass 0
         // reads them from global memory instead -- and the thread whose butterfly writes them
-        // first invalidates the barrier.
+        // first invalidates the barrier.  ROWS_SRC_SPECTRUM stages slots 0/1 only.
         {
             void* mbar = buf + 4 * RP - 1;
             ex.phase([&](int tid) {
@@ -820,12 +845,18 @@ struct RowFusedKernel {
             ex.phase([&](int tid) {
                 if (tid == 0) {
                     constexpr unsigned full = (unsigned)(M2 * sizeof(cplx));
-                    mbar_expect_tx(mbar, two ? 4u * full - 16u : 2u * full);
-                    bulk_load(buf, plane_s + (long long)k1a * M2, full, mbar);
-                    bulk_load(buf + 2 * RP, plane_p + (long long)k1a * M2, full, mbar);
-                    if (two) {
-                        bulk_load(buf + RP, plane_s + (long long)k1b * M2, full, mbar);
-                        bulk_load(buf + 3 * RP, plane_p + (long long)k1b * M2, full - 16u, mbar);
+                    if constexpr (MODE == ROWS_SRC_SPECTRUM) {
+                        mbar_expect_tx(mbar, (unsigned)nrows * full);
+                        bulk_load(buf, src_rows + (long long)k1a * M2, full, mbar);
+                        if (two) bulk_load(buf + RP, src_rows + (long long)k1b * M2, full, mbar);
+                    } else {
+                        mbar_expect_tx(mbar, two ? 4u * full - 16u : 2u * full);
+                        bulk_load(buf, src_rows + (long long)k1a * M2, full, mbar);
+                        bulk_load(buf + 2 * RP, plane_p + (long long)k1a * M2, full, mbar);
+                        if (two) {
+                            bulk_load(buf + RP, src_rows + (long long)k1b * M2, full, mbar);
+                            bulk_load(buf + 3 * RP, plane_p + (long long)k1b * M2, full - 16u, mbar);
+                        }
                     }
                 }
                 mbar_wait(mbar, 0);
@@ -886,8 +917,27 @@ struct RowFusedKernel {
             }
         };
         static_for<0, P>([&](auto PP) {
-            ex.phase([&](int tid) { fwd_pass(PP, tid, NT, 0, two ? 1 : 2, 2 * nrows); });   // slots 0,1,2,3 or 0,2
+            ex.phase([&](int tid) {
+                if constexpr (MODE == ROWS_PAIR) {
+                    fwd_pass(PP, tid, NT, 0, two ? 1 : 2, 2 * nrows);   // slots 0,1,2,3 or 0,2
+                } else if constexpr (MODE == ROWS_SRC_SPECTRUM) {
+                    fwd_pass(PP, tid, NT, 0, two ? 1 : 2, nrows);        // slots 0,1 or 0 (the pair mode's step: 60 registers, not 62)
+                    if constexpr (decltype(PP)::value == P - 1) fence_async_proxy();   // read by the bulk store below
+                } else {
+                    fwd_pass(PP, tid, NT, 2, 1, nrows);                  // slots 2,3 or 2
+                }
+            });
         });
+
+        // ---- ROWS_SRC_SPECTRUM: the transformed source rows leave in place; nothing else to do.
+        if constexpr (MODE == ROWS_SRC_SPECTRUM) {
+            ex.single([&]() {
+                bulk_store(plane_s + (long long)k1a * M2, buf, (unsigned)(M2 * sizeof(cplx)));
+                if (two) bulk_store(plane_s + (long long)k1b * M2, buf + RP, (unsigned)(M2 * sizeof(cplx)));
+                bulk_store_commit_and_drain();
+            });
+            return;
+        }
 
         // ---- split + conj-multiply + merge, in place into the source rows.
         {

@@ -37,7 +37,8 @@ ASC_HD int small_pos_of_freq(const SmallPlan& pl, int k) {
 
 // PHAT: the split step whitens the spectra (split_phat_merge); w is wn[k] as for the product.
 // WIN: the windowed twin -- only the raw indices Params::win allows compete (ArgmaxAcc::consider_win).
-template <typename InT, bool PHAT = false, bool WIN = false>
+// SHARED_SRC: every pair reads the one source at Params::sources (its pitch is not read).
+template <typename InT, bool PHAT = false, bool WIN = false, bool SHARED_SRC = false>
 struct SmallXcorrKernel {
     static constexpr int THREADS = SMALL_THREADS;
 
@@ -80,7 +81,7 @@ struct SmallXcorrKernel {
                     static_for<0, R>([&](auto Q) {
                         constexpr int q = decltype(Q)::value;
                         const long long n = i0 + q * S;
-                        if (rr == 0) v[q] = load_packed<InT>(p.sources + pair * (p.src_pitch ? p.src_pitch : 2 * M), n, p.vec_src != 0);
+                        if (rr == 0) v[q] = load_packed<InT>(p.sources + (SHARED_SRC ? 0 : pair * (p.src_pitch ? p.src_pitch : 2 * M)), n, p.vec_src != 0);
                         else v[q] = n < M / 2 ? load_packed<InT>(p.samples + pair * (p.smp_pitch ? p.smp_pitch : M), n, p.vec_smp != 0)
                                               : cmake(0.f, 0.f);
                     });

@@ -42,6 +42,12 @@ struct FftPlan {
     //  lag window: nullptr for the unwindowed kernels, else the windowed twins of the argmax step)
     std::function<int(audiosync_cuda_ctx*, DeviceState&, const void*, const void*, int, long long, long long,
                       void*, PairPeak*, int, cudaStream_t, const RawWindow*)> run_wave;
+    // Static plans only: the reuse path of a batch whose pairs share one source.  source_spectrum
+    // (ctx, d, src, dtype, spec, peaks, stream) writes the source's forward rows into spec (M complex)
+    // once per call; run_shared_wave is run_wave with spec in place of the source and its pitch.
+    std::function<int(audiosync_cuda_ctx*, DeviceState&, const void*, int, void*, PairPeak*, cudaStream_t)> source_spectrum;
+    std::function<int(audiosync_cuda_ctx*, DeviceState&, const void*, const void*, int, long long,
+                      void*, PairPeak*, int, cudaStream_t, const RawWindow*)> run_shared_wave;
     ~FftPlan() {
         col_tw.release(); col_tc.release(); row_tw.release(); row_rev.release(); row_tab.release(); m_lo.release(); m_hi.release();
         wm.release(); wn.release();
