@@ -7,11 +7,15 @@
 // plans write r and resolve it with argmax_f64_window_kernel, whose body needs warp shuffles: it is
 // restated here (the same candidates and order rule).  Every runner returns the resolved index / peak /
 // second peak at the reference's scale (x N) and the packed peak record of the fp32-argmax paths.
-// Compiled by tests/test_lag_window_emu.py; never linked into the product.
+// emulw_perturb changes one entry of a table the static plans build on the host before their kernels
+// run (tests/test_xcorr_error_emu.py: a corrupted table must fail the per-lag error bound).
+// Compiled by tests/golden/emu_build.py for the tests; never linked into the product.
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <string>
+#include <utility>
 #include <vector>
 
 #include "fft_plan.h"
@@ -59,6 +63,17 @@ struct Rec {
 
 namespace {
 
+// what: 0 none, 1 col_tw[i] *= (1 + eps), 2 row_tab[i] conjugated, 3 row_tw[i] and row_tw[j] swapped
+struct Perturb { int what; long long i, j; double eps; };
+Perturb g_perturb{0, 0, 0, 0.0};
+
+void apply_perturb(std::vector<cplx>& col_tw, std::vector<cplx>& row_tw, std::vector<cplx>& row_tab) {
+    const Perturb& q = g_perturb;
+    if (q.what == 1) col_tw.at(q.i) = cmake((float)(col_tw.at(q.i).x * (1.0 + q.eps)), (float)(col_tw.at(q.i).y * (1.0 + q.eps)));
+    else if (q.what == 2) row_tab.at(q.i).y = -row_tab.at(q.i).y;
+    else if (q.what == 3) std::swap(row_tw.at(q.i), row_tw.at(q.j));
+}
+
 void from_peak(const PairPeak& pk, double scale, Rec* r) {
     r->raw_index = (long long)argmax_key_index(pk.key);
     r->peak = (double)argmax_key_value(pk.key) * scale;
@@ -80,6 +95,7 @@ void static_plan(const double* source, const double* sample, const RawWindow& wi
     std::vector<cplx> row_rev = build_row_rev<Row>();
     std::vector<cplx> m_lo, m_hi;
     build_two_level(M, M - 1, m_lo, m_hi);
+    apply_perturb(col_tw, row_tw, row_tab);
     peak->key = 12345ull; peak->second_bits = 777u; peak->seed_bits = 777u;   // garbage: K_A must clear them
     {
         using K = ColFwdKernel<Col, Row::n, P::NT_COL, double, false>;
@@ -228,6 +244,33 @@ int generic_plan(const double* source, const double* sample, long long L, const 
 }  // namespace
 
 extern "C" {
+
+// the table entry the static plans change from now on (what = 0: none); not thread-safe against runs
+void emulw_perturb(int what, long long i, long long j, double eps) { g_perturb = Perturb{what, i, j, eps}; }
+
+// the library's description of the runtime-radix plan (kind 2 fp32, 3 fp64) at L: its length, -1 none
+int emulw_describe(int kind, long long L, char* buf, int len) {
+    GenShape sh;
+    if ((kind != 2 && kind != 3) || !gen_make_shape(L, kind == 3, &sh)) return -1;
+    const std::string d = gen_describe(sh, kind == 3);
+    if ((int)d.size() + 1 > len) return -1;
+    memcpy(buf, d.c_str(), d.size() + 1);
+    return (int)d.size();
+}
+
+// sizes of the static plan's host tables at L: col_tw, row_tw, row_tab (-1: no static plan)
+long long emulw_table_sizes(long long L, long long* out3) {
+    long long rc = -1;
+    for_each_static_plan([&](auto P) {
+        using PP = decltype(P);
+        if (PP::L != L) return;
+        out3[0] = (long long)build_pass_tables(radix_vector<typename PP::Col>()).size();
+        out3[1] = (long long)build_pass_tables(radix_vector<typename PP::Row>()).size();
+        out3[2] = (long long)build_row_tab<typename PP::Row>(PP::L, PP::Col::n).size();
+        rc = 0;
+    });
+    return rc;
+}
 
 // raw ranges of the lag window [lo, hi] at L: -1 empty, 0 all of [-L, L-1], 1 restrictive
 int emulw_window(long long lo, long long hi, long long L, unsigned* out4) {

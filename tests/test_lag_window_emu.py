@@ -2,22 +2,21 @@
 
 tests/emu/emu_lagwin.cu runs the windowed twins of the static K_C, the runtime-radix inverse column
 kernel (fp32; fp64 plans through the restated argmax_f64_window_kernel rule) and the single-CTA kernel
-on f64 inputs; this module compiles it (g++, no GPU) into a temporary directory.  The probes put a
+on f64 inputs; tests/golden/emu_build.py compiles it (g++, no GPU) into a temporary directory.  The probes put a
 one-hot sample at 0, so r[j] = N source[j] in closed form, and set each case of the windowed rule
 exactly.  Bounds as in tests/test_phat_emu.py: raw_index exact; peak / N and second / N within 1e-6
 (fp32 arithmetic) or 1e-12 (fp64).
 """
 import ctypes as C
 import os
-import subprocess
 import sys
 
 import numpy as np
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 sys.path.insert(0, os.path.join(HERE, "golden"))
+import emu_build  # noqa: E402
 import lagwin_oracle as lo  # noqa: E402
 
 STATIC, SMALL, GEN32, GEN64 = 0, 1, 2, 3
@@ -35,13 +34,8 @@ class Rec(C.Structure):
 
 
 @pytest.fixture(scope="module")
-def emu(tmp_path_factory):
-    out = str(tmp_path_factory.mktemp("emu_lagwin") / "libasc_emu_lagwin.so")
-    cuda_inc = os.environ.get("CUDA_INC", "/usr/local/cuda/include")
-    subprocess.run([os.environ.get("CXX", "g++"), "-std=c++17", "-O2", "-fPIC", "-shared", "-x", "c++",
-                    "-I" + cuda_inc, "-I" + os.path.join(ROOT, "old-audiosync_b200", "csrc"),
-                    "-o", out, os.path.join(HERE, "emu", "emu_lagwin.cu")], check=True)
-    E = C.CDLL(out)
+def emu():
+    E = C.CDLL(emu_build.build("emu_lagwin.cu"))
     E.emulw_window.argtypes = [C.c_longlong, C.c_longlong, C.c_longlong, C.POINTER(C.c_uint)]
     E.emulw_run.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_longlong, C.c_int,
                             C.POINTER(Rec)]
