@@ -83,28 +83,31 @@ int PinnedBuf::ensure(size_t need) {
 }
 void PinnedBuf::release() { if (p) cudaFreeHost(p); p = nullptr; bytes = 0; }
 
-template <typename InT, bool PHAT, bool WIN>
-static int run_small_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src,
-                          const void* smp, long long sp, long long mp, PairPeak* peaks, int pairs,
-                          cudaStream_t st, const RawWindow* win) {
-    auto go = [&](auto KK) -> int {
-        using K = decltype(KK);
-        // one load per packed point where every pair's base is aligned to two elements
-        const size_t al = 2 * sizeof(InT);
-        const int vec_src = reinterpret_cast<uintptr_t>(src) % al == 0 && sp % 2 == 0;
-        const int vec_smp = reinterpret_cast<uintptr_t>(smp) % al == 0 && mp % 2 == 0;
-        typename K::Params p{static_cast<const InT*>(src), static_cast<const InT*>(smp), peaks,
-                             static_cast<const cplx*>(plan->wm.p), static_cast<const cplx*>(plan->wn.p),
-                             plan->small, sp, mp, vec_src, vec_smp};
-        if constexpr (WIN) p.win = *win;
-        const size_t smem = K::smem_bytes(plan->small.M);
-        const dim3 grid(1, 1, pairs);
-        return launch(ctx, d, KC_SMALL_FFT, st, [&] {
-            fft_kernel_entry<K><<<grid, K::THREADS, smem, st>>>(p);
+// f(InT{}, PHAT, WIN, SHARED_SRC): the single-CTA kernel SmallXcorrKernel<InT, PHAT, WIN, SHARED_SRC>
+template <class F>
+static int with_small_kernel(int dtype, bool phat, bool win, bool shared_src, F&& f) {
+    return with_input_type(dtype, [&](auto IN) {
+        return with_bool(phat, [&](auto PHAT) {
+            return with_bool(win, [&](auto WIN) {
+                return with_bool(shared_src, [&](auto SHARED) { return f(IN, PHAT, WIN, SHARED); });
+            });
         });
-    };
-    // sp == 0: every pair reads the one source (the shared-source call; the kernel's 0 means packed)
-    return sp == 0 ? go(SmallXcorrKernel<InT, PHAT, WIN, true>{}) : go(SmallXcorrKernel<InT, PHAT, WIN>{});
+    });
+}
+
+template <typename InT, bool PHAT, bool WIN, bool SHARED>
+static int run_small_wave(FftPlan* plan, const Wave& w) {
+    using K = SmallXcorrKernel<InT, PHAT, WIN, SHARED>;
+    typename K::Params p{static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp), w.peaks,
+                         static_cast<const cplx*>(plan->wm.p), static_cast<const cplx*>(plan->wn.p),
+                         plan->small, w.src_pitch, w.smp_pitch, vec_loads<InT>(w.src, w.src_pitch),
+                         vec_loads<InT>(w.smp, w.smp_pitch)};
+    if constexpr (WIN) p.win = *w.win;
+    const size_t smem = K::smem_bytes(plan->small.M);
+    const dim3 grid(1, 1, w.pairs);
+    return launch(w.ctx, w.d, KC_SMALL_FFT, w.st, [&] {
+        fft_kernel_entry<K><<<grid, K::THREADS, smem, w.st>>>(p);
+    });
 }
 
 static int build_small_plan(FftPlan* plan, long long L) {
@@ -121,39 +124,20 @@ static int build_small_plan(FftPlan* plan, long long L) {
     const size_t smem = SmallXcorrKernel<float>::smem_bytes((int)L);
     if (smem > 48 * 1024) {
         const int cap = (int)SmallXcorrKernel<float>::smem_bytes(SMALL_MAX_M);
-        auto allow = [&](auto KK) -> int {
-            ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<decltype(KK)>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
+        auto allow = [&](auto IN, auto PHAT, auto WIN, auto SHARED) -> int {
+            using K = SmallXcorrKernel<decltype(IN), decltype(PHAT)::value, decltype(WIN)::value, decltype(SHARED)::value>;
+            ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
             return 0;
         };
-        auto allow_all = [&](auto PH, auto W) -> int {
-            constexpr bool PHAT = decltype(PH)::value, WIN = decltype(W)::value;
-            return allow(SmallXcorrKernel<float, PHAT, WIN>{}) | allow(SmallXcorrKernel<double, PHAT, WIN>{}) |
-                   allow(SmallXcorrKernel<int16_t, PHAT, WIN>{}) | allow(SmallXcorrKernel<float, PHAT, WIN, true>{}) |
-                   allow(SmallXcorrKernel<double, PHAT, WIN, true>{}) | allow(SmallXcorrKernel<int16_t, PHAT, WIN, true>{});
-        };
-        if ((plan->phat ? allow_all(std::true_type{}, std::false_type{}) | allow_all(std::true_type{}, std::true_type{})
-                        : allow_all(std::false_type{}, std::false_type{}) | allow_all(std::false_type{}, std::true_type{})) != 0)
-            return -1;
+        for (int dtype : {AUDIOSYNC_CUDA_F32, AUDIOSYNC_CUDA_F64, AUDIOSYNC_CUDA_S16})
+            for (bool win : {false, true})
+                for (bool shared_src : {false, true})
+                    if (with_small_kernel(dtype, plan->phat, win, shared_src, allow) != 0) return -1;
     }
-    auto run = [plan](auto PH, auto W, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp, int dtype,
-                      long long sp, long long mp, PairPeak* peaks, int pairs, cudaStream_t st, const RawWindow* win) -> int {
-        constexpr bool PHAT = decltype(PH)::value, WIN = decltype(W)::value;
-        switch (dtype) {
-            case AUDIOSYNC_CUDA_F32: return run_small_wave<float, PHAT, WIN>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st, win);
-            case AUDIOSYNC_CUDA_F64: return run_small_wave<double, PHAT, WIN>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st, win);
-            case AUDIOSYNC_CUDA_S16: return run_small_wave<int16_t, PHAT, WIN>(plan, ctx, d, src, smp, sp, mp, peaks, pairs, st, win);
-        }
-        set_last_error("bad dtype %d", dtype);
-        return -1;
-    };
-    plan->run_wave = [plan, run](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
-                                 int dtype, long long sp, long long mp, void*, PairPeak* peaks, int pairs,
-                                 cudaStream_t st, const RawWindow* win) {
-        auto with_phat = [&](auto PH) {
-            return win ? run(PH, std::true_type{}, ctx, d, src, smp, dtype, sp, mp, peaks, pairs, st, win)
-                       : run(PH, std::false_type{}, ctx, d, src, smp, dtype, sp, mp, peaks, pairs, st, win);
-        };
-        return plan->phat ? with_phat(std::true_type{}) : with_phat(std::false_type{});
+    plan->run_wave = [plan](const Wave& w) {
+        return with_small_kernel(w.dtype, plan->phat, w.win != nullptr, w.shared_src, [&](auto IN, auto PHAT, auto WIN, auto SHARED) {
+            return run_small_wave<decltype(IN), decltype(PHAT)::value, decltype(WIN)::value, decltype(SHARED)::value>(plan, w);
+        });
     };
     return 0;
 }
@@ -183,16 +167,12 @@ static int build_generic_plan_t(FftPlan* plan) {
                      : small_row ? GenStage<T, GEN_THREADS_SMALL>::prepare_rows(sh, plan->phat)
                                  : GenStage<T, GEN_THREADS>::prepare_rows(sh, plan->phat)) != 0)
         return -1;
-    plan->run_wave = [plan, small_col, small_row, static_rows](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
-                                                  int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,
-                                                  cudaStream_t st, const RawWindow* win) {
+    plan->run_wave = [plan, small_col, small_row, static_rows](const Wave& w) {
         using Big = GenStage<T, GEN_THREADS>;
         using Small = GenStage<T, GEN_THREADS_SMALL>;
-        if ((small_col ? Small::col_fwd(plan, ctx, d, src, smp, dtype, sp, mp, ws, peaks, pairs, st)
-                       : Big::col_fwd(plan, ctx, d, src, smp, dtype, sp, mp, ws, peaks, pairs, st)) != 0) return -1;
-        if ((static_rows ? static_rows_launch(plan, ctx, d, ws, pairs, st)
-                         : small_row ? Small::rows(plan, ctx, d, ws, pairs, st) : Big::rows(plan, ctx, d, ws, pairs, st)) != 0) return -1;
-        return small_col ? Small::col_inv(plan, ctx, d, ws, peaks, pairs, st, win) : Big::col_inv(plan, ctx, d, ws, peaks, pairs, st, win);
+        if ((small_col ? Small::col_fwd(plan, w) : Big::col_fwd(plan, w)) != 0) return -1;
+        if ((static_rows ? static_rows_launch(plan, w) : small_row ? Small::rows(plan, w) : Big::rows(plan, w)) != 0) return -1;
+        return small_col ? Small::col_inv(plan, w) : Big::col_inv(plan, w);
     };
     return 0;
 }
@@ -209,19 +189,17 @@ static int build_generic_plan(FftPlan* plan, long long L, bool precise) {
 }
 
 template <typename InT>
-static int run_direct_wave(long long L, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src,
-                           const void* smp, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,
-                           cudaStream_t st, const RawWindow* win) {
-    const long long N = 2 * L;
-    double* r = static_cast<double*>(ws);
-    const dim3 grid((unsigned)((N + DIRECT_TILE - 1) / DIRECT_TILE), pairs);
-    if (launch(ctx, d, KC_DIRECT, st, [&] {
-            direct_corr_kernel<InT><<<grid, DIRECT_TILE, 0, st>>>(static_cast<const InT*>(src),
-                                                                  static_cast<const InT*>(smp), r, L, sp, mp);
+static int run_direct_wave(FftPlan* plan, const Wave& w) {
+    const long long L = plan->L, N = 2 * L;
+    double* r = static_cast<double*>(w.ws);
+    const dim3 grid((unsigned)((N + DIRECT_TILE - 1) / DIRECT_TILE), w.pairs);
+    if (launch(w.ctx, w.d, KC_DIRECT, w.st, [&] {
+            direct_corr_kernel<InT><<<grid, DIRECT_TILE, 0, w.st>>>(static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp),
+                                                                    r, L, w.src_pitch, w.smp_pitch);
         }) != 0) return -1;
-    return launch(ctx, d, KC_ARGMAX_F64, st, [&] {
-        if (win) argmax_f64_window_kernel<<<pairs, 1024, 0, st>>>(r, N, N, peaks, *win);
-        else argmax_f64_kernel<<<pairs, 1024, 0, st>>>(r, N, N, peaks);
+    return launch(w.ctx, w.d, KC_ARGMAX_F64, w.st, [&] {
+        if (w.win) argmax_f64_window_kernel<<<w.pairs, 1024, 0, w.st>>>(r, N, N, w.peaks, *w.win);
+        else argmax_f64_kernel<<<w.pairs, 1024, 0, w.st>>>(r, N, N, w.peaks);
     });
 }
 
@@ -230,16 +208,8 @@ static int build_direct_plan(FftPlan* plan, long long L) {
     plan->L = L;
     plan->ws_bytes_per_pair = (size_t)2 * L * sizeof(double);
     plan->desc = "direct L=" + std::to_string(L) + " time-domain O(L^2) fp64";
-    plan->run_wave = [L](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
-                         int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,
-                         cudaStream_t st, const RawWindow* win) {
-        switch (dtype) {
-            case AUDIOSYNC_CUDA_F32: return run_direct_wave<float>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st, win);
-            case AUDIOSYNC_CUDA_F64: return run_direct_wave<double>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st, win);
-            case AUDIOSYNC_CUDA_S16: return run_direct_wave<int16_t>(L, ctx, d, src, smp, sp, mp, ws, peaks, pairs, st, win);
-        }
-        set_last_error("bad dtype %d", dtype);
-        return -1;
+    plan->run_wave = [plan](const Wave& w) {
+        return with_input_type(w.dtype, [&](auto IN) { return run_direct_wave<decltype(IN)>(plan, w); });
     };
     return 0;
 }
@@ -373,45 +343,30 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
     unsigned int* tickets = static_cast<unsigned int*>(work.tickets.p);
     // the source's forward rows, once per call, where the plan can reuse them (the static plans);
     // every other plan reads the one source in every pair's transform
-    const bool reuse = shared_src && plan->run_shared_wave;
-    if (reuse && !spectrum_ready &&
-        (work.spec.ensure(sizeof(cplx) * (size_t)L) != 0 || plan->source_spectrum(ctx, d, src, in_dtype, work.spec.p, peaks, st) != 0))
-        return -1;
+    const bool reuse = shared_src && plan->source_spectrum;
+    if (reuse && work.spec.ensure(sizeof(cplx) * (size_t)L) != 0) return -1;
+    Wave w{ctx, d, st, src, smp, in_dtype, src_pitch, smp_pitch, shared_src, reuse ? work.spec.p : nullptr,
+           work.ws.p, peaks, 0, win};
+    if (reuse && !spectrum_ready && plan->source_spectrum(w, work.spec.p) != 0) return -1;
     for (size_t p0 = 0; p0 < n_pairs; p0 += (size_t)wave) {
-        const int pairs = (int)std::min<size_t>((size_t)wave, n_pairs - p0);
-        const char* s = static_cast<const char*>(src) + p0 * (size_t)src_pitch * esz;
-        const char* m = static_cast<const char*>(smp) + p0 * (size_t)smp_pitch * esz;
-        if ((reuse ? plan->run_shared_wave(ctx, d, work.spec.p, m, in_dtype, smp_pitch, work.ws.p, peaks, pairs, st, win)
-                   : plan->run_wave(ctx, d, s, m, in_dtype, src_pitch, smp_pitch, work.ws.p, peaks, pairs, st, win)) != 0)
+        w.pairs = (int)std::min<size_t>((size_t)wave, n_pairs - p0);
+        w.src = static_cast<const char*>(src) + p0 * (size_t)src_pitch * esz;
+        w.smp = static_cast<const char*>(smp) + p0 * (size_t)smp_pitch * esz;
+        // EXACT: the f64 path's arithmetic, for every dtype but plain F32 (S16: on s * 2^-15)
+        auto pearson = [&](auto IN, auto EXACT) -> int {
+            using InT = decltype(IN);
+            constexpr bool EX = decltype(EXACT)::value;
+            return launch(ctx, d, KC_PEARSON, st, [&] {
+                launch_stage(plan->phat ? pearson_kernel<InT, EX, true> : pearson_kernel<InT, EX>, dim3(n_chunks, w.pairs),
+                             dim3(PEARSON_THREADS), 0, st, static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp),
+                             src_pitch, smp_pitch, L, (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets,
+                             n_chunks, d_results + p0);
+            });
+        };
+        if (plan->run_wave(w) != 0 ||
+            (dtype == AUDIOSYNC_CUDA_F32 ? pearson(float{}, std::false_type{})
+                                         : with_input_type(in_dtype, [&](auto IN) { return pearson(IN, std::true_type{}); })) != 0)
             return -1;
-        const dim3 grid(n_chunks, pairs);
-        int rc;
-        if (dtype == AUDIOSYNC_CUDA_F32) {
-            rc = launch(ctx, d, KC_PEARSON, st, [&] {
-                launch_stage(plan->phat ? pearson_kernel<float, false, true> : pearson_kernel<float, false>, grid, dim3(PEARSON_THREADS), 0, st,
-                    reinterpret_cast<const float*>(s), reinterpret_cast<const float*>(m), src_pitch, smp_pitch, L,
-                    (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
-            });
-        } else if (dtype == ASC_DTYPE_F32_EXACT) {
-            rc = launch(ctx, d, KC_PEARSON, st, [&] {
-                launch_stage(plan->phat ? pearson_kernel<float, true, true> : pearson_kernel<float, true>, grid, dim3(PEARSON_THREADS), 0, st,
-                    reinterpret_cast<const float*>(s), reinterpret_cast<const float*>(m), src_pitch, smp_pitch, L,
-                    (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
-            });
-        } else if (dtype == AUDIOSYNC_CUDA_F64) {
-            rc = launch(ctx, d, KC_PEARSON, st, [&] {
-                launch_stage(plan->phat ? pearson_kernel<double, true, true> : pearson_kernel<double, true>, grid, dim3(PEARSON_THREADS), 0, st,
-                    reinterpret_cast<const double*>(s), reinterpret_cast<const double*>(m), src_pitch, smp_pitch, L,
-                    (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
-            });
-        } else {   // S16 (esz above admits nothing else): the f64 path's arithmetic on s * 2^-15
-            rc = launch(ctx, d, KC_PEARSON, st, [&] {
-                launch_stage(plan->phat ? pearson_kernel<int16_t, true, true> : pearson_kernel<int16_t, true>, grid, dim3(PEARSON_THREADS), 0, st,
-                    reinterpret_cast<const int16_t*>(s), reinterpret_cast<const int16_t*>(m), src_pitch, smp_pitch, L,
-                    (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets, n_chunks, d_results + p0);
-            });
-        }
-        if (rc != 0) return -1;
     }
     ASC_CUDA_OK(cudaEventRecord(work.done, st));
     work.last_stream = st;
@@ -1144,18 +1099,16 @@ int audiosync_cuda_synth_pairs(audiosync_cuda_ctx* ctx, int device, uint64_t see
         const dim3 grid(bx, np);
         char* s = static_cast<char*>(d_sources) + p0 * (size_t)(2 * L) * esz;
         char* m = static_cast<char*>(d_samples) + p0 * (size_t)L * esz;
-        int rc = -1;
-        if (dtype == AUDIOSYNC_CUDA_F32)
-            rc = launch(ctx, *d, KC_SYNTH, st, [&] {
-                synth_kernel<float><<<grid, 256, 0, st>>>(reinterpret_cast<float*>(s),
-                                                          reinterpret_cast<float*>(m), seed, first_pair + p0, L);
-            });
-        else if (dtype == AUDIOSYNC_CUDA_F64)
-            rc = launch(ctx, *d, KC_SYNTH, st, [&] {
-                synth_kernel<double><<<grid, 256, 0, st>>>(reinterpret_cast<double*>(s),
-                                                           reinterpret_cast<double*>(m), seed, first_pair + p0, L);
-            });
-        if (rc != 0) return -1;
+        if (with_input_type(dtype, [&](auto IN) -> int {
+                using T = decltype(IN);
+                if constexpr (std::is_same<T, int16_t>::value) return -1;   // refused above
+                else
+                    return launch(ctx, *d, KC_SYNTH, st, [&] {
+                        synth_kernel<T><<<grid, 256, 0, st>>>(reinterpret_cast<T*>(s), reinterpret_cast<T*>(m), seed,
+                                                              first_pair + p0, L);
+                    });
+            }) != 0)
+            return -1;
     }
     return 0;
 }

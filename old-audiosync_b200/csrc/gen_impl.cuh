@@ -57,75 +57,62 @@ int GenStage<T, NT>::prepare_rows(const GenShape& sh, bool phat) {
 }
 
 template <typename T, int NT>
-int GenStage<T, NT>::col_fwd(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
-                             int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs, cudaStream_t st) {
+int GenStage<T, NT>::col_fwd(FftPlan* plan, const Wave& w) {
     typedef typename GenTraits<T>::C C;
     const GenShape& sh = plan->gen;
-    auto go = [&](auto IN) -> int {
+    return with_input_type(w.dtype, [&](auto IN) -> int {
         using InT = decltype(IN);
         return gen_for_tile_width<T>(sh.ct, [&](auto CTC) -> int {
             using K = GenColFwdKernel<T, InT, decltype(CTC)::value, NT>;
-            // two elements per load where the pairs' bases allow it
-            const size_t al = 2 * sizeof(InT);
-            const int vec_src = reinterpret_cast<uintptr_t>(src) % al == 0 && sp % 2 == 0;
-            const int vec_smp = reinterpret_cast<uintptr_t>(smp) % al == 0 && mp % 2 == 0;
-            typename K::Params p{static_cast<const InT*>(src), static_cast<const InT*>(smp), static_cast<C*>(ws), peaks,
+            typename K::Params p{static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp), static_cast<C*>(w.ws), w.peaks,
                                  static_cast<const C*>(plan->g_wcol.p), static_cast<const C*>(plan->g_lo.p),
                                  static_cast<const C*>(plan->g_hi.p), static_cast<const int*>(plan->g_p2f_col.p),
-                                 sh, sp, mp, vec_src, vec_smp};
-            const dim3 grid((sh.M2 + K::CT - 1) / K::CT, 2, pairs);
-            return launch(ctx, d, KC_COL_FWD, st, [&] {
-                launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), st, p);
+                                 sh, w.src_pitch, w.smp_pitch, vec_loads<InT>(w.src, w.src_pitch),
+                                 vec_loads<InT>(w.smp, w.smp_pitch)};
+            const dim3 grid((sh.M2 + K::CT - 1) / K::CT, 2, w.pairs);
+            return launch(w.ctx, w.d, KC_COL_FWD, w.st, [&] {
+                launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), w.st, p);
             });
         });
-    };
-    switch (dtype) {
-        case AUDIOSYNC_CUDA_F32: return go(float{});
-        case AUDIOSYNC_CUDA_F64: return go(double{});
-        case AUDIOSYNC_CUDA_S16: return go(int16_t{});
-    }
-    set_last_error("bad dtype %d", dtype);
-    return -1;
+    });
 }
 
 template <typename T, int NT>
-int GenStage<T, NT>::rows(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st) {
+int GenStage<T, NT>::rows(FftPlan* plan, const Wave& w) {
     typedef typename GenTraits<T>::C C;
     const GenShape& sh = plan->gen;
-    auto go = [&](auto KK) -> int {
-        using K = decltype(KK);
-        typename K::Params p{static_cast<C*>(ws), static_cast<const C*>(plan->g_wrow.p), static_cast<const C*>(plan->g_wpos.p),
+    return with_bool(plan->phat, [&](auto PHAT) -> int {
+        using K = GenRowFusedKernel<T, NT, decltype(PHAT)::value>;
+        typename K::Params p{static_cast<C*>(w.ws), static_cast<const C*>(plan->g_wrow.p), static_cast<const C*>(plan->g_wpos.p),
                              static_cast<const C*>(plan->g_lo.p), static_cast<const C*>(plan->g_hi.p),
                              static_cast<const int*>(plan->g_f2p_row.p), sh, static_cast<const C*>(plan->phat_rev.p),
                              static_cast<const C*>(plan->phat_lo.p), static_cast<const C*>(plan->phat_hi.p)};
-        const dim3 grid(sh.M1 / 2 + 1, 1, pairs);
-        return launch(ctx, d, KC_ROW_FUSED, st, [&] {
-            launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), st, p);
+        const dim3 grid(sh.M1 / 2 + 1, 1, w.pairs);
+        return launch(w.ctx, w.d, KC_ROW_FUSED, w.st, [&] {
+            launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), w.st, p);
         });
-    };
-    return plan->phat ? go(GenRowFusedKernel<T, NT, true>{}) : go(GenRowFusedKernel<T, NT>{});
+    });
 }
 
 template <typename T, int NT>
-int GenStage<T, NT>::col_inv(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, PairPeak* peaks, int pairs,
-                             cudaStream_t st, const RawWindow* win) {
+int GenStage<T, NT>::col_inv(FftPlan* plan, const Wave& w) {
     typedef typename GenTraits<T>::C C;
     const GenShape& sh = plan->gen;
-    C* planes = static_cast<C*>(ws);
+    C* planes = static_cast<C*>(w.ws);
     const int rc = gen_for_tile_width<T>(sh.ct, [&](auto CTC) -> int {
         auto go = [&](auto KK, auto fill) -> int {
             using K = decltype(KK);
-            typename K::Params p{planes, peaks, static_cast<const C*>(plan->g_wcol.p), static_cast<const int*>(plan->g_p2f_col.p),
+            typename K::Params p{planes, w.peaks, static_cast<const C*>(plan->g_wcol.p), static_cast<const int*>(plan->g_p2f_col.p),
                                  sh, reinterpret_cast<T*>(planes)};
             fill(p);
-            const dim3 grid(pairs, (sh.M2 + K::CT - 1) / K::CT, 1);
-            return launch(ctx, d, KC_COL_INV, st, [&] {
-                launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), st, p);
+            const dim3 grid(w.pairs, (sh.M2 + K::CT - 1) / K::CT, 1);
+            return launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
+                launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), w.st, p);
             });
         };
         constexpr int CT = decltype(CTC)::value;
         if constexpr (sizeof(T) == 4) {
-            if (win) return go(GenColInvKernel<T, CT, NT, true>{}, [&](auto& p) { p.win = *win; });
+            if (w.win) return go(GenColInvKernel<T, CT, NT, true>{}, [&](auto& p) { p.win = *w.win; });
         }
         return go(GenColInvKernel<T, CT, NT>{}, [](auto&) {});
     });
@@ -133,9 +120,9 @@ int GenStage<T, NT>::col_inv(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState
     if constexpr (sizeof(T) == 8) {
         // fp64: r[0 .. 2L) of pair i sits in its (dead) sample plane; full double keys
         const double* r = reinterpret_cast<const double*>(planes) + 2 * sh.M;
-        return launch(ctx, d, KC_ARGMAX_F64, st, [&] {
-            if (win) argmax_f64_window_kernel<<<pairs, 1024, 0, st>>>(r, 2 * sh.L, 4 * sh.M, peaks, *win);
-            else argmax_f64_kernel<<<pairs, 1024, 0, st>>>(r, 2 * sh.L, 4 * sh.M, peaks);
+        return launch(w.ctx, w.d, KC_ARGMAX_F64, w.st, [&] {
+            if (w.win) argmax_f64_window_kernel<<<w.pairs, 1024, 0, w.st>>>(r, 2 * sh.L, 4 * sh.M, w.peaks, *w.win);
+            else argmax_f64_kernel<<<w.pairs, 1024, 0, w.st>>>(r, 2 * sh.L, 4 * sh.M, w.peaks);
         });
     }
     return 0;

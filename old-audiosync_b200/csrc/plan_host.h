@@ -12,6 +12,7 @@
 #include <cstring>
 #include <functional>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "context.h"
@@ -21,6 +22,50 @@
 #include "gen_plan.h"
 
 namespace asc {
+
+// -------------------------------------------------------------------- wave
+// One launch wave of `pairs` pairs, as every plan's launchers take it.
+struct Wave {
+    audiosync_cuda_ctx* ctx;
+    DeviceState& d;
+    cudaStream_t st;
+    const void* src;
+    const void* smp;
+    int dtype;                  // what the transform loads: AUDIOSYNC_CUDA_F32 / F64 / S16
+    long long src_pitch;        // elements between consecutive pairs (0 with shared_src)
+    long long smp_pitch;
+    bool shared_src;            // every pair reads the one source at src
+    const void* spec;           // static plans: the shared source's forward rows (source_spectrum), else nullptr
+    void* ws;
+    PairPeak* peaks;
+    int pairs;
+    const RawWindow* win;       // lag window: nullptr for the unwindowed kernels
+};
+
+// f(float{}), f(double{}) or f(int16_t{}): the element type a transform loads for `dtype`.
+template <class F>
+static int with_input_type(int dtype, F&& f) {
+    switch (dtype) {
+        case AUDIOSYNC_CUDA_F32: return f(float{});
+        case AUDIOSYNC_CUDA_F64: return f(double{});
+        case AUDIOSYNC_CUDA_S16: return f(int16_t{});
+    }
+    set_last_error("bad dtype %d", dtype);
+    return -1;
+}
+
+// f(std::true_type{}) or f(std::false_type{}): a run-time choice as a template argument.
+template <class F>
+static int with_bool(bool b, F&& f) {
+    return b ? f(std::true_type{}) : f(std::false_type{});
+}
+
+// One load per packed point where every pair's base is aligned to two elements (a view at an odd
+// element offset, e.g. x[1:], is not: two element loads then).
+template <typename InT>
+static int vec_loads(const void* base, long long pitch) {
+    return reinterpret_cast<uintptr_t>(base) % (2 * sizeof(InT)) == 0 && pitch % 2 == 0;
+}
 
 // -------------------------------------------------------------------- plan
 struct FftPlan {
@@ -37,17 +82,11 @@ struct FftPlan {
     bool phat = false;                               // PHAT weighting in the split step (AUDIOSYNC_CUDA_WEIGHT_PHAT)
     DevBuf phat_rev, phat_lo, phat_hi;               // its twiddle w = W_N^k1 * phat_rev[e] (row kernel's position order)
     double peak_scale = 1.0;                         // r_reference = r_kernel * peak_scale
-    // enqueues the transform kernels for `pairs` pairs (planes/r in ws)
-    // (src, smp, dtype, src_pitch, smp_pitch [elements between pairs], workspace, peaks, pairs, stream,
-    //  lag window: nullptr for the unwindowed kernels, else the windowed twins of the argmax step)
-    std::function<int(audiosync_cuda_ctx*, DeviceState&, const void*, const void*, int, long long, long long,
-                      void*, PairPeak*, int, cudaStream_t, const RawWindow*)> run_wave;
-    // Static plans only: the reuse path of a batch whose pairs share one source.  source_spectrum
-    // (ctx, d, src, dtype, spec, peaks, stream) writes the source's forward rows into spec (M complex)
-    // once per call; run_shared_wave is run_wave with spec in place of the source and its pitch.
-    std::function<int(audiosync_cuda_ctx*, DeviceState&, const void*, int, void*, PairPeak*, cudaStream_t)> source_spectrum;
-    std::function<int(audiosync_cuda_ctx*, DeviceState&, const void*, const void*, int, long long,
-                      void*, PairPeak*, int, cudaStream_t, const RawWindow*)> run_shared_wave;
+    // enqueues the transform kernels of one wave (planes/r in ws)
+    std::function<int(const Wave&)> run_wave;
+    // Static plans only: writes the shared source's forward rows (M complex) into spec, once per
+    // call, for the waves that then reuse them.
+    std::function<int(const Wave&, void* spec)> source_spectrum;
     ~FftPlan() {
         col_tw.release(); col_tc.release(); row_tw.release(); row_rev.release(); row_tab.release(); m_lo.release(); m_hi.release();
         wm.release(); wn.release();
@@ -157,16 +196,14 @@ template <typename T, int NT>
 struct GenStage {
     static int prepare_cols(const GenShape& sh);
     static int prepare_rows(const GenShape& sh, bool phat);
-    static int col_fwd(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp, int dtype,
-                       long long sp, long long mp, void* ws, PairPeak* peaks, int pairs, cudaStream_t st);
-    static int rows(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st);
-    static int col_inv(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, PairPeak* peaks, int pairs,
-                       cudaStream_t st, const RawWindow* win);
+    static int col_fwd(FftPlan* plan, const Wave& w);
+    static int rows(FftPlan* plan, const Wave& w);
+    static int col_inv(FftPlan* plan, const Wave& w);
 };
 
 // static_rows.cu: the rows of a runtime-radix fp32 plan on a static row kernel (RowFusedKernel<RL, 0, NT>)
 // when the plan's M2 has one (GenShape::static_rows).  prepare: tables + kernel attributes.
 int static_rows_prepare(FftPlan* plan);
-int static_rows_launch(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st);
+int static_rows_launch(FftPlan* plan, const Wave& w);
 
 }  // namespace asc

@@ -6,77 +6,58 @@
 
 namespace asc {
 
-// K_A over `pairs` pairs.  SMP_ONLY: the sample planes alone (a shared-source wave); otherwise
+// K_A over the wave's pairs.  SMP_ONLY: the sample planes alone (a shared-source wave); otherwise
 // `signals` = 2 (source and sample) or 1 (the source alone: one pair whose plane 0 is a shared
 // source's column pass).
 template <class P, bool SMP_ONLY>
-static int static_col_fwd(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
-                          int dtype, long long src_pitch, long long smp_pitch, cplx* planes, PairPeak* peaks, int pairs,
-                          int signals, cudaStream_t st) {
+static int static_col_fwd(FftPlan* plan, const Wave& w, int signals) {
     using Col = typename P::Col;
     using Row = typename P::Row;
     constexpr int M1 = Col::n, M2 = Row::n;
+    cplx* planes = static_cast<cplx*>(w.ws);
     const cplx* col_tw = static_cast<const cplx*>(plan->col_tw.p);
     const cplx* col_tc = static_cast<const cplx*>(plan->col_tc.p);
     const cplx* m_lo = static_cast<const cplx*>(plan->m_lo.p);
     const cplx* m_hi = static_cast<const cplx*>(plan->m_hi.p);
-    const dim3 grid_a(M2 / COL_T, SMP_ONLY ? 1 : signals, pairs);
+    const dim3 grid_a(M2 / COL_T, SMP_ONLY ? 1 : signals, w.pairs);
     auto col_fwd = [&](auto KK, const typename decltype(KK)::Params& p) -> int {
         using K = decltype(KK);
-        return launch(ctx, d, KC_COL_FWD, st, [&] {
-            launch_stage(fft_kernel_entry<K>, grid_a, dim3(K::THREADS), K::SMEM, st, p);
+        return launch(w.ctx, w.d, KC_COL_FWD, w.st, [&] {
+            launch_stage(fft_kernel_entry<K>, grid_a, dim3(K::THREADS), K::SMEM, w.st, p);
         });
     };
-    // register path: one load per packed point where every pair's base is aligned to two elements
-    // (a view at an odd element offset, e.g. x[1:], is not: two element loads then)
-    auto vec_ok = [](const void* p, long long pitch, size_t esz) -> int {
-        return reinterpret_cast<uintptr_t>(p) % (2 * esz) == 0 && pitch % 2 == 0;
-    };
-    if (dtype == AUDIOSYNC_CUDA_F32) {
-        // TMA boxes need 16-byte aligned rows: every pair / row offset is a multiple of 16 bytes,
-        // so only the base pointers decide.  Other fp32 inputs load through registers.
-        const bool src_aligned = SMP_ONLY || ((reinterpret_cast<uintptr_t>(src) & 15u) == 0 && src_pitch % 4 == 0);
-        const bool aligned = src_aligned && (reinterpret_cast<uintptr_t>(smp) & 15u) == 0 && smp_pitch % 4 == 0;
-        const float* s_in = static_cast<const float*>(src);
-        const float* m_in = static_cast<const float*>(smp);
-        using KT = ColFwdKernel<Col, Row::n, P::NT_COL, float, true, SMP_ONLY>;
-        using KR = ColFwdKernel<Col, Row::n, P::NT_COL, float, false, SMP_ONLY>;
-        typename KT::Params pt{s_in, m_in, planes, peaks, col_tw, col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch};
-        const bool tma = aligned &&
-                         (SMP_ONLY || make_tile_map(&pt.tm_src, s_in, M2, M1, (size_t)src_pitch * sizeof(float), (size_t)pairs,
-                                                    tile_box_rows(KT::SRC_ROWS)) == 0) &&
-                         make_tile_map(&pt.tm_smp, m_in, M2, M1 / 2, (size_t)smp_pitch * sizeof(float), (size_t)pairs,
-                                       tile_box_rows(KT::SMP_ROWS)) == 0;
-        return tma ? col_fwd(KT{}, pt)
-                   : col_fwd(KR{}, {s_in, m_in, planes, peaks, col_tw, col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch,
-                                    vec_ok(src, src_pitch, sizeof(float)), vec_ok(smp, smp_pitch, sizeof(float))});
-    } else if (dtype == AUDIOSYNC_CUDA_F64) {
-        using K = ColFwdKernel<Col, Row::n, P::NT_COL, double, false, SMP_ONLY>;
-        return col_fwd(K{}, {static_cast<const double*>(src), static_cast<const double*>(smp), planes, peaks, col_tw,
-                             col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch, vec_ok(src, src_pitch, sizeof(double)),
-                             vec_ok(smp, smp_pitch, sizeof(double))});
-    } else if (dtype == AUDIOSYNC_CUDA_S16) {
-        const int vec_src = vec_ok(src, src_pitch, sizeof(int16_t));
-        const int vec_smp = vec_ok(smp, smp_pitch, sizeof(int16_t));
-        using K = ColFwdKernel<Col, Row::n, P::NT_COL, int16_t, false, SMP_ONLY>;
-        return col_fwd(K{}, {static_cast<const int16_t*>(src), static_cast<const int16_t*>(smp), planes, peaks, col_tw,
-                             col_tc, m_lo, m_hi, P::L, src_pitch, smp_pitch, vec_src, vec_smp});
-    }
-    set_last_error("bad dtype %d", dtype);
-    return -1;
+    return with_input_type(w.dtype, [&](auto IN) -> int {
+        using InT = decltype(IN);
+        const InT* s_in = static_cast<const InT*>(w.src);
+        const InT* m_in = static_cast<const InT*>(w.smp);
+        if constexpr (std::is_same<InT, float>::value) {
+            // TMA boxes need 16-byte aligned rows: every pair / row offset is a multiple of 16 bytes,
+            // so only the base pointers decide.  Other fp32 inputs load through registers.
+            const bool src_aligned = SMP_ONLY || ((reinterpret_cast<uintptr_t>(w.src) & 15u) == 0 && w.src_pitch % 4 == 0);
+            const bool aligned = src_aligned && (reinterpret_cast<uintptr_t>(w.smp) & 15u) == 0 && w.smp_pitch % 4 == 0;
+            using KT = ColFwdKernel<Col, Row::n, P::NT_COL, float, true, SMP_ONLY>;
+            typename KT::Params pt{s_in, m_in, planes, w.peaks, col_tw, col_tc, m_lo, m_hi, P::L, w.src_pitch, w.smp_pitch};
+            const bool tma = aligned &&
+                             (SMP_ONLY || make_tile_map(&pt.tm_src, s_in, M2, M1, (size_t)w.src_pitch * sizeof(float),
+                                                        (size_t)w.pairs, tile_box_rows(KT::SRC_ROWS)) == 0) &&
+                             make_tile_map(&pt.tm_smp, m_in, M2, M1 / 2, (size_t)w.smp_pitch * sizeof(float), (size_t)w.pairs,
+                                           tile_box_rows(KT::SMP_ROWS)) == 0;
+            if (tma) return col_fwd(KT{}, pt);
+        }
+        using K = ColFwdKernel<Col, Row::n, P::NT_COL, InT, false, SMP_ONLY>;
+        return col_fwd(K{}, {s_in, m_in, planes, w.peaks, col_tw, col_tc, m_lo, m_hi, P::L, w.src_pitch, w.smp_pitch,
+                             vec_loads<InT>(w.src, w.src_pitch), vec_loads<InT>(w.smp, w.smp_pitch)});
+    });
 }
 
-// One wave.  SHARED: the pairs share one source whose forward rows source_spectrum left in `spec`
-// (src and src_pitch are then unused): K_A on the samples, the shared-source K_B, K_C.
+// One wave.  SHARED: the pairs share one source whose forward rows source_spectrum left in w.spec
+// (the source itself is not read): K_A on the samples, the shared-source K_B, K_C.
 template <class P, bool SHARED>
-static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d,
-                           const void* src, const void* smp, int dtype, long long src_pitch,
-                           long long smp_pitch, void* ws, PairPeak* peaks, int pairs, cudaStream_t st,
-                           const RawWindow* win, const cplx* spec) {
+static int run_static_wave(FftPlan* plan, const Wave& w) {
     using Col = typename P::Col;
     using Row = typename P::Row;
     constexpr int M1 = Col::n, M2 = Row::n;
-    cplx* planes = static_cast<cplx*>(ws);
+    cplx* planes = static_cast<cplx*>(w.ws);
     const cplx* col_tw = static_cast<const cplx*>(plan->col_tw.p);
     const cplx* row_tw = static_cast<const cplx*>(plan->row_tw.p);
     const cplx* row_rev = static_cast<const cplx*>(plan->row_rev.p);
@@ -86,26 +67,25 @@ static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& 
     // K_C always stages its tiles through the TMA unit: its map is encoded before anything is
     // enqueued, so that a failure leaves no partial wave behind
     using KC = ColInvKernel<Col, Row::n, P::NT_COL>;
-    typename KC::Params pc{planes, peaks, col_tw, P::L};
-    if (make_tile_map(&pc.tm, planes, M2, M1, (size_t)P::L * sizeof(cplx), (size_t)2 * pairs,
+    typename KC::Params pc{planes, w.peaks, col_tw, P::L};
+    if (make_tile_map(&pc.tm, planes, M2, M1, (size_t)P::L * sizeof(cplx), (size_t)2 * w.pairs,
                       tile_box_rows(KC::TMA_ROWS)) != 0) {
         set_last_error("L = %lld: cuTensorMapEncodeTiled %s for the workspace planes", P::L,
                        tensor_map_encoder() ? "failed" : "is not exported by the driver");
         return -1;
     }
-    if (static_col_fwd<P, SHARED>(plan, ctx, d, src, smp, dtype, src_pitch, smp_pitch, planes, peaks, pairs, 2, st) != 0)
-        return -1;
+    if (static_col_fwd<P, SHARED>(plan, w, 2) != 0) return -1;
     {
         constexpr int MODE = SHARED ? ROWS_SHARED_SRC : ROWS_PAIR;
         auto rows = [&](auto KK, const cplx* rev, const cplx* lo, const cplx* hi) -> int {
             using K = decltype(KK);
             const typename K::PairParams base{planes, row_tw, rev, lo, hi, P::L, row_tab};
             typename K::Params p;
-            if constexpr (SHARED) p = {base, spec};
+            if constexpr (SHARED) p = {base, static_cast<const cplx*>(w.spec)};
             else p = base;
-            const dim3 grid(M1 / 2 + 1, 1, pairs);
-            return launch(ctx, d, KC_ROW_FUSED, st, [&] {
-                launch_stage(fft_kernel_entry<K>, grid, dim3(K::THREADS), K::SMEM, st, p);
+            const dim3 grid(M1 / 2 + 1, 1, w.pairs);
+            return launch(w.ctx, w.d, KC_ROW_FUSED, w.st, [&] {
+                launch_stage(fft_kernel_entry<K>, grid, dim3(K::THREADS), K::SMEM, w.st, p);
             });
         };
         if ((plan->phat ? rows(RowFusedKernel<Row, Col::n, P::NT_ROW, true, MODE>{}, static_cast<const cplx*>(plan->phat_rev.p),
@@ -114,15 +94,15 @@ static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& 
             return -1;
     }
     {
-        const dim3 grid(pairs, M2 / COL_T, 1);
-        if (win) {
+        const dim3 grid(w.pairs, M2 / COL_T, 1);
+        if (w.win) {
             using KCW = ColInvKernel<Col, Row::n, P::NT_COL, true, true>;
-            typename KCW::Params pw{planes, peaks, col_tw, P::L, *win, pc.tm};
-            if (launch(ctx, d, KC_COL_INV, st, [&] {
-                    launch_stage(fft_kernel_entry<KCW>, grid, dim3(KCW::THREADS), KCW::SMEM, st, pw);
+            typename KCW::Params pw{planes, w.peaks, col_tw, P::L, *w.win, pc.tm};
+            if (launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
+                    launch_stage(fft_kernel_entry<KCW>, grid, dim3(KCW::THREADS), KCW::SMEM, w.st, pw);
                 }) != 0) return -1;
-        } else if (launch(ctx, d, KC_COL_INV, st, [&] {
-                       launch_stage(fft_kernel_entry<KC>, grid, dim3(KC::THREADS), KC::SMEM, st, pc);
+        } else if (launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
+                       launch_stage(fft_kernel_entry<KC>, grid, dim3(KC::THREADS), KC::SMEM, w.st, pc);
                    }) != 0) return -1;
     }
     return 0;
@@ -131,17 +111,17 @@ static int run_static_wave(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& 
 // The shared source's forward rows, once per call: K_A on the source alone as one pair (plane 0 of
 // that pair is `spec`), then the forward passes of its rows in place.
 template <class P>
-static int static_source_spectrum(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, int dtype,
-                                  cplx* spec, PairPeak* peaks, cudaStream_t st) {
+static int static_source_spectrum(FftPlan* plan, const Wave& w, cplx* spec) {
     using Col = typename P::Col;
     using Row = typename P::Row;
-    if (static_col_fwd<P, false>(plan, ctx, d, src, src, dtype, 2 * P::L, 2 * P::L, spec, peaks, 1, 1, st) != 0) return -1;
+    const Wave src_pair{w.ctx, w.d, w.st, w.src, w.src, w.dtype, 2 * P::L, 2 * P::L, false, nullptr, spec, w.peaks, 1, nullptr};
+    if (static_col_fwd<P, false>(plan, src_pair, 1) != 0) return -1;
     using K = RowFusedKernel<Row, Col::n, P::NT_ROW, false, ROWS_SRC_SPECTRUM>;
     typename K::Params p{spec, static_cast<const cplx*>(plan->row_tw.p), static_cast<const cplx*>(plan->row_rev.p),
                          static_cast<const cplx*>(plan->m_lo.p), static_cast<const cplx*>(plan->m_hi.p), P::L,
                          static_cast<const cplx*>(plan->row_tab.p)};
-    return launch(ctx, d, KC_SRC_SPECTRUM, st, [&] {
-        launch_stage(fft_kernel_entry<K>, dim3(Col::n / 2 + 1, 1, 1), dim3(K::THREADS), K::SMEM, st, p);
+    return launch(w.ctx, w.d, KC_SRC_SPECTRUM, w.st, [&] {
+        launch_stage(fft_kernel_entry<K>, dim3(Col::n / 2 + 1, 1, 1), dim3(K::THREADS), K::SMEM, w.st, p);
     });
 }
 
@@ -203,20 +183,11 @@ int build_static_plan(FftPlan* plan) {
         prepare_kernel<KSs>(KSs::SMEM) != 0 || prepare_kernel<KBspec>(KBspec::SMEM) != 0 ||
         (plan->phat ? prepare_kernel<KBPs>(KBPs::SMEM) : prepare_kernel<KBs>(KBs::SMEM)) != 0)
         return -1;
-    plan->run_wave = [plan](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, const void* smp,
-                            int dtype, long long sp, long long mp, void* ws, PairPeak* peaks, int pairs,
-                            cudaStream_t st, const RawWindow* win) {
-        return run_static_wave<P, false>(plan, ctx, d, src, smp, dtype, sp, mp, ws, peaks, pairs, st, win, nullptr);
+    plan->run_wave = [plan](const Wave& w) {
+        return w.spec ? run_static_wave<P, true>(plan, w) : run_static_wave<P, false>(plan, w);
     };
-    plan->source_spectrum = [plan](audiosync_cuda_ctx* ctx, DeviceState& d, const void* src, int dtype, void* spec,
-                                   PairPeak* peaks, cudaStream_t st) {
-        return static_source_spectrum<P>(plan, ctx, d, src, dtype, static_cast<cplx*>(spec), peaks, st);
-    };
-    plan->run_shared_wave = [plan](audiosync_cuda_ctx* ctx, DeviceState& d, const void* spec, const void* smp,
-                                   int dtype, long long mp, void* ws, PairPeak* peaks, int pairs,
-                                   cudaStream_t st, const RawWindow* win) {
-        return run_static_wave<P, true>(plan, ctx, d, nullptr, smp, dtype, 0, mp, ws, peaks, pairs, st, win,
-                                        static_cast<const cplx*>(spec));
+    plan->source_spectrum = [plan](const Wave& w, void* spec) {
+        return static_source_spectrum<P>(plan, w, static_cast<cplx*>(spec));
     };
     return 0;
 }

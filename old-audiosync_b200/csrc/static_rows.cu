@@ -29,20 +29,19 @@ struct StaticRows {
         return prepare_kernel<KP>(KP::SMEM);
     }
     template <class KK>
-    static int launch_k(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st,
-                        const DevBuf& rev, const DevBuf& lo, const DevBuf& hi) {
+    static int launch_k(FftPlan* plan, const Wave& w, const DevBuf& rev, const DevBuf& lo, const DevBuf& hi) {
         const GenShape& sh = plan->gen;
-        typename KK::Params p{static_cast<cplx*>(ws), static_cast<const cplx*>(plan->row_tw.p),
+        typename KK::Params p{static_cast<cplx*>(w.ws), static_cast<const cplx*>(plan->row_tw.p),
                               static_cast<const cplx*>(rev.p), static_cast<const cplx*>(lo.p),
                               static_cast<const cplx*>(hi.p), sh.M, static_cast<const cplx*>(plan->row_tab.p), sh.M1};
-        const dim3 grid(sh.M1 / 2 + 1, 1, pairs);
-        return launch(ctx, d, KC_ROW_FUSED, st, [&] {
-            launch_stage(fft_kernel_entry<KK>, grid, dim3(KK::THREADS), KK::SMEM, st, p);
+        const dim3 grid(sh.M1 / 2 + 1, 1, w.pairs);
+        return launch(w.ctx, w.d, KC_ROW_FUSED, w.st, [&] {
+            launch_stage(fft_kernel_entry<KK>, grid, dim3(KK::THREADS), KK::SMEM, w.st, p);
         });
     }
-    static int launch_rows(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st) {
-        return plan->phat ? launch_k<KP>(plan, ctx, d, ws, pairs, st, plan->phat_rev, plan->phat_lo, plan->phat_hi)
-                          : launch_k<K>(plan, ctx, d, ws, pairs, st, plan->row_rev, plan->m_lo, plan->m_hi);
+    static int launch_rows(FftPlan* plan, const Wave& w) {
+        return plan->phat ? launch_k<KP>(plan, w, plan->phat_rev, plan->phat_lo, plan->phat_hi)
+                          : launch_k<K>(plan, w, plan->row_rev, plan->m_lo, plan->m_hi);
     }
 };
 
@@ -63,8 +62,8 @@ int static_rows_prepare(FftPlan* plan) {
     return for_static_rows(plan->gen.M2, [&](auto S) { return decltype(S)::prepare(plan); });
 }
 
-int static_rows_launch(FftPlan* plan, audiosync_cuda_ctx* ctx, DeviceState& d, void* ws, int pairs, cudaStream_t st) {
-    return for_static_rows(plan->gen.M2, [&](auto S) { return decltype(S)::launch_rows(plan, ctx, d, ws, pairs, st); });
+int static_rows_launch(FftPlan* plan, const Wave& w) {
+    return for_static_rows(plan->gen.M2, [&](auto S) { return decltype(S)::launch_rows(plan, w); });
 }
 
 }  // namespace asc
