@@ -229,6 +229,46 @@ int audiosync_cuda_xcorr_shared_source_device(audiosync_cuda_ctx *ctx, int devic
                                               const void *d_samples, size_t n_pairs, size_t sample_len,
                                               int dtype, audiosync_cuda_result *d_results, void *stream);
 
+/* The batch call that also returns the correlation r each record's peak is taken from, over a range of
+ * lags, for what the one argmax cannot give: sub-sample delay by interpolation around the peak, the
+ * runner-up lag, sums over channels before picking a peak, plots, a caller's own acceptance rule.
+ *   shared_source = 0: the inputs of xcorr_batch_results / xcorr_batch_device; 1: those of
+ *   xcorr_shared_source / xcorr_shared_source_device (one source of 2*sample_len elements).
+ *   results[i] is, byte for byte, the record the matching call returns for the same inputs and settings.
+ *   corr: [n_pairs][W] row-major doubles, W = corr_hi - corr_lo + 1 (a host array for the first call, a
+ *   device array on `device` for the second); corr[i][j] is pair i's correlation at the folded lag
+ *   corr_lo + j, that is at raw index lag for lag >= 0 and lag + 2L below.
+ *   The value is the one the record's peak search compared, at the record's scale: unnormalised (x N,
+ *   like FFTW's c2r), the whitened r_w under PHAT; on fp32 plans (double) of the kernel's fp32 value
+ *   times the plan's scale, the operation that gives the record's peak; the fp64 value on precise and
+ *   direct plans.  So corr[i][record.lag - corr_lo] == record.peak bit for bit when the lag is in the
+ *   range, and the argmax rule (with the lag window's restriction) over a range that holds every searched
+ *   lag gives the record's raw_index, peak and second exactly.
+ *   The range does not depend on the lag window: the window restricts the search, [corr_lo, corr_hi]
+ *   says what is written; either may be wider than, narrower than or disjoint from the other.
+ *   Every setting the batch calls honour applies, with the same refusals: dtype, memspace, path, precise
+ *   mode, weighting, lag window, wave size, host narrowing and several devices.  Under LOSSLESS
+ *   narrowing corr equals the NARROW_OFF call's; under ALWAYS it answers for the fp32 batch, as the
+ *   records do.
+ *   Returns -1 with a message, writing no record and no corr element, when corr_lo > corr_hi,
+ *   corr_lo < -sample_len or corr_hi > sample_len - 1 (no clamping: the caller's array is always
+ *   n_pairs * W), corr is NULL with n_pairs > 0, a device corr is not 8-byte aligned, or the matching
+ *   batch call refuses.  n_pairs == 0 returns 0 and launches nothing.
+ *   The host-facing call, in both memspaces, stages corr on the device in pieces of at most 256 MB per
+ *   device (one row where a row is larger) and copies each back behind its kernels.
+ * The static, runtime-radix fp32 and single-CTA plans store r in the inverse pass that computes it
+ * (kernel class "col_inv_argmax" / "small_fft"); precise and direct plans copy it from their workspace
+ * (kernel class "corr_out").  The drop-in call and pool_run do not export. */
+int audiosync_cuda_xcorr_correlation(audiosync_cuda_ctx *ctx, const void *sources, const void *samples,
+                                     size_t n_pairs, size_t sample_len, int dtype, int memspace,
+                                     int shared_source, int64_t corr_lo, int64_t corr_hi,
+                                     audiosync_cuda_result *results, double *corr);
+/* Stream-ordered form on device pointers of one device of the context (as xcorr_batch_device). */
+int audiosync_cuda_xcorr_correlation_device(audiosync_cuda_ctx *ctx, int device, const void *d_sources,
+                                            const void *d_samples, size_t n_pairs, size_t sample_len, int dtype,
+                                            int shared_source, int64_t corr_lo, int64_t corr_hi,
+                                            audiosync_cuda_result *d_results, double *d_corr, void *stream);
+
 /* ------------------------------------------------------------------------
  * Session pool (SURVEY 8f rank 1): many concurrent audiosync sessions on one device.
  * Each slot owns device-resident source / sample buffers that grow as audio arrives

@@ -52,6 +52,7 @@ EXPORTED_SYMBOLS = [
     "audiosync_cuda_create", "audiosync_cuda_destroy", "audiosync_cuda_device_count",
     "audiosync_cuda_xcorr_batch", "audiosync_cuda_xcorr_batch_results", "audiosync_cuda_xcorr_batch_device",
     "audiosync_cuda_xcorr_shared_source", "audiosync_cuda_xcorr_shared_source_device",
+    "audiosync_cuda_xcorr_correlation", "audiosync_cuda_xcorr_correlation_device",
     "audiosync_cuda_synth_pairs", "audiosync_cuda_synchronize",
     "audiosync_cuda_set_path", "audiosync_cuda_set_wave_pairs", "audiosync_cuda_set_debug", "audiosync_cuda_set_precise", "audiosync_cuda_set_weighting",
     "audiosync_cuda_set_lag_window",
@@ -118,6 +119,10 @@ def lib() -> C.CDLL:
     L.audiosync_cuda_xcorr_shared_source.argtypes = [vp, vp, vp, sz, sz, i32, i32, vp]
     L.audiosync_cuda_xcorr_shared_source_device.restype = i32
     L.audiosync_cuda_xcorr_shared_source_device.argtypes = [vp, i32, vp, vp, sz, sz, i32, vp, vp]
+    L.audiosync_cuda_xcorr_correlation.restype = i32
+    L.audiosync_cuda_xcorr_correlation.argtypes = [vp, vp, vp, sz, sz, i32, i32, i32, C.c_int64, C.c_int64, vp, vp]
+    L.audiosync_cuda_xcorr_correlation_device.restype = i32
+    L.audiosync_cuda_xcorr_correlation_device.argtypes = [vp, i32, vp, vp, sz, sz, i32, i32, C.c_int64, C.c_int64, vp, vp, vp]
     L.audiosync_cuda_synth_pairs.restype = i32
     L.audiosync_cuda_synth_pairs.argtypes = [vp, i32, u64, u64, sz, sz, i32, vp, vp, vp]
     L.audiosync_cuda_synchronize.restype = i32
@@ -610,6 +615,99 @@ class Context:
         if not sync:
             return out
         return out[: n * RESULT_DTYPE.itemsize].cpu().numpy().view(RESULT_DTYPE)
+
+    # -- correlation export -----------------------------------------------------
+    def xcorr_correlation(self, sources: np.ndarray, samples: np.ndarray, lo: int | None = None,
+                          hi: int | None = None, shared_source: bool = False):
+        """The batch call that also returns the correlation over the folded lags [lo, hi] (None: -L / L - 1).
+
+        ``sources`` [n][2L] (or, with ``shared_source``, one source of at least 2L elements) and ``samples``
+        [n][L], float32, float64 or int16 host arrays.  Returns ``(records, corr)``: the records are those of
+        ``xcorr_batch_records`` / ``xcorr_shared_source`` bit for bit, ``corr`` a float64 [n, hi - lo + 1]
+        array whose row i holds pair i's correlation at lags lo .. hi, at the records' scale (see
+        include/audiosync_cuda.h)."""
+        if sources.dtype != samples.dtype or sources.dtype not in _NP_DTYPES:
+            raise TypeError("sources/samples must both be float32, float64 or int16")
+        if samples.ndim != 2:
+            raise ValueError("expected samples [n][L]")
+        n, L = samples.shape
+        if shared_source:
+            if sources.ndim != 1 or sources.shape[0] < 2 * L:
+                raise ValueError("expected source [>= 2L] and samples [n][L]")
+            sources = sources[: 2 * L]
+        elif sources.ndim != 2 or sources.shape != (n, 2 * L):
+            raise ValueError("expected sources [n][2L] and samples [n][L]")
+        sources = np.ascontiguousarray(sources)
+        samples = np.ascontiguousarray(samples)
+        lo = -L if lo is None else int(lo)
+        hi = L - 1 if hi is None else int(hi)
+        res = np.zeros(n, RESULT_DTYPE)
+        corr = np.empty((n, max(hi - lo + 1, 0)), np.float64)
+        rc = lib().audiosync_cuda_xcorr_correlation(self._h, sources.ctypes.data, samples.ctypes.data, n, L,
+                                                    _NP_DTYPES[sources.dtype], HOST, 1 if shared_source else 0,
+                                                    lo, hi, res.ctypes.data, corr.ctypes.data)
+        self._check(rc, "xcorr_correlation")
+        return res, corr
+
+    def xcorr_correlation_torch(self, sources, samples, lo: int | None = None, hi: int | None = None, out=None,
+                                corr=None, shared_source: bool = False, sync: bool = True):
+        """``xcorr_correlation`` on torch CUDA tensors, zero copy, on torch's current stream: ``sources``
+        [n, 2L] (``shared_source``: 1-D, at least 2L elements) and ``samples`` [n, L] of one dtype on one
+        device of this context.  ``corr`` (a float64 CUDA tensor of n * W elements, allocated when omitted)
+        receives the correlation and is returned as [n, W]; ``out`` and ``sync`` as in ``xcorr_batch_torch``
+        (with ``sync`` the records come back as a NumPy array, else the uint8 device tensor):
+        returns ``(records, corr)``."""
+        import torch
+        if not (sources.is_cuda and samples.is_cuda) or sources.device != samples.device:
+            raise ValueError("sources and samples must be CUDA tensors on the same device")
+        dts = {torch.float32: F32, torch.float64: F64, torch.int16: S16}
+        if sources.dtype != samples.dtype or sources.dtype not in dts:
+            raise TypeError("sources/samples must both be float32, float64 or int16")
+        if samples.dim() != 2:
+            raise ValueError("expected samples [n, L]")
+        n, L = samples.shape
+        if shared_source:
+            if sources.dim() != 1 or sources.shape[0] < 2 * L:
+                raise ValueError("expected source [>= 2L] and samples [n, L]")
+        elif sources.dim() != 2 or tuple(sources.shape) != (n, 2 * L):
+            raise ValueError("expected sources [n, 2L] and samples [n, L]")
+        if not (sources.is_contiguous() and samples.is_contiguous()):
+            raise ValueError("tensors must be contiguous (no hidden copies on this path)")
+        lo = -L if lo is None else int(lo)
+        hi = L - 1 if hi is None else int(hi)
+        W = max(hi - lo + 1, 0)
+        dev = sources.device
+        if out is None:
+            out = torch.empty(n * RESULT_DTYPE.itemsize, dtype=torch.uint8, device=dev)
+        elif out.device != dev or out.dtype != torch.uint8 or out.numel() < n * RESULT_DTYPE.itemsize:
+            raise ValueError("out must be a uint8 tensor of n * 64 bytes on the same device")
+        if corr is None:
+            corr = torch.empty(n * W, dtype=torch.float64, device=dev)
+        elif corr.device != dev or corr.dtype != torch.float64 or corr.numel() < n * W or not corr.is_contiguous():
+            raise ValueError("corr must be a contiguous float64 tensor of n * W elements on the same device")
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        if stream == 0:
+            # as in xcorr_batch_torch: a NULL handle selects the library's own stream
+            torch.cuda.current_stream(dev).synchronize()
+        if n:
+            self.xcorr_correlation_device(dev.index, sources.data_ptr(), samples.data_ptr(), n, L, dts[sources.dtype],
+                                          lo, hi, out.data_ptr(), corr.data_ptr(), stream, shared_source)
+        if stream == 0:
+            self.synchronize(dev.index)
+        corr = corr[: n * W].view(n, W)
+        if not sync:
+            return out, corr
+        return out[: n * RESULT_DTYPE.itemsize].cpu().numpy().view(RESULT_DTYPE), corr
+
+    def xcorr_correlation_device(self, device: int, d_sources: int, d_samples: int, n_pairs: int, sample_len: int,
+                                 dtype: int, lo: int, hi: int, d_results: int, d_corr: int, stream: int = 0,
+                                 shared_source: bool = False):
+        """Stream-ordered correlation export on device pointers: records into ``d_results``, the
+        [n_pairs][hi - lo + 1] doubles into ``d_corr``; dtype F32, F64 or S16."""
+        rc = lib().audiosync_cuda_xcorr_correlation_device(self._h, device, d_sources, d_samples, n_pairs, sample_len,
+                                                           dtype, 1 if shared_source else 0, int(lo), int(hi),
+                                                           d_results, d_corr, stream or None)
+        self._check(rc, "xcorr_correlation_device")
 
     # -- stream-ordered device calls --------------------------------------------
     def xcorr_batch_device(self, device: int, d_sources: int, d_samples: int, n_pairs: int,

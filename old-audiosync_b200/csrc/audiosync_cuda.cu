@@ -55,7 +55,7 @@ static bool debug_on() { return g_debug_flag || (&global_debug != nullptr && glo
 const char* kernel_class_name(int k) {
     static const char* names[KC_COUNT] = {
         "synth", "direct_corr", "argmax_f64", "col_fwd", "row_fused",
-        "col_inv_argmax", "small_fft", "pearson", "src_spectrum"};
+        "col_inv_argmax", "small_fft", "pearson", "src_spectrum", "corr_out"};
     return (k >= 0 && k < KC_COUNT) ? names[k] : "?";
 }
 
@@ -95,14 +95,27 @@ static int with_small_kernel(int dtype, bool phat, bool win, bool shared_src, F&
     });
 }
 
-template <typename InT, bool PHAT, bool WIN, bool SHARED>
+// f(InT{}, PHAT, SHARED_SRC): the exporting twin SmallXcorrKernel<InT, PHAT, true, SHARED_SRC, true>
+template <class F>
+static int with_small_out_kernel(int dtype, bool phat, bool shared_src, F&& f) {
+    return with_input_type(dtype, [&](auto IN) {
+        return with_bool(phat, [&](auto PHAT) {
+            return with_bool(shared_src, [&](auto SHARED) { return f(IN, PHAT, SHARED); });
+        });
+    });
+}
+
+template <typename InT, bool PHAT, bool WIN, bool SHARED, bool OUT = false>
 static int run_small_wave(FftPlan* plan, const Wave& w) {
-    using K = SmallXcorrKernel<InT, PHAT, WIN, SHARED>;
-    typename K::Params p{static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp), w.peaks,
+    using K = SmallXcorrKernel<InT, PHAT, WIN, SHARED, OUT>;
+    typename K::Params p{};
+    static_cast<typename K::PlainParams&>(p) = {static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp), w.peaks,
                          static_cast<const cplx*>(plan->wm.p), static_cast<const cplx*>(plan->wn.p),
                          plan->small, w.src_pitch, w.smp_pitch, vec_loads<InT>(w.src, w.src_pitch),
                          vec_loads<InT>(w.smp, w.smp_pitch)};
-    if constexpr (WIN) p.win = *w.win;
+    // the exporting twin runs the windowed argmax, over all of [0, 2L) when no window is set
+    if constexpr (OUT) p.corr = *w.corr;
+    if constexpr (WIN) p.win = w.win ? *w.win : full_window(plan->L);
     const size_t smem = K::smem_bytes(plan->small.M);
     const dim3 grid(1, 1, w.pairs);
     return launch(w.ctx, w.d, KC_SMALL_FFT, w.st, [&] {
@@ -129,12 +142,23 @@ static int build_small_plan(FftPlan* plan, long long L) {
             ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
             return 0;
         };
+        auto allow_out = [&](auto IN, auto PHAT, auto SHARED) -> int {
+            using K = SmallXcorrKernel<decltype(IN), decltype(PHAT)::value, true, decltype(SHARED)::value, true>;
+            ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
+            return 0;
+        };
         for (int dtype : {AUDIOSYNC_CUDA_F32, AUDIOSYNC_CUDA_F64, AUDIOSYNC_CUDA_S16})
-            for (bool win : {false, true})
-                for (bool shared_src : {false, true})
+            for (bool shared_src : {false, true}) {
+                for (bool win : {false, true})
                     if (with_small_kernel(dtype, plan->phat, win, shared_src, allow) != 0) return -1;
+                if (with_small_out_kernel(dtype, plan->phat, shared_src, allow_out) != 0) return -1;
+            }
     }
     plan->run_wave = [plan](const Wave& w) {
+        if (w.corr)
+            return with_small_out_kernel(w.dtype, plan->phat, w.shared_src, [&](auto IN, auto PHAT, auto SHARED) {
+                return run_small_wave<decltype(IN), decltype(PHAT)::value, true, decltype(SHARED)::value, true>(plan, w);
+            });
         return with_small_kernel(w.dtype, plan->phat, w.win != nullptr, w.shared_src, [&](auto IN, auto PHAT, auto WIN, auto SHARED) {
             return run_small_wave<decltype(IN), decltype(PHAT)::value, decltype(WIN)::value, decltype(SHARED)::value>(plan, w);
         });
@@ -197,9 +221,31 @@ static int run_direct_wave(FftPlan* plan, const Wave& w) {
             direct_corr_kernel<InT><<<grid, DIRECT_TILE, 0, w.st>>>(static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp),
                                                                     r, L, w.src_pitch, w.smp_pitch);
         }) != 0) return -1;
-    return launch(w.ctx, w.d, KC_ARGMAX_F64, w.st, [&] {
-        if (w.win) argmax_f64_window_kernel<<<w.pairs, 1024, 0, w.st>>>(r, N, N, w.peaks, *w.win);
-        else argmax_f64_kernel<<<w.pairs, 1024, 0, w.st>>>(r, N, N, w.peaks);
+    if (launch(w.ctx, w.d, KC_ARGMAX_F64, w.st, [&] {
+            if (w.win) argmax_f64_window_kernel<<<w.pairs, 1024, 0, w.st>>>(r, N, N, w.peaks, *w.win);
+            else argmax_f64_kernel<<<w.pairs, 1024, 0, w.st>>>(r, N, N, w.peaks);
+        }) != 0)
+        return -1;
+    return w.corr ? launch_corr_gather(w, r, N) : 0;
+}
+
+// The correlation export of the plans whose r is in the workspace (precise and direct): out[pair][j]
+// = r[raw(j)] * scale, where raw(j) inverts CorrOut's map.  grid = (ceil(W / 256), pairs).
+static __global__ void __launch_bounds__(256)
+corr_gather_kernel(const double* __restrict__ r, long long pitch, CorrOut c)
+{
+    const long long pair = blockIdx.y;
+    const long long j = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (j >= c.W) return;
+    const uint32_t jj = (uint32_t)j;
+    const uint32_t i = jj - c.off0 < c.range.n0 ? c.range.lo0 + (jj - c.off0) : c.range.lo1 + (jj - c.off1);
+    c.out[pair * c.W + j] = r[pair * pitch + i] * c.scale;
+}
+
+int launch_corr_gather(const Wave& w, const double* r, long long pitch) {
+    const dim3 grid((unsigned)((w.corr->W + 255) / 256), (unsigned)w.pairs);
+    return launch(w.ctx, w.d, KC_CORR_OUT, w.st, [&] {
+        corr_gather_kernel<<<grid, 256, 0, w.st>>>(r, pitch, *w.corr);
     });
 }
 
@@ -301,10 +347,12 @@ static int ensure_tickets(WorkSet& w, size_t n) {
 // kernels then get a source pitch of 0, and a static plan transforms the source into work.spec.
 // spectrum_ready: an earlier enqueue of the same call, on this work set and stream, already left that
 // source's spectrum in work.spec (the chunks of a host-fed call), so it is not computed again.
+// corr: the correlation export (audiosync_cuda_xcorr_correlation), its out at the batch's first row of
+// [n_pairs][W] device doubles; the plan's peak_scale becomes its scale.  nullptr: no export.
 static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work, const void* src, const void* smp,
                          size_t n_pairs, long long L, int dtype, audiosync_cuda_result* d_results,
                          cudaStream_t st, long long src_pitch = 0, long long smp_pitch = 0, bool shared_src = false,
-                         bool spectrum_ready = false) {
+                         bool spectrum_ready = false, const CorrOut* corr = nullptr) {
     if (n_pairs == 0) return 0;
     if (shared_src) src_pitch = 0;
     else if (src_pitch == 0) src_pitch = 2 * L;
@@ -345,13 +393,19 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
     // every other plan reads the one source in every pair's transform
     const bool reuse = shared_src && plan->source_spectrum;
     if (reuse && work.spec.ensure(sizeof(cplx) * (size_t)L) != 0) return -1;
+    CorrOut wave_corr{};
     Wave w{ctx, d, st, src, smp, in_dtype, src_pitch, smp_pitch, shared_src, reuse ? work.spec.p : nullptr,
-           work.ws.p, peaks, 0, win};
+           work.ws.p, peaks, 0, win, corr ? &wave_corr : nullptr};
     if (reuse && !spectrum_ready && plan->source_spectrum(w, work.spec.p) != 0) return -1;
     for (size_t p0 = 0; p0 < n_pairs; p0 += (size_t)wave) {
         w.pairs = (int)std::min<size_t>((size_t)wave, n_pairs - p0);
         w.src = static_cast<const char*>(src) + p0 * (size_t)src_pitch * esz;
         w.smp = static_cast<const char*>(smp) + p0 * (size_t)smp_pitch * esz;
+        if (corr) {
+            wave_corr = *corr;
+            wave_corr.out = corr->out + p0 * (size_t)corr->W;
+            wave_corr.scale = plan->peak_scale;
+        }
         // EXACT: the f64 path's arithmetic, for every dtype but plain F32 (S16: on s * 2^-15)
         auto pearson = [&](auto IN, auto EXACT) -> int {
             using InT = decltype(IN);
@@ -395,7 +449,7 @@ static void destroy_device_state(DeviceState& d) {
     cudaSetDevice(d.device);
     cudaDeviceSynchronize();
     d.plans.clear();
-    d.work.release(); d.results.release();
+    d.work.release(); d.results.release(); d.corr.release();
     for (int i = 0; i < 2; i++) {
         d.in_src[i].release(); d.in_smp[i].release();
         d.in_src32[i].release(); d.in_smp32[i].release();
@@ -652,9 +706,19 @@ static int direct_in_flight(DeviceState& d) {
 // share the copy threads; each then feeds its device with direct uploads only).
 // shared_src: `sources` is one source for every pair; it is uploaded once (into in_src[0]) and only
 // the samples are chunked, as they are (host narrowing does not apply).
+// The host-facing correlation export stages at most this many bytes of rows per device at a time (one
+// row where a row is larger), whatever n_pairs * W is.
+constexpr size_t CORR_STAGE_BYTES = (size_t)256 << 20;
+static size_t corr_stage_pairs(long long W) {
+    return std::max<size_t>(1, CORR_STAGE_BYTES / (sizeof(double) * (size_t)W));
+}
+
+// corr: the correlation export into the host array corr_host ([n][corr->W] doubles, row p for pair p);
+// each chunk's rows are staged in d.corr and copied back after its kernels.
 static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* sources,
                           const char* samples, size_t p0, size_t p1, long long L, int dtype,
-                          audiosync_cuda_result* out, bool solo, bool shared_src = false) {
+                          audiosync_cuda_result* out, bool solo, bool shared_src = false,
+                          const CorrOut* corr = nullptr, double* corr_host = nullptr) {
     if (p1 <= p0) return 0;
     std::lock_guard<std::mutex> dlk(d.mu);
     ASC_CUDA_OK(cudaSetDevice(d.device));
@@ -674,8 +738,12 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
     const int narrowed_dtype = mode == AUDIOSYNC_CUDA_NARROW_ALWAYS ? AUDIOSYNC_CUDA_F32 : ASC_DTYPE_F32_EXACT;
     // chunk: about 192 MB of input per buffer (twice that when pairs are fed both ways), at least one pair
     const size_t src_chunk_bytes = shared_src ? 0 : src_bytes;      // source bytes per chunked pair
-    size_t chunk = std::max<size_t>(1, ((size_t)(hybrid ? 384u : 192u) << 20) / (src_chunk_bytes + smp_bytes));
+    // (and of the staged correlation, when it is exported)
+    const size_t corr_row_bytes = corr ? sizeof(double) * (size_t)corr->W : 0;
+    size_t chunk = std::max<size_t>(1, ((size_t)(hybrid ? 384u : 192u) << 20) / (src_chunk_bytes + smp_bytes + corr_row_bytes));
+    if (corr) chunk = std::min(chunk, corr_stage_pairs(corr->W));
     chunk = std::min(chunk, p1 - p0);
+    if (corr && d.corr.ensure(corr_row_bytes * chunk) != 0) return -1;
     for (int b = 0; b < 2; b++) {
         if (d.in_src[b].ensure(shared_src ? src_bytes : src_bytes * chunk) != 0 || d.in_smp[b].ensure(smp_bytes * chunk) != 0)
             return -1;
@@ -790,21 +858,33 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
         }
         // pairs [0, n_dbl): doubles (or the caller's fp32); pairs [p_nar, n): narrowed
         const size_t n_dbl = std::min(n, lo * g), p_nar = std::min(n, hi * g);
+        // the chunk's rows of the export: staged from row 0 of d.corr (the stream orders the kernels of
+        // the next chunk behind this chunk's copy back)
+        CorrOut c_dbl{}, c_nar{};
+        if (corr) {
+            c_dbl = c_nar = *corr;
+            c_dbl.out = static_cast<double*>(d.corr.p);
+            c_nar.out = c_dbl.out + p_nar * (size_t)corr->W;
+        }
         if (n_dbl > 0) {
             ASC_CUDA_OK(cudaEventRecord(d.ev_up[b], d.copy_stream));
             ASC_CUDA_OK(cudaStreamWaitEvent(d.stream, d.ev_up[b], 0));
             // shared_src: the first chunk transforms the source, the later ones reuse its spectrum
             if (enqueue_batch(ctx, d, d.work, d.in_src[shared_src ? 0 : b].p, d.in_smp[b].p, n_dbl, L, dtype, d_res + c0, d.stream,
-                              0, 0, shared_src, shared_src && c0 > 0) != 0)
+                              0, 0, shared_src, shared_src && c0 > 0, corr ? &c_dbl : nullptr) != 0)
                 return -1;
         }
         if (p_nar < n) {
             ASC_CUDA_OK(cudaEventRecord(d.ev_up32[b], d.narrow_stream));
             ASC_CUDA_OK(cudaStreamWaitEvent(d.stream, d.ev_up32[b], 0));
             if (enqueue_batch(ctx, d, d.work, static_cast<float*>(d.in_src32[b].p) + p_nar * src_n,
-                              static_cast<float*>(d.in_smp32[b].p) + p_nar * smp_n, n - p_nar, L, narrowed_dtype, d_res + c0 + p_nar, d.stream) != 0)
+                              static_cast<float*>(d.in_smp32[b].p) + p_nar * smp_n, n - p_nar, L, narrowed_dtype, d_res + c0 + p_nar, d.stream,
+                              0, 0, false, false, corr ? &c_nar : nullptr) != 0)
                 return -1;
         }
+        if (corr)
+            ASC_CUDA_OK(cudaMemcpyAsync(corr_host + (p0 + c0) * (size_t)corr->W, d.corr.p, corr_row_bytes * n,
+                                        cudaMemcpyDeviceToHost, d.stream));
         ASC_CUDA_OK(cudaEventRecord(d.ev_done[b], d.stream));
         if (dtype == AUDIOSYNC_CUDA_F64) { ctx->fed_direct += n_dbl; ctx->fed_narrowed += n - p_nar; }
     }
@@ -1113,9 +1193,10 @@ int audiosync_cuda_synth_pairs(audiosync_cuda_ctx* ctx, int device, uint64_t see
     return 0;
 }
 
-// xcorr_batch_device and xcorr_shared_source_device
+// xcorr_batch_device and xcorr_shared_source_device (corr: xcorr_correlation_device's export)
 static int batch_device(audiosync_cuda_ctx* ctx, int device, const void* d_sources, const void* d_samples, size_t n_pairs,
-                        size_t sample_len, int dtype, audiosync_cuda_result* d_results, void* stream, bool shared_src) {
+                        size_t sample_len, int dtype, audiosync_cuda_result* d_results, void* stream, bool shared_src,
+                        const CorrOut* corr = nullptr) {
     if (!ctx || !d_sources || !d_samples || !d_results) { set_last_error("null argument"); return -1; }
     if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64 && dtype != AUDIOSYNC_CUDA_S16) { set_last_error("bad dtype"); return -1; }
     DeviceState* d = ctx->find(device);
@@ -1123,7 +1204,25 @@ static int batch_device(audiosync_cuda_ctx* ctx, int device, const void* d_sourc
     std::lock_guard<std::mutex> lk(d->mu);      // per device: threads driving different devices do not serialise
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
     return enqueue_batch(ctx, *d, d->work, d_sources, d_samples, n_pairs, (long long)sample_len, dtype, d_results, st,
-                         0, 0, shared_src);
+                         0, 0, shared_src, false, corr);
+}
+
+// The export arguments of the xcorr_correlation calls: -1 (message set) when they are refused,
+// otherwise 0 with *c filled (scale left to the plan).
+static int corr_args(size_t n_pairs, size_t sample_len, int64_t corr_lo, int64_t corr_hi, double* corr, bool device, CorrOut* c) {
+    const long long L = (long long)sample_len;
+    if (corr_lo > corr_hi || corr_lo < -L || corr_hi > L - 1) {
+        set_last_error("correlation range [%lld, %lld] is not a non-empty range of the lags [%lld, %lld]",
+                       (long long)corr_lo, (long long)corr_hi, -L, L - 1);
+        return -1;
+    }
+    if (!corr && n_pairs) { set_last_error("null correlation array"); return -1; }
+    if (device && reinterpret_cast<uintptr_t>(corr) % sizeof(double) != 0) {
+        set_last_error("device correlation array is not aligned to 8 bytes");
+        return -1;
+    }
+    *c = corr_out_of(corr_lo, corr_hi, L, corr, 1.0);
+    return 0;
 }
 
 int audiosync_cuda_xcorr_batch_device(audiosync_cuda_ctx* ctx, int device, const void* d_sources,
@@ -1138,9 +1237,11 @@ int audiosync_cuda_xcorr_shared_source_device(audiosync_cuda_ctx* ctx, int devic
     return batch_device(ctx, device, d_source, d_samples, n_pairs, sample_len, dtype, d_results, stream, true);
 }
 
-// xcorr_batch_results and xcorr_shared_source
+// xcorr_batch_results and xcorr_shared_source (corr / corr_host: xcorr_correlation's export into a
+// host array)
 static int batch_results(audiosync_cuda_ctx* ctx, const void* sources, const void* samples, size_t n_pairs,
-                         size_t sample_len, int dtype, int memspace, audiosync_cuda_result* results, bool shared_src) {
+                         size_t sample_len, int dtype, int memspace, audiosync_cuda_result* results, bool shared_src,
+                         const CorrOut* corr = nullptr, double* corr_host = nullptr) {
     if (!ctx || !sources || !samples || (!results && n_pairs)) { set_last_error("null argument"); return -1; }
     if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64 && dtype != AUDIOSYNC_CUDA_S16) { set_last_error("bad dtype"); return -1; }
     if (n_pairs == 0) return 0;
@@ -1162,7 +1263,25 @@ static int batch_results(audiosync_cuda_ctx* ctx, const void* sources, const voi
         ASC_CUDA_OK(cudaSetDevice(d->device));
         if (d->results.ensure(sizeof(audiosync_cuda_result) * n_pairs) != 0) return -1;
         auto* d_res = static_cast<audiosync_cuda_result*>(d->results.p);
-        if (enqueue_batch(ctx, *d, d->work, sources, samples, n_pairs, L, dtype, d_res, d->stream, 0, 0, shared_src) != 0) return -1;
+        if (!corr) {
+            if (enqueue_batch(ctx, *d, d->work, sources, samples, n_pairs, L, dtype, d_res, d->stream, 0, 0, shared_src) != 0) return -1;
+        } else {
+            // the export is staged in pieces of at most CORR_STAGE_BYTES, each copied back behind its kernels
+            const size_t esz = dtype_bytes(dtype), piece = std::min(n_pairs, corr_stage_pairs(corr->W));
+            if (d->corr.ensure(sizeof(double) * (size_t)corr->W * piece) != 0) return -1;
+            CorrOut c = *corr;
+            c.out = static_cast<double*>(d->corr.p);
+            for (size_t q0 = 0; q0 < n_pairs; q0 += piece) {
+                const size_t n = std::min(piece, n_pairs - q0);
+                const char* s = static_cast<const char*>(sources) + (shared_src ? 0 : q0 * (size_t)(2 * L) * esz);
+                const char* m = static_cast<const char*>(samples) + q0 * (size_t)L * esz;
+                if (enqueue_batch(ctx, *d, d->work, s, m, n, L, dtype, d_res + q0, d->stream, 0, 0, shared_src,
+                                  shared_src && q0 > 0, &c) != 0)
+                    return -1;
+                ASC_CUDA_OK(cudaMemcpyAsync(corr_host + q0 * (size_t)corr->W, c.out, sizeof(double) * (size_t)corr->W * n,
+                                            cudaMemcpyDeviceToHost, d->stream));
+            }
+        }
         ASC_CUDA_OK(cudaMemcpyAsync(results, d_res, sizeof(audiosync_cuda_result) * n_pairs,
                                     cudaMemcpyDeviceToHost, d->stream));
         ASC_CUDA_OK(cudaStreamSynchronize(d->stream));
@@ -1182,7 +1301,8 @@ static int batch_results(audiosync_cuda_ctx* ctx, const void* sources, const voi
             if (cnt == 0) continue;
             auto work = [&, g, a, b] {
                 rcs[g] = run_host_range(ctx, ctx->devs[g], static_cast<const char*>(sources),
-                                        static_cast<const char*>(samples), a, b, L, dtype, results, solo, shared_src);
+                                        static_cast<const char*>(samples), a, b, L, dtype, results, solo, shared_src,
+                                        corr, corr_host);
                 if (rcs[g] != 0) errs[g] = take_last_error();   // the worker's thread-local message
             };
             if (G == 1) work(); else th.emplace_back(work);
@@ -1208,6 +1328,28 @@ int audiosync_cuda_xcorr_shared_source(audiosync_cuda_ctx* ctx, const void* sour
                                        size_t n_pairs, size_t sample_len, int dtype, int memspace,
                                        audiosync_cuda_result* results) {
     return batch_results(ctx, source, samples, n_pairs, sample_len, dtype, memspace, results, true);
+}
+
+int audiosync_cuda_xcorr_correlation(audiosync_cuda_ctx* ctx, const void* sources, const void* samples,
+                                     size_t n_pairs, size_t sample_len, int dtype, int memspace,
+                                     int shared_source, int64_t corr_lo, int64_t corr_hi,
+                                     audiosync_cuda_result* results, double* corr) {
+    if (!ctx) { set_last_error("null argument"); return -1; }
+    if (n_pairs == 0) return 0;
+    CorrOut c;
+    if (corr_args(n_pairs, sample_len, corr_lo, corr_hi, corr, false, &c) != 0) return -1;
+    return batch_results(ctx, sources, samples, n_pairs, sample_len, dtype, memspace, results, shared_source != 0, &c, corr);
+}
+
+int audiosync_cuda_xcorr_correlation_device(audiosync_cuda_ctx* ctx, int device, const void* d_sources,
+                                            const void* d_samples, size_t n_pairs, size_t sample_len, int dtype,
+                                            int shared_source, int64_t corr_lo, int64_t corr_hi,
+                                            audiosync_cuda_result* d_results, double* d_corr, void* stream) {
+    if (!ctx) { set_last_error("null argument"); return -1; }
+    if (n_pairs == 0) return 0;
+    CorrOut c;
+    if (corr_args(n_pairs, sample_len, corr_lo, corr_hi, d_corr, true, &c) != 0) return -1;
+    return batch_device(ctx, device, d_sources, d_samples, n_pairs, sample_len, dtype, d_results, stream, shared_source != 0, &c);
 }
 
 int audiosync_cuda_xcorr_batch(audiosync_cuda_ctx* ctx, const void* sources, const void* samples,

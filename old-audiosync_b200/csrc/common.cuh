@@ -115,6 +115,40 @@ struct RawWindow {
 };
 // the unwindowed kernels' (empty) window parameter
 struct NoWindow {};
+// every raw index of [0, 2L): the windowed argmax then gives the unwindowed kernels' record
+__host__ __device__ __forceinline__ RawWindow full_window(long long L) { return RawWindow{0u, (uint32_t)(2 * L), 0u, 0u}; }
+
+// Correlation export of audiosync_cuda_xcorr_correlation: pair p's value at raw index i of range k
+// of `range` is stored, as (double)value * scale, at out[p * W + off_k + (i - lo_k)].  `out` points
+// at the wave's first row; offsets are 64-bit (pairs * W can exceed 2^31).
+struct CorrOut {
+    double* out;
+    long long W;
+    RawWindow range;
+    uint32_t off0, off1;
+    double scale;
+    __host__ __device__ __forceinline__ void store(long long pair, uint32_t i, double v) const {
+        if (i - range.lo0 < range.n0) out[pair * W + (long long)(off0 + (i - range.lo0))] = v * scale;
+        else if (i - range.lo1 < range.n1) out[pair * W + (long long)(off1 + (i - range.lo1))] = v * scale;
+    }
+    // fp32 kernels: the value the peak search compared, as pearson_block scales the peak (-0 as +0,
+    // as argmax_key_value returns it)
+    __host__ __device__ __forceinline__ void store(long long pair, uint32_t i, float v) const {
+        store(pair, i, (double)(v + 0.0f));
+    }
+};
+
+// The export range [lo, hi] of folded lags (-L <= lo <= hi <= L - 1) as raw ranges and output offsets.
+__host__ __device__ __forceinline__ CorrOut corr_out_of(long long lo, long long hi, long long L, double* out, double scale) {
+    CorrOut c;
+    c.out = out;
+    c.W = hi - lo + 1;
+    c.scale = scale;
+    if (lo >= 0) { c.range = RawWindow{(uint32_t)lo, (uint32_t)c.W, 0u, 0u}; c.off0 = 0u; c.off1 = 0u; }
+    else if (hi < 0) { c.range = RawWindow{(uint32_t)(lo + 2 * L), (uint32_t)c.W, 0u, 0u}; c.off0 = 0u; c.off1 = 0u; }
+    else { c.range = RawWindow{0u, (uint32_t)(hi + 1), (uint32_t)(lo + 2 * L), (uint32_t)(-lo)}; c.off0 = (uint32_t)(-lo); c.off1 = 0u; }
+    return c;
+}
 
 // Effective window [max(lo, -L), min(hi, L - 1)] of folded lags as raw ranges: raw = lag for lag >= 0,
 // lag + 2L below.  Returns -1 when it is empty, 0 when it is all of [-L, L - 1] (the unwindowed call),

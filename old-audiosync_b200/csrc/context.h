@@ -42,6 +42,7 @@ enum KernelClass {
     KC_SMALL_FFT,    // single-CTA transform for short lengths
     KC_PEARSON,      // window statistics + coefficient + result record
     KC_SRC_SPECTRUM, // forward rows of a shared source, once per call (RowFusedKernel ROWS_SRC_SPECTRUM)
+    KC_CORR_OUT,     // correlation export of the precise and direct plans (corr_gather_kernel)
     KC_COUNT
 };
 
@@ -131,6 +132,7 @@ struct DeviceState {
     DevBuf results;       // audiosync_cuda_result for host-facing calls
     DevBuf in_src[2], in_smp[2];          // device copies of host inputs (double buffered)
     DevBuf in_src32[2], in_smp32[2];      // the host-narrowed pairs of a chunk (fp32 images of f64 inputs)
+    DevBuf corr;                          // host-facing correlation export: the staged rows of one piece
     PinnedBuf h_results;
     StageRing stage;                      // bounce buffers for pageable host inputs
     cudaEvent_t ev_up[2] = {nullptr, nullptr};

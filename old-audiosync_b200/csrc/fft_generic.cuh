@@ -557,7 +557,9 @@ struct GenRowFusedKernel {
 // by argmax_f64_kernel, which keeps full double keys.  grid = (pairs, ceil(M2 / CT)).
 // WIN (fp32 only): the windowed twin -- the raw indices Params::win allows take the place of
 // [0, limit); fp64 plans apply the window in argmax_f64_window_kernel instead.
-template <typename T, int CT_ = GenTraits<T>::CT, int NT_ = GEN_THREADS, bool WIN = false>
+// OUT (fp32, with WIN): the exporting twin -- every output Params::corr's range allows is also stored,
+// before the threshold test; fp64 plans export from r_out in corr_gather_kernel instead.
+template <typename T, int CT_ = GenTraits<T>::CT, int NT_ = GEN_THREADS, bool WIN = false, bool OUT = false>
 struct GenColInvKernel {
     typedef typename GenTraits<T>::C C;
     static constexpr int CT = CT_;
@@ -565,7 +567,7 @@ struct GenColInvKernel {
     static constexpr int TR = THREADS / CT;
     static constexpr int MIN_CTAS = gen_min_ctas(NT_, sizeof(T) == 8);
 
-    struct Params {
+    struct PlainParams {
         const C* planes;
         PairPeak* peaks;
         const C* wcol;
@@ -574,7 +576,13 @@ struct GenColInvKernel {
         T* r_out;                // fp64 only: [pair][2M] reals (aliases plane 1 of the pair)
         [[no_unique_address]] std::conditional_t<WIN, RawWindow, NoWindow> win;   // WIN only
     };
+    // OUT appends the export descriptor; the other twins keep PlainParams and their parameter block
+    struct CorrParams : PlainParams {
+        CorrOut corr;
+    };
+    using Params = std::conditional_t<OUT, CorrParams, PlainParams>;
     static_assert(!WIN || sizeof(T) == 4, "fp64 plans window in argmax_f64_window_kernel");
+    static_assert(!OUT || WIN, "the exporting twin runs the windowed argmax");
     static size_t smem_bytes(const GenShape& sh) {
         const size_t tile = (size_t)sh.M1 * CT * sizeof(C);
         return (tile > 512 ? tile : 512) + 16;
@@ -654,6 +662,14 @@ struct GenColInvKernel {
                         for (int bf = tid / CT; bf < nbf; bf += TR) {
                             C v[R];
                             const unsigned i_first = butterfly(bf, c, n2, v);
+                            if constexpr (OUT) {
+                                static_for<0, R>([&](auto K) {
+                                    constexpr int k = decltype(K)::value;
+                                    const unsigned i_re = i_first + 2u * (unsigned)k * Wt * (unsigned)M2;
+                                    p.corr.store(pair, i_re, v[k].x);
+                                    p.corr.store(pair, i_re + 1u, v[k].y);
+                                });
+                            }
                             if constexpr (WIN) {
                                 // the threshold test sees allowed outputs only (see ColInvKernel): the
                                 // unmasked bound rejects first (it is the cheap test), then the allowed

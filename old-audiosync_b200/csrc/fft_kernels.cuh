@@ -435,7 +435,9 @@ struct ColFwdKernel {
 // fixed to true, so that callers which name ColInvKernel<..., true> (tests/emu) keep building.
 // WIN: the windowed twin (audiosync_cuda_set_lag_window): only the raw indices Params::win allows
 // compete, and only they raise the threshold (see the epilogue).
-template <class RL, int M2_, int NT, bool TMA = true, bool WIN = false>
+// OUT (with WIN): the exporting twin (audiosync_cuda_xcorr_correlation): every output of the last pass
+// that Params::corr's range allows is also stored, before the threshold test.
+template <class RL, int M2_, int NT, bool TMA = true, bool WIN = false, bool OUT = false>
 struct ColInvKernel {
     static_assert(TMA, "K_C's tiles are always staged by the TMA unit");
     static constexpr int M1 = RL::n;
@@ -448,7 +450,7 @@ struct ColInvKernel {
     static_assert(NT % 32 == 0, "the argmax epilogue votes per warp");
     static_assert(P >= 2, "column plans need at least two passes");
 
-    struct Params {
+    struct PlainParams {
         const cplx* planes;      // [pair][2][M1*M2]; plane 0 holds the K_B output
         PairPeak* peaks;         // [pair]
         const cplx* tw;          // RL pass tables (forward sign; conjugated here)
@@ -457,6 +459,12 @@ struct ColInvKernel {
         [[no_unique_address]] std::conditional_t<WIN, RawWindow, NoWindow> win;
         CUtensorMap tm;          // [2 * pair][M1 rows][2*M2 floats] view of the planes
     };
+    // OUT appends the export descriptor; the other twins keep PlainParams and their parameter block
+    struct CorrParams : PlainParams {
+        CorrOut corr;
+    };
+    using Params = std::conditional_t<OUT, CorrParams, PlainParams>;
+    static_assert(!OUT || WIN, "the exporting twin runs the windowed argmax");
     static constexpr int TMA_ROWS = M1 - 1;
 
     // grid = (pairs, M2 / 16): the pair index runs fastest, so the tiles of one pair are
@@ -564,6 +572,17 @@ struct ColInvKernel {
                             v[q] = buf[(i0 + q) * COL_T + c];
                         });
                         dft_reg<R, +1>(v);
+                        if constexpr (OUT) {
+                            if (act) {
+                                const int f0 = RL::freq_of_pos(i0);
+                                static_for<0, R>([&](auto K) {
+                                    constexpr int k = decltype(K)::value;
+                                    const uint32_t i_re = 2u * ((uint32_t)(f0 + k * Wt) * (uint32_t)M2 + (uint32_t)(c0 + c));
+                                    p.corr.store(pair, i_re, v[k].x);
+                                    p.corr.store(pair, i_re + 1u, v[k].y);
+                                });
+                            }
+                        }
                         const bool has_seed = col0 && i0 == 0;          // r[0]: signed seed, exact path always
                         bool need;
                         if constexpr (WIN) {

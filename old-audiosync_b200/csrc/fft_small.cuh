@@ -38,11 +38,12 @@ ASC_HD int small_pos_of_freq(const SmallPlan& pl, int k) {
 // PHAT: the split step whitens the spectra (split_phat_merge); w is wn[k] as for the product.
 // WIN: the windowed twin -- only the raw indices Params::win allows compete (ArgmaxAcc::consider_win).
 // SHARED_SRC: every pair reads the one source at Params::sources (its pitch is not read).
-template <typename InT, bool PHAT = false, bool WIN = false, bool SHARED_SRC = false>
+// OUT (with WIN): the exporting twin -- every output Params::corr's range allows is also stored.
+template <typename InT, bool PHAT = false, bool WIN = false, bool SHARED_SRC = false, bool OUT = false>
 struct SmallXcorrKernel {
     static constexpr int THREADS = SMALL_THREADS;
 
-    struct Params {
+    struct PlainParams {
         const InT* sources;   // [pair][2M]
         const InT* samples;   // [pair][M]
         PairPeak* peaks;      // [pair]
@@ -54,6 +55,12 @@ struct SmallXcorrKernel {
         int vec_src, vec_smp; // one load per packed point (every pair's base is aligned to two elements)
         [[no_unique_address]] std::conditional_t<WIN, RawWindow, NoWindow> win;   // WIN only
     };
+    // OUT appends the export descriptor; the other twins keep PlainParams and their parameter block
+    struct CorrParams : PlainParams {
+        CorrOut corr;
+    };
+    using Params = std::conditional_t<OUT, CorrParams, PlainParams>;
+    static_assert(!OUT || WIN, "the exporting twin runs the windowed argmax");
     // two rows of M points + 512 bytes of reduction scratch (phase_argmax needs 392)
     static size_t smem_bytes(int M) { return (size_t)2 * M * sizeof(cplx) + 512; }
 
@@ -144,6 +151,10 @@ struct SmallXcorrKernel {
                 for (int n = tid; n < M; n += THREADS) {
                     const cplx v = buf[n];
                     const uint32_t i_re = (uint32_t)(2 * n);
+                    if constexpr (OUT) {
+                        p.corr.store(pair, i_re, v.x);
+                        p.corr.store(pair, i_re + 1u, v.y);
+                    }
                     if constexpr (WIN) {
                         acc.consider_win(v.x, i_re, p.win, &p.peaks[pair]);
                         acc.consider_win(v.y, i_re + 1u, p.win, &p.peaks[pair]);

@@ -22,10 +22,14 @@ static int prepare_gen_kernel(size_t smem) {
     return 0;
 }
 
-// the windowed twin of the fp32 inverse column kernel (fp64 plans window in argmax_f64_window_kernel)
+// the windowed and exporting twins of the fp32 inverse column kernel (fp64 plans window in
+// argmax_f64_window_kernel and export in corr_gather_kernel)
 template <typename T, int CT, int NT>
 static int prepare_col_inv_window(const GenShape& sh) {
-    if constexpr (sizeof(T) == 4) return prepare_gen_kernel<GenColInvKernel<T, CT, NT, true>>(GenColInvKernel<T, CT, NT, true>::smem_bytes(sh));
+    if constexpr (sizeof(T) == 4)
+        return prepare_gen_kernel<GenColInvKernel<T, CT, NT, true>>(GenColInvKernel<T, CT, NT, true>::smem_bytes(sh)) != 0 ||
+               prepare_gen_kernel<GenColInvKernel<T, CT, NT, true, true>>(GenColInvKernel<T, CT, NT, true, true>::smem_bytes(sh)) != 0
+                   ? -1 : 0;
     return 0;
 }
 
@@ -112,6 +116,12 @@ int GenStage<T, NT>::col_inv(FftPlan* plan, const Wave& w) {
         };
         constexpr int CT = decltype(CTC)::value;
         if constexpr (sizeof(T) == 4) {
+            // the exporting twin runs the windowed argmax, over all of [0, 2L) when no window is set
+            if (w.corr)
+                return go(GenColInvKernel<T, CT, NT, true, true>{}, [&](auto& p) {
+                    p.win = w.win ? *w.win : full_window(sh.L);
+                    p.corr = *w.corr;
+                });
             if (w.win) return go(GenColInvKernel<T, CT, NT, true>{}, [&](auto& p) { p.win = *w.win; });
         }
         return go(GenColInvKernel<T, CT, NT>{}, [](auto&) {});
@@ -120,10 +130,12 @@ int GenStage<T, NT>::col_inv(FftPlan* plan, const Wave& w) {
     if constexpr (sizeof(T) == 8) {
         // fp64: r[0 .. 2L) of pair i sits in its (dead) sample plane; full double keys
         const double* r = reinterpret_cast<const double*>(planes) + 2 * sh.M;
-        return launch(w.ctx, w.d, KC_ARGMAX_F64, w.st, [&] {
-            if (w.win) argmax_f64_window_kernel<<<w.pairs, 1024, 0, w.st>>>(r, 2 * sh.L, 4 * sh.M, w.peaks, *w.win);
-            else argmax_f64_kernel<<<w.pairs, 1024, 0, w.st>>>(r, 2 * sh.L, 4 * sh.M, w.peaks);
-        });
+        if (launch(w.ctx, w.d, KC_ARGMAX_F64, w.st, [&] {
+                if (w.win) argmax_f64_window_kernel<<<w.pairs, 1024, 0, w.st>>>(r, 2 * sh.L, 4 * sh.M, w.peaks, *w.win);
+                else argmax_f64_kernel<<<w.pairs, 1024, 0, w.st>>>(r, 2 * sh.L, 4 * sh.M, w.peaks);
+            }) != 0)
+            return -1;
+        if (w.corr) return launch_corr_gather(w, r, 4 * sh.M);
     }
     return 0;
 }

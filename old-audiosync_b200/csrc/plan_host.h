@@ -40,6 +40,7 @@ struct Wave {
     PairPeak* peaks;
     int pairs;
     const RawWindow* win;       // lag window: nullptr for the unwindowed kernels
+    const CorrOut* corr;        // correlation export, out at this wave's first row: nullptr when off
 };
 
 // f(float{}), f(double{}) or f(int16_t{}): the element type a transform loads for `dtype`.
@@ -205,5 +206,9 @@ struct GenStage {
 // when the plan's M2 has one (GenShape::static_rows).  prepare: tables + kernel attributes.
 int static_rows_prepare(FftPlan* plan);
 int static_rows_launch(FftPlan* plan, const Wave& w);
+
+// audiosync_cuda.cu: the correlation export of the plans whose r is in the workspace (precise and
+// direct): pair i's r[0 .. 2L) at r + i * pitch, scaled by *w.corr's scale into its rows.
+int launch_corr_gather(const Wave& w, const double* r, long long pitch);
 
 }  // namespace asc

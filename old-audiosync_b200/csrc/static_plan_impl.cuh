@@ -95,7 +95,14 @@ static int run_static_wave(FftPlan* plan, const Wave& w) {
     }
     {
         const dim3 grid(w.pairs, M2 / COL_T, 1);
-        if (w.win) {
+        if (w.corr) {
+            // the exporting twin runs the windowed argmax, over all of [0, 2L) when no window is set
+            using KCO = ColInvKernel<Col, Row::n, P::NT_COL, true, true, true>;
+            typename KCO::Params po{{planes, w.peaks, col_tw, P::L, w.win ? *w.win : full_window(P::L), pc.tm}, *w.corr};
+            if (launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
+                    launch_stage(fft_kernel_entry<KCO>, grid, dim3(KCO::THREADS), KCO::SMEM, w.st, po);
+                }) != 0) return -1;
+        } else if (w.win) {
             using KCW = ColInvKernel<Col, Row::n, P::NT_COL, true, true>;
             typename KCW::Params pw{planes, w.peaks, col_tw, P::L, *w.win, pc.tm};
             if (launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
@@ -114,7 +121,7 @@ template <class P>
 static int static_source_spectrum(FftPlan* plan, const Wave& w, cplx* spec) {
     using Col = typename P::Col;
     using Row = typename P::Row;
-    const Wave src_pair{w.ctx, w.d, w.st, w.src, w.src, w.dtype, 2 * P::L, 2 * P::L, false, nullptr, spec, w.peaks, 1, nullptr};
+    const Wave src_pair{w.ctx, w.d, w.st, w.src, w.src, w.dtype, 2 * P::L, 2 * P::L, false, nullptr, spec, w.peaks, 1, nullptr, nullptr};
     if (static_col_fwd<P, false>(plan, src_pair, 1) != 0) return -1;
     using K = RowFusedKernel<Row, Col::n, P::NT_ROW, false, ROWS_SRC_SPECTRUM>;
     typename K::Params p{spec, static_cast<const cplx*>(plan->row_tw.p), static_cast<const cplx*>(plan->row_rev.p),
@@ -166,6 +173,7 @@ int build_static_plan(FftPlan* plan) {
     using KBP = RowFusedKernel<Row, Col::n, P::NT_ROW, true>;
     using KC = ColInvKernel<Col, Row::n, P::NT_COL>;
     using KCW = ColInvKernel<Col, Row::n, P::NT_COL, true, true>;
+    using KCO = ColInvKernel<Col, Row::n, P::NT_COL, true, true, true>;
     // the shared-source path: sample-only K_A, the source-spectrum kernel and the shared K_B
     using KTs = ColFwdKernel<Col, Row::n, P::NT_COL, float, true, true>;
     using KRs = ColFwdKernel<Col, Row::n, P::NT_COL, float, false, true>;
@@ -177,7 +185,7 @@ int build_static_plan(FftPlan* plan) {
     if (prepare_kernel<KT>(KT::SMEM) != 0 || prepare_kernel<KR>(KR::SMEM) != 0 || prepare_kernel<KD>(KD::SMEM) != 0 ||
         prepare_kernel<KS>(KS::SMEM) != 0 ||
         (plan->phat ? prepare_kernel<KBP>(KBP::SMEM) : prepare_kernel<KB>(KB::SMEM)) != 0 || prepare_kernel<KC>(KC::SMEM) != 0 ||
-        prepare_kernel<KCW>(KCW::SMEM) != 0)
+        prepare_kernel<KCW>(KCW::SMEM) != 0 || prepare_kernel<KCO>(KCO::SMEM) != 0)
         return -1;
     if (prepare_kernel<KTs>(KTs::SMEM) != 0 || prepare_kernel<KRs>(KRs::SMEM) != 0 || prepare_kernel<KDs>(KDs::SMEM) != 0 ||
         prepare_kernel<KSs>(KSs::SMEM) != 0 || prepare_kernel<KBspec>(KBspec::SMEM) != 0 ||
