@@ -229,6 +229,35 @@ int audiosync_cuda_xcorr_shared_source_device(audiosync_cuda_ctx *ctx, int devic
                                               const void *d_samples, size_t n_pairs, size_t sample_len,
                                               int dtype, audiosync_cuda_result *d_results, void *stream);
 
+/* Every source against every sample: results[s * n_samples + p] is, byte for byte, record p of
+ * audiosync_cuda_xcorr_shared_source(sources[s], samples) on the same context, and so also the
+ * xcorr_batch_results record of the pair (sources[s], samples[p]).  sources: [n_sources][2*sample_len];
+ * samples: [n_samples][sample_len]; results: [n_sources][n_samples] records, row-major.
+ * For one capture against the several candidate uploads of a track, many listeners' captures against a
+ * few tracks, or every recording of an event against every reference track: each source and each sample
+ * is passed and uploaded once, and (on the six static lengths) transformed once per call and device.
+ *   Every dtype, alignment rule, context setting (path, precise mode, weighting with PHAT's refusals, lag
+ *   window, wave size) and refusal of xcorr_shared_source applies.
+ *   HOST: the samples are split in contiguous blocks over the context's devices; each device gets every
+ *   source, uploaded once per call, and its samples in chunks.  Host narrowing does not apply.
+ *   DEVICE: all pointers live on one device of the context; no input copies.
+ *   n_sources == 0 or n_samples == 0 returns 0 and launches nothing.  A record count whose bytes
+ *   overflow size_t returns -1 and writes nothing.
+ * On the static plans every source's forward rows are computed once per call and device (kernel class
+ * "src_spectrum", one launch per source) and every wave's samples' forward rows once (class
+ * "smp_spectrum", one launch per wave); the row kernel ("row_fused") then runs once per source and wave
+ * from both spectra.  Every other plan runs the shared-source call once per source.  The correlation
+ * export does not cover this call. */
+int audiosync_cuda_xcorr_cross(audiosync_cuda_ctx *ctx, const void *sources, size_t n_sources,
+                               const void *samples, size_t n_samples, size_t sample_len,
+                               int dtype, int memspace, audiosync_cuda_result *results);
+/* Stream-ordered form on device pointers of one device of the context (as xcorr_batch_device);
+ * d_results: [n_sources][n_samples] device records. */
+int audiosync_cuda_xcorr_cross_device(audiosync_cuda_ctx *ctx, int device, const void *d_sources,
+                                      size_t n_sources, const void *d_samples, size_t n_samples,
+                                      size_t sample_len, int dtype, audiosync_cuda_result *d_results,
+                                      void *stream);
+
 /* The batch call that also returns the correlation r each record's peak is taken from, over a range of
  * lags, for what the one argmax cannot give: sub-sample delay by interpolation around the peak, the
  * runner-up lag, sums over channels before picking a peak, plots, a caller's own acceptance rule.

@@ -52,6 +52,7 @@ EXPORTED_SYMBOLS = [
     "audiosync_cuda_create", "audiosync_cuda_destroy", "audiosync_cuda_device_count",
     "audiosync_cuda_xcorr_batch", "audiosync_cuda_xcorr_batch_results", "audiosync_cuda_xcorr_batch_device",
     "audiosync_cuda_xcorr_shared_source", "audiosync_cuda_xcorr_shared_source_device",
+    "audiosync_cuda_xcorr_cross", "audiosync_cuda_xcorr_cross_device",
     "audiosync_cuda_xcorr_correlation", "audiosync_cuda_xcorr_correlation_device",
     "audiosync_cuda_synth_pairs", "audiosync_cuda_synchronize",
     "audiosync_cuda_set_path", "audiosync_cuda_set_wave_pairs", "audiosync_cuda_set_debug", "audiosync_cuda_set_precise", "audiosync_cuda_set_weighting",
@@ -119,6 +120,10 @@ def lib() -> C.CDLL:
     L.audiosync_cuda_xcorr_shared_source.argtypes = [vp, vp, vp, sz, sz, i32, i32, vp]
     L.audiosync_cuda_xcorr_shared_source_device.restype = i32
     L.audiosync_cuda_xcorr_shared_source_device.argtypes = [vp, i32, vp, vp, sz, sz, i32, vp, vp]
+    L.audiosync_cuda_xcorr_cross.restype = i32
+    L.audiosync_cuda_xcorr_cross.argtypes = [vp, vp, sz, vp, sz, sz, i32, i32, vp]
+    L.audiosync_cuda_xcorr_cross_device.restype = i32
+    L.audiosync_cuda_xcorr_cross_device.argtypes = [vp, i32, vp, sz, vp, sz, sz, i32, vp, vp]
     L.audiosync_cuda_xcorr_correlation.restype = i32
     L.audiosync_cuda_xcorr_correlation.argtypes = [vp, vp, vp, sz, sz, i32, i32, i32, C.c_int64, C.c_int64, vp, vp]
     L.audiosync_cuda_xcorr_correlation_device.restype = i32
@@ -574,6 +579,71 @@ class Context:
             return out
         return out[: n * RESULT_DTYPE.itemsize].cpu().numpy().view(RESULT_DTYPE)
 
+    def xcorr_cross(self, sources: np.ndarray, samples: np.ndarray) -> np.ndarray:
+        """Every source against every sample: ``sources`` [S][2L] and ``samples`` [P][L], both float32,
+        float64 or int16 (S16) host arrays.  Returns [S, P] records; record (s, p) is, bit for bit,
+        record p of ``xcorr_shared_source(sources[s], samples)`` (see include/audiosync_cuda.h).  Each
+        source and sample is uploaded and, on the static lengths, transformed once per device."""
+        if sources.dtype != samples.dtype or sources.dtype not in _NP_DTYPES:
+            raise TypeError("sources/samples must both be float32, float64 or int16")
+        if sources.ndim != 2 or samples.ndim != 2 or sources.shape[1] != 2 * samples.shape[1]:
+            raise ValueError("expected sources [S][2L] and samples [P][L]")
+        S = sources.shape[0]
+        n, L = samples.shape
+        sources = np.ascontiguousarray(sources)
+        samples = np.ascontiguousarray(samples)
+        res = np.zeros((S, n), RESULT_DTYPE)
+        rc = lib().audiosync_cuda_xcorr_cross(self._h, sources.ctypes.data, S, samples.ctypes.data, n, L,
+                                              _NP_DTYPES[sources.dtype], HOST, res.ctypes.data)
+        self._check(rc, "xcorr_cross")
+        return res
+
+    def xcorr_cross_records(self, sources_ptr: int, n_sources: int, samples_ptr: int, n_samples: int,
+                            sample_len: int, dtype: int, memspace: int) -> np.ndarray:
+        """``xcorr_cross`` on raw pointers (host memory or one device's memory, per ``memspace``):
+        [n_sources, n_samples] records; dtype F32, F64 or S16."""
+        res = np.zeros((n_sources, n_samples), RESULT_DTYPE)
+        rc = lib().audiosync_cuda_xcorr_cross(self._h, sources_ptr, n_sources, samples_ptr, n_samples, sample_len,
+                                              dtype, memspace, res.ctypes.data)
+        self._check(rc, "xcorr_cross")
+        return res
+
+    def xcorr_cross_torch(self, sources, samples, out=None, sync: bool = True):
+        """``xcorr_cross`` on torch CUDA tensors, zero copy: ``sources`` [S, 2L] and ``samples`` [P, L]
+        of one dtype on one device of this context, enqueued on torch's current stream.  ``out``: a uint8
+        CUDA tensor of S * P * 64 bytes (allocated when omitted).  With ``sync`` the records come back as a
+        NumPy [S, P] array, otherwise ``out`` is returned, as in ``xcorr_batch_torch``."""
+        import torch
+        if not (sources.is_cuda and samples.is_cuda) or sources.device != samples.device:
+            raise ValueError("sources and samples must be CUDA tensors on the same device")
+        dts = {torch.float32: F32, torch.float64: F64, torch.int16: S16}
+        if sources.dtype != samples.dtype or sources.dtype not in dts:
+            raise TypeError("sources/samples must both be float32, float64 or int16")
+        if sources.dim() != 2 or samples.dim() != 2 or sources.shape[1] != 2 * samples.shape[1]:
+            raise ValueError("expected sources [S, 2L] and samples [P, L]")
+        if not (sources.is_contiguous() and samples.is_contiguous()):
+            raise ValueError("tensors must be contiguous (no hidden copies on this path)")
+        S = sources.shape[0]
+        n, L = samples.shape
+        nbytes = S * n * RESULT_DTYPE.itemsize
+        dev = sources.device
+        if out is None:
+            out = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        elif out.device != dev or out.dtype != torch.uint8 or out.numel() < nbytes:
+            raise ValueError("out must be a uint8 tensor of S * P * 64 bytes on the same device")
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        if stream == 0:
+            # as in xcorr_batch_torch: a NULL handle selects the library's own stream
+            torch.cuda.current_stream(dev).synchronize()
+        if S and n:
+            self.xcorr_cross_device(dev.index, sources.data_ptr(), S, samples.data_ptr(), n, L, dts[sources.dtype],
+                                    out.data_ptr(), stream)
+        if stream == 0:
+            self.synchronize(dev.index)
+        if not sync:
+            return out
+        return out[:nbytes].cpu().numpy().view(RESULT_DTYPE).reshape(S, n)
+
     def xcorr_batch_torch(self, sources, samples, out=None, sync: bool = True):
         """Zero-copy batch call on torch CUDA tensors (SURVEY 8f rank 3).
 
@@ -723,6 +793,14 @@ class Context:
         rc = lib().audiosync_cuda_xcorr_shared_source_device(self._h, device, d_source, d_samples, n_pairs,
                                                              sample_len, dtype, d_results, stream or None)
         self._check(rc, "xcorr_shared_source_device")
+
+    def xcorr_cross_device(self, device: int, d_sources: int, n_sources: int, d_samples: int, n_samples: int,
+                           sample_len: int, dtype: int, d_results: int, stream: int = 0):
+        """Stream-ordered cross call on device pointers: [n_sources][n_samples] records into
+        ``d_results``; dtype F32, F64 or S16."""
+        rc = lib().audiosync_cuda_xcorr_cross_device(self._h, device, d_sources, n_sources, d_samples, n_samples,
+                                                     sample_len, dtype, d_results, stream or None)
+        self._check(rc, "xcorr_cross_device")
 
     def synth_pairs(self, device: int, seed: int, first_pair: int, n_pairs: int, sample_len: int,
                     dtype: int, d_sources: int, d_samples: int, stream: int = 0):

@@ -55,7 +55,7 @@ static bool debug_on() { return g_debug_flag || (&global_debug != nullptr && glo
 const char* kernel_class_name(int k) {
     static const char* names[KC_COUNT] = {
         "synth", "direct_corr", "argmax_f64", "col_fwd", "row_fused",
-        "col_inv_argmax", "small_fft", "pearson", "src_spectrum", "corr_out"};
+        "col_inv_argmax", "small_fft", "pearson", "src_spectrum", "corr_out", "smp_spectrum"};
     return (k >= 0 && k < KC_COUNT) ? names[k] : "?";
 }
 
@@ -341,6 +341,25 @@ static int ensure_tickets(WorkSet& w, size_t n) {
     return 0;
 }
 
+// K_P of one wave: window statistics, coefficient and result records of w's pairs into res.
+// `dtype` is the caller's (F32_EXACT included); w.dtype what the transform loaded.
+static int launch_pearson(const Wave& w, const FftPlan* plan, int dtype, long long L, PearsonPartial* partials,
+                          unsigned int* tickets, int n_chunks, audiosync_cuda_result* res) {
+    // EXACT: the f64 path's arithmetic, for every dtype but plain F32 (S16: on s * 2^-15)
+    auto pearson = [&](auto IN, auto EXACT) -> int {
+        using InT = decltype(IN);
+        constexpr bool EX = decltype(EXACT)::value;
+        return launch(w.ctx, w.d, KC_PEARSON, w.st, [&] {
+            launch_stage(plan->phat ? pearson_kernel<InT, EX, true> : pearson_kernel<InT, EX>, dim3(n_chunks, w.pairs),
+                         dim3(PEARSON_THREADS), 0, w.st, static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp),
+                         w.src_pitch, w.smp_pitch, L, (const PairPeak*)w.peaks, 0LL, plan->peak_scale, partials, tickets,
+                         n_chunks, res);
+        });
+    };
+    return dtype == AUDIOSYNC_CUDA_F32 ? pearson(float{}, std::false_type{})
+                                       : with_input_type(w.dtype, [&](auto IN) { return pearson(IN, std::true_type{}); });
+}
+
 // Enqueue the whole path for device-resident pairs on `st` (no sync).
 // src_pitch / smp_pitch: elements between consecutive pairs (0 = packed [pair][2L] / [pair][L]).
 // shared_src: every pair reads the one source at `src` (audiosync_cuda_xcorr_shared_source); the
@@ -406,21 +425,91 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
             wave_corr.out = corr->out + p0 * (size_t)corr->W;
             wave_corr.scale = plan->peak_scale;
         }
-        // EXACT: the f64 path's arithmetic, for every dtype but plain F32 (S16: on s * 2^-15)
-        auto pearson = [&](auto IN, auto EXACT) -> int {
-            using InT = decltype(IN);
-            constexpr bool EX = decltype(EXACT)::value;
-            return launch(ctx, d, KC_PEARSON, st, [&] {
-                launch_stage(plan->phat ? pearson_kernel<InT, EX, true> : pearson_kernel<InT, EX>, dim3(n_chunks, w.pairs),
-                             dim3(PEARSON_THREADS), 0, st, static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp),
-                             src_pitch, smp_pitch, L, (const PairPeak*)peaks, 0LL, plan->peak_scale, partials, tickets,
-                             n_chunks, d_results + p0);
-            });
-        };
         if (plan->run_wave(w) != 0 ||
-            (dtype == AUDIOSYNC_CUDA_F32 ? pearson(float{}, std::false_type{})
-                                         : with_input_type(in_dtype, [&](auto IN) { return pearson(IN, std::true_type{}); })) != 0)
+            launch_pearson(w, plan, dtype, L, partials, tickets, n_chunks, d_results + p0) != 0)
             return -1;
+    }
+    ASC_CUDA_OK(cudaEventRecord(work.done, st));
+    work.last_stream = st;
+    work.used = true;
+    return 0;
+}
+
+// Source spectra a cross enqueue keeps on the device at once: the sources are taken in groups of
+// at most this many bytes of spectra (about 180 sources at 1,440,000 frames); each further group
+// transforms every sample wave again.
+constexpr size_t CROSS_SPEC_BYTES = (size_t)2 << 30;
+
+// Enqueue a cross batch on `st` (no sync): every source of srcs ([n_src][2L]) against every sample of
+// smp ([n_smp][L]).  Record (s, p) goes to d_results[s * res_pitch + p] and is record p of the
+// shared-source enqueue of source s.  Static plans transform each source once (into work.spec) and each
+// wave's samples once, then run K_B, K_C and K_P per source and wave; every other plan runs the
+// shared-source enqueue once per source.  spectra_ready: an earlier enqueue of the same call, on this
+// work set and stream, already left every source's spectrum in work.spec (the chunks of a host-fed call).
+static int enqueue_cross(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work, const void* srcs, size_t n_src,
+                         const void* smp, size_t n_smp, long long L, int dtype, audiosync_cuda_result* d_results,
+                         size_t res_pitch, cudaStream_t st, bool spectra_ready = false) {
+    if (n_src == 0 || n_smp == 0) return 0;
+    if (L <= 0 || L > (1LL << 30)) { set_last_error("unsupported sample_len %lld", L); return -1; }
+    const size_t esz = dtype_bytes(dtype);
+    if (esz == 0) { set_last_error("bad dtype %d", dtype); return -1; }
+    if (reinterpret_cast<uintptr_t>(srcs) % esz != 0 || reinterpret_cast<uintptr_t>(smp) % esz != 0) {
+        set_last_error("sources / samples base is not aligned to its %zu-byte element", esz);
+        return -1;
+    }
+    RawWindow raw_win;
+    const int windowed = lag_window(ctx, L, &raw_win);
+    if (windowed < 0) return -1;
+    ASC_CUDA_OK(cudaSetDevice(d.device));
+    FftPlan* plan = get_plan(ctx, d, L);
+    if (!plan) return -1;
+    const size_t src_bytes = (size_t)(2 * L) * esz;
+    if (!plan->cross_rows) {
+        for (size_t s = 0; s < n_src; s++)
+            if (enqueue_batch(ctx, d, work, static_cast<const char*>(srcs) + s * src_bytes, smp, n_smp, L, dtype,
+                              d_results + s * res_pitch, st, 0, 0, true) != 0)
+                return -1;
+        return 0;
+    }
+    int wave = ctx->wave_pairs > 0 ? ctx->wave_pairs : default_wave_pairs(plan, n_smp);
+    wave = (int)std::min<size_t>((size_t)wave, n_smp);
+    wave = std::min(wave, 65535);
+    const int n_chunks = (int)((L + PEARSON_CHUNK - 1) / PEARSON_CHUNK);
+    if (work.used && work.last_stream != st) ASC_CUDA_OK(cudaStreamWaitEvent(st, work.done, 0));
+    if (!work.done) ASC_CUDA_OK(cudaEventCreateWithFlags(&work.done, cudaEventDisableTiming));
+    const size_t spec_bytes = sizeof(cplx) * (size_t)L;
+    const size_t group = std::min(n_src, std::max<size_t>(1, CROSS_SPEC_BYTES / spec_bytes));
+    if (work.ws.ensure(plan->ws_bytes_per_pair * (size_t)wave + 256) != 0) return -1;
+    if (work.peaks.ensure(sizeof(PairPeak) * (size_t)wave) != 0) return -1;
+    if (work.partials.ensure(sizeof(PearsonPartial) * (size_t)wave * n_chunks) != 0) return -1;
+    if (work.spec.ensure(spec_bytes * group) != 0) return -1;
+    if (ensure_tickets(work, (size_t)wave) != 0) return -1;
+    PearsonPartial* partials = static_cast<PearsonPartial*>(work.partials.p);
+    unsigned int* tickets = static_cast<unsigned int*>(work.tickets.p);
+    char* spec = static_cast<char*>(work.spec.p);
+    Wave w{ctx, d, st, srcs, smp, dtype, 0, L, true, nullptr, work.ws.p, static_cast<PairPeak*>(work.peaks.p), 0,
+           windowed ? &raw_win : nullptr, nullptr};
+    auto source = [&](size_t s) { return static_cast<const char*>(srcs) + s * src_bytes; };
+    for (size_t g0 = 0; g0 < n_src; g0 += group) {
+        const size_t ng = std::min(group, n_src - g0);
+        if (!(spectra_ready && ng == n_src)) {
+            for (size_t s = 0; s < ng; s++) {
+                w.src = source(g0 + s);
+                if (plan->source_spectrum(w, spec + s * spec_bytes) != 0) return -1;
+            }
+        }
+        for (size_t p0 = 0; p0 < n_smp; p0 += (size_t)wave) {
+            w.pairs = (int)std::min<size_t>((size_t)wave, n_smp - p0);
+            w.smp = static_cast<const char*>(smp) + p0 * (size_t)L * esz;
+            if (plan->cross_samples(w) != 0) return -1;
+            for (size_t s = 0; s < ng; s++) {
+                w.src = source(g0 + s);
+                w.spec = spec + s * spec_bytes;
+                if (plan->cross_rows(w) != 0 ||
+                    launch_pearson(w, plan, dtype, L, partials, tickets, n_chunks, d_results + (g0 + s) * res_pitch + p0) != 0)
+                    return -1;
+            }
+        }
     }
     ASC_CUDA_OK(cudaEventRecord(work.done, st));
     work.last_stream = st;
@@ -895,6 +984,53 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
     return 0;
 }
 
+// Host-memory cross batch on one device: every source against samples [p0, p1) of n_smp.  The
+// sources are uploaded once; the samples are chunked and double buffered as for a shared-source call.
+// Records land in out[s * n_smp + p].
+static int run_host_cross(audiosync_cuda_ctx* ctx, DeviceState& d, const char* sources, size_t n_src,
+                          const char* samples, size_t n_smp, size_t p0, size_t p1, long long L, int dtype,
+                          audiosync_cuda_result* out) {
+    if (p1 <= p0) return 0;
+    std::lock_guard<std::mutex> dlk(d.mu);
+    ASC_CUDA_OK(cudaSetDevice(d.device));
+    const size_t esz = dtype_bytes(dtype);
+    const size_t src_bytes = (size_t)(2 * L) * esz, smp_bytes = (size_t)L * esz;
+    const bool pageable = host_pointer_is_pageable(sources) || host_pointer_is_pageable(samples);
+    const size_t total = p1 - p0;
+    const size_t chunk = std::min(total, std::max<size_t>(1, ((size_t)192 << 20) / smp_bytes));
+    if (d.in_src[0].ensure(src_bytes * n_src) != 0) return -1;
+    for (int b = 0; b < 2; b++) {
+        if (d.in_smp[b].ensure(smp_bytes * chunk) != 0) return -1;
+        if (!d.ev_up[b]) ASC_CUDA_OK(cudaEventCreateWithFlags(&d.ev_up[b], cudaEventDisableTiming));
+        if (!d.ev_done[b]) ASC_CUDA_OK(cudaEventCreateWithFlags(&d.ev_done[b], cudaEventDisableTiming));
+    }
+    const size_t rec = sizeof(audiosync_cuda_result);
+    if (d.results.ensure(rec * n_src * total) != 0 || d.h_results.ensure(rec * n_src * total) != 0) return -1;
+    audiosync_cuda_result* d_res = static_cast<audiosync_cuda_result*>(d.results.p);
+    if (upload_from_host(d.in_src[0].p, sources, src_bytes * n_src, d.copy_stream, d.stage, pageable) != 0) return -1;
+    int it = 0;
+    for (size_t c0 = 0; c0 < total; c0 += chunk, it++) {
+        const size_t n = std::min(chunk, total - c0);
+        const int b = it & 1;
+        if (it >= 2) ASC_CUDA_OK(cudaStreamWaitEvent(d.copy_stream, d.ev_done[b], 0));
+        if (upload_from_host(d.in_smp[b].p, samples + (p0 + c0) * smp_bytes, smp_bytes * n, d.copy_stream, d.stage, pageable) != 0)
+            return -1;
+        ASC_CUDA_OK(cudaEventRecord(d.ev_up[b], d.copy_stream));
+        ASC_CUDA_OK(cudaStreamWaitEvent(d.stream, d.ev_up[b], 0));
+        // the first chunk transforms the sources, the later ones reuse their spectra
+        if (enqueue_cross(ctx, d, d.work, d.in_src[0].p, n_src, d.in_smp[b].p, n, L, dtype, d_res + c0, total, d.stream,
+                          c0 > 0) != 0)
+            return -1;
+        ASC_CUDA_OK(cudaEventRecord(d.ev_done[b], d.stream));
+    }
+    // [n_src][total] on the device -> rows s of [n_src][n_smp], columns [p0, p1)
+    ASC_CUDA_OK(cudaMemcpyAsync(d.h_results.p, d_res, rec * n_src * total, cudaMemcpyDeviceToHost, d.stream));
+    ASC_CUDA_OK(cudaStreamSynchronize(d.stream));
+    for (size_t s = 0; s < n_src; s++)
+        memcpy(out + s * n_smp + p0, static_cast<const audiosync_cuda_result*>(d.h_results.p) + s * total, rec * total);
+    return 0;
+}
+
 }  // namespace asc
 
 using namespace asc;
@@ -1350,6 +1486,89 @@ int audiosync_cuda_xcorr_correlation_device(audiosync_cuda_ctx* ctx, int device,
     CorrOut c;
     if (corr_args(n_pairs, sample_len, corr_lo, corr_hi, d_corr, true, &c) != 0) return -1;
     return batch_device(ctx, device, d_sources, d_samples, n_pairs, sample_len, dtype, d_results, stream, shared_source != 0, &c);
+}
+
+// The record count of a cross batch, 0 (message set) when its records' bytes overflow size_t.
+static size_t cross_records(size_t n_sources, size_t n_samples) {
+    if (n_sources > std::numeric_limits<size_t>::max() / sizeof(audiosync_cuda_result) / n_samples) {
+        set_last_error("%zu sources x %zu samples: the record array's size overflows", n_sources, n_samples);
+        return 0;
+    }
+    return n_sources * n_samples;
+}
+
+int audiosync_cuda_xcorr_cross(audiosync_cuda_ctx* ctx, const void* sources, size_t n_sources, const void* samples,
+                               size_t n_samples, size_t sample_len, int dtype, int memspace,
+                               audiosync_cuda_result* results) {
+    if (!ctx || !sources || !samples || (!results && n_sources && n_samples)) { set_last_error("null argument"); return -1; }
+    if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64 && dtype != AUDIOSYNC_CUDA_S16) { set_last_error("bad dtype"); return -1; }
+    if (n_sources == 0 || n_samples == 0) return 0;
+    const size_t n_rec = cross_records(n_sources, n_samples);
+    if (n_rec == 0) return -1;
+    if (sample_len == 0) { set_last_error("sample_len must be > 0"); return -1; }
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    const long long L = (long long)sample_len;
+    RawWindow win;
+    if (lag_window(ctx, L, &win) < 0) return -1;     // before any copy: nothing is written
+    if (memspace == AUDIOSYNC_CUDA_DEVICE) {
+        cudaPointerAttributes at;
+        ASC_CUDA_OK(cudaPointerGetAttributes(&at, sources));
+        DeviceState* d = ctx->find(at.device);
+        if (at.type != cudaMemoryTypeDevice || !d) {
+            set_last_error("device-memspace pointers must live on a device of the context");
+            return -1;
+        }
+        std::lock_guard<std::mutex> dlk(d->mu);
+        ASC_CUDA_OK(cudaSetDevice(d->device));
+        if (d->results.ensure(sizeof(audiosync_cuda_result) * n_rec) != 0) return -1;
+        auto* d_res = static_cast<audiosync_cuda_result*>(d->results.p);
+        if (enqueue_cross(ctx, *d, d->work, sources, n_sources, samples, n_samples, L, dtype, d_res, n_samples, d->stream) != 0)
+            return -1;
+        ASC_CUDA_OK(cudaMemcpyAsync(results, d_res, sizeof(audiosync_cuda_result) * n_rec, cudaMemcpyDeviceToHost, d->stream));
+        ASC_CUDA_OK(cudaStreamSynchronize(d->stream));
+        return 0;
+    }
+    // the samples in contiguous blocks over the devices, every source on each; one host thread per device
+    const size_t G = ctx->devs.size();
+    std::vector<int> rcs(G, 0);
+    std::vector<std::string> errs(G);
+    std::vector<std::thread> th;
+    const size_t base = n_samples / G, rem = n_samples % G;
+    size_t p0 = 0;
+    for (size_t g = 0; g < G; g++) {
+        const size_t cnt = base + (g < rem ? 1 : 0);
+        const size_t a = p0, b = p0 + cnt;
+        p0 = b;
+        if (cnt == 0) continue;
+        auto work = [&, g, a, b] {
+            rcs[g] = run_host_cross(ctx, ctx->devs[g], static_cast<const char*>(sources), n_sources,
+                                    static_cast<const char*>(samples), n_samples, a, b, L, dtype, results);
+            if (rcs[g] != 0) errs[g] = take_last_error();
+        };
+        if (G == 1) work(); else th.emplace_back(work);
+    }
+    for (auto& t : th) t.join();
+    for (size_t g = 0; g < G; g++)
+        if (rcs[g] != 0) {
+            adopt_last_error(errs[g]);           // first failing device, for audiosync_cuda_last_error()
+            return -1;
+        }
+    return 0;
+}
+
+int audiosync_cuda_xcorr_cross_device(audiosync_cuda_ctx* ctx, int device, const void* d_sources, size_t n_sources,
+                                      const void* d_samples, size_t n_samples, size_t sample_len, int dtype,
+                                      audiosync_cuda_result* d_results, void* stream) {
+    if (!ctx || !d_sources || !d_samples || !d_results) { set_last_error("null argument"); return -1; }
+    if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64 && dtype != AUDIOSYNC_CUDA_S16) { set_last_error("bad dtype"); return -1; }
+    DeviceState* d = ctx->find(device);
+    if (!d) { set_last_error("device %d is not part of this context", device); return -1; }
+    if (n_sources == 0 || n_samples == 0) return 0;
+    if (cross_records(n_sources, n_samples) == 0) return -1;
+    std::lock_guard<std::mutex> lk(d->mu);
+    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
+    return enqueue_cross(ctx, *d, d->work, d_sources, n_sources, d_samples, n_samples, (long long)sample_len, dtype,
+                         d_results, n_samples, st);
 }
 
 int audiosync_cuda_xcorr_batch(audiosync_cuda_ctx* ctx, const void* sources, const void* samples,

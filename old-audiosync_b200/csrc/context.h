@@ -43,6 +43,7 @@ enum KernelClass {
     KC_PEARSON,      // window statistics + coefficient + result record
     KC_SRC_SPECTRUM, // forward rows of a shared source, once per call (RowFusedKernel ROWS_SRC_SPECTRUM)
     KC_CORR_OUT,     // correlation export of the precise and direct plans (corr_gather_kernel)
+    KC_SMP_SPECTRUM, // forward rows of a cross call's samples, once per wave (RowFusedKernel ROWS_SRC_SPECTRUM)
     KC_COUNT
 };
 
@@ -110,7 +111,8 @@ struct WorkSet {
     DevBuf peaks;         // PairPeak per in-flight pair
     DevBuf partials;      // PearsonPartial
     DevBuf tickets;       // per-pair completion counters of the Pearson kernel
-    DevBuf spec;          // shared-source calls on a static plan: the source's forward rows (M complex)
+    DevBuf spec;          // shared-source calls on a static plan: the source's forward rows (M complex);
+                          // cross calls: those of a group of sources ([group][M])
     cudaEvent_t done = nullptr;
     cudaStream_t last_stream = nullptr;
     bool used = false;

@@ -781,7 +781,13 @@ ASC_HD void split_phat_merge(C a, C b, C c, C d, C w, C& qk, C& qmk) {
 //   ROWS_SHARED_SRC    slots 0/1 staged from Params::spec (the rows ROWS_SRC_SPECTRUM left), the
 //                      forward passes on the sample rows only, then the split and inverse as above;
 //                      plane 0 is not read, it only receives the product.
-enum RowMode { ROWS_PAIR = 0, ROWS_SRC_SPECTRUM = 1, ROWS_SHARED_SRC = 2 };
+//   ROWS_BOTH_SPECTRA  slots 0/1 staged from Params::spec, slots 2/3 from plane 1, which already holds
+//                      the sample's forward rows (ROWS_SRC_SPECTRUM run on plane 1); no forward pass,
+//                      then the split and inverse as above.  For a batch of sources against a batch of
+//                      samples, where every sample's rows are transformed once and serve every source.
+//                      It clears the pair's peak record: K_A, which does that otherwise, runs once per
+//                      sample wave and this kernel once per source and wave.
+enum RowMode { ROWS_PAIR = 0, ROWS_SRC_SPECTRUM = 1, ROWS_SHARED_SRC = 2, ROWS_BOTH_SPECTRA = 3 };
 
 template <class RL, int M1_, int NT, bool PHAT = false, int MODE = ROWS_PAIR>
 struct RowFusedKernel {
@@ -819,7 +825,12 @@ struct RowFusedKernel {
     struct SharedParams : PairParams {
         const cplx* spec;        // [M1][M2] the source's forward rows, position order
     };
-    using Params = std::conditional_t<MODE == ROWS_SHARED_SRC, SharedParams, PairParams>;
+    // ROWS_BOTH_SPECTRA appends the peak records it clears
+    struct BothParams : SharedParams {
+        PairPeak* peaks;         // [pair]
+    };
+    using Params = std::conditional_t<MODE == ROWS_BOTH_SPECTRA, BothParams,
+                                      std::conditional_t<MODE == ROWS_SHARED_SRC, SharedParams, PairParams>>;
     // Final-pass twiddle tables of one row k1: S0 entries 0.5 * W_M^(j*k1) (the factor 1/2 of the
     // merge step rides here, exactly), then R0 entries W_M^(k*S0*k1); padded to an even count so
     // that a row is a whole number of 16-byte units for the bulk copy.
@@ -845,7 +856,7 @@ struct RowFusedKernel {
         cplx* __restrict__ plane_p = plane_s + M;
         // where slots 0/1 are staged from
         const cplx* __restrict__ src_rows = plane_s;
-        if constexpr (MODE == ROWS_SHARED_SRC) src_rows = p.spec;
+        if constexpr (MODE == ROWS_SHARED_SRC || MODE == ROWS_BOTH_SPECTRA) src_rows = p.spec;
         // final-pass twiddle tables of the two rows, copied into the (then dead) sample rows
         cplx* __restrict__ tab = buf + 2 * RP;                // [2][TABP]
         void* tabbar = buf + 2 * RP + 2 * TABP;               // mbarrier of that copy
@@ -855,11 +866,15 @@ struct RowFusedKernel {
         // The CTA's shared memory is exactly the four rows, so the 8-byte mbarrier sits on the
         // last point of slot 3; the last two points of that row are not staged -- forward pass 0
         // reads them from global memory instead -- and the thread whose butterfly writes them
-        // first invalidates the barrier.  ROWS_SRC_SPECTRUM stages slots 0/1 only.
+        // first invalidates the barrier.  ROWS_SRC_SPECTRUM stages slots 0/1 only.  ROWS_BOTH_SPECTRA
+        // runs no forward pass: its split step does both instead.
         {
             void* mbar = buf + 4 * RP - 1;
             ex.phase([&](int tid) {
                 if (tid == 0) mbar_init(mbar, 1);
+                if constexpr (MODE == ROWS_BOTH_SPECTRA) {
+                    if (tid == 0 && r == 0) p.peaks[pair] = cleared_peak();   // read by K_C, after this grid
+                }
             });
             ex.phase([&](int tid) {
                 if (tid == 0) {
@@ -935,18 +950,20 @@ struct RowFusedKernel {
                 }
             }
         };
-        static_for<0, P>([&](auto PP) {
-            ex.phase([&](int tid) {
-                if constexpr (MODE == ROWS_PAIR) {
-                    fwd_pass(PP, tid, NT, 0, two ? 1 : 2, 2 * nrows);   // slots 0,1,2,3 or 0,2
-                } else if constexpr (MODE == ROWS_SRC_SPECTRUM) {
-                    fwd_pass(PP, tid, NT, 0, two ? 1 : 2, nrows);        // slots 0,1 or 0 (the pair mode's step: 60 registers, not 62)
-                    if constexpr (decltype(PP)::value == P - 1) fence_async_proxy();   // read by the bulk store below
-                } else {
-                    fwd_pass(PP, tid, NT, 2, 1, nrows);                  // slots 2,3 or 2
-                }
+        if constexpr (MODE != ROWS_BOTH_SPECTRA) {
+            static_for<0, P>([&](auto PP) {
+                ex.phase([&](int tid) {
+                    if constexpr (MODE == ROWS_PAIR) {
+                        fwd_pass(PP, tid, NT, 0, two ? 1 : 2, 2 * nrows);   // slots 0,1,2,3 or 0,2
+                    } else if constexpr (MODE == ROWS_SRC_SPECTRUM) {
+                        fwd_pass(PP, tid, NT, 0, two ? 1 : 2, nrows);        // slots 0,1 or 0 (the pair mode's step: 60 registers, not 62)
+                        if constexpr (decltype(PP)::value == P - 1) fence_async_proxy();   // read by the bulk store below
+                    } else {
+                        fwd_pass(PP, tid, NT, 2, 1, nrows);                  // slots 2,3 or 2
+                    }
+                });
             });
-        });
+        }
 
         // ---- ROWS_SRC_SPECTRUM: the transformed source rows leave in place; nothing else to do.
         if constexpr (MODE == ROWS_SRC_SPECTRUM) {
@@ -1002,8 +1019,23 @@ struct RowFusedKernel {
                                 const int pb = M2 - 1 - e;
                                 const cplx w2 = cmul(ax[decltype(X)::value], cm[decltype(Mm)::value]);
                                 cplx qk, qmk;
-                                if constexpr (PHAT) split_phat_merge<2>(zs_a[e], zs_b[pb], zp_a[e], zp_b[pb], w2, qk, qmk);
-                                else split_mul_merge_w2(zs_a[e], zs_b[pb], zp_a[e], zp_b[pb], w2, qk, qmk);
+                                if constexpr (MODE == ROWS_BOTH_SPECTRA) {
+                                    // the two points of slot 3 the staging left out (pb = M2 - 1, M2 - 2)
+                                    // belong to items e = 0, 1: threads 0 and 1 in this (X, Mm) step.  No
+                                    // forward pass overwrote the barrier's bytes, so it is invalidated here.
+                                    cplx zb = zp_b[pb];
+                                    if constexpr (decltype(X)::value == 0 && decltype(Mm)::value == 0) {
+                                        if (tid < 2) {
+                                            zb = ldg(plane_p + (long long)k1b * M2 + pb);
+                                            if (tid == 0) mbar_inval(buf + 4 * RP - 1);
+                                        }
+                                    }
+                                    if constexpr (PHAT) split_phat_merge<2>(zs_a[e], zs_b[pb], zp_a[e], zb, w2, qk, qmk);
+                                    else split_mul_merge_w2(zs_a[e], zs_b[pb], zp_a[e], zb, w2, qk, qmk);
+                                } else {
+                                    if constexpr (PHAT) split_phat_merge<2>(zs_a[e], zs_b[pb], zp_a[e], zp_b[pb], w2, qk, qmk);
+                                    else split_mul_merge_w2(zs_a[e], zs_b[pb], zp_a[e], zp_b[pb], w2, qk, qmk);
+                                }
                                 zs_a[e] = qk;
                                 zs_b[pb] = qmk;
                             }

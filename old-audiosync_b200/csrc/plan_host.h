@@ -88,6 +88,10 @@ struct FftPlan {
     // Static plans only: writes the shared source's forward rows (M complex) into spec, once per
     // call, for the waves that then reuse them.
     std::function<int(const Wave&, void* spec)> source_spectrum;
+    // Static plans only, for a batch of sources against a batch of samples: cross_samples leaves the
+    // wave's samples' forward rows in plane 1 (w.smp, once per wave); cross_rows then correlates one
+    // source against them (w.spec: that source's forward rows), any number of times.
+    std::function<int(const Wave&)> cross_samples, cross_rows;
     ~FftPlan() {
         col_tw.release(); col_tc.release(); row_tw.release(); row_rev.release(); row_tab.release(); m_lo.release(); m_hi.release();
         wm.release(); wn.release();

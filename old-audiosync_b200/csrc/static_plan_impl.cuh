@@ -50,69 +50,113 @@ static int static_col_fwd(FftPlan* plan, const Wave& w, int signals) {
     });
 }
 
-// One wave.  SHARED: the pairs share one source whose forward rows source_spectrum left in w.spec
-// (the source itself is not read): K_A on the samples, the shared-source K_B, K_C.
-template <class P, bool SHARED>
-static int run_static_wave(FftPlan* plan, const Wave& w) {
+// K_C's parameters, its tile map encoded: -1 (message set) when the driver cannot encode it.  Encoded
+// before a wave's first launch, so that a failure leaves no partial wave behind.
+template <class P>
+static int static_col_inv_params(FftPlan* plan, const Wave& w, typename ColInvKernel<typename P::Col, P::Row::n, P::NT_COL>::Params* pc) {
     using Col = typename P::Col;
-    using Row = typename P::Row;
-    constexpr int M1 = Col::n, M2 = Row::n;
+    constexpr int M1 = Col::n, M2 = P::Row::n;
     cplx* planes = static_cast<cplx*>(w.ws);
-    const cplx* col_tw = static_cast<const cplx*>(plan->col_tw.p);
-    const cplx* row_tw = static_cast<const cplx*>(plan->row_tw.p);
-    const cplx* row_rev = static_cast<const cplx*>(plan->row_rev.p);
-    const cplx* row_tab = static_cast<const cplx*>(plan->row_tab.p);
-    const cplx* m_lo = static_cast<const cplx*>(plan->m_lo.p);
-    const cplx* m_hi = static_cast<const cplx*>(plan->m_hi.p);
-    // K_C always stages its tiles through the TMA unit: its map is encoded before anything is
-    // enqueued, so that a failure leaves no partial wave behind
-    using KC = ColInvKernel<Col, Row::n, P::NT_COL>;
-    typename KC::Params pc{planes, w.peaks, col_tw, P::L};
-    if (make_tile_map(&pc.tm, planes, M2, M1, (size_t)P::L * sizeof(cplx), (size_t)2 * w.pairs,
-                      tile_box_rows(KC::TMA_ROWS)) != 0) {
+    *pc = {planes, w.peaks, static_cast<const cplx*>(plan->col_tw.p), P::L};
+    if (make_tile_map(&pc->tm, planes, M2, M1, (size_t)P::L * sizeof(cplx), (size_t)2 * w.pairs,
+                      tile_box_rows(ColInvKernel<Col, M2, P::NT_COL>::TMA_ROWS)) != 0) {
         set_last_error("L = %lld: cuTensorMapEncodeTiled %s for the workspace planes", P::L,
                        tensor_map_encoder() ? "failed" : "is not exported by the driver");
         return -1;
     }
-    if (static_col_fwd<P, SHARED>(plan, w, 2) != 0) return -1;
-    {
-        constexpr int MODE = SHARED ? ROWS_SHARED_SRC : ROWS_PAIR;
-        auto rows = [&](auto KK, const cplx* rev, const cplx* lo, const cplx* hi) -> int {
-            using K = decltype(KK);
-            const typename K::PairParams base{planes, row_tw, rev, lo, hi, P::L, row_tab};
-            typename K::Params p;
-            if constexpr (SHARED) p = {base, static_cast<const cplx*>(w.spec)};
-            else p = base;
-            const dim3 grid(M1 / 2 + 1, 1, w.pairs);
-            return launch(w.ctx, w.d, KC_ROW_FUSED, w.st, [&] {
-                launch_stage(fft_kernel_entry<K>, grid, dim3(K::THREADS), K::SMEM, w.st, p);
-            });
-        };
-        if ((plan->phat ? rows(RowFusedKernel<Row, Col::n, P::NT_ROW, true, MODE>{}, static_cast<const cplx*>(plan->phat_rev.p),
-                               static_cast<const cplx*>(plan->phat_lo.p), static_cast<const cplx*>(plan->phat_hi.p))
-                        : rows(RowFusedKernel<Row, Col::n, P::NT_ROW, false, MODE>{}, row_rev, m_lo, m_hi)) != 0)
-            return -1;
-    }
-    {
-        const dim3 grid(w.pairs, M2 / COL_T, 1);
-        if (w.corr) {
-            // the exporting twin runs the windowed argmax, over all of [0, 2L) when no window is set
-            using KCO = ColInvKernel<Col, Row::n, P::NT_COL, true, true, true>;
-            typename KCO::Params po{{planes, w.peaks, col_tw, P::L, w.win ? *w.win : full_window(P::L), pc.tm}, *w.corr};
-            if (launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
-                    launch_stage(fft_kernel_entry<KCO>, grid, dim3(KCO::THREADS), KCO::SMEM, w.st, po);
-                }) != 0) return -1;
-        } else if (w.win) {
-            using KCW = ColInvKernel<Col, Row::n, P::NT_COL, true, true>;
-            typename KCW::Params pw{planes, w.peaks, col_tw, P::L, *w.win, pc.tm};
-            if (launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
-                    launch_stage(fft_kernel_entry<KCW>, grid, dim3(KCW::THREADS), KCW::SMEM, w.st, pw);
-                }) != 0) return -1;
-        } else if (launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
-                       launch_stage(fft_kernel_entry<KC>, grid, dim3(KC::THREADS), KC::SMEM, w.st, pc);
-                   }) != 0) return -1;
-    }
     return 0;
+}
+
+// K_B of one wave in row mode MODE: ROWS_PAIR, ROWS_SHARED_SRC or ROWS_BOTH_SPECTRA (w.spec: the
+// source's forward rows for the last two)
+template <class P, int MODE>
+static int static_rows(FftPlan* plan, const Wave& w) {
+    using Col = typename P::Col;
+    using Row = typename P::Row;
+    cplx* planes = static_cast<cplx*>(w.ws);
+    const cplx* row_tw = static_cast<const cplx*>(plan->row_tw.p);
+    const cplx* row_tab = static_cast<const cplx*>(plan->row_tab.p);
+    auto rows = [&](auto KK, const cplx* rev, const cplx* lo, const cplx* hi) -> int {
+        using K = decltype(KK);
+        const typename K::PairParams base{planes, row_tw, rev, lo, hi, P::L, row_tab};
+        typename K::Params p;
+        if constexpr (MODE == ROWS_BOTH_SPECTRA) p = {{base, static_cast<const cplx*>(w.spec)}, w.peaks};
+        else if constexpr (MODE == ROWS_SHARED_SRC) p = {base, static_cast<const cplx*>(w.spec)};
+        else p = base;
+        const dim3 grid(Col::n / 2 + 1, 1, w.pairs);
+        return launch(w.ctx, w.d, KC_ROW_FUSED, w.st, [&] {
+            launch_stage(fft_kernel_entry<K>, grid, dim3(K::THREADS), K::SMEM, w.st, p);
+        });
+    };
+    return plan->phat ? rows(RowFusedKernel<Row, Col::n, P::NT_ROW, true, MODE>{}, static_cast<const cplx*>(plan->phat_rev.p),
+                             static_cast<const cplx*>(plan->phat_lo.p), static_cast<const cplx*>(plan->phat_hi.p))
+                      : rows(RowFusedKernel<Row, Col::n, P::NT_ROW, false, MODE>{}, static_cast<const cplx*>(plan->row_rev.p),
+                             static_cast<const cplx*>(plan->m_lo.p), static_cast<const cplx*>(plan->m_hi.p));
+}
+
+// K_C of one wave: plain, windowed or exporting
+template <class P>
+static int static_col_inv(const Wave& w, const typename ColInvKernel<typename P::Col, P::Row::n, P::NT_COL>::Params& pc) {
+    using Col = typename P::Col;
+    using Row = typename P::Row;
+    using KC = ColInvKernel<Col, Row::n, P::NT_COL>;
+    const dim3 grid(w.pairs, Row::n / COL_T, 1);
+    if (w.corr) {
+        // the exporting twin runs the windowed argmax, over all of [0, 2L) when no window is set
+        using KCO = ColInvKernel<Col, Row::n, P::NT_COL, true, true, true>;
+        typename KCO::Params po{{pc.planes, pc.peaks, pc.tw, P::L, w.win ? *w.win : full_window(P::L), pc.tm}, *w.corr};
+        return launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
+            launch_stage(fft_kernel_entry<KCO>, grid, dim3(KCO::THREADS), KCO::SMEM, w.st, po);
+        });
+    }
+    if (w.win) {
+        using KCW = ColInvKernel<Col, Row::n, P::NT_COL, true, true>;
+        typename KCW::Params pw{pc.planes, pc.peaks, pc.tw, P::L, *w.win, pc.tm};
+        return launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
+            launch_stage(fft_kernel_entry<KCW>, grid, dim3(KCW::THREADS), KCW::SMEM, w.st, pw);
+        });
+    }
+    return launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
+        launch_stage(fft_kernel_entry<KC>, grid, dim3(KC::THREADS), KC::SMEM, w.st, pc);
+    });
+}
+
+// One wave.  SHARED: the pairs share one source whose forward rows source_spectrum left in w.spec
+// (the source itself is not read): K_A on the samples, the shared-source K_B, K_C.
+template <class P, bool SHARED>
+static int run_static_wave(FftPlan* plan, const Wave& w) {
+    typename ColInvKernel<typename P::Col, P::Row::n, P::NT_COL>::Params pc;
+    if (static_col_inv_params<P>(plan, w, &pc) != 0) return -1;
+    if (static_col_fwd<P, SHARED>(plan, w, 2) != 0) return -1;
+    if (static_rows<P, SHARED ? ROWS_SHARED_SRC : ROWS_PAIR>(plan, w) != 0) return -1;
+    return static_col_inv<P>(w, pc);
+}
+
+// The sample side of a cross wave (sources against samples): K_A on the samples alone, then their
+// forward rows in place in plane 1 -- the source-spectrum kernel launched on the planes one plane
+// further on, so that its plane 0 of pair i is pair i's plane 1 (the pair pitch stays 2M).
+template <class P>
+static int static_cross_samples(FftPlan* plan, const Wave& w) {
+    using Col = typename P::Col;
+    using Row = typename P::Row;
+    if (static_col_fwd<P, true>(plan, w, 2) != 0) return -1;
+    using K = RowFusedKernel<Row, Col::n, P::NT_ROW, false, ROWS_SRC_SPECTRUM>;
+    typename K::Params p{static_cast<cplx*>(w.ws) + P::L, static_cast<const cplx*>(plan->row_tw.p),
+                         static_cast<const cplx*>(plan->row_rev.p), static_cast<const cplx*>(plan->m_lo.p),
+                         static_cast<const cplx*>(plan->m_hi.p), P::L, static_cast<const cplx*>(plan->row_tab.p)};
+    return launch(w.ctx, w.d, KC_SMP_SPECTRUM, w.st, [&] {
+        launch_stage(fft_kernel_entry<K>, dim3(Col::n / 2 + 1, 1, w.pairs), dim3(K::THREADS), K::SMEM, w.st, p);
+    });
+}
+
+// One source (w.spec: its forward rows) against a wave whose samples static_cross_samples transformed:
+// K_B from both spectra, which also clears the peak records, then K_C.  Plane 1 is left as it was.
+template <class P>
+static int static_cross_rows(FftPlan* plan, const Wave& w) {
+    typename ColInvKernel<typename P::Col, P::Row::n, P::NT_COL>::Params pc;
+    if (static_col_inv_params<P>(plan, w, &pc) != 0) return -1;
+    if (static_rows<P, ROWS_BOTH_SPECTRA>(plan, w) != 0) return -1;
+    return static_col_inv<P>(w, pc);
 }
 
 // The shared source's forward rows, once per call: K_A on the source alone as one pair (plane 0 of
@@ -182,6 +226,9 @@ int build_static_plan(FftPlan* plan) {
     using KBspec = RowFusedKernel<Row, Col::n, P::NT_ROW, false, ROWS_SRC_SPECTRUM>;
     using KBs = RowFusedKernel<Row, Col::n, P::NT_ROW, false, ROWS_SHARED_SRC>;
     using KBPs = RowFusedKernel<Row, Col::n, P::NT_ROW, true, ROWS_SHARED_SRC>;
+    // the cross path: K_B from both spectra (the sample side reuses KSs..KBspec)
+    using KBb = RowFusedKernel<Row, Col::n, P::NT_ROW, false, ROWS_BOTH_SPECTRA>;
+    using KBPb = RowFusedKernel<Row, Col::n, P::NT_ROW, true, ROWS_BOTH_SPECTRA>;
     if (prepare_kernel<KT>(KT::SMEM) != 0 || prepare_kernel<KR>(KR::SMEM) != 0 || prepare_kernel<KD>(KD::SMEM) != 0 ||
         prepare_kernel<KS>(KS::SMEM) != 0 ||
         (plan->phat ? prepare_kernel<KBP>(KBP::SMEM) : prepare_kernel<KB>(KB::SMEM)) != 0 || prepare_kernel<KC>(KC::SMEM) != 0 ||
@@ -189,7 +236,8 @@ int build_static_plan(FftPlan* plan) {
         return -1;
     if (prepare_kernel<KTs>(KTs::SMEM) != 0 || prepare_kernel<KRs>(KRs::SMEM) != 0 || prepare_kernel<KDs>(KDs::SMEM) != 0 ||
         prepare_kernel<KSs>(KSs::SMEM) != 0 || prepare_kernel<KBspec>(KBspec::SMEM) != 0 ||
-        (plan->phat ? prepare_kernel<KBPs>(KBPs::SMEM) : prepare_kernel<KBs>(KBs::SMEM)) != 0)
+        (plan->phat ? prepare_kernel<KBPs>(KBPs::SMEM) : prepare_kernel<KBs>(KBs::SMEM)) != 0 ||
+        (plan->phat ? prepare_kernel<KBPb>(KBPb::SMEM) : prepare_kernel<KBb>(KBb::SMEM)) != 0)
         return -1;
     plan->run_wave = [plan](const Wave& w) {
         return w.spec ? run_static_wave<P, true>(plan, w) : run_static_wave<P, false>(plan, w);
@@ -197,6 +245,8 @@ int build_static_plan(FftPlan* plan) {
     plan->source_spectrum = [plan](const Wave& w, void* spec) {
         return static_source_spectrum<P>(plan, w, static_cast<cplx*>(spec));
     };
+    plan->cross_samples = [plan](const Wave& w) { return static_cross_samples<P>(plan, w); };
+    plan->cross_rows = [plan](const Wave& w) { return static_cross_rows<P>(plan, w); };
     return 0;
 }
 
