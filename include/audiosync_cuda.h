@@ -298,6 +298,49 @@ int audiosync_cuda_xcorr_correlation_device(audiosync_cuda_ctx *ctx, int device,
                                             int shared_source, int64_t corr_lo, int64_t corr_hi,
                                             audiosync_cuda_result *d_results, double *d_corr, void *stream);
 
+/* The batch call that also returns each pair's runner-up: the best peak at least min_separation lags
+ * from the record's lag, with its own coefficient.  A song with a repeated bar, chorus or loop can
+ * match two offsets almost equally well; `second` cannot show it, since on band-limited audio it is
+ * almost always r[raw_index +- 1], the other side of the same peak.  A caller rejects an ambiguous
+ * interval, or waits for the next one, when the runner-up comes close to the record.
+ *   shared_source = 0: the inputs of xcorr_batch_results / xcorr_batch_device; 1: those of
+ *   xcorr_shared_source / xcorr_shared_source_device.  results[i] is, byte for byte, the record the
+ *   matching call returns for the same inputs and settings.
+ *   D = min_separation >= 1.  With p the folded lag of results[i], pair i's runner-up set is
+ *       A(p) = { lags l of the effective lag window [max(lag_lo, -L), min(lag_hi, L - 1)] : |l - p| >= D }
+ *   (plain distance on folded lags, no wrap-around), and runner_up[i] is the record the batch call
+ *   would return if its search were restricted to A(p), under the lag window's rule: raw = lag for
+ *   lag >= 0 and lag + 2L below; r[0] is the signed seed only when A(p) holds lag 0, otherwise every
+ *   allowed index competes by |r|; strict >, the first raw index wins ties; a NaN never wins, and when
+ *   no allowed value is a number the lowest allowed index is chosen; second and margin are taken over
+ *   A(p) without the runner-up; lag, coef, ret, success and ncc are the usual functions of raw_index.
+ *   Under PHAT the search runs over r_w and ncc = peak / N.
+ *   With D = 1, |runner_up.peak| equals the record's second, except when A(p) holds lag 0 with a
+ *   negative r[0]: the seed rule lets r[0] lose to every |r[i]|, while second counts |r[0]|.
+ *   An empty A(p) (D too large for the window) is a per-pair outcome: the call still succeeds and
+ *   writes raw_index = -1, lag = 0, peak = second = margin = 0, coef = ncc = NaN, ret = -1,
+ *   success = 0.
+ *   Every setting the batch calls honour applies, with the same refusals: dtype, memspace, path, precise
+ *   mode, weighting, lag window, wave size, host narrowing and several devices.  Returns -1 with a
+ *   message, writing nothing, when min_separation < 1, runner_up is NULL with n_pairs > 0, or the
+ *   matching call refuses.  n_pairs == 0 returns 0 and launches nothing.
+ * Each wave runs a second search over the correlation its batch search read, which is still on the
+ * device, then a second Pearson step (kernel classes "runner_up_argmax" and "runner_up_pearson"): the
+ * static and runtime-radix fp32 plans run their last inverse pass again, the single-CTA plan its
+ * whole transform, and the precise and direct plans search the r their workspace holds.  The cross
+ * call, the correlation export, pool_run and the drop-in call have no runner-up. */
+int audiosync_cuda_xcorr_runner_up(audiosync_cuda_ctx *ctx, const void *sources, const void *samples,
+                                   size_t n_pairs, size_t sample_len, int dtype, int memspace,
+                                   int shared_source, int64_t min_separation,
+                                   audiosync_cuda_result *results, audiosync_cuda_result *runner_up);
+/* Stream-ordered form on device pointers of one device of the context (as xcorr_batch_device);
+ * d_runner_up: n_pairs device records. */
+int audiosync_cuda_xcorr_runner_up_device(audiosync_cuda_ctx *ctx, int device, const void *d_sources,
+                                          const void *d_samples, size_t n_pairs, size_t sample_len, int dtype,
+                                          int shared_source, int64_t min_separation,
+                                          audiosync_cuda_result *d_results, audiosync_cuda_result *d_runner_up,
+                                          void *stream);
+
 /* ------------------------------------------------------------------------
  * Session pool (SURVEY 8f rank 1): many concurrent audiosync sessions on one device.
  * Each slot owns device-resident source / sample buffers that grow as audio arrives

@@ -54,6 +54,7 @@ EXPORTED_SYMBOLS = [
     "audiosync_cuda_xcorr_shared_source", "audiosync_cuda_xcorr_shared_source_device",
     "audiosync_cuda_xcorr_cross", "audiosync_cuda_xcorr_cross_device",
     "audiosync_cuda_xcorr_correlation", "audiosync_cuda_xcorr_correlation_device",
+    "audiosync_cuda_xcorr_runner_up", "audiosync_cuda_xcorr_runner_up_device",
     "audiosync_cuda_synth_pairs", "audiosync_cuda_synchronize",
     "audiosync_cuda_set_path", "audiosync_cuda_set_wave_pairs", "audiosync_cuda_set_debug", "audiosync_cuda_set_precise", "audiosync_cuda_set_weighting",
     "audiosync_cuda_set_lag_window",
@@ -128,6 +129,10 @@ def lib() -> C.CDLL:
     L.audiosync_cuda_xcorr_correlation.argtypes = [vp, vp, vp, sz, sz, i32, i32, i32, C.c_int64, C.c_int64, vp, vp]
     L.audiosync_cuda_xcorr_correlation_device.restype = i32
     L.audiosync_cuda_xcorr_correlation_device.argtypes = [vp, i32, vp, vp, sz, sz, i32, i32, C.c_int64, C.c_int64, vp, vp, vp]
+    L.audiosync_cuda_xcorr_runner_up.restype = i32
+    L.audiosync_cuda_xcorr_runner_up.argtypes = [vp, vp, vp, sz, sz, i32, i32, i32, C.c_int64, vp, vp]
+    L.audiosync_cuda_xcorr_runner_up_device.restype = i32
+    L.audiosync_cuda_xcorr_runner_up_device.argtypes = [vp, i32, vp, vp, sz, sz, i32, i32, C.c_int64, vp, vp, vp]
     L.audiosync_cuda_synth_pairs.restype = i32
     L.audiosync_cuda_synth_pairs.argtypes = [vp, i32, u64, u64, sz, sz, i32, vp, vp, vp]
     L.audiosync_cuda_synchronize.restype = i32
@@ -778,6 +783,91 @@ class Context:
                                                            dtype, 1 if shared_source else 0, int(lo), int(hi),
                                                            d_results, d_corr, stream or None)
         self._check(rc, "xcorr_correlation_device")
+
+    # -- runner-up ----------------------------------------------------------------
+    def xcorr_runner_up(self, sources: np.ndarray, samples: np.ndarray, min_separation: int,
+                        shared_source: bool = False):
+        """The batch call that also returns each pair's runner-up: the best peak at least ``min_separation``
+        lags from the record's lag, with its own coefficient (see include/audiosync_cuda.h).
+
+        Inputs as in ``xcorr_correlation``.  Returns ``(records, runner_up)``, two ``RESULT_DTYPE`` arrays of
+        n records; the records are those of ``xcorr_batch_records`` / ``xcorr_shared_source`` bit for bit.
+        A pair without a runner-up (its set is empty) gets raw_index -1 and ret -1."""
+        if sources.dtype != samples.dtype or sources.dtype not in _NP_DTYPES:
+            raise TypeError("sources/samples must both be float32, float64 or int16")
+        if samples.ndim != 2:
+            raise ValueError("expected samples [n][L]")
+        n, L = samples.shape
+        if shared_source:
+            if sources.ndim != 1 or sources.shape[0] < 2 * L:
+                raise ValueError("expected source [>= 2L] and samples [n][L]")
+            sources = sources[: 2 * L]
+        elif sources.ndim != 2 or sources.shape != (n, 2 * L):
+            raise ValueError("expected sources [n][2L] and samples [n][L]")
+        sources = np.ascontiguousarray(sources)
+        samples = np.ascontiguousarray(samples)
+        res = np.zeros(n, RESULT_DTYPE)
+        ru = np.zeros(n, RESULT_DTYPE)
+        rc = lib().audiosync_cuda_xcorr_runner_up(self._h, sources.ctypes.data, samples.ctypes.data, n, L,
+                                                  _NP_DTYPES[sources.dtype], HOST, 1 if shared_source else 0,
+                                                  int(min_separation), res.ctypes.data, ru.ctypes.data)
+        self._check(rc, "xcorr_runner_up")
+        return res, ru
+
+    def xcorr_runner_up_torch(self, sources, samples, min_separation: int, out=None, out_runner_up=None,
+                              shared_source: bool = False, sync: bool = True):
+        """``xcorr_runner_up`` on torch CUDA tensors, zero copy, on torch's current stream: ``sources``
+        [n, 2L] (``shared_source``: 1-D, at least 2L elements) and ``samples`` [n, L] of one dtype on one
+        device of this context.  ``out`` / ``out_runner_up``: uint8 CUDA tensors of n * 64 bytes (allocated
+        when omitted).  Returns ``(records, runner_up)``: NumPy arrays with ``sync``, else the device tensors."""
+        import torch
+        if not (sources.is_cuda and samples.is_cuda) or sources.device != samples.device:
+            raise ValueError("sources and samples must be CUDA tensors on the same device")
+        dts = {torch.float32: F32, torch.float64: F64, torch.int16: S16}
+        if sources.dtype != samples.dtype or sources.dtype not in dts:
+            raise TypeError("sources/samples must both be float32, float64 or int16")
+        if samples.dim() != 2:
+            raise ValueError("expected samples [n, L]")
+        n, L = samples.shape
+        if shared_source:
+            if sources.dim() != 1 or sources.shape[0] < 2 * L:
+                raise ValueError("expected source [>= 2L] and samples [n, L]")
+        elif sources.dim() != 2 or tuple(sources.shape) != (n, 2 * L):
+            raise ValueError("expected sources [n, 2L] and samples [n, L]")
+        if not (sources.is_contiguous() and samples.is_contiguous()):
+            raise ValueError("tensors must be contiguous (no hidden copies on this path)")
+        dev = sources.device
+        nbytes = n * RESULT_DTYPE.itemsize
+        bufs = []
+        for t in (out, out_runner_up):
+            if t is None:
+                t = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+            elif t.device != dev or t.dtype != torch.uint8 or t.numel() < nbytes:
+                raise ValueError("out / out_runner_up must be uint8 tensors of n * 64 bytes on the same device")
+            bufs.append(t)
+        out, out_runner_up = bufs
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        if stream == 0:
+            # as in xcorr_batch_torch: a NULL handle selects the library's own stream
+            torch.cuda.current_stream(dev).synchronize()
+        if n:
+            self.xcorr_runner_up_device(dev.index, sources.data_ptr(), samples.data_ptr(), n, L, dts[sources.dtype],
+                                        min_separation, out.data_ptr(), out_runner_up.data_ptr(), stream, shared_source)
+        if stream == 0:
+            self.synchronize(dev.index)
+        if not sync:
+            return out, out_runner_up
+        return (out[:nbytes].cpu().numpy().view(RESULT_DTYPE), out_runner_up[:nbytes].cpu().numpy().view(RESULT_DTYPE))
+
+    def xcorr_runner_up_device(self, device: int, d_sources: int, d_samples: int, n_pairs: int, sample_len: int,
+                               dtype: int, min_separation: int, d_results: int, d_runner_up: int, stream: int = 0,
+                               shared_source: bool = False):
+        """Stream-ordered runner-up call on device pointers: records into ``d_results``, runner-up records
+        into ``d_runner_up``; dtype F32, F64 or S16."""
+        rc = lib().audiosync_cuda_xcorr_runner_up_device(self._h, device, d_sources, d_samples, n_pairs, sample_len,
+                                                         dtype, 1 if shared_source else 0, int(min_separation),
+                                                         d_results, d_runner_up, stream or None)
+        self._check(rc, "xcorr_runner_up_device")
 
     # -- stream-ordered device calls --------------------------------------------
     def xcorr_batch_device(self, device: int, d_sources: int, d_samples: int, n_pairs: int,

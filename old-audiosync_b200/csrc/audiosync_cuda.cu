@@ -55,7 +55,8 @@ static bool debug_on() { return g_debug_flag || (&global_debug != nullptr && glo
 const char* kernel_class_name(int k) {
     static const char* names[KC_COUNT] = {
         "synth", "direct_corr", "argmax_f64", "col_fwd", "row_fused",
-        "col_inv_argmax", "small_fft", "pearson", "src_spectrum", "corr_out", "smp_spectrum"};
+        "col_inv_argmax", "small_fft", "pearson", "src_spectrum", "corr_out", "smp_spectrum",
+        "runner_up_argmax", "runner_up_pearson"};
     return (k >= 0 && k < KC_COUNT) ? names[k] : "?";
 }
 
@@ -105,9 +106,9 @@ static int with_small_out_kernel(int dtype, bool phat, bool shared_src, F&& f) {
     });
 }
 
-template <typename InT, bool PHAT, bool WIN, bool SHARED, bool OUT = false>
+template <typename InT, bool PHAT, bool WIN, bool SHARED, bool OUT = false, bool RU = false>
 static int run_small_wave(FftPlan* plan, const Wave& w) {
-    using K = SmallXcorrKernel<InT, PHAT, WIN, SHARED, OUT>;
+    using K = SmallXcorrKernel<InT, PHAT, WIN, SHARED, OUT, RU>;
     typename K::Params p{};
     static_cast<typename K::PlainParams&>(p) = {static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp), w.peaks,
                          static_cast<const cplx*>(plan->wm.p), static_cast<const cplx*>(plan->wn.p),
@@ -116,9 +117,10 @@ static int run_small_wave(FftPlan* plan, const Wave& w) {
     // the exporting twin runs the windowed argmax, over all of [0, 2L) when no window is set
     if constexpr (OUT) p.corr = *w.corr;
     if constexpr (WIN) p.win = w.win ? *w.win : full_window(plan->L);
+    if constexpr (RU) p.ru = *w.ru;
     const size_t smem = K::smem_bytes(plan->small.M);
     const dim3 grid(1, 1, w.pairs);
-    return launch(w.ctx, w.d, KC_SMALL_FFT, w.st, [&] {
+    return launch(w.ctx, w.d, RU ? KC_RU_ARGMAX : KC_SMALL_FFT, w.st, [&] {
         fft_kernel_entry<K><<<grid, K::THREADS, smem, w.st>>>(p);
     });
 }
@@ -147,11 +149,18 @@ static int build_small_plan(FftPlan* plan, long long L) {
             ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
             return 0;
         };
+        auto allow_ru = [&](auto IN, auto PHAT, auto SHARED) -> int {
+            using K = SmallXcorrKernel<decltype(IN), decltype(PHAT)::value, true, decltype(SHARED)::value, false, true>;
+            ASC_CUDA_OK(cudaFuncSetAttribute(fft_kernel_entry<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
+            return 0;
+        };
         for (int dtype : {AUDIOSYNC_CUDA_F32, AUDIOSYNC_CUDA_F64, AUDIOSYNC_CUDA_S16})
             for (bool shared_src : {false, true}) {
                 for (bool win : {false, true})
                     if (with_small_kernel(dtype, plan->phat, win, shared_src, allow) != 0) return -1;
-                if (with_small_out_kernel(dtype, plan->phat, shared_src, allow_out) != 0) return -1;
+                if (with_small_out_kernel(dtype, plan->phat, shared_src, allow_out) != 0 ||
+                    with_small_out_kernel(dtype, plan->phat, shared_src, allow_ru) != 0)
+                    return -1;
             }
     }
     plan->run_wave = [plan](const Wave& w) {
@@ -161,6 +170,13 @@ static int build_small_plan(FftPlan* plan, long long L) {
             });
         return with_small_kernel(w.dtype, plan->phat, w.win != nullptr, w.shared_src, [&](auto IN, auto PHAT, auto WIN, auto SHARED) {
             return run_small_wave<decltype(IN), decltype(PHAT)::value, decltype(WIN)::value, decltype(SHARED)::value>(plan, w);
+        });
+    };
+    // the single-CTA kernel keeps r in shared memory only: its runner-up twin is a second launch that
+    // transforms the wave again and searches each pair's runner-up set
+    plan->runner_up = [plan](const Wave& w) {
+        return with_small_out_kernel(w.dtype, plan->phat, w.shared_src, [&](auto IN, auto PHAT, auto SHARED) {
+            return run_small_wave<decltype(IN), decltype(PHAT)::value, true, decltype(SHARED)::value, false, true>(plan, w);
         });
     };
     return 0;
@@ -197,6 +213,9 @@ static int build_generic_plan_t(FftPlan* plan) {
         if ((small_col ? Small::col_fwd(plan, w) : Big::col_fwd(plan, w)) != 0) return -1;
         if ((static_rows ? static_rows_launch(plan, w) : small_row ? Small::rows(plan, w) : Big::rows(plan, w)) != 0) return -1;
         return small_col ? Small::col_inv(plan, w) : Big::col_inv(plan, w);
+    };
+    plan->runner_up = [plan, small_col](const Wave& w) {
+        return small_col ? GenStage<T, GEN_THREADS_SMALL>::runner_up(plan, w) : GenStage<T, GEN_THREADS>::runner_up(plan, w);
     };
     return 0;
 }
@@ -256,6 +275,13 @@ static int build_direct_plan(FftPlan* plan, long long L) {
     plan->desc = "direct L=" + std::to_string(L) + " time-domain O(L^2) fp64";
     plan->run_wave = [plan](const Wave& w) {
         return with_input_type(w.dtype, [&](auto IN) { return run_direct_wave<decltype(IN)>(plan, w); });
+    };
+    // r stays in the workspace after the batch search
+    plan->runner_up = [plan](const Wave& w) {
+        const double* r = static_cast<const double*>(w.ws);
+        return launch(w.ctx, w.d, KC_RU_ARGMAX, w.st, [&] {
+            argmax_f64_runner_up_kernel<<<w.pairs, 1024, 0, w.st>>>(r, 2 * plan->L, w.peaks, *w.ru);
+        });
     };
     return 0;
 }
@@ -349,6 +375,13 @@ static int launch_pearson(const Wave& w, const FftPlan* plan, int dtype, long lo
     auto pearson = [&](auto IN, auto EXACT) -> int {
         using InT = decltype(IN);
         constexpr bool EX = decltype(EXACT)::value;
+        if (w.ru)      // the runner-up records, from the runner-up search's peaks
+            return launch(w.ctx, w.d, KC_RU_PEARSON, w.st, [&] {
+                launch_stage(plan->phat ? pearson_runner_up_kernel<InT, EX, true> : pearson_runner_up_kernel<InT, EX>,
+                             dim3(n_chunks, w.pairs), dim3(PEARSON_THREADS), 0, w.st, static_cast<const InT*>(w.src),
+                             static_cast<const InT*>(w.smp), w.src_pitch, w.smp_pitch, L, (const PairPeak*)w.peaks, *w.ru,
+                             plan->peak_scale, partials, tickets, n_chunks, res);
+            });
         return launch(w.ctx, w.d, KC_PEARSON, w.st, [&] {
             launch_stage(plan->phat ? pearson_kernel<InT, EX, true> : pearson_kernel<InT, EX>, dim3(n_chunks, w.pairs),
                          dim3(PEARSON_THREADS), 0, w.st, static_cast<const InT*>(w.src), static_cast<const InT*>(w.smp),
@@ -368,10 +401,13 @@ static int launch_pearson(const Wave& w, const FftPlan* plan, int dtype, long lo
 // source's spectrum in work.spec (the chunks of a host-fed call), so it is not computed again.
 // corr: the correlation export (audiosync_cuda_xcorr_correlation), its out at the batch's first row of
 // [n_pairs][W] device doubles; the plan's peak_scale becomes its scale.  nullptr: no export.
+// d_ru: the runner-up records (audiosync_cuda_xcorr_runner_up) at min_separation min_sep: after each
+// wave's Pearson step, the plan's runner-up search and the runner-up Pearson step.  nullptr: none.
 static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work, const void* src, const void* smp,
                          size_t n_pairs, long long L, int dtype, audiosync_cuda_result* d_results,
                          cudaStream_t st, long long src_pitch = 0, long long smp_pitch = 0, bool shared_src = false,
-                         bool spectrum_ready = false, const CorrOut* corr = nullptr) {
+                         bool spectrum_ready = false, const CorrOut* corr = nullptr,
+                         long long min_sep = 0, audiosync_cuda_result* d_ru = nullptr) {
     if (n_pairs == 0) return 0;
     if (shared_src) src_pitch = 0;
     else if (src_pitch == 0) src_pitch = 2 * L;
@@ -403,6 +439,7 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
     if (!work.done) ASC_CUDA_OK(cudaEventCreateWithFlags(&work.done, cudaEventDisableTiming));
     if (work.ws.ensure(plan->ws_bytes_per_pair * (size_t)wave + 256) != 0) return -1;
     if (work.peaks.ensure(sizeof(PairPeak) * (size_t)wave) != 0) return -1;
+    if (d_ru && work.peaks_ru.ensure(sizeof(PairPeak) * (size_t)wave) != 0) return -1;
     if (work.partials.ensure(sizeof(PearsonPartial) * (size_t)wave * n_chunks) != 0) return -1;
     PairPeak* peaks = static_cast<PairPeak*>(work.peaks.p);
     PearsonPartial* partials = static_cast<PearsonPartial*>(work.partials.p);
@@ -428,6 +465,17 @@ static int enqueue_batch(audiosync_cuda_ctx* ctx, DeviceState& d, WorkSet& work,
         if (plan->run_wave(w) != 0 ||
             launch_pearson(w, plan, dtype, L, partials, tickets, n_chunks, d_results + p0) != 0)
             return -1;
+        if (d_ru) {
+            // the centres are the records just written; the search gets its own cleared PairPeak array
+            const RunnerUp ru{d_results + p0, std::max(ctx->lag_lo, -L), std::min(ctx->lag_hi, L - 1), min_sep, L};
+            Wave wr = w;
+            wr.peaks = static_cast<PairPeak*>(work.peaks_ru.p);
+            wr.ru = &ru;
+            ASC_CUDA_OK(cudaMemsetAsync(wr.peaks, 0, sizeof(PairPeak) * (size_t)w.pairs, st));
+            if (plan->runner_up(wr) != 0 ||
+                launch_pearson(wr, plan, dtype, L, partials, tickets, n_chunks, d_ru + p0) != 0)
+                return -1;
+        }
     }
     ASC_CUDA_OK(cudaEventRecord(work.done, st));
     work.last_stream = st;
@@ -804,10 +852,12 @@ static size_t corr_stage_pairs(long long W) {
 
 // corr: the correlation export into the host array corr_host ([n][corr->W] doubles, row p for pair p);
 // each chunk's rows are staged in d.corr and copied back after its kernels.
+// ru_out: the runner-up records at min_separation min_sep, gathered like `out` (nullptr: none).
 static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* sources,
                           const char* samples, size_t p0, size_t p1, long long L, int dtype,
                           audiosync_cuda_result* out, bool solo, bool shared_src = false,
-                          const CorrOut* corr = nullptr, double* corr_host = nullptr) {
+                          const CorrOut* corr = nullptr, double* corr_host = nullptr,
+                          long long min_sep = 0, audiosync_cuda_result* ru_out = nullptr) {
     if (p1 <= p0) return 0;
     std::lock_guard<std::mutex> dlk(d.mu);
     ASC_CUDA_OK(cudaSetDevice(d.device));
@@ -848,9 +898,11 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
     if (mode != AUDIOSYNC_CUDA_NARROW_OFF && !d.narrow_stream)
         ASC_CUDA_OK(cudaStreamCreateWithFlags(&d.narrow_stream, cudaStreamNonBlocking));
     const size_t total = p1 - p0;
-    if (d.results.ensure(sizeof(audiosync_cuda_result) * total) != 0) return -1;
-    if (d.h_results.ensure(sizeof(audiosync_cuda_result) * total) != 0) return -1;
+    const size_t n_rec = ru_out ? 2 * total : total;        // the runner-up records follow the batch records
+    if (d.results.ensure(sizeof(audiosync_cuda_result) * n_rec) != 0) return -1;
+    if (d.h_results.ensure(sizeof(audiosync_cuda_result) * n_rec) != 0) return -1;
     audiosync_cuda_result* d_res = static_cast<audiosync_cuda_result*>(d.results.p);
+    audiosync_cuda_result* d_ru = ru_out ? d_res + total : nullptr;
     if (shared_src && upload_from_host(d.in_src[0].p, sources, src_bytes, d.copy_stream, d.stage, pageable) != 0) return -1;
     int it = 0;
     for (size_t c0 = 0; c0 < total; c0 += chunk, it++) {
@@ -960,7 +1012,8 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
             ASC_CUDA_OK(cudaStreamWaitEvent(d.stream, d.ev_up[b], 0));
             // shared_src: the first chunk transforms the source, the later ones reuse its spectrum
             if (enqueue_batch(ctx, d, d.work, d.in_src[shared_src ? 0 : b].p, d.in_smp[b].p, n_dbl, L, dtype, d_res + c0, d.stream,
-                              0, 0, shared_src, shared_src && c0 > 0, corr ? &c_dbl : nullptr) != 0)
+                              0, 0, shared_src, shared_src && c0 > 0, corr ? &c_dbl : nullptr, min_sep,
+                              d_ru ? d_ru + c0 : nullptr) != 0)
                 return -1;
         }
         if (p_nar < n) {
@@ -968,7 +1021,7 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
             ASC_CUDA_OK(cudaStreamWaitEvent(d.stream, d.ev_up32[b], 0));
             if (enqueue_batch(ctx, d, d.work, static_cast<float*>(d.in_src32[b].p) + p_nar * src_n,
                               static_cast<float*>(d.in_smp32[b].p) + p_nar * smp_n, n - p_nar, L, narrowed_dtype, d_res + c0 + p_nar, d.stream,
-                              0, 0, false, false, corr ? &c_nar : nullptr) != 0)
+                              0, 0, false, false, corr ? &c_nar : nullptr, min_sep, d_ru ? d_ru + c0 + p_nar : nullptr) != 0)
                 return -1;
         }
         if (corr)
@@ -977,10 +1030,11 @@ static int run_host_range(audiosync_cuda_ctx* ctx, DeviceState& d, const char* s
         ASC_CUDA_OK(cudaEventRecord(d.ev_done[b], d.stream));
         if (dtype == AUDIOSYNC_CUDA_F64) { ctx->fed_direct += n_dbl; ctx->fed_narrowed += n - p_nar; }
     }
-    ASC_CUDA_OK(cudaMemcpyAsync(d.h_results.p, d_res, sizeof(audiosync_cuda_result) * total,
+    ASC_CUDA_OK(cudaMemcpyAsync(d.h_results.p, d_res, sizeof(audiosync_cuda_result) * n_rec,
                                 cudaMemcpyDeviceToHost, d.stream));
     ASC_CUDA_OK(cudaStreamSynchronize(d.stream));
     memcpy(out + p0, d.h_results.p, sizeof(audiosync_cuda_result) * total);
+    if (ru_out) memcpy(ru_out + p0, static_cast<audiosync_cuda_result*>(d.h_results.p) + total, sizeof(audiosync_cuda_result) * total);
     return 0;
 }
 
@@ -1330,9 +1384,10 @@ int audiosync_cuda_synth_pairs(audiosync_cuda_ctx* ctx, int device, uint64_t see
 }
 
 // xcorr_batch_device and xcorr_shared_source_device (corr: xcorr_correlation_device's export)
+// (min_sep, d_ru: xcorr_runner_up_device's runner-up records)
 static int batch_device(audiosync_cuda_ctx* ctx, int device, const void* d_sources, const void* d_samples, size_t n_pairs,
                         size_t sample_len, int dtype, audiosync_cuda_result* d_results, void* stream, bool shared_src,
-                        const CorrOut* corr = nullptr) {
+                        const CorrOut* corr = nullptr, long long min_sep = 0, audiosync_cuda_result* d_ru = nullptr) {
     if (!ctx || !d_sources || !d_samples || !d_results) { set_last_error("null argument"); return -1; }
     if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64 && dtype != AUDIOSYNC_CUDA_S16) { set_last_error("bad dtype"); return -1; }
     DeviceState* d = ctx->find(device);
@@ -1340,7 +1395,7 @@ static int batch_device(audiosync_cuda_ctx* ctx, int device, const void* d_sourc
     std::lock_guard<std::mutex> lk(d->mu);      // per device: threads driving different devices do not serialise
     cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : d->stream;
     return enqueue_batch(ctx, *d, d->work, d_sources, d_samples, n_pairs, (long long)sample_len, dtype, d_results, st,
-                         0, 0, shared_src, false, corr);
+                         0, 0, shared_src, false, corr, min_sep, d_ru);
 }
 
 // The export arguments of the xcorr_correlation calls: -1 (message set) when they are refused,
@@ -1375,9 +1430,11 @@ int audiosync_cuda_xcorr_shared_source_device(audiosync_cuda_ctx* ctx, int devic
 
 // xcorr_batch_results and xcorr_shared_source (corr / corr_host: xcorr_correlation's export into a
 // host array)
+// (min_sep, ru_host: xcorr_runner_up's runner-up records into a host array)
 static int batch_results(audiosync_cuda_ctx* ctx, const void* sources, const void* samples, size_t n_pairs,
                          size_t sample_len, int dtype, int memspace, audiosync_cuda_result* results, bool shared_src,
-                         const CorrOut* corr = nullptr, double* corr_host = nullptr) {
+                         const CorrOut* corr = nullptr, double* corr_host = nullptr,
+                         long long min_sep = 0, audiosync_cuda_result* ru_host = nullptr) {
     if (!ctx || !sources || !samples || (!results && n_pairs)) { set_last_error("null argument"); return -1; }
     if (dtype != AUDIOSYNC_CUDA_F32 && dtype != AUDIOSYNC_CUDA_F64 && dtype != AUDIOSYNC_CUDA_S16) { set_last_error("bad dtype"); return -1; }
     if (n_pairs == 0) return 0;
@@ -1397,9 +1454,15 @@ static int batch_results(audiosync_cuda_ctx* ctx, const void* sources, const voi
         }
         std::lock_guard<std::mutex> dlk(d->mu);
         ASC_CUDA_OK(cudaSetDevice(d->device));
-        if (d->results.ensure(sizeof(audiosync_cuda_result) * n_pairs) != 0) return -1;
+        if (d->results.ensure(sizeof(audiosync_cuda_result) * n_pairs * (ru_host ? 2 : 1)) != 0) return -1;
         auto* d_res = static_cast<audiosync_cuda_result*>(d->results.p);
-        if (!corr) {
+        if (ru_host) {
+            auto* d_ru = d_res + n_pairs;
+            if (enqueue_batch(ctx, *d, d->work, sources, samples, n_pairs, L, dtype, d_res, d->stream, 0, 0, shared_src, false,
+                              nullptr, min_sep, d_ru) != 0)
+                return -1;
+            ASC_CUDA_OK(cudaMemcpyAsync(ru_host, d_ru, sizeof(audiosync_cuda_result) * n_pairs, cudaMemcpyDeviceToHost, d->stream));
+        } else if (!corr) {
             if (enqueue_batch(ctx, *d, d->work, sources, samples, n_pairs, L, dtype, d_res, d->stream, 0, 0, shared_src) != 0) return -1;
         } else {
             // the export is staged in pieces of at most CORR_STAGE_BYTES, each copied back behind its kernels
@@ -1438,7 +1501,7 @@ static int batch_results(audiosync_cuda_ctx* ctx, const void* sources, const voi
             auto work = [&, g, a, b] {
                 rcs[g] = run_host_range(ctx, ctx->devs[g], static_cast<const char*>(sources),
                                         static_cast<const char*>(samples), a, b, L, dtype, results, solo, shared_src,
-                                        corr, corr_host);
+                                        corr, corr_host, min_sep, ru_host);
                 if (rcs[g] != 0) errs[g] = take_last_error();   // the worker's thread-local message
             };
             if (G == 1) work(); else th.emplace_back(work);
@@ -1486,6 +1549,39 @@ int audiosync_cuda_xcorr_correlation_device(audiosync_cuda_ctx* ctx, int device,
     CorrOut c;
     if (corr_args(n_pairs, sample_len, corr_lo, corr_hi, d_corr, true, &c) != 0) return -1;
     return batch_device(ctx, device, d_sources, d_samples, n_pairs, sample_len, dtype, d_results, stream, shared_source != 0, &c);
+}
+
+// The arguments the runner-up calls add: -1 (message set) when they are refused.
+static int runner_up_args(size_t n_pairs, int64_t min_separation, const audiosync_cuda_result* runner_up) {
+    if (min_separation < 1) {
+        set_last_error("min_separation %lld: the runner-up must be at least 1 lag from the peak", (long long)min_separation);
+        return -1;
+    }
+    if (!runner_up && n_pairs) { set_last_error("null runner-up array"); return -1; }
+    return 0;
+}
+
+int audiosync_cuda_xcorr_runner_up(audiosync_cuda_ctx* ctx, const void* sources, const void* samples,
+                                   size_t n_pairs, size_t sample_len, int dtype, int memspace,
+                                   int shared_source, int64_t min_separation,
+                                   audiosync_cuda_result* results, audiosync_cuda_result* runner_up) {
+    if (!ctx) { set_last_error("null argument"); return -1; }
+    if (runner_up_args(n_pairs, min_separation, runner_up) != 0) return -1;
+    if (n_pairs == 0) return 0;
+    return batch_results(ctx, sources, samples, n_pairs, sample_len, dtype, memspace, results, shared_source != 0,
+                         nullptr, nullptr, (long long)min_separation, runner_up);
+}
+
+int audiosync_cuda_xcorr_runner_up_device(audiosync_cuda_ctx* ctx, int device, const void* d_sources,
+                                          const void* d_samples, size_t n_pairs, size_t sample_len, int dtype,
+                                          int shared_source, int64_t min_separation,
+                                          audiosync_cuda_result* d_results, audiosync_cuda_result* d_runner_up,
+                                          void* stream) {
+    if (!ctx) { set_last_error("null argument"); return -1; }
+    if (runner_up_args(n_pairs, min_separation, d_runner_up) != 0) return -1;
+    if (n_pairs == 0) return 0;
+    return batch_device(ctx, device, d_sources, d_samples, n_pairs, sample_len, dtype, d_results, stream, shared_source != 0,
+                        nullptr, (long long)min_separation, d_runner_up);
 }
 
 // The record count of a cross batch, 0 (message set) when its records' bytes overflow size_t.

@@ -187,6 +187,64 @@ __host__ __device__ __forceinline__ Window fold_index(long long idx, long long L
     return w;
 }
 
+// Runner-up search of audiosync_cuda_xcorr_runner_up: the raw indices pair i may pick from, as at most
+// three ranges in ascending raw order (lo0 the lowest allowed index).  An empty set has n0 = n1 = n2 = 0
+// and lo0 = 0xffffffff, which is no index.
+struct PairWindow {
+    uint32_t lo0, n0, lo1, n1, lo2, n2;
+    __host__ __device__ __forceinline__ bool allows(uint32_t i) const {
+        return i - lo0 < n0 || i - lo1 < n1 || i - lo2 < n2;
+    }
+    __host__ __device__ __forceinline__ bool empty() const { return n0 == 0u; }
+};
+
+// A(p) = { l in [lo, hi] : |l - p| >= D } ([lo, hi] the effective lag window, D >= 1) as raw ranges.
+// Its two folded intervals [lo, p - D] and [p + D, hi] each have a part at lags >= 0 (raw = lag) and
+// one below (raw = lag + 2L); only one interval can hold lag 0, so at most three parts are non-empty.
+__host__ __device__ __forceinline__ PairWindow runner_up_window(long long p, long long lo, long long hi, long long D,
+                                                                long long L) {
+    if (D > 2 * L) D = 2 * L;                      // every pair of lags is closer than 2L
+    const long long a0 = lo, b0 = p - D < hi ? p - D : hi;          // [lo, p - D]
+    const long long a1 = p + D > lo ? p + D : lo, b1 = hi;          // [p + D, hi]
+    PairWindow w{0xffffffffu, 0u, 0u, 0u, 0u, 0u};
+    auto put = [&](long long s, long long n) {     // the next non-empty range, in ascending raw order
+        if (n <= 0) return;
+        if (w.n0 == 0u) { w.lo0 = (uint32_t)s; w.n0 = (uint32_t)n; }
+        else if (w.n1 == 0u) { w.lo1 = (uint32_t)s; w.n1 = (uint32_t)n; }
+        else { w.lo2 = (uint32_t)s; w.n2 = (uint32_t)n; }
+    };
+    // lags >= 0 (raw = lag), then lags < 0 (raw = lag + 2L, above every lag >= 0)
+    put(a0 > 0 ? a0 : 0, b0 - (a0 > 0 ? a0 : 0) + 1);
+    put(a1 > 0 ? a1 : 0, b1 - (a1 > 0 ? a1 : 0) + 1);
+    put(a0 + 2 * L, (b0 < -1 ? b0 : -1) - a0 + 1);
+    put(a1 + 2 * L, (b1 < -1 ? b1 : -1) - a1 + 1);
+    return w;
+}
+
+// The runner-up twins' descriptor: pair i's centre p is the folded lag of first[i].raw_index, the wave's
+// records of the batch call (written by the preceding Pearson step).
+struct RunnerUp {
+    const audiosync_cuda_result* first;
+    long long lo, hi;               // the effective lag window
+    long long D;                    // min_separation >= 1
+    long long L;
+    __host__ __device__ __forceinline__ PairWindow window(long long pair) const {
+        return runner_up_window(fold_index(first[pair].raw_index, L).lag, lo, hi, D, L);
+    }
+};
+
+// What a windowed kernel searches for `pair`: the call's lag window, or (RU: the runner-up twins, whose
+// parameters add a RunnerUp `ru`) the pair's runner-up set.
+template <bool RU, class Pm>
+__host__ __device__ __forceinline__ decltype(auto) search_window(const Pm& p, long long pair) {
+    if constexpr (RU) {
+        return p.ru.window(pair);
+    } else {
+        (void)pair;
+        return (p.win);
+    }
+}
+
 // splitmix64 finaliser used by the seeded generator (oracle/xcorr_oracle.c).
 __host__ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
     uint64_t z = x + 0x9E3779B97F4A7C15ULL;

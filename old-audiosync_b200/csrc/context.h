@@ -44,6 +44,8 @@ enum KernelClass {
     KC_SRC_SPECTRUM, // forward rows of a shared source, once per call (RowFusedKernel ROWS_SRC_SPECTRUM)
     KC_CORR_OUT,     // correlation export of the precise and direct plans (corr_gather_kernel)
     KC_SMP_SPECTRUM, // forward rows of a cross call's samples, once per wave (RowFusedKernel ROWS_SRC_SPECTRUM)
+    KC_RU_ARGMAX,    // runner-up search over each pair's runner-up set (audiosync_cuda_xcorr_runner_up)
+    KC_RU_PEARSON,   // the runner-up records (pearson_runner_up_kernel)
     KC_COUNT
 };
 
@@ -109,6 +111,7 @@ struct FftPlan;   // fft_plan.h
 struct WorkSet {
     DevBuf ws;            // transform workspace (direct: r[]; fft: A/B planes)
     DevBuf peaks;         // PairPeak per in-flight pair
+    DevBuf peaks_ru;      // the runner-up search's PairPeak per in-flight pair (cleared before each search)
     DevBuf partials;      // PearsonPartial
     DevBuf tickets;       // per-pair completion counters of the Pearson kernel
     DevBuf spec;          // shared-source calls on a static plan: the source's forward rows (M complex);
@@ -117,7 +120,7 @@ struct WorkSet {
     cudaStream_t last_stream = nullptr;
     bool used = false;
     void release() {
-        ws.release(); peaks.release(); partials.release(); tickets.release(); spec.release();
+        ws.release(); peaks.release(); peaks_ru.release(); partials.release(); tickets.release(); spec.release();
         if (done) cudaEventDestroy(done);
         done = nullptr; used = false;
     }

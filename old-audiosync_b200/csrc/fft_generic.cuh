@@ -559,7 +559,9 @@ struct GenRowFusedKernel {
 // [0, limit); fp64 plans apply the window in argmax_f64_window_kernel instead.
 // OUT (fp32, with WIN): the exporting twin -- every output Params::corr's range allows is also stored,
 // before the threshold test; fp64 plans export from r_out in corr_gather_kernel instead.
-template <typename T, int CT_ = GenTraits<T>::CT, int NT_ = GEN_THREADS, bool WIN = false, bool OUT = false>
+// RU (fp32, with WIN): the runner-up twin -- the windowed search over each pair's runner-up set
+// (Params::ru); fp64 plans search it in argmax_f64_runner_up_kernel instead.
+template <typename T, int CT_ = GenTraits<T>::CT, int NT_ = GEN_THREADS, bool WIN = false, bool OUT = false, bool RU = false>
 struct GenColInvKernel {
     typedef typename GenTraits<T>::C C;
     static constexpr int CT = CT_;
@@ -580,9 +582,14 @@ struct GenColInvKernel {
     struct CorrParams : PlainParams {
         CorrOut corr;
     };
-    using Params = std::conditional_t<OUT, CorrParams, PlainParams>;
+    // RU appends the runner-up descriptor
+    struct RunnerUpParams : PlainParams {
+        RunnerUp ru;
+    };
+    using Params = std::conditional_t<OUT, CorrParams, std::conditional_t<RU, RunnerUpParams, PlainParams>>;
     static_assert(!WIN || sizeof(T) == 4, "fp64 plans window in argmax_f64_window_kernel");
     static_assert(!OUT || WIN, "the exporting twin runs the windowed argmax");
+    static_assert(!RU || (WIN && !OUT), "the runner-up twin runs the windowed argmax and exports nothing");
     static size_t smem_bytes(const GenShape& sh) {
         const size_t tile = (size_t)sh.M1 * CT * sizeof(C);
         return (tile > 512 ? tile : 512) + 16;
@@ -658,6 +665,7 @@ struct GenColInvKernel {
                         if (seen != 0u) acc.thr = float_from_order_bits(seen);
                         const int c = tid % CT;
                         const int n2 = c0 + c;
+                        [[maybe_unused]] decltype(auto) win = search_window<RU>(p, pair);
                         if (n2 < M2)
                         for (int bf = tid / CT; bf < nbf; bf += TR) {
                             C v[R];
@@ -676,8 +684,8 @@ struct GenColInvKernel {
                                 // outputs are tested; the butterfly of the lowest allowed index always
                                 // takes the exact path
                                 const unsigned step = 2u * Wt * (unsigned)M2;
-                                const bool has_floor = p.win.lo0 - i_first < (unsigned)R * step &&
-                                                       (p.win.lo0 - i_first) % step < 2u;
+                                const bool has_floor = win.lo0 - i_first < (unsigned)R * step &&
+                                                       (win.lo0 - i_first) % step < 2u;
                                 if (!has_floor) {
                                     float gm = fmaxf(fabsf(v[0].x), fabsf(v[0].y));
                                     static_for<1, R>([&](auto K) { gm = fmaxf(gm, fmaxf(fabsf(v[decltype(K)::value].x), fabsf(v[decltype(K)::value].y))); });
@@ -686,16 +694,16 @@ struct GenColInvKernel {
                                     static_for<0, R>([&](auto K) {
                                         constexpr int k = decltype(K)::value;
                                         const unsigned i_re = i_first + (unsigned)k * step;
-                                        if (p.win.allows(i_re)) gm = fmaxf(gm, fabsf(v[k].x));
-                                        if (p.win.allows(i_re + 1u)) gm = fmaxf(gm, fabsf(v[k].y));
+                                        if (win.allows(i_re)) gm = fmaxf(gm, fabsf(v[k].x));
+                                        if (win.allows(i_re + 1u)) gm = fmaxf(gm, fabsf(v[k].y));
                                     });
                                     if (!(gm >= acc.thr)) continue;
                                 }
                                 static_for<0, R>([&](auto K) {
                                     constexpr int k = decltype(K)::value;
                                     const unsigned i_re = i_first + 2u * (unsigned)k * Wt * (unsigned)M2;
-                                    acc.consider_win(v[k].x, i_re, p.win, &p.peaks[pair]);
-                                    acc.consider_win(v[k].y, i_re + 1u, p.win, &p.peaks[pair]);
+                                    acc.consider_win(v[k].x, i_re, win, &p.peaks[pair]);
+                                    acc.consider_win(v[k].y, i_re + 1u, win, &p.peaks[pair]);
                                 });
                                 continue;
                             }

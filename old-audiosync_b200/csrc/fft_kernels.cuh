@@ -139,7 +139,9 @@ struct ArgmaxAcc {
     // lowest real key (argmax_key_abs maps it to 0 high bits), below every number, so when no
     // allowed value is a number the pair resolves to that index with a NaN peak, as a NaN seed does.
     // A NaN's magnitude never joins `second` (fmaxf drops it).
-    ASC_HD void consider_win(float v, uint32_t index, const RawWindow& w, PairPeak* pk) {
+    // W: RawWindow (the lag window) or PairWindow (a runner-up set).
+    template <class W>
+    ASC_HD void consider_win(float v, uint32_t index, const W& w, PairPeak* pk) {
         if (index == w.lo0) {
             if (index == 0u) consider_seed(v, pk);
             else update(argmax_key_abs(v, index), fabsf(v));
@@ -437,7 +439,9 @@ struct ColFwdKernel {
 // compete, and only they raise the threshold (see the epilogue).
 // OUT (with WIN): the exporting twin (audiosync_cuda_xcorr_correlation): every output of the last pass
 // that Params::corr's range allows is also stored, before the threshold test.
-template <class RL, int M2_, int NT, bool TMA = true, bool WIN = false, bool OUT = false>
+// RU (with WIN): the runner-up twin (audiosync_cuda_xcorr_runner_up): the windowed search over each
+// pair's runner-up set (Params::ru) instead of the lag window.
+template <class RL, int M2_, int NT, bool TMA = true, bool WIN = false, bool OUT = false, bool RU = false>
 struct ColInvKernel {
     static_assert(TMA, "K_C's tiles are always staged by the TMA unit");
     static constexpr int M1 = RL::n;
@@ -463,8 +467,13 @@ struct ColInvKernel {
     struct CorrParams : PlainParams {
         CorrOut corr;
     };
-    using Params = std::conditional_t<OUT, CorrParams, PlainParams>;
+    // RU appends the runner-up descriptor
+    struct RunnerUpParams : PlainParams {
+        RunnerUp ru;
+    };
+    using Params = std::conditional_t<OUT, CorrParams, std::conditional_t<RU, RunnerUpParams, PlainParams>>;
     static_assert(!OUT || WIN, "the exporting twin runs the windowed argmax");
+    static_assert(!RU || (WIN && !OUT), "the runner-up twin runs the windowed argmax and exports nothing");
     static constexpr int TMA_ROWS = M1 - 1;
 
     // grid = (pairs, M2 / 16): the pair index runs fastest, so the tiles of one pair are
@@ -554,12 +563,13 @@ struct ColInvKernel {
                     if (seen != 0u) acc.thr = float_from_order_bits(seen);
                     const int c = tid & (COL_T - 1);
                     const bool col0 = (c0 + c) == 0;
+                    [[maybe_unused]] decltype(auto) win = search_window<RU>(p, pair);
                     // WIN: the column and row n1 of the packed point of the lowest allowed index
                     [[maybe_unused]] bool floor_col = false;
                     [[maybe_unused]] int floor_n1 = 0;
                     if constexpr (WIN) {
-                        floor_col = (p.win.lo0 >> 1) % (uint32_t)M2 == (uint32_t)(c0 + c);
-                        floor_n1 = (int)((p.win.lo0 >> 1) / (uint32_t)M2);
+                        floor_col = (win.lo0 >> 1) % (uint32_t)M2 == (uint32_t)(c0 + c);
+                        floor_n1 = (int)((win.lo0 >> 1) / (uint32_t)M2);
                     }
                     for (int w0 = 0; w0 < items; w0 += NT) {      // warp-uniform trip count
                         const int w = w0 + tid;
@@ -609,8 +619,8 @@ struct ColInvKernel {
                                 static_for<0, R>([&](auto K) {
                                     constexpr int k = decltype(K)::value;
                                     const uint32_t i_re = 2u * ((uint32_t)(f0 + k * Wt) * (uint32_t)M2 + (uint32_t)(c0 + c));
-                                    if (p.win.allows(i_re)) gm = fmaxf(gm, fabsf(v[k].x));
-                                    if (p.win.allows(i_re + 1u)) gm = fmaxf(gm, fabsf(v[k].y));
+                                    if (win.allows(i_re)) gm = fmaxf(gm, fabsf(v[k].x));
+                                    if (win.allows(i_re + 1u)) gm = fmaxf(gm, fabsf(v[k].y));
                                 });
                                 pass = gm >= acc.thr;
                             }
@@ -631,8 +641,8 @@ struct ColInvKernel {
                                     const int n1 = f0 + k * Wt;
                                     const uint32_t i_re = 2u * ((uint32_t)n1 * (uint32_t)M2 + (uint32_t)(c0 + c));
                                     if constexpr (WIN) {
-                                        acc.consider_win(v[k].x, i_re, p.win, &p.peaks[pair]);
-                                        acc.consider_win(v[k].y, i_re + 1u, p.win, &p.peaks[pair]);
+                                        acc.consider_win(v[k].x, i_re, win, &p.peaks[pair]);
+                                        acc.consider_win(v[k].y, i_re + 1u, win, &p.peaks[pair]);
                                     } else {
                                         if (has_seed && n1 == 0) acc.consider_seed(v[k].x, &p.peaks[pair]);
                                         else acc.consider(v[k].x, i_re);

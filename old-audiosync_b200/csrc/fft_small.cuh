@@ -39,7 +39,9 @@ ASC_HD int small_pos_of_freq(const SmallPlan& pl, int k) {
 // WIN: the windowed twin -- only the raw indices Params::win allows compete (ArgmaxAcc::consider_win).
 // SHARED_SRC: every pair reads the one source at Params::sources (its pitch is not read).
 // OUT (with WIN): the exporting twin -- every output Params::corr's range allows is also stored.
-template <typename InT, bool PHAT = false, bool WIN = false, bool SHARED_SRC = false, bool OUT = false>
+// RU (with WIN): the runner-up twin -- a second launch over the wave after the batch records are
+// written, the windowed search over each pair's runner-up set (Params::ru).
+template <typename InT, bool PHAT = false, bool WIN = false, bool SHARED_SRC = false, bool OUT = false, bool RU = false>
 struct SmallXcorrKernel {
     static constexpr int THREADS = SMALL_THREADS;
 
@@ -59,8 +61,13 @@ struct SmallXcorrKernel {
     struct CorrParams : PlainParams {
         CorrOut corr;
     };
-    using Params = std::conditional_t<OUT, CorrParams, PlainParams>;
+    // RU appends the runner-up descriptor
+    struct RunnerUpParams : PlainParams {
+        RunnerUp ru;
+    };
+    using Params = std::conditional_t<OUT, CorrParams, std::conditional_t<RU, RunnerUpParams, PlainParams>>;
     static_assert(!OUT || WIN, "the exporting twin runs the windowed argmax");
+    static_assert(!RU || (WIN && !OUT), "the runner-up twin runs the windowed argmax and exports nothing");
     // two rows of M points + 512 bytes of reduction scratch (phase_argmax needs 392)
     static size_t smem_bytes(int M) { return (size_t)2 * M * sizeof(cplx) + 512; }
 
@@ -148,6 +155,7 @@ struct SmallXcorrKernel {
         ex.phase_argmax(
             [&](int tid) -> ArgmaxPair {
                 ArgmaxAcc acc;
+                [[maybe_unused]] decltype(auto) win = search_window<RU>(p, pair);
                 for (int n = tid; n < M; n += THREADS) {
                     const cplx v = buf[n];
                     const uint32_t i_re = (uint32_t)(2 * n);
@@ -156,8 +164,8 @@ struct SmallXcorrKernel {
                         p.corr.store(pair, i_re + 1u, v.y);
                     }
                     if constexpr (WIN) {
-                        acc.consider_win(v.x, i_re, p.win, &p.peaks[pair]);
-                        acc.consider_win(v.y, i_re + 1u, p.win, &p.peaks[pair]);
+                        acc.consider_win(v.x, i_re, win, &p.peaks[pair]);
+                        acc.consider_win(v.y, i_re + 1u, win, &p.peaks[pair]);
                     } else {
                         if (n == 0) acc.consider_seed(v.x, &p.peaks[pair]);
                         else acc.consider(v.x, i_re);

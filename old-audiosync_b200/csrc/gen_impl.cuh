@@ -22,13 +22,15 @@ static int prepare_gen_kernel(size_t smem) {
     return 0;
 }
 
-// the windowed and exporting twins of the fp32 inverse column kernel (fp64 plans window in
-// argmax_f64_window_kernel and export in corr_gather_kernel)
+// the windowed, exporting and runner-up twins of the fp32 inverse column kernel (fp64 plans window in
+// argmax_f64_window_kernel, export in corr_gather_kernel and search runner-ups in argmax_f64_runner_up_kernel)
 template <typename T, int CT, int NT>
 static int prepare_col_inv_window(const GenShape& sh) {
     if constexpr (sizeof(T) == 4)
         return prepare_gen_kernel<GenColInvKernel<T, CT, NT, true>>(GenColInvKernel<T, CT, NT, true>::smem_bytes(sh)) != 0 ||
-               prepare_gen_kernel<GenColInvKernel<T, CT, NT, true, true>>(GenColInvKernel<T, CT, NT, true, true>::smem_bytes(sh)) != 0
+               prepare_gen_kernel<GenColInvKernel<T, CT, NT, true, true>>(GenColInvKernel<T, CT, NT, true, true>::smem_bytes(sh)) != 0 ||
+               prepare_gen_kernel<GenColInvKernel<T, CT, NT, true, false, true>>(
+                   GenColInvKernel<T, CT, NT, true, false, true>::smem_bytes(sh)) != 0
                    ? -1 : 0;
     return 0;
 }
@@ -138,6 +140,35 @@ int GenStage<T, NT>::col_inv(FftPlan* plan, const Wave& w) {
         if (w.corr) return launch_corr_gather(w, r, 4 * sh.M);
     }
     return 0;
+}
+
+// The runner-up search of a wave into w.peaks.  fp32: the inverse column kernel's runner-up twin over
+// plane 0, which G_C only reads (the rows' static or runtime-radix kernel wrote it, and nothing since);
+// fp64: over r in the pairs' sample planes, which nothing writes after G_C.
+template <typename T, int NT>
+int GenStage<T, NT>::runner_up(FftPlan* plan, const Wave& w) {
+    typedef typename GenTraits<T>::C C;
+    const GenShape& sh = plan->gen;
+    C* planes = static_cast<C*>(w.ws);
+    if constexpr (sizeof(T) == 8) {
+        const double* r = reinterpret_cast<const double*>(planes) + 2 * sh.M;
+        return launch(w.ctx, w.d, KC_RU_ARGMAX, w.st, [&] {
+            argmax_f64_runner_up_kernel<<<w.pairs, 1024, 0, w.st>>>(r, 4 * sh.M, w.peaks, *w.ru);
+        });
+    } else {
+        return gen_for_tile_width<T>(sh.ct, [&](auto CTC) -> int {
+            using K = GenColInvKernel<T, decltype(CTC)::value, NT, true, false, true>;
+            typename K::Params p{};
+            static_cast<typename K::PlainParams&>(p) = {planes, w.peaks, static_cast<const C*>(plan->g_wcol.p),
+                                                        static_cast<const int*>(plan->g_p2f_col.p), sh, reinterpret_cast<T*>(planes),
+                                                        w.win ? *w.win : full_window(sh.L)};
+            p.ru = *w.ru;
+            const dim3 grid(w.pairs, (sh.M2 + K::CT - 1) / K::CT, 1);
+            return launch(w.ctx, w.d, KC_RU_ARGMAX, w.st, [&] {
+                launch_stage(gen_kernel_entry<K>, grid, dim3(K::THREADS), K::smem_bytes(sh), w.st, p);
+            });
+        });
+    }
 }
 
 }  // namespace asc

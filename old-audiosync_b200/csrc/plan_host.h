@@ -41,6 +41,7 @@ struct Wave {
     int pairs;
     const RawWindow* win;       // lag window: nullptr for the unwindowed kernels
     const CorrOut* corr;        // correlation export, out at this wave's first row: nullptr when off
+    const RunnerUp* ru = nullptr;   // runner_up: the wave's runner-up descriptor (first: its batch records)
 };
 
 // f(float{}), f(double{}) or f(int16_t{}): the element type a transform loads for `dtype`.
@@ -92,6 +93,11 @@ struct FftPlan {
     // wave's samples' forward rows in plane 1 (w.smp, once per wave); cross_rows then correlates one
     // source against them (w.spec: that source's forward rows), any number of times.
     std::function<int(const Wave&)> cross_samples, cross_rows;
+    // The runner-up search of a wave whose run_wave and Pearson step have run (w.ru set, w.peaks the
+    // cleared second PairPeak array): the inverse pass that holds r again (static, runtime-radix fp32,
+    // single-CTA) or the search over the r the workspace still holds (precise, direct).  Nothing between
+    // the two passes writes plane 0 or r.
+    std::function<int(const Wave&)> runner_up;
     ~FftPlan() {
         col_tw.release(); col_tc.release(); row_tw.release(); row_rev.release(); row_tab.release(); m_lo.release(); m_hi.release();
         wm.release(); wn.release();
@@ -204,6 +210,7 @@ struct GenStage {
     static int col_fwd(FftPlan* plan, const Wave& w);
     static int rows(FftPlan* plan, const Wave& w);
     static int col_inv(FftPlan* plan, const Wave& w);
+    static int runner_up(FftPlan* plan, const Wave& w);
 };
 
 // static_rows.cu: the rows of a runtime-radix fp32 plan on a static row kernel (RowFusedKernel<RL, 0, NT>)

@@ -202,6 +202,52 @@ argmax_f64_window_kernel(const double* __restrict__ r, long long N, long long pi
     }
 }
 
+// The runner-up twin (audiosync_cuda_xcorr_runner_up): the window kernel's rule over pair i's runner-up
+// set, at most three ranges; an empty set writes nothing (the runner-up Pearson step reports it).
+static __global__ void __launch_bounds__(1024)
+argmax_f64_runner_up_kernel(const double* __restrict__ r, long long pitch, PairPeak* __restrict__ peaks, RunnerUp ru)
+{
+    const PairWindow win = ru.window(blockIdx.x);
+    if (win.empty()) return;
+    __shared__ KeyF64 s_k[32];
+    const double* rp = r + (size_t)blockIdx.x * (size_t)pitch;
+    const double ninf = -INFINITY, pinf = INFINITY;
+    KeyF64 best; best.v = ninf; best.i = 0x7fffffffffffffffLL; best.a = 0.0; best.s = 0.0;
+    for (int g = 0; g < 3; g++) {
+        const long long beg = g == 0 ? win.lo0 : g == 1 ? win.lo1 : win.lo2;
+        const long long end = beg + (g == 0 ? win.n0 : g == 1 ? win.n1 : win.n2);
+        for (long long i = beg + threadIdx.x; i < end; i += blockDim.x) {
+            const double x = rp[i];
+            KeyF64 c;
+            c.i = i;
+            const double a = fabs(x);
+            c.a = (a != a) ? 0.0 : a;
+            c.s = 0.0;
+            if (i == 0) c.v = (x != x) ? pinf : x;
+            else c.v = (a != a) ? ninf : a;
+            best = key_better(best, c);
+        }
+    }
+    for (int o = 16; o > 0; o >>= 1) best = key_better(best, key_shfl_xor(best, o));
+    const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+    if (l == 0) s_k[w] = best;
+    __syncthreads();
+    if (w == 0) {
+        const int nw = (blockDim.x + 31) >> 5;
+        if (l < nw) best = s_k[l];
+        else { best.v = ninf; best.i = 0x7fffffffffffffffLL; best.a = 0.0; best.s = 0.0; }
+        for (int o = 16; o > 0; o >>= 1) best = key_better(best, key_shfl_xor(best, o));
+        if (l == 0) {
+            PairPeak p = cleared_peak();
+            p.raw_index = best.i;
+            p.peak = rp[best.i];
+            p.second = best.s;
+            p.resolved = 1;
+            peaks[blockIdx.x] = p;
+        }
+    }
+}
+
 // ---------------------------------------------------------------------------
 // Pearson coefficient of the aligned windows (reference
 // src/cross_correlation.c:74-116 on the windows of :256-271).
@@ -457,6 +503,36 @@ pearson_kernel(const T* __restrict__ sources, const T* __restrict__ samples,
     __shared__ PearsonShared<PEARSON_THREADS> sh;
     pdl_prologue();
     pearson_block<T, PEARSON_THREADS, WIDE, PHAT>(sources, samples, src_pitch, smp_pitch, L, peaks, explicit_n, peak_scale, partials,
+                                      tickets, n_chunks, results, (int)blockIdx.y, (int)blockIdx.x,
+                                      (int)threadIdx.x, sh);
+}
+
+// The record of a pair whose runner-up set is empty (audiosync_cuda_xcorr_runner_up).
+__host__ __device__ __forceinline__ audiosync_cuda_result no_runner_up() {
+    audiosync_cuda_result r;
+    r.lag = 0; r.coef = NAN; r.peak = 0.0; r.ret = -1; r.success = 0;
+    r.raw_index = -1; r.second = 0.0; r.margin = 0.0; r.ncc = NAN;
+    return r;
+}
+
+// The runner-up twin of pearson_kernel: pair i's record from the second search's peaks, or
+// no_runner_up() when its runner-up set is empty (every CTA of that pair returns at once, so its
+// ticket counter is not touched).
+template <typename T, bool WIDE = !std::is_same<T, float>::value, bool PHAT = false>
+__global__ void __launch_bounds__(PEARSON_THREADS)
+pearson_runner_up_kernel(const T* __restrict__ sources, const T* __restrict__ samples,
+                         long long src_pitch, long long smp_pitch, long long L,
+                         const PairPeak* __restrict__ peaks, RunnerUp ru, double peak_scale,
+                         PearsonPartial* __restrict__ partials, unsigned int* __restrict__ tickets,
+                         int n_chunks, audiosync_cuda_result* __restrict__ results)
+{
+    __shared__ PearsonShared<PEARSON_THREADS> sh;
+    pdl_prologue();
+    if (ru.window(blockIdx.y).empty()) {
+        if (blockIdx.x == 0 && threadIdx.x == 0) results[blockIdx.y] = no_runner_up();
+        return;
+    }
+    pearson_block<T, PEARSON_THREADS, WIDE, PHAT>(sources, samples, src_pitch, smp_pitch, L, peaks, 0LL, peak_scale, partials,
                                       tickets, n_chunks, results, (int)blockIdx.y, (int)blockIdx.x,
                                       (int)threadIdx.x, sh);
 }

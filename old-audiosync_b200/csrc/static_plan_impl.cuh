@@ -104,6 +104,7 @@ static int static_col_inv(const Wave& w, const typename ColInvKernel<typename P:
     if (w.corr) {
         // the exporting twin runs the windowed argmax, over all of [0, 2L) when no window is set
         using KCO = ColInvKernel<Col, Row::n, P::NT_COL, true, true, true>;
+    using KCR = ColInvKernel<Col, Row::n, P::NT_COL, true, true, false, true>;
         typename KCO::Params po{{pc.planes, pc.peaks, pc.tw, P::L, w.win ? *w.win : full_window(P::L), pc.tm}, *w.corr};
         return launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
             launch_stage(fft_kernel_entry<KCO>, grid, dim3(KCO::THREADS), KCO::SMEM, w.st, po);
@@ -118,6 +119,22 @@ static int static_col_inv(const Wave& w, const typename ColInvKernel<typename P:
     }
     return launch(w.ctx, w.d, KC_COL_INV, w.st, [&] {
         launch_stage(fft_kernel_entry<KC>, grid, dim3(KC::THREADS), KC::SMEM, w.st, pc);
+    });
+}
+
+// The runner-up search of a wave: K_C's runner-up twin over the planes run_static_wave left (K_C only
+// reads them), into w.peaks.
+template <class P>
+static int static_runner_up(FftPlan* plan, const Wave& w) {
+    using Col = typename P::Col;
+    using Row = typename P::Row;
+    typename ColInvKernel<Col, Row::n, P::NT_COL>::Params pc;
+    if (static_col_inv_params<P>(plan, w, &pc) != 0) return -1;
+    using KCR = ColInvKernel<Col, Row::n, P::NT_COL, true, true, false, true>;
+    typename KCR::Params pr{{pc.planes, pc.peaks, pc.tw, P::L, w.win ? *w.win : full_window(P::L), pc.tm}, *w.ru};
+    const dim3 grid(w.pairs, Row::n / COL_T, 1);
+    return launch(w.ctx, w.d, KC_RU_ARGMAX, w.st, [&] {
+        launch_stage(fft_kernel_entry<KCR>, grid, dim3(KCR::THREADS), KCR::SMEM, w.st, pr);
     });
 }
 
@@ -218,6 +235,7 @@ int build_static_plan(FftPlan* plan) {
     using KC = ColInvKernel<Col, Row::n, P::NT_COL>;
     using KCW = ColInvKernel<Col, Row::n, P::NT_COL, true, true>;
     using KCO = ColInvKernel<Col, Row::n, P::NT_COL, true, true, true>;
+    using KCR = ColInvKernel<Col, Row::n, P::NT_COL, true, true, false, true>;
     // the shared-source path: sample-only K_A, the source-spectrum kernel and the shared K_B
     using KTs = ColFwdKernel<Col, Row::n, P::NT_COL, float, true, true>;
     using KRs = ColFwdKernel<Col, Row::n, P::NT_COL, float, false, true>;
@@ -232,7 +250,7 @@ int build_static_plan(FftPlan* plan) {
     if (prepare_kernel<KT>(KT::SMEM) != 0 || prepare_kernel<KR>(KR::SMEM) != 0 || prepare_kernel<KD>(KD::SMEM) != 0 ||
         prepare_kernel<KS>(KS::SMEM) != 0 ||
         (plan->phat ? prepare_kernel<KBP>(KBP::SMEM) : prepare_kernel<KB>(KB::SMEM)) != 0 || prepare_kernel<KC>(KC::SMEM) != 0 ||
-        prepare_kernel<KCW>(KCW::SMEM) != 0 || prepare_kernel<KCO>(KCO::SMEM) != 0)
+        prepare_kernel<KCW>(KCW::SMEM) != 0 || prepare_kernel<KCO>(KCO::SMEM) != 0 || prepare_kernel<KCR>(KCR::SMEM) != 0)
         return -1;
     if (prepare_kernel<KTs>(KTs::SMEM) != 0 || prepare_kernel<KRs>(KRs::SMEM) != 0 || prepare_kernel<KDs>(KDs::SMEM) != 0 ||
         prepare_kernel<KSs>(KSs::SMEM) != 0 || prepare_kernel<KBspec>(KBspec::SMEM) != 0 ||
@@ -247,6 +265,7 @@ int build_static_plan(FftPlan* plan) {
     };
     plan->cross_samples = [plan](const Wave& w) { return static_cross_samples<P>(plan, w); };
     plan->cross_rows = [plan](const Wave& w) { return static_cross_rows<P>(plan, w); };
+    plan->runner_up = [plan](const Wave& w) { return static_runner_up<P>(plan, w); };
     return 0;
 }
 
